@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (N > 1: launched under torch.distributed.run)
   python bench.py --impl reference ...                     (the reference's CPU path on the host cores)
+  python bench.py ... --dump-outputs DIR                   (also write the last timed step's output to DIR)
 
 A "step" is one full likelihood evaluation (one MCMC proposal): orbit velocities -> Doppler-shifted covariance
 fill -> FP64 Cholesky + solve + log-determinant for every chunk of the workload, and the cross-rank reduction of
@@ -161,7 +162,15 @@ def main():
     ap.add_argument("--workload", default="C4", choices=sorted(WORKLOADS))
     ap.add_argument("--nbranch", type=int, default=0, help="chunks in flight per GPU (0: 64; 128 for the small chunks of C6)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (the per-chunk log-likelihood "
+                         "vector, float64) to DIR/chunk_lnlikes.npy; the inputs depend only on the arguments, so two "
+                         "builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     if args.nbranch <= 0:   # measured: C4 4.60 evals/s with 32 branches, 4.62 with 64 (4.66 with rank-1024 updates), 4.60 with 96;
         args.nbranch = 128 if args.workload == "C6" else 64   # C6 (N = 1600) 31.0 / 34.2 / 34.9 with 32 / 64 / 128
     if args.impl == "reference":
@@ -231,7 +240,7 @@ def main():
     barrier()
     e0.record()
     for k in range(args.warmup, args.warmup + args.steps):
-        farm.chunk_lnlikes_device(p_dev[k])
+        lnl_last = farm.chunk_lnlikes_device(p_dev[k])
     e1.record()
     barrier()
     t_wall1 = time.time()
@@ -245,6 +254,11 @@ def main():
     ms_total = float(ms.item())
     clocks = sampler.stop(t_wall0, t_wall1) if rank == 0 else None
     value = args.steps / (ms_total * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # read before the next evaluation overwrites the farm's result buffer (with several ranks the all-reduce has
+        # already filled in every chunk)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "chunk_lnlikes.npy"), lnl_last.cpu().numpy())
     lnl_check = float(np.sum(farm.chunk_lnlikes_device(p_dev[-1]).cpu().numpy()))
 
     # ---- parity, asserted in the same run: the chunks the CPU arm sampled, same parameter vector ----------

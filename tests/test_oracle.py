@@ -1,7 +1,6 @@
 """CPU: pin the oracle (oracle/oracle.py + oracle/psoap_oracle.c) against the golden vectors produced by the
 unmodified reference (tests/golden/make_golden.py)."""
 import numpy as np
-import pytest
 
 from conftest import rel_close
 
@@ -23,17 +22,6 @@ def test_fill_bit_exact(golden, oracle):
     m = np.empty((33, 33)); oracle.fill_V11_f(m, g["far_lwl"], 0.5, 5.0)
     assert np.array_equal(m, g["far_V11_f"])
     assert (g["far_V11_f"] == 0).any()  # the fixture reaches exp underflow
-
-
-def test_ref_compiled_fill_matches_c_port(golden, oracle):
-    mod = oracle.ref_matrix_functions()
-    if mod is None:
-        pytest.skip("oracle/_ref not built (reference absent)")
-    g = golden["fills"]
-    lw, amp, l = g["lwl"], g["amp"], g["l"]
-    N = lw.shape[1]
-    m = np.empty((N, N)); mod.fill_V11_f_g(m, lw[0], lw[1], amp[0], l[0], amp[1], l[1])
-    assert np.array_equal(m, g["V11_f_g"])
 
 
 def test_orbits(golden, oracle):
