@@ -70,35 +70,29 @@ std::once_flag g_attr_once;
 int g_attr_status = 0;
 int g_attr_device = 0;
 int g_num_sms = 148;
-int g_ctas_per_sm = 2;
-int g_yield_lookahead = -1;  // PSOAP_YIELD_LOOKAHEAD: how the bulk update shares the SMs with the links under look-ahead (see the syrk launch); -1 = by size
+int g_yield_lookahead = 0;  // PSOAP_YIELD_LOOKAHEAD=1|2: how the bulk update shares the SMs with the links under look-ahead (see the syrk launch); 0 = by size
 // Chain links (diagonal block + panel solve): 7 = potrf_diag7 + trsm7 (chain.cuh: blocked factorisation with one chain
 // warp, blocked substitution), 3 = potrf_diag3 + trsm3 (explicit 128 x 128 inverse, GEMM panel solve).  7 is the faster
 // chain for a matrix factored on its own (N = 2000: 0.88 vs 1.22 ms, N = 4000: 2.11 vs 2.74 ms); inside the graph farm,
 // where chain latency is hidden by the other chunks and SM-time is what counts, 3 wins (trsm7 keeps a whole SM per
-// 32-row tile).  PSOAP_POTRF sets both, PSOAP_FARM_POTRF the farm's.
+// 32-row tile: see farm_issue).  PSOAP_POTRF sets this default of the direct API.
 int g_potrf_version = 7;
-int g_farm_potrf_version = 3;
 // PSOAP_TAIL=1: the partial last round of a trailing update is dealt out as quarter tiles (syrk_split).  Measured on
 // a B200: the kernel ALONE gains (m = 4096, K = 512: 29.4 -> 31.7 TFLOP/s, m = 8192: 33.0 -> 33.9), every path that
 // ships loses, because there the partial round is already covered by other work: the 256-chunk farm 217.7 -> 224.1 ms
 // (the other branches' kernels), a lone N = 6000 matrix 3.71 -> 3.74 ms (the look-ahead's next panels).  Off.
 int g_tail_split = 0;
-int g_single_rows = 24;  // PSOAP_SINGLE_ROWS: a lone matrix goes to single-panel groups once this many row blocks remain (0: never)
-int g_small_tiles = 1;   // PSOAP_SMALL_TILES=0: keep 128 x 64 tiles for the critical block-column updates too
-int g_pf_mode = 2;
 int g_lookahead = 1;   // direct API: next group's head on a high-priority side stream
 int g_pdl = 256;       // direct issue: grids up to this many CTAs are launched with programmatic stream serialization
                        // (64 -> 256 with the 32-row panel-solve tiles and 64 x 32 update tiles: N = 2000 0.78 -> 0.72 ms)
 int g_group = 0;  // 0: automatic (see launch_factor); PSOAP_GROUP=2|4|8 forces it
-int g_farm_group = 8;   // PSOAP_FARM_GROUP: panels per trailing update inside the graph farm
-inline int persistent_ctas(int ntiles) { return std::max(1, std::min(ntiles, g_ctas_per_sm * g_num_sms)); }
+inline int persistent_ctas(int ntiles) { return std::max(1, std::min(ntiles, CTAS_PER_SM * g_num_sms)); }
 // How a trailing update of `ntiles` 128 x 64 tiles is dealt out: `nmain` tiles to `nctas` CTAs (persistent round-robin,
 // or one tile each when `one_per_cta`), and the partial last round, `ntiles - nmain` tiles, as 4 quarter-tile CTAs each
 // when that is shorter than one more whole-tile round (3 quarter rounds or fewer).
 struct SyrkSplit { int nmain, nctas, nquarters; };
 inline SyrkSplit syrk_split(int ntiles, bool one_per_cta, bool allow_tail) {
-    const int slots = g_ctas_per_sm * g_num_sms;
+    const int slots = CTAS_PER_SM * g_num_sms;
     SyrkSplit sp{ntiles, 0, 0};
     const int rem = ntiles % slots;
     if (allow_tail && rem > 0 && 4 * rem <= 3 * slots) { sp.nmain = ntiles - rem; sp.nquarters = 4 * rem; }
@@ -126,15 +120,9 @@ int set_kernel_attributes() {
         if (e == cudaSuccess) e = cudaDeviceGetAttribute(&g_num_sms, cudaDevAttrMultiProcessorCount, dev);
         g_attr_device = dev;
         g_attr_status = (int)e;
-        if (const char* c = getenv("PSOAP_CTAS_PER_SM")) g_ctas_per_sm = std::max(1, std::min(2, atoi(c)));
-        if (const char* c = getenv("PSOAP_YIELD_LOOKAHEAD")) g_yield_lookahead = atoi(c);
-        if (const char* c = getenv("PSOAP_POTRF")) g_potrf_version = g_farm_potrf_version = (atoi(c) == 7) ? 7 : 3;
-        if (const char* c = getenv("PSOAP_SMALL_TILES")) g_small_tiles = atoi(c);
+        if (const char* c = getenv("PSOAP_YIELD_LOOKAHEAD")) g_yield_lookahead = (atoi(c) == 1 || atoi(c) == 2) ? atoi(c) : 0;
+        if (const char* c = getenv("PSOAP_POTRF")) g_potrf_version = (atoi(c) == 7) ? 7 : 3;
         if (const char* c = getenv("PSOAP_TAIL")) g_tail_split = atoi(c);
-        if (const char* c = getenv("PSOAP_SINGLE_ROWS")) g_single_rows = atoi(c);
-        if (const char* c = getenv("PSOAP_FARM_GROUP")) g_farm_group = (atoi(c) >= 8) ? 8 : (atoi(c) >= 4) ? 4 : 2;
-        if (const char* c = getenv("PSOAP_FARM_POTRF")) g_farm_potrf_version = (atoi(c) == 7) ? 7 : 3;
-        if (const char* c = getenv("PSOAP_PF_MODE")) g_pf_mode = atoi(c);
         if (e == cudaSuccess) {
             void* fn = nullptr;
             cudaDriverEntryPointQueryResult qres;
@@ -310,23 +298,23 @@ int launch_factor(const Lanes& ln, double* W, int64_t ld, int T_elim, int T_tota
         const int R = T_total - row0;
         // part 1 (the block columns the next diagonal blocks wait for) of a matrix factored on its own: 64 x 32 tiles,
         // four times the CTAs at a quarter of the latency each
-        const int sh = (part == 1 && chain == 7 && g_small_tiles) ? 2 : 1;
+        const int sh = (part == 1 && chain == 7) ? 2 : 1;
         SyrkSrc src;
         src.W = W; src.ld = ld; src.row0 = sh * row0; src.res_row0 = row0; src.kbeg = kbeg_of(q); src.kend = kend;
-        src.P = pbuf(q); src.ldp = ldp; src.part = part; src.ncol1 = sh * ncol1; src.pf_mode = g_pf_mode;
+        src.P = pbuf(q); src.ldp = ldp; src.part = part; src.ncol1 = sh * ncol1;
         const int ntiles = syrk_ntiles(sh * R, part, sh * ncol1);
         const int nres = (part == 2 || ykb < 0) ? 0 : R;
         if (ntiles + nres == 0) return;
         // Under look-ahead the bulk update (part 2) must leave room for the links of the next group (high-priority side
-        // stream).  Mode 2 (default): it stays persistent but takes ONE slot per SM and leaves one SM empty, so that every
-        // link finds a slot on every SM at once (a panel-solve CTA, 126 KB of shared memory, fits beside an update CTA,
+        // stream).  Mode 2: it stays persistent but takes ONE slot per SM and leaves one SM empty, so that every link
+        // finds a slot on every SM at once (a panel-solve CTA, 126 KB of shared memory, fits beside an update CTA,
         // 102 KB, and not beside two) and the one-CTA diagonal block, which needs a whole SM's shared memory, an empty SM
         // instead of waiting 20-40 us for two update CTAs to retire.  Mode 1: one tile per CTA on all slots, which free
-        // up continuously.  Mode 0: persistent on all slots (the links then wait for the update to end).  N = 4000 / 6000
-        // / 9000: 1.70 / 3.50 / 9.31 ms in mode 2, 1.75 / 3.64 / 9.39 in mode 1; where the bulk dominates mode 1 wins
-        // (N = 16384: 47.4 vs 47.7 ms, N = 32768: 349 vs 364 ms), so by default mode 2 below 96 panels and mode 1 from there.
-        const int yield_mode = g_yield_lookahead >= 0 ? g_yield_lookahead : (T_total >= 96 ? 1 : 2);
-        const bool yield_slots = (part == 2 && ln.side != nullptr && yield_mode);
+        // up continuously.  N = 4000 / 6000 / 9000: 1.70 / 3.50 / 9.31 ms in mode 2, 1.75 / 3.64 / 9.39 in mode 1; where
+        // the bulk dominates mode 1 wins (N = 16384: 47.4 vs 47.7 ms, N = 32768: 349 vs 364 ms), so by default mode 2
+        // below 96 panels and mode 1 from there.
+        const int yield_mode = g_yield_lookahead ? g_yield_lookahead : (T_total >= 96 ? 1 : 2);
+        const bool yield_slots = (part == 2 && ln.side != nullptr);
         const double* yk = ws.y + (int64_t)std::max(ykb, 0) * NB;
         if (sh == 2) {
             const int nctas = persistent_ctas(ntiles);
@@ -334,9 +322,6 @@ int launch_factor(const Lanes& ln, double* W, int64_t ld, int T_elim, int T_tota
                      res_col0, mapPas[q & 1], mapPbs[q & 1], mapPas[q & 1], mapPbs[q & 1]);
         } else {
             SyrkSplit sp = syrk_split(ntiles, yield_slots && yield_mode == 1, part != 1 && g_tail_split != 0);
-            // mode 2: the bulk update under look-ahead stays persistent but takes ONE slot per SM and leaves one SM empty:
-            // the links find a slot on every SM at once and the one-CTA diagonal block (which needs a whole SM's shared
-            // memory) an empty SM, instead of waiting for update CTAs to retire
             if (yield_slots && yield_mode == 2) sp.nctas = std::min(sp.nmain, g_num_sms - 1);
             launch_k(syrk3_kernel<1>, nres + sp.nctas + sp.nquarters, 256, sp.nquarters ? SYRK1_SMEM : GEMM_SMEM, s, ln.pdl, src, sp.nmain, sp.nctas, nres,
                      yk, ws.rvec, res_col0, mapPa[q & 1], mapPb[q & 1], mapPas[q & 1], mapPbs[q & 1]);
@@ -344,15 +329,16 @@ int launch_factor(const Lanes& ln, double* W, int64_t ld, int T_elim, int T_tota
         ++g_launches;
     };
     // Group boundaries.  Uniform groups of G, except at the END of a matrix factored on its own (look-ahead, chain 7):
-    // once fewer than g_single_rows row blocks remain the trailing update is shorter than the links it runs beside,
+    // once fewer than SINGLE_ROWS row blocks remain the trailing update is shorter than the links it runs beside,
     // the chain is all there is, and single panels (no in-group column update, a rank-128 update of ONE block column
     // before the next diagonal block) make the shortest chain: 38 us per panel against 48.  Measured with 0 / 16 / 24 / 36
     // such rows: N = 4000 1.706 / 1.675 / 1.647 / 1.625 ms, N = 6000 3.514 / 3.491 / 3.442 / 3.526, N = 9000 9.31 / 9.29 / 9.25 / 9.33.
+    constexpr int SINGLE_ROWS = 24;
     std::vector<int> gstart;
     {
         const bool lone = ln.side != nullptr && chain == 7 && g_group == 0;
         for (int a = 0; a < T_elim;) {
-            const int g = (lone && T_total - a <= g_single_rows) ? 1 : G;
+            const int g = (lone && T_total - a <= SINGLE_ROWS) ? 1 : G;
             gstart.push_back(a);
             a += std::min(g, T_elim - a);
         }
@@ -888,12 +874,11 @@ int farm_issue(psoap_farm* f, cudaStream_t s0, int pdl) {
             // x 8 proposals on 8 branches: 1121 evals/s against 1149 with rank-512)
             ln.group = f->lookahead ? 0
                      : (f->group_hint == 2 || f->group_hint == 4 || f->group_hint == 8) ? f->group_hint
-                     : (nbranch >= 32 ? g_farm_group : std::min(g_farm_group, 4));
+                     : (nbranch >= 32 ? 8 : 4);
             ln.pdl = pdl;
             // chain links: the caller's choice (psoap_chunk.reserved = 3 | 7, the same on every rank of a partitioned
             // farm so that the bits do not depend on the number of GPUs), else by exposure of the chain latency
-            ln.chain = (f->chain_hint == 3 || f->chain_hint == 7) ? f->chain_hint
-                                                                  : (f->lookahead ? 0 : g_farm_potrf_version);
+            ln.chain = (f->chain_hint == 3 || f->chain_hint == 7) ? f->chain_hint : (f->lookahead ? 0 : 3);
             rc = launch_chunk(ln, f->ncomp, ch.N, zs, ch.fl, ch.sigma, f->mu, gp, ws, f->flags + it, f->results + 4 * it);
             if (rc) break;
         }
@@ -1010,18 +995,16 @@ int psoap_farm_create_batched(psoap_farm** out, int model, int nchunks, const ps
     f->events.resize(nbranch + 1);
     {
         // Branch b carries the b-th largest items first (LPT order): its stream gets the matching priority level, which a
-        // captured kernel node inherits (PSOAP_FARM_PRIO=0: all equal).  Measured neutral on a B200 (one rank's share of
+        // captured kernel node inherits.  Measured neutral on a B200 against all-equal priorities (one rank's share of
         // an 8-GPU run: 28.50 ms either way; a launch-attribute variant likewise): the drain at the end of an evaluation
         // is not a matter of which chunk gets the free SM slots first.
         int lo = 0, hi = 0;
         cudaDeviceGetStreamPriorityRange(&lo, &hi);
-        const char* pe = getenv("PSOAP_FARM_PRIO");
-        const int mode = pe ? (atoi(pe) != 0) : 1;
         const int nlev = lo - hi + 1;
         for (int b = 0; b <= nbranch; ++b) {
             // (a look-ahead farm's branch streams carry the bulk updates: lowest priority, below their side streams, where
             // the chain links run; with both at the top C2 ran at 95.5 instead of 104 evals/s)
-            const int pr = (mode == 1 && b < nbranch && nlev > 1 && !f->lookahead) ? hi + (int)((int64_t)b * nlev / nbranch) : lo;
+            const int pr = (b < nbranch && nlev > 1 && !f->lookahead) ? hi + (int)((int64_t)b * nlev / nbranch) : lo;
             cudaStreamCreateWithPriority(&f->streams[b], cudaStreamNonBlocking, pr);
         }
     }
@@ -1137,7 +1120,6 @@ int psoap_bench_syrk_split(int64_t m, int K, int reps, int tail_split, double* a
     const int R = (int)(m / NB), ntiles = R * (R + 1);
     SyrkSrc src;
     src.W = W; src.ld = m; src.row0 = 0; src.res_row0 = 0; src.kbeg = 0; src.kend = K; src.P = P; src.ldp = m; src.part = 0; src.ncol1 = 2;
-    src.pf_mode = g_pf_mode;
     const SyrkSplit sp = syrk_split(ntiles, false, tail_split != 0);
     CUtensorMap mapPa, mapPb, mapQa, mapQb;
     rc = make_tensor_map(&mapPa, P, (uint64_t)m, (uint64_t)K, (uint64_t)m, SA);

@@ -62,7 +62,6 @@ __device__ __forceinline__ void tma_load_2d(void* smem_dst, const CUtensorMap* m
         "l"(map), "r"(c0), "r"(c1), "r"(smem_u32(bar))
         : "memory");
 }
-__device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];\n" ::"l"(p)); }
 __device__ __forceinline__ void tma_prefetch_l2(const void* p, uint32_t bytes) {
     asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;\n" ::"l"(p), "r"(bytes) : "memory");
 }
@@ -122,7 +121,7 @@ struct SyrkSrc {
     const double* P;
     int64_t ldp;
     int part, ncol1;
-    int pf_mode;     // how the next tile's C lines are pulled towards L2: 0 none, 1 prefetch.global.L2 per thread, 2 TMA bulk prefetch
+    static constexpr bool PREFETCH_C = true;   // the next tile's C lines are pulled towards L2 (gemm_persistent)
     // tile index -> (row r, 64-column tile jrel); host-callable so the CPU tests can check the coverage
     __host__ __device__ __forceinline__ void decode(int t, int& r, int& jrel) const {
         if (part == 0) {
@@ -179,7 +178,7 @@ struct SyrkSrc {
 struct SyrkTailSrc {
     SyrkSrc base;
     int first;
-    int pf_mode;
+    static constexpr bool PREFETCH_C = false;   // each quarter CTA reads its one C tile without an L2 prefetch
     template <int SH = 2>
     __device__ __forceinline__ TileDesc tile(int t) const {
         TileDesc d = base.template tile<1>(first + (t >> 2));
@@ -259,18 +258,12 @@ __device__ __forceinline__ void gemm_persistent(const Src& src, int ntiles, int 
 
     const int64_t coff0 = (wi * 8 * NI + tq * 2);
     const int joff0 = wj * 8 * NJ + g4;
-    // pull a tile's C lines (128 rows x 64 columns, read-modify-written by this CTA) towards L2 ahead of use
+    // pull a tile's C lines (TI rows x TJ columns, read-modify-written by this CTA) towards L2 ahead of use: one TMA
+    // bulk prefetch per column, where the tile source asks for it
     auto prefetch_c = [&](const TileDesc& t) {
-        int mode = 1;
-        if constexpr (MODE == 1) mode = src.pf_mode;
-        if (mode == 1) {
-            const double* c0 = t.C + coff0 + (int64_t)joff0 * t.ldc;
-#pragma unroll
-            for (int mj = 0; mj < NJ; ++mj)
-#pragma unroll
-                for (int ni = 0; ni < NI; ni += 2) prefetch_l2(c0 + ni * 8 + (int64_t)(mj * 8) * t.ldc);
-        } else if (mode == 2) {
-            if (lane < TS::TJ / 8) tma_prefetch_l2(t.C + (int64_t)(warp * (TS::TJ / 8) + lane) * t.ldc, TS::TI * 8);
+        if constexpr (MODE == 1) {
+            if constexpr (Src::PREFETCH_C)
+                if (lane < TS::TJ / 8) tma_prefetch_l2(t.C + (int64_t)(warp * (TS::TJ / 8) + lane) * t.ldc, TS::TI * 8);
         }
     };
     if (MODE == 1 && first_tile < ntiles) prefetch_c(src.template tile<SH>(first_tile));
@@ -362,8 +355,10 @@ __device__ __forceinline__ void gemm_persistent(const Src& src, int ntiles, int 
     }
 }
 
-// Persistent launch geometry: `nctas` CTAs walk the tiles round-robin.
-__global__ void __launch_bounds__(256, 2)
+// Persistent launch geometry: `nctas` CTAs walk the tiles round-robin, CTAS_PER_SM of them resident per SM (the
+// kernels are compiled for that occupancy; persistent_ctas and syrk_split in api.cu fill that many slots per SM).
+constexpr int CTAS_PER_SM = 2;
+__global__ void __launch_bounds__(256, CTAS_PER_SM)
 trsm3_kernel(TrsmSrc src, int ntiles, const __grid_constant__ CUtensorMap mapW, const __grid_constant__ CUtensorMap mapLinv) {
     extern __shared__ __align__(128) double sm[];
     TL_IN();
@@ -396,7 +391,7 @@ __device__ __forceinline__ void syrk_residual_block(const SyrkSrc& src, const do
 // 64 x 32 pieces that the block scheduler deals out as the persistent CTAs retire (m = 4096, K = 512: 1056 tiles on
 // 296 slots are 3 rounds + 168 tiles; as a 4th round those keep 57 % of the slots busy for a whole tile time).
 template <int SH>
-__global__ void __launch_bounds__(256, 2)
+__global__ void __launch_bounds__(256, CTAS_PER_SM)
 syrk3_kernel(SyrkSrc src, int ntiles, int nctas, int nres, const double* __restrict__ yk, double* __restrict__ rvec,
              int res_col0, const __grid_constant__ CUtensorMap mapPa, const __grid_constant__ CUtensorMap mapPb,
              const __grid_constant__ CUtensorMap mapQa, const __grid_constant__ CUtensorMap mapQb) {
@@ -412,7 +407,7 @@ syrk3_kernel(SyrkSrc src, int ntiles, int nctas, int nres, const double* __restr
         gemm_persistent<1, SH>(src, ntiles, b, nctas, sm, &mapPa, &mapPb);
     } else if constexpr (SH == 1) {
         SyrkTailSrc tail;
-        tail.base = src; tail.first = ntiles; tail.pf_mode = 0;
+        tail.base = src; tail.first = ntiles;
         const int q = b - nctas;
         gemm_persistent<1, 2>(tail, q + 1, q, 1 << 30, sm, &mapQa, &mapQb);
     }

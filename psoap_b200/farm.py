@@ -11,7 +11,6 @@ per-chunk log-likelihoods are combined with a single all-reduce of a length-n_ch
 filled, others zero: exact and order independent), then summed in chunk order like the reference's np.sum.
 """
 import ctypes
-import os
 
 import numpy as np
 
@@ -109,8 +108,8 @@ class ChunkFarm:
             # ... and the panels per trailing update likewise: rank-1024 updates (8) when there are at least 64 pairs to
             # hide their long heads behind, else rank-512 (4)
             n_pairs = self.n_chunks * self.n_proposals
-            chain = int(os.environ.get("PSOAP_FARM_CHAIN", 7 if n_pairs < 8 else 3))
-            group = int(os.environ.get("PSOAP_FARM_GROUP", 8 if n_pairs >= 64 else 4))
+            chain = 7 if n_pairs < 8 else 3
+            group = 8 if n_pairs >= 64 else 4
             d.reserved = chain | (group << 8)
             d.N, d.n_epochs = len(host["fl"]), len(host["dates"])
             d.lwl, d.epoch, d.fl = base + off["lwl"], base + off["epoch"], base + off["fl"]

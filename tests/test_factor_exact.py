@@ -164,17 +164,16 @@ def direct_plan(n, m, nsm, env=None):
     g = int(env.get("PSOAP_GROUP", 0))
     g_group = 8 if g >= 8 else 4 if g >= 4 else 2 if g >= 2 else 1 if g == 1 else 0
     potrf = 7 if int(env.get("PSOAP_POTRF", 7)) == 7 else 3
-    single_rows = int(env.get("PSOAP_SINGLE_ROWS", 24))
-    slots = max(1, min(2, int(env.get("PSOAP_CTAS_PER_SM", 2)))) * nsm
-    yl = int(env.get("PSOAP_YIELD_LOOKAHEAD", -1))
-    yield_mode = yl if yl >= 0 else (1 if Tt >= 96 else 2)
+    slots = 2 * nsm                                       # CTAS_PER_SM (gemm.cuh)
+    yl = int(env.get("PSOAP_YIELD_LOOKAHEAD", 0))
+    yield_mode = yl if yl in (1, 2) else (1 if Tt >= 96 else 2)
     tail = int(env.get("PSOAP_TAIL", 0)) != 0
     G = g_group or (4 if Tt >= 96 else 2)
     chain = 3 if Tt >= 192 else potrf
     lone = lookahead and chain == 7 and g_group == 0
     groups, a = [], 0
     while a < Te:
-        size = min(1 if (lone and Tt - a <= single_rows) else G, Te - a)
+        size = min(1 if (lone and Tt - a <= 24) else G, Te - a)   # SINGLE_ROWS = 24
         groups.append((a, size))
         a += size
     updates = []
@@ -222,17 +221,23 @@ CONFIGS = {
     "group4": {"PSOAP_GROUP": "4"},
     "group8": {"PSOAP_GROUP": "8"},
     "farm-sequence": {"PSOAP_LOOKAHEAD": "0", "PSOAP_POTRF": "3", "PSOAP_GROUP": "8", "PSOAP_PDL": "0"},
-    "no-small-tiles": {"PSOAP_SMALL_TILES": "0"},
     "quarter-tail": {"PSOAP_TAIL": "1"},
-    "yield0": {"PSOAP_YIELD_LOOKAHEAD": "0"},
     "yield1": {"PSOAP_YIELD_LOOKAHEAD": "1"},
     "yield2": {"PSOAP_YIELD_LOOKAHEAD": "2"},
-    "no-single-rows": {"PSOAP_SINGLE_ROWS": "0"},
-    "one-cta-per-sm": {"PSOAP_CTAS_PER_SM": "1"},
-    "prefetch0": {"PSOAP_PF_MODE": "0"},
-    "prefetch1": {"PSOAP_PF_MODE": "1"},
     "no-pdl": {"PSOAP_PDL": "0"},
     "pdl-everywhere": {"PSOAP_PDL": "100000"},
+    # uniform groups of 2 to the end (no single panels): the plan below 96 blocks without the single-panel tail
+    "group2": {"PSOAP_GROUP": "2"},
+    # chain 7 without the side stream: part-0 updates only, small tiles in the in-group column updates
+    "no-lookahead": {"PSOAP_LOOKAHEAD": "0"},
+    # the graph farm's sequence with rank-512 updates (ChunkFarm below 64 (proposal, chunk) pairs)
+    "farm-sequence-rank512": {"PSOAP_LOOKAHEAD": "0", "PSOAP_POTRF": "3", "PSOAP_GROUP": "4", "PSOAP_PDL": "0"},
+    # a captured look-ahead farm (fewer than 8 branches) that was given chain 3: side stream, no PDL
+    "lookahead-farm-sequence": {"PSOAP_POTRF": "3", "PSOAP_PDL": "0"},
+    # the direct plan from 192 blocks on (chain 3, G = 4, one tile per CTA in the bulk update)
+    "plan-from-192-blocks": {"PSOAP_POTRF": "3", "PSOAP_GROUP": "4", "PSOAP_YIELD_LOOKAHEAD": "1"},
+    # the direct plan from 96 blocks on without its single-panel end (chain 7, G = 4, one tile per CTA)
+    "group4-yield1": {"PSOAP_GROUP": "4", "PSOAP_YIELD_LOOKAHEAD": "1"},
 }
 # the pivot-failure cases run under both chains: potrf_diag7 + trsm7 (default below 192 blocks) and potrf_diag3 + trsm3
 PIVOT_CONFIGS = ("inverse-chain", "farm-sequence")

@@ -684,10 +684,9 @@ def test_farm_many_proposals(oracle, torch_cuda):
 @pytest.mark.gpu
 @pytest.mark.parametrize("env", [{"PSOAP_POTRF": "3"}, {"PSOAP_POTRF": "7", "PSOAP_GROUP": "4"},
                                  {"PSOAP_PDL": "0", "PSOAP_LOOKAHEAD": "0"}, {"PSOAP_PDL": "100000"},
-                                 {"PSOAP_FARM_PRIO": "0", "PSOAP_FARM_GROUP": "4"}, {"PSOAP_TAIL": "1"},
-                                 {"PSOAP_YIELD_LOOKAHEAD": "1"}],
+                                 {"PSOAP_TAIL": "1"}, {"PSOAP_YIELD_LOOKAHEAD": "1"}, {"PSOAP_FARM_LOOKAHEAD": "0"}],
                          ids=["inverse-chain-everywhere", "blocked-chain-everywhere-group4", "no-pdl-no-lookahead", "pdl-everywhere",
-                              "farm-without-priorities-rank512", "quarter-tile-tail", "one-tile-per-cta-bulk"])
+                              "quarter-tile-tail", "one-tile-per-cta-bulk", "farm-without-lookahead"])
 def test_alternative_kernel_paths(env, torch_cuda):
     """The library's environment switches select alternative kernels / launch modes for the same contract (the blocked
     diagonal factorisation + blocked panel solve of csrc/chain.cuh, launch attributes).  They are read once at load
