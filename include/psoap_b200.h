@@ -153,6 +153,35 @@ int psoap_predict_host(int ncomp, int mode, int64_t n, int64_t m, const double *
                        const double *sigma, const double *const *lwl_predict, const double *amp, const double *l,
                        double resid_mu, double nugget, double *delta_out, double *Sigma_out, psoap_result *result);
 
+/* ---- gradient of the log-likelihood ------------------------------------------------------------------- */
+/* lnlike_f / _f_g / _f_g_h (as psoap_lnlike) together with its exact gradient:
+ *   grad_hyp_dev [2 ncomp + 1]    d lnlike / d(amp_f, l_f, amp_g, l_g, amp_h, l_h (first 2 ncomp), mu_GP)
+ *   grad_lwl_dev [ncomp, N]       d lnlike / d lwl_c[i] (the shifted ln-wavelengths), or NULL when not wanted.
+ * K^-1 comes from eliminating the data block of [[K, I], [I, 0]] with the likelihood's kernels (about three times the
+ * work of psoap_lnlike for large N); every sum runs in a fixed order, so the result is bit-identical from run to run.
+ * Arguments, the negative-hyper-parameter and N = 0 conventions and the stream use are those of psoap_lnlike; when
+ * lnlike is -inf (negative hyper-parameters, info != 0) every gradient entry is NaN; N = 0 gives -0.0 and zeros.
+ * workspace_dev: >= psoap_lnlike_grad_workspace_bytes(ncomp, N) bytes, 256-byte aligned. */
+size_t psoap_lnlike_grad_workspace_bytes(int ncomp, int64_t N);
+int psoap_lnlike_grad(int ncomp, int64_t N, const double *lwl_f_dev, const double *lwl_g_dev, const double *lwl_h_dev,
+                      const double *fl_dev, const double *sigma_dev, const double *amp, const double *l, double mu_GP,
+                      void *workspace_dev, size_t workspace_bytes, psoap_result *result_dev, double *grad_hyp_dev,
+                      double *grad_lwl_dev, void *stream);
+/* Views into a gradient workspace after psoap_lnlike_grad (their offsets depend on N alone): -K^-1 as the lower
+ * triangle of a column-major [N, N] block with leading dimension *ld (data order), and -alpha = -K^-1 (fl - mu) [N]. */
+int psoap_lnlike_grad_views(void *workspace_dev, int64_t N, double **neg_kinv_dev, int64_t *ld, double **neg_alpha_dev);
+/* One chunk of the farm with its gradient for the full registered parameter vector p_dev (orbital then GP,
+ * utils.py:4-8; on the device): orbit velocities and sentinel, the Doppler-shifted fill, the identity-bordered
+ * elimination, the contraction, the per-epoch sum and the orbit Jacobian.  grad_p_dev [norb + 2 ncomp]; NaN when
+ * lnlike is -inf (|v| >= c, a negative GP hyper-parameter, info != 0).  chunk->reserved is ignored (the direct API's
+ * launch choices apply).  workspace_dev: >= psoap_chunk_lnprob_grad_workspace_bytes(model, N, n_epochs) bytes. */
+size_t psoap_chunk_lnprob_grad_workspace_bytes(int model, int64_t N, int32_t n_epochs);
+int psoap_chunk_lnprob_grad(int model, const psoap_chunk *chunk, const double *p_dev, double mu_GP, void *workspace_dev,
+                            size_t workspace_bytes, psoap_result *result_dev, double *grad_p_dev, void *stream);
+/* d v_c[ep] / d p_k of psoap_orbit_velocities: jac_dev [ncomp][n_epochs][norb], p_orb_dev in registered order. */
+int psoap_orbit_jacobian(int model, const double *p_orb_dev, const double *dates_dev, int n_epochs, double *jac_dev,
+                         void *stream);
+
 /* ---- chunk farm: psoap/sample_parallel.py:168-198, :371-390 ------------------------------------------ */
 typedef struct psoap_farm psoap_farm;
 size_t psoap_farm_workspace_bytes(int nchunks, const int64_t *N, const int32_t *n_epochs, int nbranch);

@@ -9,6 +9,7 @@ Everything runs in the CUDA library (csrc/): fill + blocked FP64 Cholesky with t
 quadratic form fused in.  predict_* build the bordered matrix [[K + s^2 I, C^T], [C, A]] on the device and take
 its Schur complement with the same factorisation kernels (A - C K^-1 C^T, and mu from the carried residual).
 """
+import collections
 import ctypes
 
 import numpy as np
@@ -86,6 +87,42 @@ def lnlike_host(lwls, fl, sigma, amps, ls, mu_GP=1.):
                                      sigma.ctypes.data_as(_lib.c_double_p), _lib.dbl_array(amps), _lib.dbl_array(ls),
                                      float(mu_GP), ctypes.byref(res)))
     return res.lnlike
+
+
+LnlikeGrad = collections.namedtuple("LnlikeGrad", ["lnlike", "amp", "l", "mu_GP", "lwl"])
+
+
+def lnlike_grad(lwls, fl, sigma, amps, ls, mu_GP=1.0):
+    """The log-likelihood of `_lnlike` and its exact gradient (psoap_lnlike_grad): returns
+    LnlikeGrad(lnlike, amp [ncomp], l [ncomp], mu_GP, lwl [ncomp, N]) with d lnlike / d(amp_c, l_c, mu_GP) as numpy
+    arrays / float and d lnlike / d lwls[c][i] as numpy or CUDA tensor like `fl`.  Inputs as in lnlike_f / _f_g / _f_g_h.
+    When lnlike is -inf (negative hyper-parameters, K not positive definite) every gradient entry is NaN."""
+    lib = _lib.load()
+    torch = _lib.torch_cuda()
+    on_dev = _is_dev(fl)
+    vecs = [_lib.dev_f64(v) for v in lwls]
+    fl_d, sg_d = _lib.dev_f64(fl), _lib.dev_f64(sigma)
+    ncomp, N = len(vecs), fl_d.numel()
+    if not 1 <= ncomp <= 3 or len(amps) != ncomp or len(ls) != ncomp:
+        raise ValueError("lnlike_grad takes 1 to 3 components, one amp and one l each")
+    for v in vecs + [sg_d]:
+        if v.dim() != 1 or v.numel() != N:
+            raise ValueError("wavelength, flux and sigma vectors must be 1-D with the same length")
+    nbytes = lib.psoap_lnlike_grad_workspace_bytes(ncomp, N)
+    ws = _lib.workspace(nbytes + 256, "lnlike_grad")
+    res = torch.empty(4, dtype=torch.float64, device="cuda")
+    g_hyp = torch.empty(2 * ncomp + 1, dtype=torch.float64, device="cuda")
+    g_lwl = torch.empty((ncomp, N), dtype=torch.float64, device="cuda")
+    ptrs = [_lib.ptr(v) for v in vecs] + [_lib.vp(None)] * (3 - ncomp)
+    _lib.check(lib.psoap_lnlike_grad(ncomp, N, ptrs[0], ptrs[1], ptrs[2], _lib.ptr(fl_d), _lib.ptr(sg_d),
+                                     _lib.dbl_array(amps), _lib.dbl_array(ls), float(mu_GP), _lib.ptr(ws), nbytes,
+                                     _lib.ptr(res), _lib.ptr(g_hyp), _lib.ptr(g_lwl) if N else _lib.vp(None),
+                                     _lib.stream_ptr()))
+    h = g_hyp.cpu().numpy()
+    if N == 0:
+        g_lwl.zero_()
+    return LnlikeGrad(float(res[0].item()), h[0:2 * ncomp:2].copy(), h[1:2 * ncomp:2].copy(), float(h[-1]),
+                      _out(g_lwl, on_dev))
 
 
 # --------------------------------------------------------------------------------------------------

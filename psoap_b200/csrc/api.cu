@@ -19,6 +19,7 @@
 #include "common.cuh"
 #include "fill.cuh"
 #include "gemm.cuh"
+#include "grad.cuh"
 #include "orbit.cuh"
 #include "predict.cuh"
 
@@ -237,8 +238,18 @@ cudaError_t launch_k(void (*kernel)(KArgs...), unsigned grid, unsigned block, si
 // traffic and the per-tile overhead of the dominant kernel by G.
 // Look-ahead: the big update first covers the next group's block columns (part 1); the next group's head
 // (potrf, trsm, column update, ...) then runs on the side stream under the rest of the update.
+//
+// identity_border: the border is the identity in data order (m = n, border row a is 1 at column pad + a; the gradient
+// entries).  C L^-T is then upper triangular, so border row block T_elim + b is zero in every panel before panel b, and
+// in the panel group that ends at block g1 only border row blocks [T_elim, T_elim + g1) are non-zero.  Every launch of
+// group q (the panel solves, the in-group column updates, both parts of the group update and the residual blocks) then
+// ends at row block T_elim + gstart[q + 1] instead of T_total: the rows it leaves out would only subtract exact zeros.
+// Each panel solve of a group covers up to the group's end, not only its own reach, because the group update reads the
+// group's panels side by side.  The elimination drops from 7 N^3 / 3 to N^3 flops.  Tile shapes, the group size, the
+// chain and the yield mode are still chosen from T_total, and every tile runs the same k loop as without the
+// restriction: the trailing block and the residual are the same bits.
 int launch_factor(const Lanes& ln, double* W, int64_t ld, int T_elim, int T_total, int pad, const FactorWs& ws,
-                  const int* sentinel, double* result) {
+                  const int* sentinel, double* result, bool identity_border = false) {
     const int64_t ldp = ws.Nt;
     CUtensorMap mapW, mapLinv, mapPa[2], mapPb[2], mapPas[2], mapPbs[2];   // ..s: boxes of the small tile shape
     CUtensorMap mapWblk, mapWt, mapL7[3];                                   // chain 7: diagonal block, panel tile, L_kk below its sub-blocks
@@ -277,8 +288,10 @@ int launch_factor(const Lanes& ln, double* W, int64_t ld, int T_elim, int T_tota
             launch_k(potrf_diag3_kernel, 1, 256, POTRF_SMEM, s, ln.pdl, (const double*)W, ld, kb, pad, ws.Linv, ws.rvec,
                      ws.y + (int64_t)kb * NB, ws.acc, ws.info, sentinel, (int)(kb == T_elim - 1), result);
     };
+    // last row block (exclusive) of the launches of group q; set once the group boundaries are known
+    std::vector<int> tend;
     auto trsm = [&](cudaStream_t s, int kb, int q, int col0) {
-        const int R = T_total - kb - 1;
+        const int R = tend[q] - kb - 1;
         if (chain == 7) {   // blocked substitution against L_kk and its 32 x 32 diagonal inverses (chain.cuh)
             Trsm7Args a;
             a.W = W; a.ld = ld; a.kb = kb; a.Lfac = ws.Linv; a.Xd = ws.Xd;
@@ -295,7 +308,7 @@ int launch_factor(const Lanes& ln, double* W, int64_t ld, int T_elim, int T_tota
     // update of row tiles [row0, T_total) with k range [kbeg, kend) of group buffer q; the residual blocks (if
     // ykb >= 0) apply panel ykb, whose columns start at res_col0 in the buffer
     auto syrk = [&](cudaStream_t s, int q, int row0, int kend, int part, int ncol1, int ykb, int res_col0) {
-        const int R = T_total - row0;
+        const int R = tend[q] - row0;
         // part 1 (the block columns the next diagonal blocks wait for) of a matrix factored on its own: 64 x 32 tiles,
         // four times the CTAs at a quarter of the latency each
         const int sh = (part == 1 && chain == 7) ? 2 : 1;
@@ -345,6 +358,7 @@ int launch_factor(const Lanes& ln, double* W, int64_t ld, int T_elim, int T_tota
         gstart.push_back(T_elim);
     }
     const int ngroups = (int)gstart.size() - 1;
+    for (int q = 0; q < ngroups; ++q) tend.push_back(identity_border ? T_elim + gstart[q + 1] : T_total);
     auto group_size = [&](int q) { return gstart[q + 1] - gstart[q]; };
     // everything of group q that precedes its big update: for each panel g: (column update with the group's
     // earlier panels, which also carries the residual update of panel g-1), potrf, trsm
@@ -354,7 +368,7 @@ int launch_factor(const Lanes& ln, double* W, int64_t ld, int T_elim, int T_tota
             const int kb = a + g;
             if (g > 0) syrk(s, q, kb, g * NB, 1, 2, kb - 1, (g - 1) * NB);   // block column kb, K = 128 g
             potrf(s, kb); LAUNCH_CHECK();
-            if (T_total - kb - 1 > 0) { trsm(s, kb, q, g * NB); LAUNCH_CHECK(); }
+            if (tend[q] - kb - 1 > 0) { trsm(s, kb, q, g * NB); LAUNCH_CHECK(); }
         }
         return PSOAP_OK;
     };
@@ -463,7 +477,7 @@ ZSource direct_z(const double* f, const double* g, const double* h) {
 extern "C" {
 
 const char* psoap_last_error(void) { return g_err.c_str(); }
-int psoap_version(void) { return 100; }
+int psoap_version(void) { return 101; }
 int psoap_device_count(void) {
     int n = 0;
     if (cudaGetDeviceCount(&n) != cudaSuccess) { cudaGetLastError(); return 0; }
@@ -692,6 +706,193 @@ extern "C" int psoap_schur_views(void* workspace, int64_t n, int64_t m, double**
     if (rvec) *rvec = ws.rvec;
     if (acc) *acc = ws.acc;
     if (info) *info = ws.info;
+    return PSOAP_OK;
+}
+
+// ---- gradient of the log-likelihood (grad.cuh) -----------------------------------------------------------
+namespace {
+// The gradient entries factor the identity-bordered matrix S = [[K, I], [I, 0]]: data block front-padded to Nn, a
+// border of Nn rows after it (no front padding), Nt = 2 Nn.  Workspace: S and the factorisation scratch first, so
+// that their offsets depend on N alone (psoap_lnlike_grad_views), then the contraction partials, then (chunk entry)
+// the velocity table, sentinel, orbit Jacobian and the per-pixel / per-epoch gradients.
+struct GradWs {
+    double* S;
+    FactorWs f;
+    double* tile;   // [ntiles][2 ncomp]
+    double* slot;   // [Tb][Tb][ncomp][128]
+    double* hyp;    // [2 ncomp + 1]
+    double* vel;    // [3][n_epochs]
+    int* flag;
+    double* jac;    // [3][n_epochs][norb]
+    double* gz;     // [ncomp][N]
+    double* gv;     // [3][n_epochs]
+    int64_t Nn, Nt;
+    int Tb, ntiles;
+};
+size_t carve_grad_ws(char* base, int ncomp, int64_t N, int n_epochs, int norb, GradWs* g) {
+    g->Nn = padded_dim(std::max<int64_t>(N, 1));
+    g->Nt = 2 * g->Nn;
+    g->Tb = (int)(g->Nn / NB);
+    g->ntiles = g->Tb * (g->Tb + 1) / 2;
+    size_t off = 0;
+    auto take = [&](size_t bytes) { char* r = base ? base + off : nullptr; off += align_up(bytes, 256); return r; };
+    g->S = (double*)take((size_t)g->Nt * g->Nt * 8);
+    const size_t fbytes = factor_ws_bytes(g->Nt) - align_up((size_t)g->Nt * g->Nt * 8, 256);
+    char* fb = take(fbytes);
+    if (base) carve_factor_ws(fb, g->Nt, &g->f, false);
+    g->tile = (double*)take((size_t)g->ntiles * 2 * ncomp * 8);
+    g->slot = (double*)take((size_t)g->Tb * g->Tb * ncomp * NB * 8);
+    g->hyp = (double*)take(8 * 8);
+    g->vel = (double*)take((size_t)3 * n_epochs * 8);
+    g->flag = (int*)take(4);
+    g->jac = (double*)take((size_t)3 * n_epochs * norb * 8);
+    g->gz = (double*)take((size_t)ncomp * N * 8);
+    g->gv = (double*)take((size_t)3 * n_epochs * 8);
+    return off;
+}
+
+// fill, identity border, restricted elimination, contraction and the hyper-parameter reduction (+ the per-pixel
+// gradient when grad_z is given) of one problem on ln.main
+int launch_grad(const Lanes& ln, int ncomp, int64_t N, const ZSource& zs, const double* fl, const double* sigma,
+                double mu, const GpParams& gp, const GradWs& g, const int* sentinel, double* result, double* grad_hyp,
+                double* grad_z) {
+    const int Tn = (int)(g.Nn / NB), Tt = 2 * Tn, pad = (int)(g.Nn - N);
+    cudaStream_t st = ln.main;
+    int rc = launch_fill_lower(ncomp, st, g.S, g.Nt, Tn, pad, zs, sigma, fl, mu, gp, g.f);
+    if (rc) return rc;
+    const unsigned nborder = (unsigned)((int64_t)Tt * (Tt + 1) / 2 - (int64_t)Tn * (Tn + 1) / 2);
+    grad_border_kernel<<<nborder, 256, 0, st>>>(g.S, g.Nt, (int)g.Nn, (int)N, pad, g.f.rvec);
+    LAUNCH_CHECK();
+    rc = launch_factor(ln, g.S, g.Nt, Tn, Tt, pad, g.f, sentinel, result, true);
+    if (rc) return rc;
+    const GradOut out{g.tile, g.slot, g.Tb};
+    if (ncomp == 1) lnlike_grad_kernel<1><<<g.ntiles, 256, 0, st>>>(g.S, g.Nt, (int)g.Nn, (int)N, g.f.rvec, zs, gp, out);
+    else if (ncomp == 2) lnlike_grad_kernel<2><<<g.ntiles, 256, 0, st>>>(g.S, g.Nt, (int)g.Nn, (int)N, g.f.rvec, zs, gp, out);
+    else lnlike_grad_kernel<3><<<g.ntiles, 256, 0, st>>>(g.S, g.Nt, (int)g.Nn, (int)N, g.f.rvec, zs, gp, out);
+    LAUNCH_CHECK();
+    grad_hyp_kernel<<<1, 256, 0, st>>>(g.tile, g.ntiles, ncomp, g.f.rvec, (int)g.Nn, (int)N, gp, g.f.info, sentinel, grad_hyp);
+    LAUNCH_CHECK();
+    if (grad_z) {
+        grad_pixel_kernel<<<(unsigned)(ncomp * g.Tb), NB, 0, st>>>(g.slot, g.Tb, ncomp, (int)N, gp, g.f.info, sentinel, grad_z);
+        LAUNCH_CHECK();
+    }
+    return PSOAP_OK;
+}
+
+int fill_value(double* p, int64_t n, double v, cudaStream_t st) {
+    if (n <= 0 || !p) return PSOAP_OK;
+    grad_fill_kernel<<<(unsigned)std::min<int64_t>((n + 255) / 256, 1024), 256, 0, st>>>(p, n, v);
+    LAUNCH_CHECK();
+    return PSOAP_OK;
+}
+}  // namespace
+
+extern "C" size_t psoap_lnlike_grad_workspace_bytes(int ncomp, int64_t N) {
+    if (ncomp < 1 || ncomp > 3 || N < 0) return 0;
+    GradWs g;
+    return carve_grad_ws(nullptr, ncomp, N, 0, 0, &g);
+}
+
+extern "C" int psoap_lnlike_grad(int ncomp, int64_t N, const double* lwl_f, const double* lwl_g, const double* lwl_h,
+                                 const double* fl, const double* sigma, const double* amp, const double* l, double mu_GP,
+                                 void* workspace, size_t workspace_bytes, psoap_result* result, double* grad_hyp,
+                                 double* grad_lwl, void* stream) {
+    if (ncomp < 1 || ncomp > 3 || N < 0 || N > 200000 || !amp || !l || !result || !grad_hyp)
+        return fail(PSOAP_ERR_ARG, "psoap_lnlike_grad: bad arguments");
+    cudaStream_t st = (cudaStream_t)stream;
+    const int nh = 2 * ncomp + 1;
+    GpParams gp;
+    if (make_gp(ncomp, amp, l, &gp)) {  // negative hyper-parameters: -inf, and no gradient
+        write_result_kernel<<<1, 1, 0, st>>>((double*)result, -INFINITY, 0.0, 0.0, 0.0);
+        LAUNCH_CHECK();
+        int rc = fill_value(grad_hyp, nh, NAN, st);
+        if (!rc) rc = fill_value(grad_lwl, (int64_t)ncomp * N, NAN, st);
+        return rc;
+    }
+    if (N == 0) {  // empty chunk: -0.0 (see psoap_lnlike), nothing depends on the parameters
+        write_result_kernel<<<1, 1, 0, st>>>((double*)result, -0.0, 0.0, 0.0, 0.0);
+        LAUNCH_CHECK();
+        return fill_value(grad_hyp, nh, 0.0, st);
+    }
+    if (!lwl_f || (ncomp > 1 && !lwl_g) || (ncomp > 2 && !lwl_h) || !fl || !sigma)
+        return fail(PSOAP_ERR_ARG, "psoap_lnlike_grad: null vector");
+    if (!workspace || workspace_bytes < psoap_lnlike_grad_workspace_bytes(ncomp, N) || ((uintptr_t)workspace & 255))
+        return fail(PSOAP_ERR_WORKSPACE, "psoap_lnlike_grad: workspace too small or not 256-byte aligned");
+    int rc = set_kernel_attributes();
+    if (rc) return rc;
+    GradWs g;
+    carve_grad_ws((char*)workspace, ncomp, N, 0, 0, &g);
+    Lanes ln;
+    rc = get_lanes(st, &ln);
+    if (rc) return rc;
+    return launch_grad(ln, ncomp, N, direct_z(lwl_f, lwl_g, lwl_h), fl, sigma, mu_GP, gp, g, nullptr, (double*)result,
+                       grad_hyp, grad_lwl);
+}
+
+extern "C" int psoap_lnlike_grad_views(void* workspace, int64_t N, double** neg_kinv_dev, int64_t* ld,
+                                       double** neg_alpha_dev) {
+    if (!workspace || N < 0) return fail(PSOAP_ERR_ARG, "psoap_lnlike_grad_views: bad arguments");
+    GradWs g;
+    carve_grad_ws((char*)workspace, 1, N, 0, 0, &g);
+    if (neg_kinv_dev) *neg_kinv_dev = g.S + g.Nn + g.Nn * g.Nt;
+    if (ld) *ld = g.Nt;
+    if (neg_alpha_dev) *neg_alpha_dev = g.f.rvec + g.Nn;
+    return PSOAP_OK;
+}
+
+extern "C" size_t psoap_chunk_lnprob_grad_workspace_bytes(int model, int64_t N, int32_t n_epochs) {
+    if (model < 1 || model > 5 || N < 1 || n_epochs < 1) return 0;
+    GradWs g;
+    return carve_grad_ws(nullptr, model_ncomp(model), N, n_epochs, model_norb(model), &g);
+}
+
+extern "C" int psoap_chunk_lnprob_grad(int model, const psoap_chunk* chunk, const double* p_dev, double mu_GP,
+                                       void* workspace, size_t workspace_bytes, psoap_result* result, double* grad_p,
+                                       void* stream) {
+    if (model < 1 || model > 5 || !chunk || !p_dev || !result || !grad_p || chunk->N < 1 || chunk->N > 200000 ||
+        chunk->n_epochs < 1 || !chunk->lwl || !chunk->epoch || !chunk->fl || !chunk->sigma || !chunk->dates)
+        return fail(PSOAP_ERR_ARG, "psoap_chunk_lnprob_grad: bad arguments");
+    const int64_t N = chunk->N;
+    const int ne = chunk->n_epochs, ncomp = model_ncomp(model), norb = model_norb(model);
+    if (!workspace || workspace_bytes < psoap_chunk_lnprob_grad_workspace_bytes(model, N, ne) ||
+        ((uintptr_t)workspace & 255))
+        return fail(PSOAP_ERR_WORKSPACE, "psoap_chunk_lnprob_grad: workspace too small or not 256-byte aligned");
+    int rc = set_kernel_attributes();
+    if (rc) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    GradWs g;
+    carve_grad_ws((char*)workspace, ncomp, N, ne, norb, &g);
+    // orbit velocities and the sentinel (|v| >= c, or a negative GP hyper-parameter), as the farm's orbit kernel
+    orbit_kernel<<<1, 128, 0, st>>>(model, p_dev, chunk->dates, ne, g.vel, g.flag, 1);
+    LAUNCH_CHECK();
+    // the farm's fused Doppler-shifted fill (farm_issue): base vector + epoch + velocity table, GP values on the device
+    ZSource zs;
+    zs.lwl[0] = chunk->lwl; zs.lwl[1] = nullptr; zs.lwl[2] = nullptr;
+    zs.epoch = chunk->epoch; zs.vel = g.vel; zs.n_epochs = ne; zs.shift = 1;
+    GpParams gp;
+    gp.dev = p_dev + norb;
+    for (int c = 0; c < 3; ++c) { gp.amp[c] = 0; gp.l[c] = 1; }
+    Lanes ln;
+    rc = get_lanes(st, &ln);
+    if (rc) return rc;
+    rc = launch_grad(ln, ncomp, N, zs, chunk->fl, chunk->sigma, mu_GP, gp, g, g.flag, (double*)result, g.hyp, g.gz);
+    if (rc) return rc;
+    grad_epoch_kernel<<<(unsigned)(ncomp * ne), 256, 0, st>>>(g.gz, chunk->epoch, N, ne, g.gv);
+    LAUNCH_CHECK();
+    orbit_jacobian_kernel<<<1, 128, 0, st>>>(model, p_dev, chunk->dates, ne, g.jac);
+    LAUNCH_CHECK();
+    grad_chain_kernel<<<1, 32, 0, st>>>(g.gv, g.jac, g.hyp, ncomp, ne, norb, g.f.info, g.flag, grad_p);
+    LAUNCH_CHECK();
+    return PSOAP_OK;
+}
+
+extern "C" int psoap_orbit_jacobian(int model, const double* p_orb_dev, const double* dates_dev, int n_epochs,
+                                    double* jac_dev, void* stream) {
+    if (model < 1 || model > 5 || !p_orb_dev || !dates_dev || !jac_dev || n_epochs < 0)
+        return fail(PSOAP_ERR_ARG, "psoap_orbit_jacobian: bad arguments");
+    if (n_epochs == 0) return PSOAP_OK;
+    orbit_jacobian_kernel<<<1, 128, 0, (cudaStream_t)stream>>>(model, p_orb_dev, dates_dev, n_epochs, jac_dev);
+    LAUNCH_CHECK();
     return PSOAP_OK;
 }
 

@@ -25,7 +25,8 @@ __device__ __forceinline__ double py_mod(double a, double b) {
 // True anomaly, orbit.py:47-72: t' = (t - T0) % P; solve E - e sin E = 2 pi t'/P; f = 2 atan(sqrt((1+e)/(1-e))
 // tan(E/2)), + 2 pi when E >= pi.  The reference calls scipy fsolve from E0 = M (lands within 2.8e-13 rad of
 // the root, SURVEY.md §7); here: Newton safeguarded by the bracket [0, 2 pi] (the function is monotone).
-__device__ inline double true_anomaly(double t, double T0, double P, double e) {
+// E_out (may be null) receives the eccentric anomaly E, for the orbit Jacobian.
+__device__ inline double true_anomaly(double t, double T0, double P, double e, double* E_out = nullptr) {
     const double PI = 3.141592653589793;
     const double tp = py_mod(t - T0, P);
     const double Mn = 2 * PI * tp / P;
@@ -39,6 +40,7 @@ __device__ inline double true_anomaly(double t, double T0, double P, double e) {
         E = En;
         if (dE <= 4.5e-16 * fmax(1.0, fabs(E))) break;
     }
+    if (E_out) *E_out = E;
     const double th = 2 * atan(sqrt((1 + e) / (1 - e)) * tan(E / 2.));
     return (E < PI) ? th : th + 2 * PI;
 }
@@ -98,6 +100,79 @@ __device__ inline void orbit_block(int model, const double* __restrict__ p, cons
     }
     __syncthreads();
     if (threadIdx.x == 0 && flag) flag[0] = s_flag;
+}
+
+// Derivatives of rv(K, e, omega, f(t; T0, P, e)) with respect to (K, e, omega, P, T0) at true anomaly f and eccentric
+// anomaly E.  M = 2 pi ((t - T0) mod P) / P: dM/dP = -2 pi (t - T0) / P^2, dM/dT0 = -2 pi / P (the modulus drops out);
+// dE/dM = 1 / (1 - e cos E), dE/de|M = sin E / (1 - e cos E), df/dE = sqrt(1 - e^2) / (1 - e cos E),
+// df/de|E = sin f / (1 - e^2).  The + 2 pi branch of true_anomaly changes no derivative.
+__device__ inline void rv_grad(double K, double e, double omega_deg, double P, double T0, double t, double f, double E,
+                               double g[5]) {
+    const double PI = 3.141592653589793;
+    const double w = omega_deg * PI / 180;
+    const double swf = sin(w + f), cw = cos(w);
+    const double den = 1.0 - e * cos(E);
+    const double se = sqrt(1.0 - e * e);
+    const double dfdM = se / (den * den);
+    const double dfde = se * sin(E) / (den * den) + sin(f) / (1.0 - e * e);
+    const double dvdf = -K * swf;
+    g[0] = cos(w + f) + e * cw;
+    g[1] = dvdf * dfde + K * cw;
+    g[2] = -K * (swf + e * sin(w)) * (PI / 180);
+    g[3] = dvdf * dfdM * (-2 * PI * (t - T0) / (P * P));
+    g[4] = dvdf * dfdM * (-2 * PI / P);
+}
+
+// dv_c[ep] / dp_k for every model, as orbit_block computes v: jac [ncomp][n_epochs][norb] (p in utils.registered_params
+// order).  The secondary of a pair uses K / q and omega + 180, the triples sum these terms.  One block; threads stride
+// over epochs.
+__device__ inline void orbit_jacobian_block(int model, const double* __restrict__ p, const double* __restrict__ dates,
+                                            int n_epochs, double* __restrict__ jac) {
+    const int ncomp = model_ncomp(model), norb = model_norb(model);
+    for (int ep = threadIdx.x; ep < n_epochs; ep += blockDim.x) {
+        const double t = dates[ep];
+        for (int c = 0; c < ncomp; ++c) {
+            double* Jc = jac + ((int64_t)c * n_epochs + ep) * norb;
+            for (int k = 0; k < norb; ++k) Jc[k] = 0.0;
+            Jc[norb - 1] = 1.0;                                              // gamma
+        }
+        double* J0 = jac + (int64_t)ep * norb;                               // rows of components 0, 1, 2
+        double* J1 = J0 + (int64_t)n_epochs * norb;
+        double* J2 = J1 + (int64_t)n_epochs * norb;
+        // Kepler term with scale K / q (q = 1: primary): derivatives into J at K index ik (and q index iq >= 0)
+        auto term = [&](double* Jc, int o, int iq, double q, double K, double e, double om, double P, double T0, double f,
+                        double E) {
+            double g[5];
+            rv_grad(K / q, e, om, P, T0, t, f, E, g);
+            Jc[o] += g[0] / q;
+            if (iq >= 0) Jc[iq] += -K / (q * q) * g[0];
+#pragma unroll
+            for (int k = 1; k < 5; ++k) Jc[o + k] += g[k];
+        };
+        if (model == SB1 || model == SB2) {
+            const int o = (model == SB2) ? 1 : 0;
+            const double K = p[o + 0], e = p[o + 1], om = p[o + 2], P = p[o + 3], T0 = p[o + 4];
+            double E;
+            const double f = true_anomaly(t, T0, P, e, &E);
+            term(J0, o, -1, 1.0, K, e, om, P, T0, f, E);
+            if (model == SB2) term(J1, o, 0, p[0], K, e, om + 180, P, T0, f, E);
+        } else {
+            const int o = (model == ST1) ? 0 : 1;
+            const double K_in = p[o + 0], e_in = p[o + 1], om_in = p[o + 2], P_in = p[o + 3], T0_in = p[o + 4];
+            const int oo = o + 5 + ((model == ST3) ? 1 : 0);
+            const double K_out = p[oo + 0], e_out = p[oo + 1], om_out = p[oo + 2], P_out = p[oo + 3], T0_out = p[oo + 4];
+            double Ei, Eo;
+            const double fi = true_anomaly(t, T0_in, P_in, e_in, &Ei);
+            const double fo = true_anomaly(t, T0_out, P_out, e_out, &Eo);
+            term(J0, o, -1, 1.0, K_in, e_in, om_in, P_in, T0_in, fi, Ei);
+            term(J0, oo, -1, 1.0, K_out, e_out, om_out, P_out, T0_out, fo, Eo);
+            if (model != ST1) {
+                term(J1, o, 0, p[0], K_in, e_in, om_in + 180, P_in, T0_in, fi, Ei);
+                term(J1, oo, -1, 1.0, K_out, e_out, om_out, P_out, T0_out, fo, Eo);
+            }
+            if (model == ST3) term(J2, oo, o + 5, p[o + 5], K_out, e_out, om_out + 180, P_out, T0_out, fo, Eo);
+        }
+    }
 }
 
 __global__ void orbit_kernel(int model, const double* __restrict__ p, const double* __restrict__ dates,

@@ -120,6 +120,10 @@ class ChunkFarm:
         self._dev_buf.copy_(self._host_buf, non_blocking=True)
         torch.cuda.synchronize()
         self.Ns = Ns
+        self.mu_GP = float(mu_GP)
+        self._descs = descs          # kept for the gradient entry, which takes one chunk at a time
+        self._n_epochs = nes
+        self._grad_ws = None         # allocated by the first lnprob_and_grad call
         self._farm = _lib.vp(None)
         K = self.n_proposals
         self._results = torch.zeros((K, max(1, len(self.mine)), 4), dtype=torch.float64, device="cuda")
@@ -203,6 +207,44 @@ class ChunkFarm:
         self._lnl_pin.copy_(self._lnl_all, non_blocking=False)
         sums = np.sum(self._lnl_pin.numpy(), axis=1)
         return float(sums[0]) if self.n_proposals == 1 else sums
+
+    def chunk_lnlike_grads(self, p):
+        """Per-chunk (lnlike, gradient) rows for the full registered vector p (orbital then GP, utils.py:4-8): device
+        tensor [n_chunks, n_params + 1].  This rank's chunks go one at a time through psoap_chunk_lnprob_grad, each
+        writing its row at its global chunk index; the other rows are zero, and with world_size > 1 the tensor is
+        all-reduced (exact: every row has one contributor).  The first call allocates one workspace for the largest
+        own chunk; a farm that never asks for a gradient holds none.  Gradient rows are NaN where lnlike is -inf."""
+        lib = _lib.load()
+        torch = _lib.torch_cuda()
+        p = np.asarray(p, dtype=np.float64)
+        if p.size != self.n_params:
+            raise ValueError("p must hold the %d registered parameters of %s" % (self.n_params, self.model))
+        npar = self.n_params
+        rows = torch.zeros((self.n_chunks, npar + 1), dtype=torch.float64, device="cuda")
+        if self.mine:
+            model = _lib.MODELS[self.model]
+            if self._grad_ws is None:
+                need = max(lib.psoap_chunk_lnprob_grad_workspace_bytes(model, N, ne)
+                           for N, ne in zip(self.Ns, self._n_epochs))
+                self._grad_ws = (torch.empty(need + 256, dtype=torch.uint8, device="cuda"), need)
+            ws, nbytes = self._grad_ws
+            p_dev = torch.from_numpy(p.reshape(-1).copy()).cuda()
+            res = torch.empty((len(self.mine), 4), dtype=torch.float64, device="cuda")
+            base, stride = rows.data_ptr(), (npar + 1) * 8
+            for k, idx in enumerate(self.mine):
+                _lib.check(lib.psoap_chunk_lnprob_grad(model, ctypes.byref(self._descs[k]), _lib.ptr(p_dev),
+                                                       self.mu_GP, _lib.ptr(ws), nbytes, _lib.ptr(res[k]),
+                                                       _lib.vp(base + idx * stride + 8), _lib.stream_ptr()))
+            rows[:, 0].index_copy_(0, self._mine_idx, res[:, 0])
+        if self.world_size > 1:
+            self._allreduce(rows)
+        return rows
+
+    def lnprob_and_grad(self, p):
+        """lnprob(p) and its gradient with respect to p: (float, ndarray [n_params]).  The per-chunk rows of
+        chunk_lnlike_grads are summed in chunk order on the host, so the bits do not depend on the number of GPUs."""
+        h = self.chunk_lnlike_grads(p).cpu().numpy()
+        return float(np.sum(h[:, 0])), np.sum(h[:, 1:], axis=0)
 
     def lnprob_many(self, P):
         """Ensemble evaluation (SURVEY.md §8f-2): P is [n_proposals, n_params]; one graph launch evaluates every

@@ -72,6 +72,22 @@ def velocities(model, p_orb, dates):
     return out
 
 
+def velocity_jacobian(model, p_orb, dates):
+    """d v_c[ep] / d p_orb[k] of `velocities` on the device: CUDA tensor [ncomp, n_dates, n_orb] (p_orb in
+    utils.registered_params order)."""
+    lib = _lib.load()
+    torch = _lib.torch_cuda()
+    p = _lib.dev_f64(p_orb)
+    d = _lib.dev_f64(np.atleast_1d(np.asarray(dates, dtype=np.float64)) if not isinstance(dates, torch.Tensor) else dates)
+    norb = _lib.N_ORB[model]
+    if p.numel() != norb:
+        raise ValueError("%s takes %d orbital parameters" % (model, norb))
+    out = torch.empty((_lib.NCOMP[model], d.numel(), norb), dtype=torch.float64, device="cuda")
+    _lib.check(lib.psoap_orbit_jacobian(_lib.MODELS[model], _lib.ptr(p), _lib.ptr(d), d.numel(), _lib.ptr(out),
+                                        _lib.stream_ptr()))
+    return out
+
+
 class SB1(_Orbit):
     """orbit.py:20-115: SB1(K, e, omega, P, T0, gamma, obs_dates=None)"""
     model = "SB1"
