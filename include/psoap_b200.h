@@ -201,7 +201,27 @@ size_t psoap_farm_workspace_bytes_batched(int nchunks, const int64_t *N, const i
 int psoap_farm_create_batched(psoap_farm **farm, int model, int nchunks, const psoap_chunk *chunks, int nprop,
                               int nbranch, double mu_GP, void *workspace_dev, size_t workspace_bytes);
 int psoap_farm_launches_per_eval(const psoap_farm *farm);
+/* Frees the farm's streams, events and graph, and its gradient graph when one is attached (not the workspaces). */
 int psoap_farm_destroy(psoap_farm *farm);
+
+/* Gradient graph of a farm: every (proposal, chunk) pair through the steps of psoap_chunk_lnprob_grad, nbranch pairs in
+ * flight, captured into a second CUDA graph beside the likelihood's (which, with its workspace and launch count, is left
+ * as it is).  A farm that never attaches one allocates and captures nothing for it.
+ * psoap_farm_grad_workspace_bytes: bytes the attach needs for nbranch branches (each holds the identity-bordered
+ * matrix of the largest chunk, 8 (2 padded(N))^2 bytes, plus its group buffers), 0 for a null farm or nbranch < 1.
+ * psoap_farm_grad_attach: captures the graph (once per farm); workspace_dev >= psoap_farm_grad_workspace_bytes(farm,
+ * nbranch) bytes, 256-byte aligned, valid for the farm's life.  Launch choices follow psoap_chunk.reserved as the
+ * likelihood graph's do; look-ahead is taken where the reserved chain is 7, so that with the reserved value set the
+ * gradient's bits depend neither on nbranch nor on how the chunks are partitioned over ranks. */
+size_t psoap_farm_grad_workspace_bytes(const psoap_farm *farm, int nbranch);
+int psoap_farm_grad_attach(psoap_farm *farm, int nbranch, void *workspace_dev, size_t workspace_bytes);
+/* p_dev: [nprop][n_params] contiguous, as psoap_farm_lnprob.  results_dev: [nprop][nchunks] records.
+ * grad_dev: [nprop][nchunks][n_params], the gradient of each pair's lnlike for the full registered vector (orbital then
+ * GP); a row is NaN where that pair's lnlike is -inf (|v| >= c, a negative GP value, info != 0), other rows are
+ * unaffected.  PSOAP_ERR_ARG before psoap_farm_grad_attach.  Every sum runs in a fixed order: the rows are
+ * bit-identical from call to call. */
+int psoap_farm_lnprob_grad(psoap_farm *farm, const double *p_dev, psoap_result *results_dev, double *grad_dev,
+                           void *stream);
 
 /* ---- measurement helpers ----------------------------------------------------------------------------- */
 /* Register-resident DMMA.8x8x4 loop on all SMs: measured FP64 tensor-pipe peak in TFLOP/s (synchronous). */

@@ -86,6 +86,9 @@ SIGNATURES = {
     "psoap_farm_lnprob": (ctypes.c_int, [vp, vp, vp, vp]),
     "psoap_farm_launches_per_eval": (ctypes.c_int, [vp]),
     "psoap_farm_destroy": (ctypes.c_int, [vp]),
+    "psoap_farm_grad_workspace_bytes": (ctypes.c_size_t, [vp, ctypes.c_int]),
+    "psoap_farm_grad_attach": (ctypes.c_int, [vp, ctypes.c_int, vp, ctypes.c_size_t]),
+    "psoap_farm_lnprob_grad": (ctypes.c_int, [vp, vp, vp, vp, vp]),
     "psoap_fp64_peak_tflops": (ctypes.c_int, [c_double_p]),
     "psoap_bench_syrk": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int, ctypes.c_int, c_double_p, c_double_p]),
     "psoap_bench_syrk_split": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int, ctypes.c_int, ctypes.c_int, c_double_p, c_double_p]),

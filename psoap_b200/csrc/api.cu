@@ -477,7 +477,7 @@ ZSource direct_z(const double* f, const double* g, const double* h) {
 extern "C" {
 
 const char* psoap_last_error(void) { return g_err.c_str(); }
-int psoap_version(void) { return 101; }
+int psoap_version(void) { return 102; }
 int psoap_device_count(void) {
     int n = 0;
     if (cudaGetDeviceCount(&n) != cudaSuccess) { cudaGetLastError(); return 0; }
@@ -1017,6 +1017,34 @@ extern "C" int psoap_predict_host(int ncomp, int mode, int64_t n, int64_t m, con
 // Chunk farm
 // ======================================================================================================
 constexpr int P_STRIDE = 32;  // doubles reserved per proposal in the parameter buffer
+namespace {
+// The optional gradient graph of a farm (psoap_farm_grad_attach): its own parameter buffer, velocity tables,
+// sentinels, orbit Jacobians and outputs per (proposal, chunk) item, and one GradWs region per branch, carved for
+// each item in turn (items of a branch run in stream order).
+struct FarmGrad {
+    int nbranch = 0;
+    bool lookahead = false;
+    bool direct = false;
+    double* p_buf = nullptr;          // [nprop][P_STRIDE]
+    double* results = nullptr;        // [nitems][4]
+    double* grad = nullptr;           // [nitems][n_params]
+    int* flags = nullptr;             // per item sentinel
+    OrbitDesc* descs = nullptr;       // device, per item
+    JacDesc* jdescs = nullptr;        // device, per item
+    std::vector<double*> item_vel;    // [ncomp][n_epochs] per item
+    std::vector<double*> item_jac;    // [ncomp][n_epochs][norb] per item
+    std::vector<char*> branch_base;   // GradWs region of each branch
+    std::vector<std::vector<int>> branch_items;
+    cudaGraph_t graph = nullptr;
+    cudaGraphExec_t exec = nullptr;
+    std::vector<cudaStream_t> streams;
+    std::vector<cudaStream_t> side_streams;
+    std::vector<cudaEvent_t> events;
+    std::vector<cudaEvent_t> side_events;
+    int launches = 0;
+};
+}  // namespace
+
 struct psoap_farm {
     int model = 0, ncomp = 0, norb = 0, nchunks = 0, nprop = 1, nitems = 0, nbranch = 0;
     double mu = 1.0;
@@ -1041,9 +1069,31 @@ struct psoap_farm {
     int chain_hint = 0;               // psoap_chunk.reserved of the first chunk, low byte: 3 | 7 forces the chain links
     int group_hint = 0;               // ... bits 8 and up: 2 | 4 | 8 forces the panels per trailing update
     int launches = 0;
+    FarmGrad* grad = nullptr;         // psoap_farm_grad_attach; null until then
 };
 
 namespace {
+// The launch plan of one work item on branch b, shared by the likelihood graph and the gradient graph so that the two
+// cannot drift apart.  `nbranch` and `lookahead` are the issuing graph's.
+Lanes farm_lanes(const psoap_farm* f, int nbranch, bool lookahead, cudaStream_t main, cudaStream_t side, cudaEvent_t e1,
+                 cudaEvent_t e2, int pdl) {
+    Lanes ln;
+    ln.main = main;
+    ln.side = lookahead ? side : nullptr;
+    ln.e1 = e1; ln.e2 = e2;
+    // panels per update: the caller's choice (bits 8.. of psoap_chunk.reserved: 2, 4 or 8, again the same on every
+    // rank), else by the number of chunks in flight: rank-1024 updates need many to hide their 8-panel heads (C1
+    // x 8 proposals on 8 branches: 1121 evals/s against 1149 with rank-512)
+    ln.group = lookahead ? 0
+             : (f->group_hint == 2 || f->group_hint == 4 || f->group_hint == 8) ? f->group_hint
+             : (nbranch >= 32 ? 8 : 4);
+    ln.pdl = pdl;
+    // chain links: the caller's choice (psoap_chunk.reserved = 3 | 7, the same on every rank of a partitioned
+    // farm so that the bits do not depend on the number of GPUs), else by exposure of the chain latency
+    ln.chain = (f->chain_hint == 3 || f->chain_hint == 7) ? f->chain_hint : (lookahead ? 0 : 3);
+    return ln;
+}
+
 // Issues one evaluation onto the farm's streams, rooted at s0: the orbit kernel for every item, then the per-chunk
 // pipelines on the branch streams, joined back into s0.  Runs under stream capture (graph mode) or for real
 // (direct mode, which adds programmatic dependent launch on the small grids).
@@ -1066,20 +1116,8 @@ int farm_issue(psoap_farm* f, cudaStream_t s0, int pdl) {
             zs.epoch = ch.epoch; zs.vel = f->item_vel[it]; zs.n_epochs = ch.n_epochs; zs.shift = 1;
             FactorWs ws = f->branch_ws[b];
             ws.Nt = padded_dim(ch.N);
-            Lanes ln;
-            ln.main = sb;
-            ln.side = f->lookahead ? f->side_streams[b] : nullptr;
-            ln.e1 = f->side_events[2 * b]; ln.e2 = f->side_events[2 * b + 1];
-            // panels per update: the caller's choice (bits 8.. of psoap_chunk.reserved: 2, 4 or 8, again the same on every
-            // rank), else by the number of chunks in flight: rank-1024 updates need many to hide their 8-panel heads (C1
-            // x 8 proposals on 8 branches: 1121 evals/s against 1149 with rank-512)
-            ln.group = f->lookahead ? 0
-                     : (f->group_hint == 2 || f->group_hint == 4 || f->group_hint == 8) ? f->group_hint
-                     : (nbranch >= 32 ? 8 : 4);
-            ln.pdl = pdl;
-            // chain links: the caller's choice (psoap_chunk.reserved = 3 | 7, the same on every rank of a partitioned
-            // farm so that the bits do not depend on the number of GPUs), else by exposure of the chain latency
-            ln.chain = (f->chain_hint == 3 || f->chain_hint == 7) ? f->chain_hint : (f->lookahead ? 0 : 3);
+            const Lanes ln = farm_lanes(f, nbranch, f->lookahead, sb, f->side_streams[b], f->side_events[2 * b],
+                                        f->side_events[2 * b + 1], pdl);
             rc = launch_chunk(ln, f->ncomp, ch.N, zs, ch.fl, ch.sigma, f->mu, gp, ws, f->flags + it, f->results + 4 * it);
             if (rc) break;
         }
@@ -1087,6 +1125,155 @@ int farm_issue(psoap_farm* f, cudaStream_t s0, int pdl) {
         cudaStreamWaitEvent(s0, f->events[b], 0);
     }
     return rc;
+}
+
+// the per-epoch sums and the chain rule of one gradient item (steps 7 and 8 of psoap_chunk_lnprob_grad)
+int launch_grad_chain(cudaStream_t st, int ncomp, int norb, const psoap_chunk& ch, const GradWs& w, const double* jac,
+                      const int* sentinel, double* grad_p) {
+    grad_epoch_kernel<<<(unsigned)(ncomp * ch.n_epochs), 256, 0, st>>>(w.gz, ch.epoch, ch.N, ch.n_epochs, w.gv);
+    LAUNCH_CHECK();
+    grad_chain_kernel<<<1, 32, 0, st>>>(w.gv, jac, w.hyp, ncomp, ch.n_epochs, norb, w.f.info, sentinel, grad_p);
+    LAUNCH_CHECK();
+    return PSOAP_OK;
+}
+
+// The gradient counterpart of farm_issue: velocities, sentinels and orbit Jacobians of every item, then per branch,
+// item after item in LPT order, the steps of psoap_chunk_lnprob_grad into the item's result and gradient rows.
+int farm_grad_issue(psoap_farm* f, cudaStream_t s0, int pdl) {
+    FarmGrad& g = *f->grad;
+    const int nbranch = g.nbranch, nchunks = f->nchunks, np = f->norb + 2 * f->ncomp;
+    orbit_farm_kernel<<<f->nitems, 64, 0, s0>>>(f->model, g.p_buf, g.descs);
+    ++g_launches;
+    orbit_jacobian_farm_kernel<<<f->nitems, 64, 0, s0>>>(f->model, g.p_buf, g.jdescs);
+    ++g_launches;
+    cudaEventRecord(g.events[nbranch], s0);
+    int rc = PSOAP_OK;
+    for (int b = 0; b < nbranch && rc == PSOAP_OK; ++b) {
+        cudaStream_t sb = g.streams[b];
+        cudaStreamWaitEvent(sb, g.events[nbranch], 0);
+        for (int it : g.branch_items[b]) {
+            const psoap_chunk& ch = f->chunks[it % nchunks];
+            GpParams gp;
+            gp.dev = g.p_buf + (size_t)(it / nchunks) * P_STRIDE + f->norb;
+            for (int c = 0; c < 3; ++c) { gp.amp[c] = 0; gp.l[c] = 1; }
+            ZSource zs;
+            zs.lwl[0] = ch.lwl; zs.lwl[1] = nullptr; zs.lwl[2] = nullptr;
+            zs.epoch = ch.epoch; zs.vel = g.item_vel[it]; zs.n_epochs = ch.n_epochs; zs.shift = 1;
+            GradWs w;
+            carve_grad_ws(g.branch_base[b], f->ncomp, ch.N, ch.n_epochs, f->norb, &w);
+            const Lanes ln = farm_lanes(f, nbranch, g.lookahead, sb, g.side_streams[b], g.side_events[2 * b],
+                                        g.side_events[2 * b + 1], pdl);
+            rc = launch_grad(ln, f->ncomp, ch.N, zs, ch.fl, ch.sigma, f->mu, gp, w, g.flags + it, g.results + 4 * it,
+                             w.hyp, w.gz);
+            if (!rc) rc = launch_grad_chain(sb, f->ncomp, f->norb, ch, w, g.item_jac[it], g.flags + it,
+                                            g.grad + (size_t)it * np);
+            if (rc) break;
+        }
+        cudaEventRecord(g.events[b], sb);
+        cudaStreamWaitEvent(s0, g.events[b], 0);
+    }
+    return rc;
+}
+
+// LPT (longest processing time first) assignment of work items (item = prop * nchunks + chunk) to branches by N^3
+std::vector<std::vector<int>> lpt_items(const std::vector<int64_t>& Ns, int nitems, int nbranch) {
+    const int nchunks = (int)Ns.size();
+    std::vector<int> order(nitems);
+    std::iota(order.begin(), order.end(), 0);
+    std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return Ns[a % nchunks] > Ns[b % nchunks]; });
+    std::vector<double> load(nbranch, 0.0);
+    std::vector<std::vector<int>> items(nbranch);
+    for (int it : order) {
+        int b = (int)(std::min_element(load.begin(), load.end()) - load.begin());
+        items[b].push_back(it);
+        const double n = (double)Ns[it % nchunks];
+        load[b] += n * n * n;
+    }
+    return items;
+}
+
+// Branch streams (+ the root stream at index nbranch), their events, and the high-priority side streams of look-ahead
+void create_farm_streams(int nbranch, bool lookahead, std::vector<cudaStream_t>& streams,
+                         std::vector<cudaEvent_t>& events, std::vector<cudaStream_t>& side_streams,
+                         std::vector<cudaEvent_t>& side_events) {
+    streams.resize(nbranch + 1);
+    events.resize(nbranch + 1);
+    {
+        // Branch b carries the b-th largest items first (LPT order): its stream gets the matching priority level, which a
+        // captured kernel node inherits.  Measured neutral on a B200 against all-equal priorities (one rank's share of
+        // an 8-GPU run: 28.50 ms either way; a launch-attribute variant likewise): the drain at the end of an evaluation
+        // is not a matter of which chunk gets the free SM slots first.
+        int lo = 0, hi = 0;
+        cudaDeviceGetStreamPriorityRange(&lo, &hi);
+        const int nlev = lo - hi + 1;
+        for (int b = 0; b <= nbranch; ++b) {
+            // (a look-ahead farm's branch streams carry the bulk updates: lowest priority, below their side streams, where
+            // the chain links run; with both at the top C2 ran at 95.5 instead of 104 evals/s)
+            const int pr = (b < nbranch && nlev > 1 && !lookahead) ? hi + (int)((int64_t)b * nlev / nbranch) : lo;
+            cudaStreamCreateWithPriority(&streams[b], cudaStreamNonBlocking, pr);
+        }
+    }
+    for (auto& ev : events) cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
+    side_streams.resize(nbranch);
+    side_events.resize(2 * nbranch);
+    {
+        int lo = 0, hi = 0;
+        cudaDeviceGetStreamPriorityRange(&lo, &hi);
+        for (auto& s : side_streams) cudaStreamCreateWithPriority(&s, cudaStreamNonBlocking, hi);
+        for (auto& ev : side_events) cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
+    }
+}
+
+void destroy_farm_streams(std::vector<cudaStream_t>& streams, std::vector<cudaEvent_t>& events,
+                          std::vector<cudaStream_t>& side_streams, std::vector<cudaEvent_t>& side_events) {
+    for (auto& s : streams) if (s) cudaStreamDestroy(s);
+    for (auto& s : side_streams) if (s) cudaStreamDestroy(s);
+    for (auto& ev : events) if (ev) cudaEventDestroy(ev);
+    for (auto& ev : side_events) if (ev) cudaEventDestroy(ev);
+}
+
+// Layout of a gradient workspace (base null: sizes only): the per-item buffers, then nbranch GradWs regions sized for
+// the largest chunk and the most epochs (every GradWs buffer grows with N and with n_epochs, so an item's carve fits).
+size_t carve_farm_grad(const psoap_farm* f, int nbranch, char* base, FarmGrad* g) {
+    const int nitems = f->nitems, np = f->norb + 2 * f->ncomp;
+    size_t off = 0;
+    auto take = [&](size_t bytes) { char* r = base ? base + off : nullptr; off += align_up(bytes, 256); return r; };
+    char* p_buf = take((size_t)f->nprop * P_STRIDE * 8);
+    char* results = take((size_t)nitems * 4 * 8);
+    char* grad = take((size_t)nitems * np * 8);
+    char* flags = take((size_t)nitems * 4);
+    char* descs = take((size_t)nitems * sizeof(OrbitDesc));
+    char* jdescs = take((size_t)nitems * sizeof(JacDesc));
+    if (g) {
+        g->p_buf = (double*)p_buf; g->results = (double*)results; g->grad = (double*)grad; g->flags = (int*)flags;
+        g->descs = (OrbitDesc*)descs; g->jdescs = (JacDesc*)jdescs;
+        g->item_vel.resize(nitems); g->item_jac.resize(nitems); g->branch_base.resize(nbranch);
+    }
+    int64_t nmax = 1;
+    int nemax = 1;
+    for (int it = 0; it < nitems; ++it) {
+        const psoap_chunk& ch = f->chunks[it % f->nchunks];
+        nmax = std::max<int64_t>(nmax, ch.N);
+        nemax = std::max(nemax, (int)ch.n_epochs);
+        char* vel = take((size_t)f->ncomp * ch.n_epochs * 8);
+        char* jac = take((size_t)f->ncomp * ch.n_epochs * f->norb * 8);
+        if (g) { g->item_vel[it] = (double*)vel; g->item_jac[it] = (double*)jac; }
+    }
+    GradWs probe;
+    const size_t per_branch = carve_grad_ws(nullptr, f->ncomp, nmax, nemax, f->norb, &probe);
+    for (int b = 0; b < nbranch; ++b) {
+        char* r = take(per_branch);
+        if (g) g->branch_base[b] = r;
+    }
+    return off;
+}
+
+void destroy_farm_grad(FarmGrad* g) {
+    if (!g) return;
+    if (g->exec) cudaGraphExecDestroy(g->exec);
+    if (g->graph) cudaGraphDestroy(g->graph);
+    destroy_farm_streams(g->streams, g->events, g->side_streams, g->side_events);
+    delete g;
 }
 }  // namespace
 
@@ -1176,48 +1363,12 @@ int psoap_farm_create_batched(psoap_farm** out, int model, int nchunks, const ps
     cudaError_t e = cudaMemcpy(f->descs, hd.data(), (size_t)nitems * sizeof(OrbitDesc), cudaMemcpyHostToDevice);
     if (e != cudaSuccess) { delete f; return fail(PSOAP_ERR_CUDA, std::string("farm descs: ") + cudaGetErrorString(e)); }
 
-    // LPT (longest processing time first) assignment of work items to branches by N^3
-    std::vector<int> order(nitems);
-    std::iota(order.begin(), order.end(), 0);
-    std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return Ns[a % nchunks] > Ns[b % nchunks]; });
-    std::vector<double> load(nbranch, 0.0);
-    f->branch_items.assign(nbranch, {});
-    for (int it : order) {
-        int b = (int)(std::min_element(load.begin(), load.end()) - load.begin());
-        f->branch_items[b].push_back(it);
-        const double n = (double)Ns[it % nchunks];
-        load[b] += n * n * n;
-    }
+    f->branch_items = lpt_items(Ns, nitems, nbranch);
 
     const char* la_env = getenv("PSOAP_FARM_LOOKAHEAD");
     f->lookahead = la_env ? (atoi(la_env) != 0) : (nbranch < 8);
     // capture the whole evaluation into one CUDA graph
-    f->streams.resize(nbranch + 1);
-    f->events.resize(nbranch + 1);
-    {
-        // Branch b carries the b-th largest items first (LPT order): its stream gets the matching priority level, which a
-        // captured kernel node inherits.  Measured neutral on a B200 against all-equal priorities (one rank's share of
-        // an 8-GPU run: 28.50 ms either way; a launch-attribute variant likewise): the drain at the end of an evaluation
-        // is not a matter of which chunk gets the free SM slots first.
-        int lo = 0, hi = 0;
-        cudaDeviceGetStreamPriorityRange(&lo, &hi);
-        const int nlev = lo - hi + 1;
-        for (int b = 0; b <= nbranch; ++b) {
-            // (a look-ahead farm's branch streams carry the bulk updates: lowest priority, below their side streams, where
-            // the chain links run; with both at the top C2 ran at 95.5 instead of 104 evals/s)
-            const int pr = (b < nbranch && nlev > 1 && !f->lookahead) ? hi + (int)((int64_t)b * nlev / nbranch) : lo;
-            cudaStreamCreateWithPriority(&f->streams[b], cudaStreamNonBlocking, pr);
-        }
-    }
-    for (auto& ev : f->events) cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
-    f->side_streams.resize(nbranch);
-    f->side_events.resize(2 * nbranch);
-    {
-        int lo = 0, hi = 0;
-        cudaDeviceGetStreamPriorityRange(&lo, &hi);
-        for (auto& s : f->side_streams) cudaStreamCreateWithPriority(&s, cudaStreamNonBlocking, hi);
-        for (auto& ev : f->side_events) cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
-    }
+    create_farm_streams(nbranch, f->lookahead, f->streams, f->events, f->side_streams, f->side_events);
     cudaStream_t s0 = f->streams[nbranch];
     const int64_t before = g_launches.load();
     f->item_vel.resize(nitems);
@@ -1281,11 +1432,101 @@ int psoap_farm_destroy(psoap_farm* f) {
     if (!f) return PSOAP_OK;
     if (f->exec) cudaGraphExecDestroy(f->exec);
     if (f->graph) cudaGraphDestroy(f->graph);
-    for (auto& s : f->streams) if (s) cudaStreamDestroy(s);
-    for (auto& s : f->side_streams) if (s) cudaStreamDestroy(s);
-    for (auto& ev : f->events) if (ev) cudaEventDestroy(ev);
-    for (auto& ev : f->side_events) if (ev) cudaEventDestroy(ev);
+    destroy_farm_streams(f->streams, f->events, f->side_streams, f->side_events);
+    destroy_farm_grad(f->grad);
     delete f;
+    return PSOAP_OK;
+}
+
+// ---- gradient graph of a farm -----------------------------------------------------------------------------------
+size_t psoap_farm_grad_workspace_bytes(const psoap_farm* f, int nbranch) {
+    if (!f || nbranch < 1) return 0;
+    return carve_farm_grad(f, std::min(nbranch, f->nitems), nullptr, nullptr);
+}
+
+int psoap_farm_grad_attach(psoap_farm* f, int nbranch, void* workspace, size_t workspace_bytes) {
+    if (!f || nbranch < 1 || !workspace) return fail(PSOAP_ERR_ARG, "psoap_farm_grad_attach: bad arguments");
+    if (f->grad) return fail(PSOAP_ERR_ARG, "psoap_farm_grad_attach: the farm already has a gradient graph");
+    nbranch = std::min(nbranch, f->nitems);
+    if (((uintptr_t)workspace & 255) || workspace_bytes < psoap_farm_grad_workspace_bytes(f, nbranch))
+        return fail(PSOAP_ERR_WORKSPACE, "psoap_farm_grad_attach: workspace too small or not 256-byte aligned");
+    int rc = set_kernel_attributes();
+    if (rc) return rc;
+    FarmGrad* g = new FarmGrad();
+    g->nbranch = nbranch;
+    carve_farm_grad(f, nbranch, (char*)workspace, g);
+    const int nitems = f->nitems, nchunks = f->nchunks;
+    std::vector<OrbitDesc> hd(nitems);
+    std::vector<JacDesc> hj(nitems);
+    std::vector<int64_t> Ns(nchunks);
+    int64_t nmax = 0;
+    for (int i = 0; i < nchunks; ++i) { Ns[i] = f->chunks[i].N; nmax = std::max(nmax, Ns[i]); }
+    for (int it = 0; it < nitems; ++it) {
+        const psoap_chunk& ch = f->chunks[it % nchunks];
+        const int k = it / nchunks;
+        hd[it].dates = ch.dates; hd[it].vel = g->item_vel[it]; hd[it].flag = g->flags + it;
+        hd[it].n_epochs = ch.n_epochs; hd[it].p_off = k * P_STRIDE;
+        hj[it].dates = ch.dates; hj[it].jac = g->item_jac[it]; hj[it].n_epochs = ch.n_epochs; hj[it].p_off = k * P_STRIDE;
+    }
+    cudaError_t e = cudaMemcpy(g->descs, hd.data(), (size_t)nitems * sizeof(OrbitDesc), cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) e = cudaMemcpy(g->jdescs, hj.data(), (size_t)nitems * sizeof(JacDesc), cudaMemcpyHostToDevice);
+    if (e != cudaSuccess) { delete g; return fail(PSOAP_ERR_CUDA, std::string("farm grad descs: ") + cudaGetErrorString(e)); }
+    g->branch_items = lpt_items(Ns, nitems, nbranch);
+    // Look-ahead changes the panel groups of the elimination, hence its bits.  When the caller passes the chain links
+    // (psoap_chunk.reserved, chosen from the global problem: 7 for fewer than 8 (proposal, chunk) pairs in all), the
+    // gradient graph takes look-ahead exactly there, so that its rows depend neither on the branch count nor on the
+    // number of GPUs; without that hint it decides by branch count, as the likelihood graph does.
+    const char* la_env = getenv("PSOAP_FARM_LOOKAHEAD");
+    g->lookahead = la_env ? (atoi(la_env) != 0)
+                 : (f->chain_hint == 3 || f->chain_hint == 7) ? (f->chain_hint == 7) : (nbranch < 8);
+    const char* de = getenv("PSOAP_FARM_DIRECT");
+    g->direct = de ? (atoi(de) != 0) : (g->lookahead && nmax >= 7000);
+    create_farm_streams(nbranch, g->lookahead, g->streams, g->events, g->side_streams, g->side_events);
+    f->grad = g;
+    cudaStream_t s0 = g->streams[nbranch];
+    const int64_t before = g_launches.load();
+    e = cudaStreamBeginCapture(s0, cudaStreamCaptureModeThreadLocal);
+    if (e != cudaSuccess) {
+        destroy_farm_grad(g); f->grad = nullptr;
+        return fail(PSOAP_ERR_CUDA, std::string("begin capture: ") + cudaGetErrorString(e));
+    }
+    rc = farm_grad_issue(f, s0, 0);
+    e = cudaStreamEndCapture(s0, &g->graph);
+    g->launches = (int)(g_launches.load() - before);
+    g_launches = before;  // capture is not execution
+    if (rc == PSOAP_OK && e != cudaSuccess) rc = fail(PSOAP_ERR_CUDA, std::string("end capture: ") + cudaGetErrorString(e));
+    if (rc == PSOAP_OK) {
+        e = cudaGraphInstantiate(&g->exec, g->graph, 0);
+        if (e != cudaSuccess) rc = fail(PSOAP_ERR_CUDA, std::string("graph instantiate: ") + cudaGetErrorString(e));
+    }
+    if (rc != PSOAP_OK) { destroy_farm_grad(g); f->grad = nullptr; }
+    return rc;
+}
+
+int psoap_farm_lnprob_grad(psoap_farm* f, const double* p_dev, psoap_result* results_dev, double* grad_dev,
+                           void* stream) {
+    if (!f || !p_dev || !results_dev || !grad_dev) return fail(PSOAP_ERR_ARG, "psoap_farm_lnprob_grad: bad arguments");
+    if (!f->grad) return fail(PSOAP_ERR_ARG, "psoap_farm_lnprob_grad: no gradient graph (psoap_farm_grad_attach first)");
+    FarmGrad& g = *f->grad;
+    cudaStream_t st = (cudaStream_t)stream;
+    const int np = f->norb + 2 * f->ncomp;
+    CUDA_TRY(cudaMemcpy2DAsync(g.p_buf, P_STRIDE * 8, p_dev, (size_t)np * 8, (size_t)np * 8, f->nprop,
+                               cudaMemcpyDeviceToDevice, st));
+    if (g.direct) {
+        cudaStream_t s0 = g.streams[g.nbranch];
+        cudaEvent_t fork = g.events[g.nbranch];
+        CUDA_TRY(cudaEventRecord(fork, st));
+        CUDA_TRY(cudaStreamWaitEvent(s0, fork, 0));
+        int rc = farm_grad_issue(f, s0, g_pdl);
+        if (rc) return rc;
+        CUDA_TRY(cudaEventRecord(fork, s0));
+        CUDA_TRY(cudaStreamWaitEvent(st, fork, 0));
+    } else {
+        CUDA_TRY(cudaGraphLaunch(g.exec, st));
+        g_launches += g.launches;
+    }
+    CUDA_TRY(cudaMemcpyAsync(results_dev, g.results, (size_t)f->nitems * sizeof(psoap_result), cudaMemcpyDeviceToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(grad_dev, g.grad, (size_t)f->nitems * np * 8, cudaMemcpyDeviceToDevice, st));
     return PSOAP_OK;
 }
 

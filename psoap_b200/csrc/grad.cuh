@@ -286,4 +286,17 @@ __global__ void orbit_jacobian_kernel(int model, const double* __restrict__ p, c
     orbit_jacobian_block(model, p, dates, n_epochs, jac);
 }
 
+// Farm gradient graph: block b writes work item b's orbit Jacobian [ncomp][n_epochs][norb] for the parameter vector at
+// p + p_off (the Jacobian counterpart of orbit_farm_kernel's OrbitDesc).
+struct JacDesc {
+    const double* dates;
+    double* jac;
+    int n_epochs;
+    int p_off;
+};
+__global__ void orbit_jacobian_farm_kernel(int model, const double* __restrict__ p, const JacDesc* __restrict__ descs) {
+    const JacDesc d = descs[blockIdx.x];
+    orbit_jacobian_block(model, p + d.p_off, d.dates, d.n_epochs, d.jac);
+}
+
 }  // namespace psoap

@@ -45,15 +45,26 @@ def chunk_cost(N):
     return n ** 3 + ALPHA2 * n * n + ALPHA1 * n
 
 
+# Default (proposal, chunk) pairs in flight in the gradient graph (capped by nbranch).  Measured on a B200 (1000 W), C4,
+# one proposal (tools/time_grad_farm.py): 16 / 32 / 64 branches 784 / 781 / 780 ms for 21.8 / 43.5 / 87.1 GB; the
+# branches beyond 16 buy nothing the SMs could use, so 16, at half the memory of 32.
+GRAD_NBRANCH = 16
+
+
 class ChunkFarm:
     """model: "SB1" | "SB2" | "ST1" | "ST2" | "ST3".
     chunks: list of dicts with lwl, fl, sigma (masked 1-D), mask [n_epochs, n_pix] (or `epoch` int32 [N]) and
     date1D — the attributes a reference Chunk exposes after apply_mask() (data.py:120-147).
     rank/world_size: static partition of the chunks over GPUs; process_group: torch.distributed group (or None).
+    grad_nbranch: (proposal, chunk) pairs in flight in the gradient graph of chunk_lnlike_grads_many (default
+    GRAD_NBRANCH, at most nbranch); each branch holds the identity-bordered matrix of the largest chunk, 8 (2 N)^2 bytes.
     """
 
     def __init__(self, model, chunks, mu_GP=1.0, soften=1.0, nbranch=32, rank=0, world_size=1, process_group=None,
-                 n_proposals=1):
+                 n_proposals=1, grad_nbranch=None):
+        self.grad_nbranch = int(grad_nbranch) if grad_nbranch is not None else min(nbranch, GRAD_NBRANCH)
+        if self.grad_nbranch < 1:
+            raise ValueError("grad_nbranch must be at least 1")
         lib = _lib.load()
         torch = _lib.torch_cuda()
         self.model = model
@@ -124,6 +135,7 @@ class ChunkFarm:
         self._descs = descs          # kept for the gradient entry, which takes one chunk at a time
         self._n_epochs = nes
         self._grad_ws = None         # allocated by the first lnprob_and_grad call
+        self._grad_farm_ws = None    # allocated, and the gradient graph attached, by the first *_many gradient call
         self._farm = _lib.vp(None)
         K = self.n_proposals
         self._results = torch.zeros((K, max(1, len(self.mine)), 4), dtype=torch.float64, device="cuda")
@@ -251,10 +263,59 @@ class ChunkFarm:
         (proposal, chunk) pair; returns the n_proposals summed log-likelihoods."""
         return np.atleast_1d(self.lnprob(P))
 
+    def _attach_grad_graph(self):
+        lib = _lib.load()
+        torch = _lib.torch_cuda()
+        nbytes = lib.psoap_farm_grad_workspace_bytes(self._farm, self.grad_nbranch)
+        try:
+            ws = torch.empty(nbytes + 256, dtype=torch.uint8, device="cuda")
+        except torch.cuda.OutOfMemoryError as e:
+            raise MemoryError("the gradient graph needs %d bytes of device memory for grad_nbranch = %d (one "
+                              "identity-bordered matrix of the largest chunk per branch); pass a smaller grad_nbranch"
+                              % (nbytes, self.grad_nbranch)) from e
+        _lib.check(lib.psoap_farm_grad_attach(self._farm, self.grad_nbranch, _lib.ptr(ws), nbytes))
+        self._grad_farm_ws = ws
+
+    def chunk_lnlike_grads_many(self, P):
+        """Per-(proposal, chunk) (lnlike, gradient) rows for the n_proposals registered vectors P ([n_proposals,
+        n_params]): device tensor [n_proposals, n_chunks, n_params + 1].  One launch of the farm's gradient graph
+        evaluates every (proposal, chunk) pair of this rank, grad_nbranch of them in flight; the rows go at their
+        global chunk index, the other rows are zero, and with world_size > 1 the tensor is all-reduced (exact: every
+        row has one contributor).  The first call allocates the graph's workspace and captures it; a farm that never
+        asks for it holds neither.  Gradient rows are NaN where lnlike is -inf."""
+        lib = _lib.load()
+        torch = _lib.torch_cuda()
+        P = np.asarray(P, dtype=np.float64)
+        K, npar = self.n_proposals, self.n_params
+        if P.size != K * npar:
+            raise ValueError("P must hold %d x %d registered parameters of %s" % (K, npar, self.model))
+        rows = torch.zeros((K, self.n_chunks, npar + 1), dtype=torch.float64, device="cuda")
+        if self.mine:
+            if self._grad_farm_ws is None:
+                self._attach_grad_graph()
+            p_dev = torch.from_numpy(np.ascontiguousarray(P.reshape(K, npar))).cuda()
+            res = torch.empty((K, len(self.mine), 4), dtype=torch.float64, device="cuda")
+            grad = torch.empty((K, len(self.mine), npar), dtype=torch.float64, device="cuda")
+            _lib.check(lib.psoap_farm_lnprob_grad(self._farm, _lib.ptr(p_dev), _lib.ptr(res), _lib.ptr(grad),
+                                                  _lib.stream_ptr()))
+            rows.index_copy_(1, self._mine_idx, torch.cat([res[:, :, :1], grad], dim=2))
+        if self.world_size > 1:
+            self._allreduce(rows)
+        return rows
+
+    def lnprob_and_grad_many(self, P):
+        """lnprob and its gradient for each of the n_proposals vectors P: (ndarray [n_proposals], ndarray
+        [n_proposals, n_params]).  Each proposal's rows are summed in chunk order on the host as lnprob_and_grad
+        sums them, so the bits do not depend on the number of GPUs."""
+        h = self.chunk_lnlike_grads_many(P).cpu().numpy()
+        lnp = np.array([float(np.sum(hk[:, 0])) for hk in h])
+        return lnp, np.stack([np.sum(hk[:, 1:], axis=0) for hk in h])
+
     def close(self):
         if self._farm:
             _lib.load().psoap_farm_destroy(self._farm)
             self._farm = _lib.vp(None)
+        self._grad_farm_ws = None
 
     def __del__(self):
         try:
