@@ -115,6 +115,10 @@ int psoap_lnlike(int ncomp, int64_t N, const double *lwl_f_dev, const double *lw
 int psoap_lnlike_host(int ncomp, int64_t N, const double *lwl_f, const double *lwl_g, const double *lwl_h,
                       const double *fl, const double *sigma, const double *amp, const double *l, double mu_GP,
                       psoap_result *result);
+/* The envelope the last psoap_lnlike call on this workspace computed on the device: *tend_dev points at int[T + 1]
+ * (T = padded(N) / 128 row blocks); tend[e], e >= 1, is the first row block from which every row of K is exactly zero
+ * in block columns [0, e).  The factorisation's launches for panels before e stop there. */
+int psoap_lnlike_envelope_view(void *workspace_dev, int64_t N, int **tend_dev, int *T);
 
 /* ---- prediction: psoap/covariance.py:81-297 (Schur complement of a bordered matrix) ------------------- */
 /* In place on a column-major device matrix S [n + m, ld]: the leading n x n block (lower triangle) is

@@ -57,6 +57,7 @@ SIGNATURES = {
                                          ctypes.POINTER(PsoapResult)]),
     "psoap_schur_workspace_bytes": (ctypes.c_size_t, [ctypes.c_int64, ctypes.c_int64]),
     "psoap_schur": (ctypes.c_int, [vp, ctypes.c_int64, ctypes.c_int64, ctypes.c_int64, vp, ctypes.c_size_t, vp, vp]),
+    "psoap_lnlike_envelope_view": (ctypes.c_int, [vp, ctypes.c_int64, ctypes.POINTER(vp), c_int_p]),
     "psoap_schur_views": (ctypes.c_int, [vp, ctypes.c_int64, ctypes.c_int64, ctypes.POINTER(vp), ctypes.POINTER(vp),
                                          ctypes.POINTER(vp)]),
     "psoap_lnlike_grad_workspace_bytes": (ctypes.c_size_t, [ctypes.c_int, ctypes.c_int64]),

@@ -151,7 +151,7 @@ int set_kernel_attributes() {
 }
 
 // Device scratch of one factorisation: W [Nt x Nt] (Nt = padded total dimension), two panel buffers,
-// L_kk^-1, residual, y, accumulators, info.
+// L_kk^-1, residual, y, accumulators, info, the fill's exact-zero tile flags and the envelope computed from them.
 constexpr int MAX_GROUP = 8;  // panels per trailing update (rank 128 * G)
 struct FactorWs {
     double* W;
@@ -162,6 +162,8 @@ struct FactorWs {
     double* y;
     double* acc;
     int* info;
+    uint8_t* nz;    // fill_lower_kernel: one byte per lower tile, T (T + 1) / 2 (T = Nt / 128)
+    int* tend;      // envelope_kernel: int[T + 1], tend[e] = first row block of the envelope of panels [0, e)
     int64_t Nt;
 };
 
@@ -174,6 +176,9 @@ size_t factor_ws_bytes(int64_t Nt) {
     b += 2 * align_up((size_t)Nt * 8, 256);
     b += align_up(8 * 8, 256);
     b += align_up(2 * 4, 256);
+    const int64_t T = Nt / NB;
+    b += align_up((size_t)(T * (T + 1) / 2), 256);
+    b += align_up((size_t)(T + 1) * 4, 256);
     return b;
 }
 
@@ -190,6 +195,9 @@ void carve_factor_ws(char* base, int64_t Nt, FactorWs* ws, bool with_W) {
     ws->y = (double*)take((size_t)Nt * 8);
     ws->acc = (double*)take(8 * 8);
     ws->info = (int*)take(2 * 4);
+    const int64_t T = Nt / NB;
+    ws->nz = (uint8_t*)take((size_t)(T * (T + 1) / 2));
+    ws->tend = (int*)take((size_t)(T + 1) * 4);
 }
 
 // Streams of one factorisation pipeline: the caller's stream plus a high-priority side stream on which the next
@@ -248,8 +256,19 @@ cudaError_t launch_k(void (*kernel)(KArgs...), unsigned grid, unsigned block, si
 // group's panels side by side.  The elimination drops from 7 N^3 / 3 to N^3 flops.  Tile shapes, the group size, the
 // chain and the yield mode are still chosen from T_total, and every tile runs the same k loop as without the
 // restriction: the trailing block and the residual are the same bits.
+//
+// envelope (T_elim == T_total only; may be null): envelope[e] (fill.cuh envelope_kernel, on the device) is the first row
+// block from which every row is exactly zero in block columns [0, e) of the filled matrix.  Cholesky keeps a row's
+// leading zeros (L_ij = 0 for j before the row's first non-zero in K), so in the group that ends at panel e those rows
+// have exact-zero panel-solve inputs, exact +0 panels, and every product they would take part in has a +-0 factor:
+// the update C - 0 leaves C as it is, except that the sign of a zero can differ inside entries that stay zero and are
+// never pivoted.  The kernels read the entry after pdl_wait() and stop their rows there (gemm.cuh row_limit); the grids,
+// the group boundaries and every other host-side choice stay those of the full launch, which bound them from above.
+// The likelihood is the same bits as the unrestricted factorisation in the same row order.  Rows sorted by wavelength
+// give a narrow envelope (squared-exponential entries underflow to +0 beyond about 38.6 length scales); in any other
+// order it is T_total everywhere and every launch runs in full.
 int launch_factor(const Lanes& ln, double* W, int64_t ld, int T_elim, int T_total, int pad, const FactorWs& ws,
-                  const int* sentinel, double* result, bool identity_border = false) {
+                  const int* sentinel, double* result, bool identity_border = false, const int* envelope = nullptr) {
     const int64_t ldp = ws.Nt;
     CUtensorMap mapW, mapLinv, mapPa[2], mapPb[2], mapPas[2], mapPbs[2];   // ..s: boxes of the small tile shape
     CUtensorMap mapWblk, mapWt, mapL7[3];                                   // chain 7: diagonal block, panel tile, L_kk below its sub-blocks
@@ -290,12 +309,14 @@ int launch_factor(const Lanes& ln, double* W, int64_t ld, int T_elim, int T_tota
     };
     // last row block (exclusive) of the launches of group q; set once the group boundaries are known
     std::vector<int> tend;
+    std::vector<int> gstart;
     auto trsm = [&](cudaStream_t s, int kb, int q, int col0) {
         const int R = tend[q] - kb - 1;
         if (chain == 7) {   // blocked substitution against L_kk and its 32 x 32 diagonal inverses (chain.cuh)
             Trsm7Args a;
             a.W = W; a.ld = ld; a.kb = kb; a.Lfac = ws.Linv; a.Xd = ws.Xd;
             a.P = pbuf(q) + (int64_t)col0 * ldp; a.ldp = ldp; a.ntiles = 4 * R;
+            a.tend = envelope; a.tend_at = gstart[q + 1];
             launch_k(trsm7_kernel, std::min(4 * R, g_num_sms), T7_THREADS, TRSM7_SMEM, s, ln.pdl, a, mapWt, mapL7[0], mapL7[1],
                      mapL7[2]);
             return;
@@ -303,6 +324,7 @@ int launch_factor(const Lanes& ln, double* W, int64_t ld, int T_elim, int T_tota
         TrsmSrc src;
         src.W = W; src.ld = ld; src.kb = kb; src.kbeg = (kb == 0) ? (pad / BK) * BK : 0;
         src.Linv = ws.Linv; src.P = pbuf(q) + (int64_t)col0 * ldp; src.ldp = ldp;
+        src.tend = envelope; src.tend_at = gstart[q + 1];
         launch_k(trsm3_kernel, persistent_ctas(2 * R), 256, GEMM_SMEM, s, ln.pdl, src, 2 * R, mapW, mapLinv);
     };
     // update of row tiles [row0, T_total) with k range [kbeg, kend) of group buffer q; the residual blocks (if
@@ -315,6 +337,7 @@ int launch_factor(const Lanes& ln, double* W, int64_t ld, int T_elim, int T_tota
         SyrkSrc src;
         src.W = W; src.ld = ld; src.row0 = sh * row0; src.res_row0 = row0; src.kbeg = kbeg_of(q); src.kend = kend;
         src.P = pbuf(q); src.ldp = ldp; src.part = part; src.ncol1 = sh * ncol1;
+        src.tend = envelope; src.tend_at = gstart[q + 1];
         const int ntiles = syrk_ntiles(sh * R, part, sh * ncol1);
         const int nres = (part == 2 || ykb < 0) ? 0 : R;
         if (ntiles + nres == 0) return;
@@ -347,7 +370,6 @@ int launch_factor(const Lanes& ln, double* W, int64_t ld, int T_elim, int T_tota
     // before the next diagonal block) make the shortest chain: 38 us per panel against 48.  Measured with 0 / 16 / 24 / 36
     // such rows: N = 4000 1.706 / 1.675 / 1.647 / 1.625 ms, N = 6000 3.514 / 3.491 / 3.442 / 3.526, N = 9000 9.31 / 9.29 / 9.25 / 9.33.
     constexpr int SINGLE_ROWS = 24;
-    std::vector<int> gstart;
     {
         const bool lone = ln.side != nullptr && chain == 7 && g_group == 0;
         for (int a = 0; a < T_elim;) {
@@ -405,7 +427,7 @@ template <int NCOMP>
 void launch_fill_lower_t(cudaStream_t st, double* W, int64_t ld, int T, int pad, const ZSource& zs,
                          const double* sigma, const double* fl, double mu, const GpParams& gp, const FactorWs& ws) {
     launch_k(fill_lower_kernel<NCOMP>, (unsigned)(T * (T + 1) / 2), 256, 0, st, 0, W, ld, pad, zs, sigma, fl, mu, gp, ws.rvec,
-             ws.acc, ws.info);
+             ws.acc, ws.info, ws.nz);
 }
 
 int launch_fill_lower(int ncomp, cudaStream_t st, double* W, int64_t ld, int T, int pad, const ZSource& zs,
@@ -425,7 +447,10 @@ int launch_chunk(const Lanes& ln, int ncomp, int64_t N, const ZSource& zs, const
     const int pad = (int)(Np - N);
     int rc = launch_fill_lower(ncomp, ln.main, ws.W, Np, T, pad, zs, sigma, fl, mu, gp, ws);
     if (rc) return rc;
-    return launch_factor(ln, ws.W, Np, T, T, pad, ws, sentinel, result);
+    if (T > ENV_MAX_T) return fail(PSOAP_ERR_ARG, "launch_chunk: matrix too large for the envelope");
+    launch_k(envelope_kernel, 1, 256, 0, ln.main, ln.pdl, (const uint8_t*)ws.nz, T, ws.tend);
+    LAUNCH_CHECK();
+    return launch_factor(ln, ws.W, Np, T, T, pad, ws, sentinel, result, false, ws.tend);
 }
 
 // Side stream + events for calls on a caller-provided stream (one set per host thread).
@@ -618,6 +643,15 @@ int psoap_lnlike(int ncomp, int64_t N, const double* lwl_f, const double* lwl_g,
     rc = get_lanes(st, &ln);
     if (rc) return rc;
     return launch_chunk(ln, ncomp, N, direct_z(lwl_f, lwl_g, lwl_h), fl, sigma, mu_GP, gp, ws, nullptr, (double*)result);
+}
+
+int psoap_lnlike_envelope_view(void* workspace, int64_t N, int** tend, int* T) {
+    if (!workspace || N < 1 || !tend || !T) return fail(PSOAP_ERR_ARG, "psoap_lnlike_envelope_view: bad arguments");
+    FactorWs ws;
+    carve_factor_ws((char*)workspace, padded_dim(N), &ws, true);
+    *tend = ws.tend;
+    *T = (int)(padded_dim(N) / NB);
+    return PSOAP_OK;
 }
 
 namespace {

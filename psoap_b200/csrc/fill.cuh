@@ -11,16 +11,23 @@ namespace psoap {
 //   One CTA per 128x128 tile with bi >= bj (1-D grid over the T (T+1) / 2 lower tiles); thread = 2 consecutive rows
 //   (double2 stores, 512 B per warp).  Diagonal tiles also initialise the residual r = fl - mu_GP (zero in the
 //   padding) and tile (0,0) resets the accumulators of the factorisation.
+//   nz (may be null): one byte per tile, in launch order, 1 when the tile as stored holds an entry != 0.0 (NaN included):
+//   the exact-zero pattern the factorisation's envelope is computed from (envelope_kernel).  Every lower tile is rewritten
+//   by every fill, so the flags need no reset.
 //   (Skipping the exponentials that are known to underflow to an exact +0 — a warp-uniform test of a 64-row strip's z
 //   range against the column — was measured SLOWER, 71 vs 64 us at N = 6000: with 2.8 km/s pixels and l = 5..7 km/s only
 //   a quarter of the strips qualify, and the test's branch keeps the unrolled evaluations from interleaving.)
 // ------------------------------------------------------------------------------------------------------
+__device__ __forceinline__ unsigned nonzero_bits(double v) {
+    return ((unsigned)__double2hiint(v) << 1) | (unsigned)__double2loint(v);
+}
 template <int NCOMP>
 __global__ void __launch_bounds__(256) fill_lower_kernel(double* __restrict__ W, int64_t ld, int pad, ZSource zs,
                                                          const double* __restrict__ sigma,
                                                          const double* __restrict__ fl, double mu_GP,
                                                          GpParams gp, double* __restrict__ rvec,
-                                                         double* __restrict__ acc, int* __restrict__ info) {
+                                                         double* __restrict__ acc, int* __restrict__ info,
+                                                         uint8_t* __restrict__ nz) {
     // lower-triangular tile index t -> (bi, bj), bi (bi + 1) / 2 + bj = t
     const int t = blockIdx.x;
     int bi = (int)((sqrtf(8.0f * (float)t + 1.0f) - 1.0f) * 0.5f);
@@ -61,6 +68,8 @@ __global__ void __launch_bounds__(256) fill_lower_kernel(double* __restrict__ W,
     }
     __syncthreads();
     const int cg = tid >> 6;
+    // OR over this thread's entries of their bits below the sign: non-zero unless every entry is +-0 (integer pipe)
+    unsigned bits = 0;
     // Interior tiles (strictly below the diagonal, clear of the identity padding) are 95 % of the tiles of a large
     // matrix: no per-entry case analysis there.
     if (bi != bj && (bj > 0 || pad == 0)) {
@@ -75,30 +84,68 @@ __global__ void __launch_bounds__(256) fill_lower_kernel(double* __restrict__ W,
                 for (int c = 1; c < NCOMP; ++c) cov = __dadd_rn(cov, se_term(amp2[c], p2[c], zi[c][e], zj[c][jl], etab));
                 v[e] = cov;
             }
+            bits |= nonzero_bits(v[0]) | nonzero_bits(v[1]);
             *reinterpret_cast<double2*>(W + pi0 + (int64_t)(bj * NB + jl) * ld) = make_double2(v[0], v[1]);
         }
-        return;
-    }
+    } else {
 #pragma unroll 4
-    for (int cc = 0; cc < 32; ++cc) {
-        const int jl = cc * 4 + cg;
-        const int pj = bj * NB + jl;
-        double v[2];
+        for (int cc = 0; cc < 32; ++cc) {
+            const int jl = cc * 4 + cg;
+            const int pj = bj * NB + jl;
+            double v[2];
 #pragma unroll
-        for (int e = 0; e < 2; ++e) {
-            const int pi = pi0 + e;
-            if (pi < pad || pj < pad) {
-                v[e] = (pi == pj) ? 1.0 : 0.0;
-            } else if (pi == pj) {
-                v[e] = dg[e];
-            } else {
-                double cov = se_term(amp2[0], p2[0], zi[0][e], zj[0][jl], etab);
+            for (int e = 0; e < 2; ++e) {
+                const int pi = pi0 + e;
+                if (pi < pad || pj < pad) {
+                    v[e] = (pi == pj) ? 1.0 : 0.0;
+                } else if (pi == pj) {
+                    v[e] = dg[e];
+                } else {
+                    double cov = se_term(amp2[0], p2[0], zi[0][e], zj[0][jl], etab);
 #pragma unroll
-                for (int c = 1; c < NCOMP; ++c) cov = __dadd_rn(cov, se_term(amp2[c], p2[c], zi[c][e], zj[c][jl], etab));
-                v[e] = cov;
+                    for (int c = 1; c < NCOMP; ++c) cov = __dadd_rn(cov, se_term(amp2[c], p2[c], zi[c][e], zj[c][jl], etab));
+                    v[e] = cov;
+                }
             }
+            bits |= nonzero_bits(v[0]) | nonzero_bits(v[1]);
+            *reinterpret_cast<double2*>(W + pi0 + (int64_t)pj * ld) = make_double2(v[0], v[1]);
         }
-        *reinterpret_cast<double2*>(W + pi0 + (int64_t)pj * ld) = make_double2(v[0], v[1]);
+    }
+    if (nz) {
+        const int any = __syncthreads_or(bits != 0u);
+        if (tid == 0) nz[t] = (uint8_t)any;
+    }
+}
+
+// ------------------------------------------------------------------------------------------------------
+// The envelope of a factorisation, from the fill's exact-zero tile flags (one CTA, right after the fill):
+//   f[I]   = first block column J <= I whose tile (I, J) holds a non-zero (I itself when none does)
+//   F[I]   = min_{I' >= I} f[I']                 (suffix minimum: row order is only nearly monotone in the shifted z)
+//   tend[e] = min{I >= e : F[I] >= e}, or T      (e = 1 .. T; tend[0] = T)
+// Row blocks I >= tend[e] are exactly zero in block columns < e, in K and so in L (Cholesky keeps a row's leading
+// zeros), so the launches of a panel group ending at panel e stop at row block tend[e] (api.cu launch_factor).
+// tend does not decrease with e.  Unsorted data has tend = T everywhere: every launch runs in full.
+// ------------------------------------------------------------------------------------------------------
+constexpr int ENV_MAX_T = 2048;   // shared-memory suffix minima: matrices up to 262144 rows
+__global__ void __launch_bounds__(256) envelope_kernel(const uint8_t* __restrict__ nz, int T, int* __restrict__ tend) {
+    __shared__ int F[ENV_MAX_T];
+    pdl_wait();
+    const int tid = threadIdx.x;
+    for (int I = tid; I < T; I += blockDim.x) {
+        const uint8_t* row = nz + (int64_t)I * (I + 1) / 2;
+        int J = 0;
+        while (J < I && !row[J]) ++J;
+        F[I] = J;
+    }
+    __syncthreads();
+    if (tid == 0)
+        for (int I = T - 2; I >= 0; --I) F[I] = min(F[I], F[I + 1]);
+    __syncthreads();
+    for (int e = tid; e <= T; e += blockDim.x) {
+        int I = e;
+        if (e > 0)
+            while (I < T && F[I] < e) ++I;
+        tend[e] = (e == 0) ? T : I;
     }
 }
 

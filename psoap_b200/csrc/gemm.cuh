@@ -87,6 +87,8 @@ struct TrsmSrc {
     const double* Linv;
     double* P;
     int64_t ldp;
+    const int* tend = nullptr;   // envelope (may be null): row blocks from tend[tend_at] on are skipped (see row_limit)
+    int tend_at = 0;
     template <int SH = 1>
     __device__ __forceinline__ TileDesc tile(int t) const {
         const int I = kb + 1 + (t >> 1), jh = t & 1;
@@ -121,6 +123,8 @@ struct SyrkSrc {
     const double* P;
     int64_t ldp;
     int part, ncol1;
+    const int* tend = nullptr;   // envelope (may be null): row blocks from tend[tend_at] on are skipped (see row_limit)
+    int tend_at = 0;
     static constexpr bool PREFETCH_C = true;   // the next tile's C lines are pulled towards L2 (gemm_persistent)
     // tile index -> (row r, 64-column tile jrel); host-callable so the CPU tests can check the coverage
     __host__ __device__ __forceinline__ void decode(int t, int& r, int& jrel) const {
@@ -196,6 +200,13 @@ __host__ __device__ inline int syrk_ntiles(int R, int part, int ncol1) {
     if (part == 0) return R * (R + 1);
     if (part == 1) return R <= h ? R * (R + 1) : h * (h + 1) + (R - h) * ncol1;
     return R > h ? (R - h) * (R - h + 1) : 0;
+}
+
+// Row blocks [row0, row0 + R) of a launch over R row blocks that lie inside the envelope: R, or fewer when the
+// envelope (written on the device after the fill, api.cu launch_chunk) says the rows from tend[tend_at] on are exactly
+// zero in every panel of the group.  Read after pdl_wait().  The grid and the host's launch plan stay sized for R.
+__device__ __forceinline__ int row_limit(const int* tend, int tend_at, int row0, int R) {
+    return tend ? max(0, min(R, tend[tend_at] - row0)) : R;
 }
 
 __device__ __forceinline__ double flip_sign(double x) {  // integer pipe, keeps the FP64 pipe for DMMA
@@ -365,6 +376,7 @@ trsm3_kernel(TrsmSrc src, int ntiles, const __grid_constant__ CUtensorMap mapW, 
     pdl_trigger();   // small grid: let the trailing update become resident behind it
     pdl_wait();
     TL_GO(6);
+    ntiles = 2 * row_limit(src.tend, src.tend_at, src.kb + 1, ntiles >> 1);
     gemm_persistent<0, 1>(src, ntiles, blockIdx.x, gridDim.x, sm, &mapW, &mapLinv);
     TL_OUT();
 }
@@ -400,16 +412,23 @@ syrk3_kernel(SyrkSrc src, int ntiles, int nctas, int nres, const double* __restr
     pdl_wait();
     TL_GO(SH == 1 ? (src.part == 1 ? 8 : 3) : 4);
     const int b = (int)blockIdx.x - nres;
+    // tiles of the rows inside the envelope: a prefix of the launch's tile order (every part enumerates row by row)
+    int ntot = 1 << 30;
+    if (src.tend) {
+        const int R = row_limit(src.tend, src.tend_at, src.res_row0, 1 << 30);
+        ntot = syrk_ntiles(SH * R, src.part, src.ncol1);
+        nres = min(nres, R);
+    }
     if (b < 0) {
-        syrk_residual_block(src, yk, rvec, res_col0, sm);
+        if ((int)blockIdx.x < nres) syrk_residual_block(src, yk, rvec, res_col0, sm);
     } else if (b < nctas) {
         // same buffer, two boxes: TI + 4 rows for the i operand, TJ + 4 rows for the j operand
-        gemm_persistent<1, SH>(src, ntiles, b, nctas, sm, &mapPa, &mapPb);
+        gemm_persistent<1, SH>(src, min(ntiles, ntot), b, nctas, sm, &mapPa, &mapPb);
     } else if constexpr (SH == 1) {
         SyrkTailSrc tail;
         tail.base = src; tail.first = ntiles;
         const int q = b - nctas;
-        gemm_persistent<1, 2>(tail, q + 1, q, 1 << 30, sm, &mapQa, &mapQb);
+        if (ntiles + (q >> 2) < ntot) gemm_persistent<1, 2>(tail, q + 1, q, 1 << 30, sm, &mapQa, &mapQb);
     }
     TL_OUT();
 }

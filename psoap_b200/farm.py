@@ -98,6 +98,12 @@ class ChunkFarm:
                                  % (idx, np.asarray(ch["mask"]).shape[0], len(host["dates"])))
             if N and (host["epoch"].min() < 0 or host["epoch"].max() >= len(host["dates"])):
                 raise ValueError("chunk %d: epoch indices must lie in [0, %d)" % (idx, len(host["dates"])))
+            # pixels in wavelength order, epochs interleaved: the covariance is then exactly zero outside a narrow
+            # envelope that the factorisation skips (DESIGN §9).  The likelihood and its parameter gradient do not
+            # depend on the pixel order; every farm path reads these buffers, so all of them see the same order.
+            order = np.argsort(host["lwl"], kind="stable")
+            for k2 in ("lwl", "fl", "sigma", "epoch"):
+                host[k2] = np.ascontiguousarray(host[k2][order])
             off = {}
             for k2, v in host.items():
                 off[k2] = total
