@@ -186,6 +186,24 @@ int psoap_chunk_lnprob_grad(int model, const psoap_chunk *chunk, const double *p
 int psoap_orbit_jacobian(int model, const double *p_orb_dev, const double *dates_dev, int n_epochs, double *jac_dev,
                          void *stream);
 
+/* ---- expected Fisher information of one chunk ---------------------------------------------------------- */
+/* psoap_chunk_lnprob_grad plus fisher_dev [n_params][n_params] (row-major, symmetric bit for bit, n_params =
+ * norb + 2 ncomp):  F_ab = 1/2 tr(K^-1 dK/dp_a K^-1 dK/dp_b) in the full registered parameter vector.  NaN everywhere
+ * when lnlike is -inf.  The gamma row and column are exactly zero (the covariance depends on velocity differences
+ * only).  result_dev and grad_p_dev receive exactly what psoap_chunk_lnprob_grad writes; grad_p_dev may be NULL.
+ * Bit-reproducible: no floating-point atomics.  workspace_dev: >= psoap_chunk_fisher_workspace_bytes(model, N,
+ * n_epochs) bytes, 256-byte aligned: the gradient's identity-bordered matrix plus one N x N product per parameter,
+ * about (4 + n_params) 8 N^2 bytes. */
+size_t psoap_chunk_fisher_workspace_bytes(int model, int64_t N, int32_t n_epochs);
+int psoap_chunk_fisher(int model, const psoap_chunk *chunk, const double *p_dev, double mu_GP, void *workspace_dev,
+                       size_t workspace_bytes, psoap_result *result_dev, double *grad_p_dev, double *fisher_dev,
+                       void *stream);
+/* Views into a Fisher workspace after psoap_chunk_fisher: *Tb = padded N / 128, the tile flags [Tb][Tb] (1 where an
+ * exponential factor of the covariance is non-zero in the 128 x 128 tile) and the k range [Tb][2] (first and last
+ * flagged row block of each block column) that the products run over. */
+int psoap_chunk_fisher_views(void *workspace_dev, int model, int64_t N, int32_t n_epochs, uint8_t **flags_dev,
+                             int **krange_dev, int *Tb);
+
 /* ---- chunk farm: psoap/sample_parallel.py:168-198, :371-390 ------------------------------------------ */
 typedef struct psoap_farm psoap_farm;
 size_t psoap_farm_workspace_bytes(int nchunks, const int64_t *N, const int32_t *n_epochs, int nbranch);

@@ -6,7 +6,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(CSRC, "libpsoap_b200.so")
 SOURCES = ["api.cu"]
-HEADERS = ["common.cuh", "fill.cuh", "chain.cuh", "chol.cuh", "gemm.cuh", "orbit.cuh", "predict.cuh", "grad.cuh", os.path.join("..", "..", "include", "psoap_b200.h")]
+HEADERS = ["common.cuh", "fill.cuh", "chain.cuh", "chol.cuh", "gemm.cuh", "orbit.cuh", "predict.cuh", "grad.cuh", "fisher.cuh", os.path.join("..", "..", "include", "psoap_b200.h")]
 NVCC_FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
               "-Xcompiler", "-fPIC", "-shared", "-Xptxas", "-v"]
 

@@ -68,6 +68,11 @@ SIGNATURES = {
     "psoap_chunk_lnprob_grad": (ctypes.c_int, [ctypes.c_int, ctypes.POINTER(PsoapChunk), vp, ctypes.c_double, vp,
                                                ctypes.c_size_t, vp, vp, vp]),
     "psoap_orbit_jacobian": (ctypes.c_int, [ctypes.c_int, vp, vp, ctypes.c_int, vp, vp]),
+    "psoap_chunk_fisher_workspace_bytes": (ctypes.c_size_t, [ctypes.c_int, ctypes.c_int64, ctypes.c_int32]),
+    "psoap_chunk_fisher": (ctypes.c_int, [ctypes.c_int, ctypes.POINTER(PsoapChunk), vp, ctypes.c_double, vp,
+                                          ctypes.c_size_t, vp, vp, vp, vp]),
+    "psoap_chunk_fisher_views": (ctypes.c_int, [vp, ctypes.c_int, ctypes.c_int64, ctypes.c_int32, ctypes.POINTER(vp),
+                                                ctypes.POINTER(vp), c_int_p]),
     "psoap_predict_workspace_bytes": (ctypes.c_size_t, [ctypes.c_int, ctypes.c_int, ctypes.c_int64, ctypes.c_int64]),
     "psoap_predict": (ctypes.c_int, [ctypes.c_int, ctypes.c_int, ctypes.c_int64, ctypes.c_int64, ctypes.POINTER(vp), vp,
                                      vp, ctypes.POINTER(vp), c_double_p, c_double_p, ctypes.c_double, ctypes.c_double,

@@ -18,6 +18,7 @@
 #include "chol.cuh"
 #include "common.cuh"
 #include "fill.cuh"
+#include "fisher.cuh"
 #include "gemm.cuh"
 #include "grad.cuh"
 #include "orbit.cuh"
@@ -108,6 +109,9 @@ int set_kernel_attributes() {
         if (e == cudaSuccess) e = cudaFuncSetAttribute(trsm3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM);
         if (e == cudaSuccess) e = cudaFuncSetAttribute(syrk3_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, SYRK1_SMEM);
         if (e == cudaSuccess) e = cudaFuncSetAttribute(syrk3_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, Shape<2>::SMEM);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(fisher_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM);
+        if (e == cudaSuccess)
+            e = cudaFuncSetAttribute(fisher_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, fisher_pair_smem(FISHER_MAXP));
         // every kernel of the chain asks for the same (maximal) shared-memory carve-out: CTAs of kernels with different
         // carve-outs do not share an SM, and the links are meant to run beside the trailing update's CTAs
         if (e == cudaSuccess) e = cudaFuncSetAttribute(potrf_diag3_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
@@ -502,7 +506,7 @@ ZSource direct_z(const double* f, const double* g, const double* h) {
 extern "C" {
 
 const char* psoap_last_error(void) { return g_err.c_str(); }
-int psoap_version(void) { return 102; }
+int psoap_version(void) { return 103; }
 int psoap_device_count(void) {
     int n = 0;
     if (cudaGetDeviceCount(&n) != cudaSuccess) { cudaGetLastError(); return 0; }
@@ -880,11 +884,57 @@ extern "C" size_t psoap_chunk_lnprob_grad_workspace_bytes(int model, int64_t N, 
     return carve_grad_ws(nullptr, model_ncomp(model), N, n_epochs, model_norb(model), &g);
 }
 
+namespace {
+// the chunk's pixels shifted by its epoch velocities (the farm's fused Doppler-shifted fill, farm_issue) and its GP
+// values on the device, as psoap_chunk_lnprob_grad and psoap_chunk_fisher see them
+ZSource chunk_zsource(const psoap_chunk* chunk, const GradWs& g) {
+    ZSource zs;
+    zs.lwl[0] = chunk->lwl; zs.lwl[1] = nullptr; zs.lwl[2] = nullptr;
+    zs.epoch = chunk->epoch; zs.vel = g.vel; zs.n_epochs = chunk->n_epochs; zs.shift = 1;
+    return zs;
+}
+GpParams chunk_gp(const double* p_dev, int norb) {
+    GpParams gp;
+    gp.dev = p_dev + norb;
+    for (int c = 0; c < 3; ++c) { gp.amp[c] = 0; gp.l[c] = 1; }
+    return gp;
+}
+
+// The launches of psoap_chunk_lnprob_grad on a carved workspace: orbit velocities and sentinel, fill, identity border,
+// restricted elimination, contraction, reductions, per-epoch sum, orbit Jacobian and chain rule.
+int launch_chunk_grad(int model, const psoap_chunk* chunk, const double* p_dev, double mu_GP, const GradWs& g,
+                      cudaStream_t st, double* result, double* grad_p) {
+    const int64_t N = chunk->N;
+    const int ne = chunk->n_epochs, ncomp = model_ncomp(model), norb = model_norb(model);
+    // orbit velocities and the sentinel (|v| >= c, or a negative GP hyper-parameter), as the farm's orbit kernel
+    orbit_kernel<<<1, 128, 0, st>>>(model, p_dev, chunk->dates, ne, g.vel, g.flag, 1);
+    LAUNCH_CHECK();
+    const ZSource zs = chunk_zsource(chunk, g);
+    const GpParams gp = chunk_gp(p_dev, norb);
+    Lanes ln;
+    int rc = get_lanes(st, &ln);
+    if (rc) return rc;
+    rc = launch_grad(ln, ncomp, N, zs, chunk->fl, chunk->sigma, mu_GP, gp, g, g.flag, result, g.hyp, g.gz);
+    if (rc) return rc;
+    grad_epoch_kernel<<<(unsigned)(ncomp * ne), 256, 0, st>>>(g.gz, chunk->epoch, N, ne, g.gv);
+    LAUNCH_CHECK();
+    orbit_jacobian_kernel<<<1, 128, 0, st>>>(model, p_dev, chunk->dates, ne, g.jac);
+    LAUNCH_CHECK();
+    grad_chain_kernel<<<1, 32, 0, st>>>(g.gv, g.jac, g.hyp, ncomp, ne, norb, g.f.info, g.flag, grad_p);
+    LAUNCH_CHECK();
+    return PSOAP_OK;
+}
+
+bool chunk_args_ok(int model, const psoap_chunk* chunk) {
+    return model >= 1 && model <= 5 && chunk && chunk->N >= 1 && chunk->N <= 200000 && chunk->n_epochs >= 1 &&
+           chunk->lwl && chunk->epoch && chunk->fl && chunk->sigma && chunk->dates;
+}
+}  // namespace
+
 extern "C" int psoap_chunk_lnprob_grad(int model, const psoap_chunk* chunk, const double* p_dev, double mu_GP,
                                        void* workspace, size_t workspace_bytes, psoap_result* result, double* grad_p,
                                        void* stream) {
-    if (model < 1 || model > 5 || !chunk || !p_dev || !result || !grad_p || chunk->N < 1 || chunk->N > 200000 ||
-        chunk->n_epochs < 1 || !chunk->lwl || !chunk->epoch || !chunk->fl || !chunk->sigma || !chunk->dates)
+    if (!chunk_args_ok(model, chunk) || !p_dev || !result || !grad_p)
         return fail(PSOAP_ERR_ARG, "psoap_chunk_lnprob_grad: bad arguments");
     const int64_t N = chunk->N;
     const int ne = chunk->n_epochs, ncomp = model_ncomp(model), norb = model_norb(model);
@@ -893,30 +943,120 @@ extern "C" int psoap_chunk_lnprob_grad(int model, const psoap_chunk* chunk, cons
         return fail(PSOAP_ERR_WORKSPACE, "psoap_chunk_lnprob_grad: workspace too small or not 256-byte aligned");
     int rc = set_kernel_attributes();
     if (rc) return rc;
-    cudaStream_t st = (cudaStream_t)stream;
     GradWs g;
     carve_grad_ws((char*)workspace, ncomp, N, ne, norb, &g);
-    // orbit velocities and the sentinel (|v| >= c, or a negative GP hyper-parameter), as the farm's orbit kernel
-    orbit_kernel<<<1, 128, 0, st>>>(model, p_dev, chunk->dates, ne, g.vel, g.flag, 1);
+    return launch_chunk_grad(model, chunk, p_dev, mu_GP, g, (cudaStream_t)stream, (double*)result, grad_p);
+}
+
+// ---- Fisher information of one chunk (fisher.cuh) ---------------------------------------------------------------
+namespace {
+// After the chunk's gradient workspace: the tile flags, the k ranges, the contraction partials, a gradient row for
+// callers that want none, and the P products A_a = K^-1 D_a (the only O(N^2) addition: P Nn^2 doubles).
+struct FisherWs {
+    uint8_t* flags;   // [Tb][Tb]
+    int* krange;      // [Tb][2]
+    double* part;     // [Tb (Tb + 1) / 2][P (P + 1) / 2]
+    double* grad_p;   // [P]
+    double* prod;     // [P][Nn][Nn]
+    int P, npairs;
+};
+size_t carve_fisher_ws(char* base, int model, int64_t N, int n_epochs, GradWs* g, FisherWs* f) {
+    const int ncomp = model_ncomp(model), norb = model_norb(model);
+    size_t off = carve_grad_ws(base, ncomp, N, n_epochs, norb, g);
+    auto take = [&](size_t bytes) { char* r = base ? base + off : nullptr; off += align_up(bytes, 256); return r; };
+    const int64_t Tb = g->Tb;
+    f->P = norb + 2 * ncomp;
+    f->npairs = (int)(Tb * (Tb + 1) / 2);
+    f->flags = (uint8_t*)take((size_t)(Tb * Tb));
+    f->krange = (int*)take((size_t)Tb * 2 * 4);
+    f->part = (double*)take((size_t)f->npairs * (f->P * (f->P + 1) / 2) * 8);
+    f->grad_p = (double*)take((size_t)f->P * 8);
+    f->prod = (double*)take((size_t)f->P * g->Nn * g->Nn * 8);
+    return off;
+}
+
+template <int NCOMP>
+void launch_dk(cudaStream_t st, const GradWs& g, int N, const ZSource& zs, const GpParams& gp, int norb, int a,
+               uint8_t* flags) {
+    fisher_dk_kernel<NCOMP><<<(unsigned)(g.Tb * g.Tb), 256, 0, st>>>(g.S, g.Nt, g.Tb, N, zs, gp, g.jac, norb, a, flags);
+}
+
+// the Fisher steps after launch_chunk_grad (fisher.cuh): mirror K^-1, then per parameter D_a and A_a = K^-1 D_a, then
+// the tile-pair contraction and the fixed-order reduction into fisher [P][P]
+int launch_fisher(int model, const psoap_chunk* chunk, const double* p_dev, const GradWs& g, const FisherWs& f,
+                  cudaStream_t st, double* fisher) {
+    const int N = (int)chunk->N, ncomp = model_ncomp(model), norb = model_norb(model), P = f.P;
+    const int64_t Nn = g.Nn;
+    double* kinv = g.S + Nn + Nn * g.Nt;
+    const int T32 = (int)(Nn / 32);
+    fisher_mirror_kernel<<<(unsigned)((int64_t)T32 * (T32 + 1) / 2), 256, 0, st>>>(kinv, g.Nt, N);
     LAUNCH_CHECK();
-    // the farm's fused Doppler-shifted fill (farm_issue): base vector + epoch + velocity table, GP values on the device
-    ZSource zs;
-    zs.lwl[0] = chunk->lwl; zs.lwl[1] = nullptr; zs.lwl[2] = nullptr;
-    zs.epoch = chunk->epoch; zs.vel = g.vel; zs.n_epochs = ne; zs.shift = 1;
-    GpParams gp;
-    gp.dev = p_dev + norb;
-    for (int c = 0; c < 3; ++c) { gp.amp[c] = 0; gp.l[c] = 1; }
-    Lanes ln;
-    rc = get_lanes(st, &ln);
+    CUtensorMap mapS, mapD;
+    int rc = make_tensor_map(&mapS, kinv, (uint64_t)Nn, (uint64_t)Nn, (uint64_t)g.Nt, SA);
+    if (!rc) rc = make_tensor_map(&mapD, g.S, (uint64_t)Nn, (uint64_t)Nn, (uint64_t)g.Nt, SB);
     if (rc) return rc;
-    rc = launch_grad(ln, ncomp, N, zs, chunk->fl, chunk->sigma, mu_GP, gp, g, g.flag, (double*)result, g.hyp, g.gz);
+    const ZSource zs = chunk_zsource(chunk, g);
+    const GpParams gp = chunk_gp(p_dev, norb);
+    const int ntiles = g.Tb * 2 * g.Tb;
+    for (int a = 0; a < P; ++a) {
+        uint8_t* flags = (a == 0) ? f.flags : nullptr;   // the zero pattern is the same for every parameter
+        if (ncomp == 1) launch_dk<1>(st, g, N, zs, gp, norb, a, flags);
+        else if (ncomp == 2) launch_dk<2>(st, g, N, zs, gp, norb, a, flags);
+        else launch_dk<3>(st, g, N, zs, gp, norb, a, flags);
+        LAUNCH_CHECK();
+        if (a == 0) {
+            fisher_krange_kernel<<<1, 256, 0, st>>>(f.flags, g.Tb, f.krange);
+            LAUNCH_CHECK();
+        }
+        FisherSrc src;
+        src.krange = f.krange; src.C = f.prod + (int64_t)a * Nn * Nn; src.ldc = Nn; src.Tb = g.Tb;
+        fisher_gemm_kernel<<<persistent_ctas(ntiles), 256, GEMM_SMEM, st>>>(src, ntiles, mapS, mapD);
+        LAUNCH_CHECK();
+    }
+    fisher_pair_kernel<<<(unsigned)f.npairs, 256, fisher_pair_smem(P), st>>>(f.prod, Nn * Nn, Nn, P, f.part);
+    LAUNCH_CHECK();
+    fisher_reduce_kernel<<<1, 256, 0, st>>>(f.part, f.npairs, P, g.f.info, g.flag, fisher);
+    LAUNCH_CHECK();
+    return PSOAP_OK;
+}
+}  // namespace
+
+extern "C" size_t psoap_chunk_fisher_workspace_bytes(int model, int64_t N, int32_t n_epochs) {
+    if (model < 1 || model > 5 || N < 1 || N > 200000 || n_epochs < 1) return 0;
+    GradWs g;
+    FisherWs f;
+    return carve_fisher_ws(nullptr, model, N, n_epochs, &g, &f);
+}
+
+extern "C" int psoap_chunk_fisher(int model, const psoap_chunk* chunk, const double* p_dev, double mu_GP,
+                                  void* workspace, size_t workspace_bytes, psoap_result* result, double* grad_p,
+                                  double* fisher, void* stream) {
+    if (!chunk_args_ok(model, chunk) || !p_dev || !result || !fisher)
+        return fail(PSOAP_ERR_ARG, "psoap_chunk_fisher: bad arguments");
+    if (!workspace || workspace_bytes < psoap_chunk_fisher_workspace_bytes(model, chunk->N, chunk->n_epochs) ||
+        ((uintptr_t)workspace & 255))
+        return fail(PSOAP_ERR_WORKSPACE, "psoap_chunk_fisher: workspace too small or not 256-byte aligned");
+    int rc = set_kernel_attributes();
     if (rc) return rc;
-    grad_epoch_kernel<<<(unsigned)(ncomp * ne), 256, 0, st>>>(g.gz, chunk->epoch, N, ne, g.gv);
-    LAUNCH_CHECK();
-    orbit_jacobian_kernel<<<1, 128, 0, st>>>(model, p_dev, chunk->dates, ne, g.jac);
-    LAUNCH_CHECK();
-    grad_chain_kernel<<<1, 32, 0, st>>>(g.gv, g.jac, g.hyp, ncomp, ne, norb, g.f.info, g.flag, grad_p);
-    LAUNCH_CHECK();
+    GradWs g;
+    FisherWs f;
+    carve_fisher_ws((char*)workspace, model, chunk->N, chunk->n_epochs, &g, &f);
+    const cudaStream_t st = (cudaStream_t)stream;
+    rc = launch_chunk_grad(model, chunk, p_dev, mu_GP, g, st, (double*)result, grad_p ? grad_p : f.grad_p);
+    if (rc) return rc;
+    return launch_fisher(model, chunk, p_dev, g, f, st, fisher);
+}
+
+extern "C" int psoap_chunk_fisher_views(void* workspace, int model, int64_t N, int32_t n_epochs, uint8_t** flags,
+                                        int** krange, int* Tb) {
+    if (!workspace || model < 1 || model > 5 || N < 1 || n_epochs < 1)
+        return fail(PSOAP_ERR_ARG, "psoap_chunk_fisher_views: bad arguments");
+    GradWs g;
+    FisherWs f;
+    carve_fisher_ws((char*)workspace, model, N, n_epochs, &g, &f);
+    if (flags) *flags = f.flags;
+    if (krange) *krange = f.krange;
+    if (Tb) *Tb = g.Tb;
     return PSOAP_OK;
 }
 

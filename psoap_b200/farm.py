@@ -264,6 +264,44 @@ class ChunkFarm:
         h = self.chunk_lnlike_grads(p).cpu().numpy()
         return float(np.sum(h[:, 0])), np.sum(h[:, 1:], axis=0)
 
+    def chunk_fishers(self, p):
+        """Per-chunk expected Fisher information F_ab = 1/2 tr(K^-1 dK/dp_a K^-1 dK/dp_b) at the full registered vector p
+        (orbital then GP): device tensor [n_chunks, n_params, n_params].  This rank's chunks go one at a time through
+        psoap_chunk_fisher (each chunk's n_params products fill the GPU), each written at its global chunk index; the
+        other entries are zero, and with world_size > 1 the tensor is all-reduced (exact: every entry has one
+        contributor).  The workspace, (4 + n_params) 8 N^2 bytes for the largest own chunk, is allocated for the call
+        and released after it.  A chunk's matrix is NaN where its lnlike is -inf."""
+        lib = _lib.load()
+        torch = _lib.torch_cuda()
+        p = np.asarray(p, dtype=np.float64)
+        if p.size != self.n_params:
+            raise ValueError("p must hold the %d registered parameters of %s" % (self.n_params, self.model))
+        npar = self.n_params
+        out = torch.zeros((self.n_chunks, npar, npar), dtype=torch.float64, device="cuda")
+        if self.mine:
+            model = _lib.MODELS[self.model]
+            nbytes = max(lib.psoap_chunk_fisher_workspace_bytes(model, N, ne) for N, ne in zip(self.Ns, self._n_epochs))
+            try:
+                ws = torch.empty(nbytes, dtype=torch.uint8, device="cuda")
+            except torch.cuda.OutOfMemoryError as e:
+                raise MemoryError("the Fisher information of the largest chunk needs %d bytes of device memory"
+                                  % nbytes) from e
+            p_dev = torch.from_numpy(p.reshape(-1).copy()).cuda()
+            res = torch.empty(4, dtype=torch.float64, device="cuda")
+            for k, idx in enumerate(self.mine):
+                _lib.check(lib.psoap_chunk_fisher(model, ctypes.byref(self._descs[k]), _lib.ptr(p_dev), self.mu_GP,
+                                                  _lib.ptr(ws), nbytes, _lib.ptr(res), None, _lib.ptr(out[idx]),
+                                                  _lib.stream_ptr()))
+        if self.world_size > 1:
+            self._allreduce(out)
+        return out
+
+    def fisher(self, p):
+        """Expected Fisher information of the farm's likelihood at p: ndarray [n_params, n_params], the per-chunk
+        matrices of chunk_fishers summed in chunk order on the host (as lnprob_and_grad sums), so the bits do not
+        depend on the number of GPUs.  Chunks are independent, so this is the Fisher information of the whole data."""
+        return np.sum(self.chunk_fishers(p).cpu().numpy(), axis=0)
+
     def lnprob_many(self, P):
         """Ensemble evaluation (SURVEY.md §8f-2): P is [n_proposals, n_params]; one graph launch evaluates every
         (proposal, chunk) pair; returns the n_proposals summed log-likelihoods."""

@@ -160,9 +160,31 @@ def make_lnprob(farm, model, fix_params, pars, prior=None, user_prior=None):
     return lnprob
 
 
+def fisher_jump(F, model, fix_params):
+    """Gaussian jump covariance for MHSampler from the expected Fisher information F [n_params, n_params] of the full
+    registered vector (ChunkFarm.fisher): 2.38^2/d * inv(F_fit), F_fit = F restricted to the d sampled parameters
+    (registry order, fix_params left out), the scaling utils.estimate_covariance gives a pilot chain's covariance.
+    Raises ValueError when F_fit has an exactly zero row (the likelihood does not depend on that parameter: gamma,
+    whose row is zero because the covariance depends on velocity differences only) or is not positive definite."""
+    names = [n for n in utils.registered_params[model] if n not in fix_params]
+    idx = [utils.registered_params[model].index(n) for n in names]
+    F = np.asarray(F, dtype=np.float64)
+    F_fit = F[np.ix_(idx, idx)]
+    zero = [n for n, row in zip(names, F_fit) if not np.any(row)]
+    if zero:
+        raise ValueError("the Fisher information has an exactly zero row for %s: the likelihood does not depend on %s; "
+                         "fix it (fix_params)" % (", ".join(zero), "it" if len(zero) == 1 else "them"))
+    try:
+        np.linalg.cholesky(F_fit)
+    except np.linalg.LinAlgError as e:
+        raise ValueError("the Fisher information of the sampled parameters %s is not positive definite" % names) from e
+    return 2.38 ** 2 / len(idx) * np.linalg.inv(F_fit)
+
+
 def run(config, chunks, run_index=0, seed=0, rank=0, world_size=1, process_group=None, verbose=True, workdir=None):
     """Run the chain described by a PSOAP config (a dict, or the path of a config.yaml; psoap/data/config.SB2.yaml
-    keys: model, parameters, jumps, fix_params, samples, opt_jump, outdir, soften).  A `prior.py` in `workdir`
+    keys: model, parameters, jumps, fix_params, samples, opt_jump, outdir, soften; `fisher_jump: true` takes the jump
+    covariance from fisher_jump(farm.fisher(p0), ...) instead of opt_jump / jumps).  A `prior.py` in `workdir`
     (default: the current directory, as in the reference) overrides the default prior.  Returns the sampler."""
     from .farm import ChunkFarm
     if isinstance(config, str):
@@ -180,10 +202,17 @@ def run(config, chunks, run_index=0, seed=0, rank=0, world_size=1, process_group
     if lnp0 == -np.inf:  # sample_parallel.py:406-422
         farm.close()
         raise RuntimeError("Starting position for Markov Chain evaluates to -np.inf")
-    try:
-        cov = np.load(config.get("opt_jump", ""))  # sample_parallel.py:427-432
-    except Exception:
-        cov = utils.convert_dict(model, fix, **config["jumps"]) ** 2 * np.eye(dim)
+    if config.get("fisher_jump"):  # the local shape of the posterior at p0, without a pilot chain
+        try:
+            cov = fisher_jump(farm.fisher(np.concatenate(utils.convert_vector(p0, model, fix, **pars))), model, fix)
+        except Exception:
+            farm.close()
+            raise
+    else:
+        try:
+            cov = np.load(config.get("opt_jump", ""))  # sample_parallel.py:427-432
+        except Exception:
+            cov = utils.convert_dict(model, fix, **config["jumps"]) ** 2 * np.eye(dim)
     sampler = MHSampler(cov, dim, lnprob, seed=seed)
     for i, _ in enumerate(sampler.sample(p0, lnprob0=lnp0, iterations=config["samples"])):
         if verbose and rank == 0 and (i + 1) % 20 == 0:
