@@ -223,7 +223,7 @@ size_t psoap_farm_workspace_bytes_batched(int nchunks, const int64_t *N, const i
 int psoap_farm_create_batched(psoap_farm **farm, int model, int nchunks, const psoap_chunk *chunks, int nprop,
                               int nbranch, double mu_GP, void *workspace_dev, size_t workspace_bytes);
 int psoap_farm_launches_per_eval(const psoap_farm *farm);
-/* Frees the farm's streams, events and graph, and its gradient graph when one is attached (not the workspaces). */
+/* Frees the farm's streams, events and graph, and its gradient and prediction graphs when attached (not the workspaces). */
 int psoap_farm_destroy(psoap_farm *farm);
 
 /* Gradient graph of a farm: every (proposal, chunk) pair through the steps of psoap_chunk_lnprob_grad, nbranch pairs in
@@ -244,6 +244,35 @@ int psoap_farm_grad_attach(psoap_farm *farm, int nbranch, void *workspace_dev, s
  * bit-identical from call to call. */
 int psoap_farm_lnprob_grad(psoap_farm *farm, const double *p_dev, psoap_result *results_dev, double *grad_dev,
                            void *stream);
+
+/* Prediction graph of a farm: the component spectra of every chunk at every proposal, psoap_predict mode 0
+ * (psoap/covariance.py:81-148 predict_f_g, :190-251 predict_f_g_h, as scripts/psoap_retrieve_SB2.py / _ST3.py call them)
+ * on the farm's resident pixels shifted by each proposal's velocities, nbranch (proposal, chunk) items in flight,
+ * captured into a third CUDA graph beside the likelihood's and the gradient's (both left as they are).  A farm that
+ * never attaches one allocates and captures nothing for it.
+ * m: [nchunks] grid points per component of each chunk (0: the chunk takes no work; a chunk without pixels must have 0).
+ * grids: [nchunks][ncomp] DEVICE pointers to each chunk's rest-frame ln-wavelength grid of each component, m[i] values
+ * each; captured into the graph, so they stay valid for the farm's life.  sigma_mode 0 writes Sigma, 1 only its diagonal.
+ * psoap_farm_predict_workspace_bytes: bytes the attach needs, 0 for bad arguments.  Each branch holds the bordered matrix
+ * of the largest item, 8 (padded(N) + padded(ncomp m))^2 bytes, plus its factorisation scratch; the graph's outputs are
+ * held as well.
+ * psoap_farm_predict_attach: captures the graph (once per farm).  workspace_dev >= the bytes above, 256-byte aligned,
+ * valid for the farm's life.  offsets_out: int64 [2][nitems + 1], item = proposal * nchunks + chunk: row 0 where each
+ * item's delta starts in delta_dev, row 1 where its Sigma (or diagonal) starts in sigma_dev, in doubles; entry nitems of
+ * each row is that buffer's length.  A chunk's items are contiguous, proposal after proposal.  Launch choices and
+ * look-ahead follow psoap_chunk.reserved as the gradient graph's do, so that with the reserved value set the outputs
+ * depend neither on nbranch nor on how the chunks are partitioned over ranks. */
+size_t psoap_farm_predict_workspace_bytes(const psoap_farm *farm, int nbranch, const int64_t *m, int sigma_mode);
+int psoap_farm_predict_attach(psoap_farm *farm, int nbranch, const int64_t *m, const double *const *grids_dev,
+                              int sigma_mode, void *workspace_dev, size_t workspace_bytes, int64_t *offsets_out);
+/* p_dev: [nprop][n_params] contiguous, as psoap_farm_lnprob.  Per item: delta = C K^-1 (fl - mu_GP), the components
+ * stacked [ncomp * m] (the caller adds the component means), Sigma row-major [ncomp m][ncomp m] or its diagonal, and
+ * the item's record in results_dev [nprop][nchunks] (lnlike, logdet, quad, info of the chunk's data block).  Every output
+ * of an item is NaN when its sentinel fired (|v| >= c, a negative GP value; lnlike -inf, info 0) or info != 0; other
+ * items are unaffected.  No floating-point atomics: the outputs are bit-identical from call to call.  PSOAP_ERR_ARG
+ * before psoap_farm_predict_attach. */
+int psoap_farm_predict(psoap_farm *farm, const double *p_dev, double *delta_dev, double *sigma_dev,
+                       psoap_result *results_dev, void *stream);
 
 /* ---- measurement helpers ----------------------------------------------------------------------------- */
 /* Register-resident DMMA.8x8x4 loop on all SMs: measured FP64 tensor-pipe peak in TFLOP/s (synchronous). */

@@ -95,6 +95,10 @@ SIGNATURES = {
     "psoap_farm_grad_workspace_bytes": (ctypes.c_size_t, [vp, ctypes.c_int]),
     "psoap_farm_grad_attach": (ctypes.c_int, [vp, ctypes.c_int, vp, ctypes.c_size_t]),
     "psoap_farm_lnprob_grad": (ctypes.c_int, [vp, vp, vp, vp, vp]),
+    "psoap_farm_predict_workspace_bytes": (ctypes.c_size_t, [vp, ctypes.c_int, c_i64_p, ctypes.c_int]),
+    "psoap_farm_predict_attach": (ctypes.c_int, [vp, ctypes.c_int, c_i64_p, ctypes.POINTER(vp), ctypes.c_int, vp,
+                                                 ctypes.c_size_t, c_i64_p]),
+    "psoap_farm_predict": (ctypes.c_int, [vp, vp, vp, vp, vp, vp]),
     "psoap_fp64_peak_tflops": (ctypes.c_int, [c_double_p]),
     "psoap_bench_syrk": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int, ctypes.c_int, c_double_p, c_double_p]),
     "psoap_bench_syrk_split": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int, ctypes.c_int, ctypes.c_int, c_double_p, c_double_p]),

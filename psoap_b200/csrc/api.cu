@@ -8,6 +8,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <mutex>
 #include <numeric>
 #include <string>
@@ -506,7 +507,7 @@ ZSource direct_z(const double* f, const double* g, const double* h) {
 extern "C" {
 
 const char* psoap_last_error(void) { return g_err.c_str(); }
-int psoap_version(void) { return 103; }
+int psoap_version(void) { return 104; }
 int psoap_device_count(void) {
     int n = 0;
     if (cudaGetDeviceCount(&n) != cudaSuccess) { cudaGetLastError(); return 0; }
@@ -1192,13 +1193,27 @@ extern "C" int psoap_predict_host(int ncomp, int mode, int64_t n, int64_t m, con
 // ======================================================================================================
 constexpr int P_STRIDE = 32;  // doubles reserved per proposal in the parameter buffer
 namespace {
+// One CUDA graph of a farm and what issues it: the branch streams (+ the root stream at index nbranch), their events,
+// the high-priority side streams of look-ahead, and whether calls replay the captured graph or issue the kernels
+// directly.  The likelihood graph, the gradient graph and the prediction graph each own one.
+struct FarmGraph {
+    int nbranch = 0;
+    bool lookahead = false;
+    bool direct = false;              // issue the kernels on every call instead of replaying the captured graph
+    cudaGraph_t graph = nullptr;
+    cudaGraphExec_t exec = nullptr;
+    std::vector<cudaStream_t> streams;
+    std::vector<cudaStream_t> side_streams;
+    std::vector<cudaEvent_t> events;
+    std::vector<cudaEvent_t> side_events;
+    int launches = 0;                 // kernels one evaluation launches
+};
+
 // The optional gradient graph of a farm (psoap_farm_grad_attach): its own parameter buffer, velocity tables,
 // sentinels, orbit Jacobians and outputs per (proposal, chunk) item, and one GradWs region per branch, carved for
 // each item in turn (items of a branch run in stream order).
 struct FarmGrad {
-    int nbranch = 0;
-    bool lookahead = false;
-    bool direct = false;
+    FarmGraph g;
     double* p_buf = nullptr;          // [nprop][P_STRIDE]
     double* results = nullptr;        // [nitems][4]
     double* grad = nullptr;           // [nitems][n_params]
@@ -1209,18 +1224,34 @@ struct FarmGrad {
     std::vector<double*> item_jac;    // [ncomp][n_epochs][norb] per item
     std::vector<char*> branch_base;   // GradWs region of each branch
     std::vector<std::vector<int>> branch_items;
-    cudaGraph_t graph = nullptr;
-    cudaGraphExec_t exec = nullptr;
-    std::vector<cudaStream_t> streams;
-    std::vector<cudaStream_t> side_streams;
-    std::vector<cudaEvent_t> events;
-    std::vector<cudaEvent_t> side_events;
-    int launches = 0;
+};
+
+// The optional prediction graph of a farm (psoap_farm_predict_attach): its own parameter buffer, velocity tables,
+// sentinels and result records per (proposal, chunk) item, the caller's grids, the output offsets of every item, and
+// one bordered-matrix region per branch (S of the largest item, then its FactorWs), carved for each item in turn.
+struct FarmPredict {
+    FarmGraph g;
+    int sigma_mode = 0;               // 0: Sigma [M][M], 1: its diagonal [M]
+    double* p_buf = nullptr;          // [nprop][P_STRIDE]
+    double* results = nullptr;        // [nitems][4]
+    int* flags = nullptr;             // per item sentinel
+    OrbitDesc* descs = nullptr;       // device, per item
+    std::vector<double*> item_vel;    // [ncomp][n_epochs] per item
+    std::vector<int64_t> m;           // grid points per component, per chunk
+    std::vector<const double*> grids; // [nchunks][ncomp] device pointers
+    std::vector<int64_t> delta_off;   // [nitems + 1] offsets (doubles) into delta_dev; the last one is its length
+    std::vector<int64_t> sigma_off;   // [nitems + 1] the same into sigma_dev
+    std::vector<char*> branch_base;
+    std::vector<std::vector<int>> branch_items;
+    double* delta = nullptr;          // the caller's buffers of the call being issued (direct issue)
+    double* sigma = nullptr;
+    double* cap_delta = nullptr;      // scratch outputs the captured graph writes; copied out after a replay
+    double* cap_sigma = nullptr;
 };
 }  // namespace
 
 struct psoap_farm {
-    int model = 0, ncomp = 0, norb = 0, nchunks = 0, nprop = 1, nitems = 0, nbranch = 0;
+    int model = 0, ncomp = 0, norb = 0, nchunks = 0, nprop = 1, nitems = 0;
     double mu = 1.0;
     std::vector<psoap_chunk> chunks;
     std::vector<FactorWs> branch_ws;
@@ -1231,23 +1262,16 @@ struct psoap_farm {
     int* flags = nullptr;             // per item sentinel
     OrbitDesc* descs = nullptr;       // device, per item
     std::vector<size_t> vel_off;
-    cudaGraph_t graph = nullptr;
-    cudaGraphExec_t exec = nullptr;
-    std::vector<cudaStream_t> streams;
-    std::vector<cudaStream_t> side_streams;
-    std::vector<cudaEvent_t> events;
-    std::vector<cudaEvent_t> side_events;
     std::vector<double*> item_vel;    // device velocity table of each item
-    bool lookahead = false;
-    bool direct = false;              // issue the kernels on every call instead of replaying the captured graph
+    FarmGraph g;                      // the likelihood graph
     int chain_hint = 0;               // psoap_chunk.reserved of the first chunk, low byte: 3 | 7 forces the chain links
     int group_hint = 0;               // ... bits 8 and up: 2 | 4 | 8 forces the panels per trailing update
-    int launches = 0;
     FarmGrad* grad = nullptr;         // psoap_farm_grad_attach; null until then
+    FarmPredict* pred = nullptr;      // psoap_farm_predict_attach; null until then
 };
 
 namespace {
-// The launch plan of one work item on branch b, shared by the likelihood graph and the gradient graph so that the two
+// The launch plan of one work item on branch b, shared by the likelihood, gradient and prediction graphs so that they
 // cannot drift apart.  `nbranch` and `lookahead` are the issuing graph's.
 Lanes farm_lanes(const psoap_farm* f, int nbranch, bool lookahead, cudaStream_t main, cudaStream_t side, cudaEvent_t e1,
                  cudaEvent_t e2, int pdl) {
@@ -1267,36 +1291,49 @@ Lanes farm_lanes(const psoap_farm* f, int nbranch, bool lookahead, cudaStream_t 
     ln.chain = (f->chain_hint == 3 || f->chain_hint == 7) ? f->chain_hint : (lookahead ? 0 : 3);
     return ln;
 }
+Lanes farm_lanes(const psoap_farm* f, const FarmGraph& g, int b, int pdl) {
+    return farm_lanes(f, g.nbranch, g.lookahead, g.streams[b], g.side_streams[b], g.side_events[2 * b],
+                      g.side_events[2 * b + 1], pdl);
+}
+
+// The GP values of proposal k and the chunk's pixels shifted by the item's velocity table, as every farm graph reads them
+GpParams farm_gp(const psoap_farm* f, const double* p_buf, int k) {
+    GpParams gp;
+    gp.dev = p_buf + (size_t)k * P_STRIDE + f->norb;
+    for (int c = 0; c < 3; ++c) { gp.amp[c] = 0; gp.l[c] = 1; }
+    return gp;
+}
+ZSource farm_z(const psoap_chunk& ch, const double* vel) {
+    ZSource zs;
+    zs.lwl[0] = ch.lwl; zs.lwl[1] = nullptr; zs.lwl[2] = nullptr;
+    zs.epoch = ch.epoch; zs.vel = vel; zs.n_epochs = ch.n_epochs; zs.shift = 1;
+    return zs;
+}
 
 // Issues one evaluation onto the farm's streams, rooted at s0: the orbit kernel for every item, then the per-chunk
 // pipelines on the branch streams, joined back into s0.  Runs under stream capture (graph mode) or for real
 // (direct mode, which adds programmatic dependent launch on the small grids).
 int farm_issue(psoap_farm* f, cudaStream_t s0, int pdl) {
-    const int nbranch = f->nbranch, nchunks = f->nchunks;
+    const int nbranch = f->g.nbranch, nchunks = f->nchunks;
     orbit_farm_kernel<<<f->nitems, 64, 0, s0>>>(f->model, f->p_buf, f->descs);
     ++g_launches;
-    cudaEventRecord(f->events[nbranch], s0);
+    cudaEventRecord(f->g.events[nbranch], s0);
     int rc = PSOAP_OK;
     for (int b = 0; b < nbranch && rc == PSOAP_OK; ++b) {
-        cudaStream_t sb = f->streams[b];
-        cudaStreamWaitEvent(sb, f->events[nbranch], 0);
+        cudaStream_t sb = f->g.streams[b];
+        cudaStreamWaitEvent(sb, f->g.events[nbranch], 0);
         for (int it : f->branch_items[b]) {
             const psoap_chunk& ch = f->chunks[it % nchunks];
-            GpParams gp;
-            gp.dev = f->p_buf + (size_t)(it / nchunks) * P_STRIDE + f->norb;
-            for (int c = 0; c < 3; ++c) { gp.amp[c] = 0; gp.l[c] = 1; }
-            ZSource zs;
-            zs.lwl[0] = ch.lwl; zs.lwl[1] = nullptr; zs.lwl[2] = nullptr;
-            zs.epoch = ch.epoch; zs.vel = f->item_vel[it]; zs.n_epochs = ch.n_epochs; zs.shift = 1;
+            const GpParams gp = farm_gp(f, f->p_buf, it / nchunks);
+            const ZSource zs = farm_z(ch, f->item_vel[it]);
             FactorWs ws = f->branch_ws[b];
             ws.Nt = padded_dim(ch.N);
-            const Lanes ln = farm_lanes(f, nbranch, f->lookahead, sb, f->side_streams[b], f->side_events[2 * b],
-                                        f->side_events[2 * b + 1], pdl);
-            rc = launch_chunk(ln, f->ncomp, ch.N, zs, ch.fl, ch.sigma, f->mu, gp, ws, f->flags + it, f->results + 4 * it);
+            rc = launch_chunk(farm_lanes(f, f->g, b, pdl), f->ncomp, ch.N, zs, ch.fl, ch.sigma, f->mu, gp, ws, f->flags + it,
+                              f->results + 4 * it);
             if (rc) break;
         }
-        cudaEventRecord(f->events[b], sb);
-        cudaStreamWaitEvent(s0, f->events[b], 0);
+        cudaEventRecord(f->g.events[b], sb);
+        cudaStreamWaitEvent(s0, f->g.events[b], 0);
     }
     return rc;
 }
@@ -1315,45 +1352,101 @@ int launch_grad_chain(cudaStream_t st, int ncomp, int norb, const psoap_chunk& c
 // item after item in LPT order, the steps of psoap_chunk_lnprob_grad into the item's result and gradient rows.
 int farm_grad_issue(psoap_farm* f, cudaStream_t s0, int pdl) {
     FarmGrad& g = *f->grad;
-    const int nbranch = g.nbranch, nchunks = f->nchunks, np = f->norb + 2 * f->ncomp;
+    const int nbranch = g.g.nbranch, nchunks = f->nchunks, np = f->norb + 2 * f->ncomp;
     orbit_farm_kernel<<<f->nitems, 64, 0, s0>>>(f->model, g.p_buf, g.descs);
     ++g_launches;
     orbit_jacobian_farm_kernel<<<f->nitems, 64, 0, s0>>>(f->model, g.p_buf, g.jdescs);
     ++g_launches;
-    cudaEventRecord(g.events[nbranch], s0);
+    cudaEventRecord(g.g.events[nbranch], s0);
     int rc = PSOAP_OK;
     for (int b = 0; b < nbranch && rc == PSOAP_OK; ++b) {
-        cudaStream_t sb = g.streams[b];
-        cudaStreamWaitEvent(sb, g.events[nbranch], 0);
+        cudaStream_t sb = g.g.streams[b];
+        cudaStreamWaitEvent(sb, g.g.events[nbranch], 0);
         for (int it : g.branch_items[b]) {
             const psoap_chunk& ch = f->chunks[it % nchunks];
-            GpParams gp;
-            gp.dev = g.p_buf + (size_t)(it / nchunks) * P_STRIDE + f->norb;
-            for (int c = 0; c < 3; ++c) { gp.amp[c] = 0; gp.l[c] = 1; }
-            ZSource zs;
-            zs.lwl[0] = ch.lwl; zs.lwl[1] = nullptr; zs.lwl[2] = nullptr;
-            zs.epoch = ch.epoch; zs.vel = g.item_vel[it]; zs.n_epochs = ch.n_epochs; zs.shift = 1;
+            const GpParams gp = farm_gp(f, g.p_buf, it / nchunks);
+            const ZSource zs = farm_z(ch, g.item_vel[it]);
             GradWs w;
             carve_grad_ws(g.branch_base[b], f->ncomp, ch.N, ch.n_epochs, f->norb, &w);
-            const Lanes ln = farm_lanes(f, nbranch, g.lookahead, sb, g.side_streams[b], g.side_events[2 * b],
-                                        g.side_events[2 * b + 1], pdl);
-            rc = launch_grad(ln, f->ncomp, ch.N, zs, ch.fl, ch.sigma, f->mu, gp, w, g.flags + it, g.results + 4 * it,
-                             w.hyp, w.gz);
+            rc = launch_grad(farm_lanes(f, g.g, b, pdl), f->ncomp, ch.N, zs, ch.fl, ch.sigma, f->mu, gp, w, g.flags + it,
+                             g.results + 4 * it, w.hyp, w.gz);
             if (!rc) rc = launch_grad_chain(sb, f->ncomp, f->norb, ch, w, g.item_jac[it], g.flags + it,
                                             g.grad + (size_t)it * np);
             if (rc) break;
         }
-        cudaEventRecord(g.events[b], sb);
-        cudaStreamWaitEvent(s0, g.events[b], 0);
+        cudaEventRecord(g.g.events[b], sb);
+        cudaStreamWaitEvent(s0, g.g.events[b], 0);
     }
     return rc;
 }
 
-// LPT (longest processing time first) assignment of work items (item = prop * nchunks + chunk) to branches by N^3
+// Bordered dimensions of one prediction item: data block Nn (front-padded), border M = ncomp m, total Nt.
+struct PredictDims { int64_t Nn, M, Nt; };
+PredictDims predict_item_dims(int ncomp, int64_t N, int64_t m) {
+    const int64_t Nn = padded_dim(N), M = ncomp * m;
+    return {Nn, M, Nn + padded_dim(M)};
+}
+
+template <int NCOMP>
+void launch_predict_border_farm(cudaStream_t st, double* S, int64_t ld, const PredictFarmSrc& ps, const GpParams& gp,
+                                double* rvec, unsigned ntile) {
+    predict_border_farm_kernel<NCOMP><<<ntile, 256, 0, st>>>(S, ld, ps, gp, rvec);
+}
+
+// The prediction counterpart of farm_issue: velocities and sentinels of every item, then per branch, item after item in
+// LPT order, the steps of psoap_predict (mode 0) on the item's shifted pixels: data fill, border fill, elimination of
+// the data block, read-out into the item's offsets of delta and sigma.
+int farm_predict_issue(psoap_farm* f, cudaStream_t s0, int pdl, double* delta, double* sigma) {
+    FarmPredict& q = *f->pred;
+    const int nbranch = q.g.nbranch, nchunks = f->nchunks, ncomp = f->ncomp;
+    orbit_farm_kernel<<<f->nitems, 64, 0, s0>>>(f->model, q.p_buf, q.descs);
+    ++g_launches;
+    cudaEventRecord(q.g.events[nbranch], s0);
+    int rc = PSOAP_OK;
+    for (int b = 0; b < nbranch && rc == PSOAP_OK; ++b) {
+        cudaStream_t sb = q.g.streams[b];
+        cudaStreamWaitEvent(sb, q.g.events[nbranch], 0);
+        for (int it : q.branch_items[b]) {
+            const int ci = it % nchunks;
+            const psoap_chunk& ch = f->chunks[ci];
+            const PredictDims d = predict_item_dims(ncomp, ch.N, q.m[ci]);
+            const int Tn = (int)(d.Nn / NB), Tt = (int)(d.Nt / NB), pad = (int)(d.Nn - ch.N);
+            FactorWs ws;
+            carve_factor_ws(q.branch_base[b], d.Nt, &ws, true);
+            const GpParams gp = farm_gp(f, q.p_buf, it / nchunks);
+            const ZSource zs = farm_z(ch, q.item_vel[it]);
+            rc = launch_fill_lower(ncomp, sb, ws.W, d.Nt, Tn, pad, zs, ch.sigma, ch.fl, f->mu, gp, ws);
+            if (rc) break;
+            PredictFarmSrc ps;
+            for (int c = 0; c < 3; ++c) { ps.data[c] = nullptr; ps.pred[c] = c < ncomp ? q.grids[(size_t)ci * ncomp + c] : nullptr; }
+            ps.ncomp = ncomp; ps.mode = 0; ps.n = (int)ch.N; ps.m = (int)q.m[ci]; ps.M = (int)d.M;
+            ps.pad = pad; ps.Nn = (int)d.Nn; ps.Nt = (int)d.Nt; ps.nugget = 0.0; ps.zs = zs;
+            const unsigned ntile = (unsigned)((int64_t)Tt * (Tt + 1) / 2 - (int64_t)Tn * (Tn + 1) / 2);
+            if (ncomp == 1) launch_predict_border_farm<1>(sb, ws.W, d.Nt, ps, gp, ws.rvec, ntile);
+            else if (ncomp == 2) launch_predict_border_farm<2>(sb, ws.W, d.Nt, ps, gp, ws.rvec, ntile);
+            else launch_predict_border_farm<3>(sb, ws.W, d.Nt, ps, gp, ws.rvec, ntile);
+            LAUNCH_CHECK();
+            rc = launch_factor(farm_lanes(f, q.g, b, pdl), ws.W, d.Nt, Tn, Tt, pad, ws, q.flags + it, q.results + 4 * it);
+            if (rc) break;
+            const unsigned nb = (unsigned)((d.M + 31) / 32);
+            predict_farm_readout_kernel<<<dim3(q.sigma_mode ? 1u : nb, nb), 256, 0, sb>>>(
+                ws.W, d.Nt, (int)d.Nn, (int)d.M, ws.rvec, ws.info, q.flags + it, q.sigma_mode, sigma + q.sigma_off[it],
+                delta + q.delta_off[it]);
+            LAUNCH_CHECK();
+        }
+        cudaEventRecord(q.g.events[b], sb);
+        cudaStreamWaitEvent(s0, q.g.events[b], 0);
+    }
+    return rc;
+}
+
+// LPT (longest processing time first) assignment of work items (item = prop * nchunks + chunk) to branches by N^3;
+// items of chunks with N = 0 are left out
 std::vector<std::vector<int>> lpt_items(const std::vector<int64_t>& Ns, int nitems, int nbranch) {
     const int nchunks = (int)Ns.size();
-    std::vector<int> order(nitems);
-    std::iota(order.begin(), order.end(), 0);
+    std::vector<int> order;
+    for (int it = 0; it < nitems; ++it)
+        if (Ns[it % nchunks] > 0) order.push_back(it);
     std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return Ns[a % nchunks] > Ns[b % nchunks]; });
     std::vector<double> load(nbranch, 0.0);
     std::vector<std::vector<int>> items(nbranch);
@@ -1367,11 +1460,10 @@ std::vector<std::vector<int>> lpt_items(const std::vector<int64_t>& Ns, int nite
 }
 
 // Branch streams (+ the root stream at index nbranch), their events, and the high-priority side streams of look-ahead
-void create_farm_streams(int nbranch, bool lookahead, std::vector<cudaStream_t>& streams,
-                         std::vector<cudaEvent_t>& events, std::vector<cudaStream_t>& side_streams,
-                         std::vector<cudaEvent_t>& side_events) {
-    streams.resize(nbranch + 1);
-    events.resize(nbranch + 1);
+void create_farm_streams(FarmGraph& g) {
+    const int nbranch = g.nbranch;
+    g.streams.resize(nbranch + 1);
+    g.events.resize(nbranch + 1);
     {
         // Branch b carries the b-th largest items first (LPT order): its stream gets the matching priority level, which a
         // captured kernel node inherits.  Measured neutral on a B200 against all-equal priorities (one rank's share of
@@ -1383,27 +1475,81 @@ void create_farm_streams(int nbranch, bool lookahead, std::vector<cudaStream_t>&
         for (int b = 0; b <= nbranch; ++b) {
             // (a look-ahead farm's branch streams carry the bulk updates: lowest priority, below their side streams, where
             // the chain links run; with both at the top C2 ran at 95.5 instead of 104 evals/s)
-            const int pr = (b < nbranch && nlev > 1 && !lookahead) ? hi + (int)((int64_t)b * nlev / nbranch) : lo;
-            cudaStreamCreateWithPriority(&streams[b], cudaStreamNonBlocking, pr);
+            const int pr = (b < nbranch && nlev > 1 && !g.lookahead) ? hi + (int)((int64_t)b * nlev / nbranch) : lo;
+            cudaStreamCreateWithPriority(&g.streams[b], cudaStreamNonBlocking, pr);
         }
     }
-    for (auto& ev : events) cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
-    side_streams.resize(nbranch);
-    side_events.resize(2 * nbranch);
+    for (auto& ev : g.events) cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
+    g.side_streams.resize(nbranch);
+    g.side_events.resize(2 * nbranch);
     {
         int lo = 0, hi = 0;
         cudaDeviceGetStreamPriorityRange(&lo, &hi);
-        for (auto& s : side_streams) cudaStreamCreateWithPriority(&s, cudaStreamNonBlocking, hi);
-        for (auto& ev : side_events) cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
+        for (auto& s : g.side_streams) cudaStreamCreateWithPriority(&s, cudaStreamNonBlocking, hi);
+        for (auto& ev : g.side_events) cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
     }
 }
 
-void destroy_farm_streams(std::vector<cudaStream_t>& streams, std::vector<cudaEvent_t>& events,
-                          std::vector<cudaStream_t>& side_streams, std::vector<cudaEvent_t>& side_events) {
-    for (auto& s : streams) if (s) cudaStreamDestroy(s);
-    for (auto& s : side_streams) if (s) cudaStreamDestroy(s);
-    for (auto& ev : events) if (ev) cudaEventDestroy(ev);
-    for (auto& ev : side_events) if (ev) cudaEventDestroy(ev);
+void destroy_farm_graph(FarmGraph& g) {
+    if (g.exec) cudaGraphExecDestroy(g.exec);
+    if (g.graph) cudaGraphDestroy(g.graph);
+    g.exec = nullptr; g.graph = nullptr;
+    for (auto& s : g.streams) if (s) cudaStreamDestroy(s);
+    for (auto& s : g.side_streams) if (s) cudaStreamDestroy(s);
+    for (auto& ev : g.events) if (ev) cudaEventDestroy(ev);
+    for (auto& ev : g.side_events) if (ev) cudaEventDestroy(ev);
+}
+
+using FarmIssue = std::function<int(cudaStream_t s0, int pdl)>;
+
+// Captures one evaluation, issued by `issue` onto g's streams, into g's graph and instantiates it.  The launches it
+// counts are g.launches (capture is not execution: the library's launch counter is left as it was).
+int capture_farm_graph(FarmGraph& g, const FarmIssue& issue) {
+    cudaStream_t s0 = g.streams[g.nbranch];
+    const int64_t before = g_launches.load();
+    cudaError_t e = cudaStreamBeginCapture(s0, cudaStreamCaptureModeThreadLocal);
+    if (e != cudaSuccess) return fail(PSOAP_ERR_CUDA, std::string("begin capture: ") + cudaGetErrorString(e));
+    int rc = issue(s0, 0);
+    e = cudaStreamEndCapture(s0, &g.graph);
+    g.launches = (int)(g_launches.load() - before);
+    g_launches = before;
+    if (rc != PSOAP_OK) return rc;
+    if (e != cudaSuccess) return fail(PSOAP_ERR_CUDA, std::string("end capture: ") + cudaGetErrorString(e));
+    e = cudaGraphInstantiate(&g.exec, g.graph, 0);
+    if (e != cudaSuccess) return fail(PSOAP_ERR_CUDA, std::string("graph instantiate: ") + cudaGetErrorString(e));
+    return PSOAP_OK;
+}
+
+// One evaluation on the caller's stream st: the captured graph's replay, or (direct mode) the kernels issued on g's
+// own streams, forked from st and joined back into it.
+int run_farm_graph(FarmGraph& g, cudaStream_t st, const FarmIssue& issue) {
+    if (g.direct) {
+        cudaStream_t s0 = g.streams[g.nbranch];
+        cudaEvent_t fork = g.events[g.nbranch];
+        CUDA_TRY(cudaEventRecord(fork, st));
+        CUDA_TRY(cudaStreamWaitEvent(s0, fork, 0));
+        int rc = issue(s0, g_pdl);
+        if (rc) return rc;
+        CUDA_TRY(cudaEventRecord(fork, s0));
+        CUDA_TRY(cudaStreamWaitEvent(st, fork, 0));
+    } else {
+        CUDA_TRY(cudaGraphLaunch(g.exec, st));
+        g_launches += g.launches;
+    }
+    return PSOAP_OK;
+}
+
+// Look-ahead and direct issue of a graph attached to a farm (gradient, prediction).  Look-ahead changes the panel
+// groups of the elimination, hence its bits.  When the caller passes the chain links (psoap_chunk.reserved, chosen from
+// the global problem: 7 for fewer than 8 (proposal, chunk) pairs in all), the attached graph takes look-ahead exactly
+// there, so that its outputs depend neither on the branch count nor on the number of GPUs; without that hint it decides
+// by branch count, as the likelihood graph does.
+void attached_graph_modes(const psoap_farm* f, FarmGraph& g, int64_t nmax) {
+    const char* la_env = getenv("PSOAP_FARM_LOOKAHEAD");
+    g.lookahead = la_env ? (atoi(la_env) != 0)
+                : (f->chain_hint == 3 || f->chain_hint == 7) ? (f->chain_hint == 7) : (g.nbranch < 8);
+    const char* de = getenv("PSOAP_FARM_DIRECT");
+    g.direct = de ? (atoi(de) != 0) : (g.lookahead && nmax >= 7000);
 }
 
 // Layout of a gradient workspace (base null: sizes only): the per-item buffers, then nbranch GradWs regions sized for
@@ -1444,10 +1590,57 @@ size_t carve_farm_grad(const psoap_farm* f, int nbranch, char* base, FarmGrad* g
 
 void destroy_farm_grad(FarmGrad* g) {
     if (!g) return;
-    if (g->exec) cudaGraphExecDestroy(g->exec);
-    if (g->graph) cudaGraphDestroy(g->graph);
-    destroy_farm_streams(g->streams, g->events, g->side_streams, g->side_events);
+    destroy_farm_graph(g->g);
     delete g;
+}
+
+// Layout of a prediction workspace (base null: sizes only): the per-item buffers, the graph's scratch outputs, then
+// nbranch regions of factor_ws_bytes(Nt) for the largest bordered item (S first, then its FactorWs).
+size_t carve_farm_predict(const psoap_farm* f, int nbranch, const int64_t* m, int sigma_mode, char* base, FarmPredict* q) {
+    const int nitems = f->nitems, nchunks = f->nchunks;
+    size_t off = 0;
+    auto take = [&](size_t bytes) { char* r = base ? base + off : nullptr; off += align_up(bytes, 256); return r; };
+    char* p_buf = take((size_t)f->nprop * P_STRIDE * 8);
+    char* results = take((size_t)nitems * 4 * 8);
+    char* flags = take((size_t)nitems * 4);
+    char* descs = take((size_t)nitems * sizeof(OrbitDesc));
+    // output layout: chunk after chunk, each chunk's proposals side by side, so that a chunk's outputs are contiguous
+    std::vector<int64_t> doff(nitems + 1), soff(nitems + 1);
+    int64_t nd = 0, ns = 0, ntmax = 0;
+    for (int ci = 0; ci < nchunks; ++ci) {
+        const PredictDims d = predict_item_dims(f->ncomp, f->chunks[ci].N, m[ci]);
+        if (m[ci] > 0) ntmax = std::max(ntmax, d.Nt);
+        for (int k = 0; k < f->nprop; ++k) {
+            const int it = k * nchunks + ci;
+            doff[it] = nd; soff[it] = ns;
+            nd += d.M; ns += sigma_mode ? d.M : d.M * d.M;
+        }
+    }
+    doff[nitems] = nd; soff[nitems] = ns;
+    char* cap_delta = take((size_t)nd * 8);
+    char* cap_sigma = take((size_t)ns * 8);
+    if (q) {
+        q->p_buf = (double*)p_buf; q->results = (double*)results; q->flags = (int*)flags; q->descs = (OrbitDesc*)descs;
+        q->cap_delta = (double*)cap_delta; q->cap_sigma = (double*)cap_sigma;
+        q->delta_off = doff; q->sigma_off = soff;
+        q->item_vel.resize(nitems); q->branch_base.resize(nbranch);
+    }
+    for (int it = 0; it < nitems; ++it) {
+        char* vel = take((size_t)f->ncomp * f->chunks[it % nchunks].n_epochs * 8);
+        if (q) q->item_vel[it] = (double*)vel;
+    }
+    const size_t per_branch = ntmax ? factor_ws_bytes(ntmax) : 0;
+    for (int b = 0; b < nbranch; ++b) {
+        char* r = take(per_branch);
+        if (q) q->branch_base[b] = r;
+    }
+    return off;
+}
+
+void destroy_farm_predict(FarmPredict* q) {
+    if (!q) return;
+    destroy_farm_graph(q->g);
+    delete q;
 }
 }  // namespace
 
@@ -1506,7 +1699,7 @@ int psoap_farm_create_batched(psoap_farm** out, int model, int nchunks, const ps
 
     psoap_farm* f = new psoap_farm();
     f->model = model; f->ncomp = model_ncomp(model); f->norb = model_norb(model);
-    f->nchunks = nchunks; f->nprop = nprop; f->nitems = nitems; f->nbranch = nbranch; f->mu = mu_GP;
+    f->nchunks = nchunks; f->nprop = nprop; f->nitems = nitems; f->g.nbranch = nbranch; f->mu = mu_GP;
     f->chunks.assign(chunks, chunks + nchunks);
     f->chain_hint = chunks[0].reserved & 0xff;
     f->group_hint = (chunks[0].reserved >> 8) & 0xff;
@@ -1540,32 +1733,20 @@ int psoap_farm_create_batched(psoap_farm** out, int model, int nchunks, const ps
     f->branch_items = lpt_items(Ns, nitems, nbranch);
 
     const char* la_env = getenv("PSOAP_FARM_LOOKAHEAD");
-    f->lookahead = la_env ? (atoi(la_env) != 0) : (nbranch < 8);
+    f->g.lookahead = la_env ? (atoi(la_env) != 0) : (nbranch < 8);
     // capture the whole evaluation into one CUDA graph
-    create_farm_streams(nbranch, f->lookahead, f->streams, f->events, f->side_streams, f->side_events);
-    cudaStream_t s0 = f->streams[nbranch];
-    const int64_t before = g_launches.load();
+    create_farm_streams(f->g);
     f->item_vel.resize(nitems);
     for (int it = 0; it < nitems; ++it) f->item_vel[it] = hd[it].vel;
     // Graph replay removes every launch gap, which wins for short chains (N = 4000: 2.57 vs 2.75 ms); for a farm of
     // a few LARGE chunks the directly issued pipeline is faster (N = 9000: 10.5 vs 11.3 ms: the side stream's
     // priority and the pre-staged small grids do their job there).  PSOAP_FARM_DIRECT=0|1 overrides.
     {
-        int64_t nmax = 0;
-        for (int i = 0; i < nchunks; ++i) nmax = std::max<int64_t>(nmax, chunks[i].N);
         const char* de = getenv("PSOAP_FARM_DIRECT");
-        f->direct = de ? (atoi(de) != 0) : (f->lookahead && nmax >= 7000);
+        f->g.direct = de ? (atoi(de) != 0) : (f->g.lookahead && nmax >= 7000);
     }
-    e = cudaStreamBeginCapture(s0, cudaStreamCaptureModeThreadLocal);
-    if (e != cudaSuccess) { psoap_farm_destroy(f); return fail(PSOAP_ERR_CUDA, std::string("begin capture: ") + cudaGetErrorString(e)); }
-    rc = farm_issue(f, s0, 0);
-    e = cudaStreamEndCapture(s0, &f->graph);
-    f->launches = (int)(g_launches.load() - before);
-    g_launches = before;  // capture is not execution
+    rc = capture_farm_graph(f->g, [f](cudaStream_t s0, int pdl) { return farm_issue(f, s0, pdl); });
     if (rc != PSOAP_OK) { psoap_farm_destroy(f); return rc; }
-    if (e != cudaSuccess) { psoap_farm_destroy(f); return fail(PSOAP_ERR_CUDA, std::string("end capture: ") + cudaGetErrorString(e)); }
-    e = cudaGraphInstantiate(&f->exec, f->graph, 0);
-    if (e != cudaSuccess) { psoap_farm_destroy(f); return fail(PSOAP_ERR_CUDA, std::string("graph instantiate: ") + cudaGetErrorString(e)); }
     *out = f;
     return PSOAP_OK;
 }
@@ -1582,32 +1763,19 @@ int psoap_farm_lnprob(psoap_farm* f, const double* p_dev, psoap_result* results_
     // p_dev: [nprop][np] contiguous -> [nprop][P_STRIDE]
     CUDA_TRY(cudaMemcpy2DAsync(f->p_buf, P_STRIDE * 8, p_dev, (size_t)np * 8, (size_t)np * 8, f->nprop,
                                cudaMemcpyDeviceToDevice, st));
-    if (f->direct) {
-        // the pipelines run on the farm's own streams: fork from the caller's stream and join back into it
-        cudaStream_t s0 = f->streams[f->nbranch];
-        cudaEvent_t fork = f->events[f->nbranch];
-        CUDA_TRY(cudaEventRecord(fork, st));
-        CUDA_TRY(cudaStreamWaitEvent(s0, fork, 0));
-        int rc = farm_issue(f, s0, g_pdl);
-        if (rc) return rc;
-        CUDA_TRY(cudaEventRecord(fork, s0));
-        CUDA_TRY(cudaStreamWaitEvent(st, fork, 0));
-    } else {
-        CUDA_TRY(cudaGraphLaunch(f->exec, st));
-        g_launches += f->launches;
-    }
+    int rc = run_farm_graph(f->g, st, [f](cudaStream_t s0, int pdl) { return farm_issue(f, s0, pdl); });
+    if (rc) return rc;
     CUDA_TRY(cudaMemcpyAsync(results_dev, f->results, (size_t)f->nitems * sizeof(psoap_result), cudaMemcpyDeviceToDevice, st));
     return PSOAP_OK;
 }
 
-int psoap_farm_launches_per_eval(const psoap_farm* f) { return f ? f->launches : 0; }
+int psoap_farm_launches_per_eval(const psoap_farm* f) { return f ? f->g.launches : 0; }
 
 int psoap_farm_destroy(psoap_farm* f) {
     if (!f) return PSOAP_OK;
-    if (f->exec) cudaGraphExecDestroy(f->exec);
-    if (f->graph) cudaGraphDestroy(f->graph);
-    destroy_farm_streams(f->streams, f->events, f->side_streams, f->side_events);
+    destroy_farm_graph(f->g);
     destroy_farm_grad(f->grad);
+    destroy_farm_predict(f->pred);
     delete f;
     return PSOAP_OK;
 }
@@ -1627,7 +1795,7 @@ int psoap_farm_grad_attach(psoap_farm* f, int nbranch, void* workspace, size_t w
     int rc = set_kernel_attributes();
     if (rc) return rc;
     FarmGrad* g = new FarmGrad();
-    g->nbranch = nbranch;
+    g->g.nbranch = nbranch;
     carve_farm_grad(f, nbranch, (char*)workspace, g);
     const int nitems = f->nitems, nchunks = f->nchunks;
     std::vector<OrbitDesc> hd(nitems);
@@ -1646,33 +1814,10 @@ int psoap_farm_grad_attach(psoap_farm* f, int nbranch, void* workspace, size_t w
     if (e == cudaSuccess) e = cudaMemcpy(g->jdescs, hj.data(), (size_t)nitems * sizeof(JacDesc), cudaMemcpyHostToDevice);
     if (e != cudaSuccess) { delete g; return fail(PSOAP_ERR_CUDA, std::string("farm grad descs: ") + cudaGetErrorString(e)); }
     g->branch_items = lpt_items(Ns, nitems, nbranch);
-    // Look-ahead changes the panel groups of the elimination, hence its bits.  When the caller passes the chain links
-    // (psoap_chunk.reserved, chosen from the global problem: 7 for fewer than 8 (proposal, chunk) pairs in all), the
-    // gradient graph takes look-ahead exactly there, so that its rows depend neither on the branch count nor on the
-    // number of GPUs; without that hint it decides by branch count, as the likelihood graph does.
-    const char* la_env = getenv("PSOAP_FARM_LOOKAHEAD");
-    g->lookahead = la_env ? (atoi(la_env) != 0)
-                 : (f->chain_hint == 3 || f->chain_hint == 7) ? (f->chain_hint == 7) : (nbranch < 8);
-    const char* de = getenv("PSOAP_FARM_DIRECT");
-    g->direct = de ? (atoi(de) != 0) : (g->lookahead && nmax >= 7000);
-    create_farm_streams(nbranch, g->lookahead, g->streams, g->events, g->side_streams, g->side_events);
+    attached_graph_modes(f, g->g, nmax);
+    create_farm_streams(g->g);
     f->grad = g;
-    cudaStream_t s0 = g->streams[nbranch];
-    const int64_t before = g_launches.load();
-    e = cudaStreamBeginCapture(s0, cudaStreamCaptureModeThreadLocal);
-    if (e != cudaSuccess) {
-        destroy_farm_grad(g); f->grad = nullptr;
-        return fail(PSOAP_ERR_CUDA, std::string("begin capture: ") + cudaGetErrorString(e));
-    }
-    rc = farm_grad_issue(f, s0, 0);
-    e = cudaStreamEndCapture(s0, &g->graph);
-    g->launches = (int)(g_launches.load() - before);
-    g_launches = before;  // capture is not execution
-    if (rc == PSOAP_OK && e != cudaSuccess) rc = fail(PSOAP_ERR_CUDA, std::string("end capture: ") + cudaGetErrorString(e));
-    if (rc == PSOAP_OK) {
-        e = cudaGraphInstantiate(&g->exec, g->graph, 0);
-        if (e != cudaSuccess) rc = fail(PSOAP_ERR_CUDA, std::string("graph instantiate: ") + cudaGetErrorString(e));
-    }
+    rc = capture_farm_graph(g->g, [f](cudaStream_t s0, int pdl) { return farm_grad_issue(f, s0, pdl); });
     if (rc != PSOAP_OK) { destroy_farm_grad(g); f->grad = nullptr; }
     return rc;
 }
@@ -1686,21 +1831,100 @@ int psoap_farm_lnprob_grad(psoap_farm* f, const double* p_dev, psoap_result* res
     const int np = f->norb + 2 * f->ncomp;
     CUDA_TRY(cudaMemcpy2DAsync(g.p_buf, P_STRIDE * 8, p_dev, (size_t)np * 8, (size_t)np * 8, f->nprop,
                                cudaMemcpyDeviceToDevice, st));
-    if (g.direct) {
-        cudaStream_t s0 = g.streams[g.nbranch];
-        cudaEvent_t fork = g.events[g.nbranch];
-        CUDA_TRY(cudaEventRecord(fork, st));
-        CUDA_TRY(cudaStreamWaitEvent(s0, fork, 0));
-        int rc = farm_grad_issue(f, s0, g_pdl);
-        if (rc) return rc;
-        CUDA_TRY(cudaEventRecord(fork, s0));
-        CUDA_TRY(cudaStreamWaitEvent(st, fork, 0));
-    } else {
-        CUDA_TRY(cudaGraphLaunch(g.exec, st));
-        g_launches += g.launches;
-    }
+    int rc = run_farm_graph(g.g, st, [f](cudaStream_t s0, int pdl) { return farm_grad_issue(f, s0, pdl); });
+    if (rc) return rc;
     CUDA_TRY(cudaMemcpyAsync(results_dev, g.results, (size_t)f->nitems * sizeof(psoap_result), cudaMemcpyDeviceToDevice, st));
     CUDA_TRY(cudaMemcpyAsync(grad_dev, g.grad, (size_t)f->nitems * np * 8, cudaMemcpyDeviceToDevice, st));
+    return PSOAP_OK;
+}
+
+// ---- prediction graph of a farm ---------------------------------------------------------------------------------
+namespace {
+// the checks both prediction entries make on their arguments, on the host only
+bool predict_args_ok(const psoap_farm* f, int nbranch, const int64_t* m, int sigma_mode) {
+    if (!f || nbranch < 1 || !m || (sigma_mode != 0 && sigma_mode != 1)) return false;
+    for (int i = 0; i < f->nchunks; ++i)
+        if (m[i] < 0 || m[i] > 200000 || (f->chunks[i].N < 1 && m[i] != 0)) return false;
+    return true;
+}
+}  // namespace
+
+size_t psoap_farm_predict_workspace_bytes(const psoap_farm* f, int nbranch, const int64_t* m, int sigma_mode) {
+    if (!predict_args_ok(f, nbranch, m, sigma_mode)) return 0;
+    return carve_farm_predict(f, std::min(nbranch, f->nitems), m, sigma_mode, nullptr, nullptr);
+}
+
+int psoap_farm_predict_attach(psoap_farm* f, int nbranch, const int64_t* m, const double* const* grids, int sigma_mode,
+                              void* workspace, size_t workspace_bytes, int64_t* offsets_out) {
+    if (!predict_args_ok(f, nbranch, m, sigma_mode) || !grids || !workspace || !offsets_out)
+        return fail(PSOAP_ERR_ARG, "psoap_farm_predict_attach: bad arguments");
+    for (int i = 0; i < f->nchunks; ++i)
+        for (int c = 0; c < f->ncomp; ++c)
+            if (m[i] > 0 && !grids[(size_t)i * f->ncomp + c])
+                return fail(PSOAP_ERR_ARG, "psoap_farm_predict_attach: null grid of chunk " + std::to_string(i));
+    if (f->pred) return fail(PSOAP_ERR_ARG, "psoap_farm_predict_attach: the farm already has a prediction graph");
+    nbranch = std::min(nbranch, f->nitems);
+    if (((uintptr_t)workspace & 255) || workspace_bytes < psoap_farm_predict_workspace_bytes(f, nbranch, m, sigma_mode))
+        return fail(PSOAP_ERR_WORKSPACE, "psoap_farm_predict_attach: workspace too small or not 256-byte aligned");
+    int rc = set_kernel_attributes();
+    if (rc) return rc;
+    FarmPredict* q = new FarmPredict();
+    q->g.nbranch = nbranch;
+    q->sigma_mode = sigma_mode;
+    const int nitems = f->nitems, nchunks = f->nchunks;
+    q->m.assign(m, m + nchunks);
+    q->grids.assign(grids, grids + (size_t)nchunks * f->ncomp);
+    carve_farm_predict(f, nbranch, m, sigma_mode, (char*)workspace, q);
+    std::vector<OrbitDesc> hd(nitems);
+    // the LPT weight of an item is its bordered dimension Nt (cubed by lpt_items); items of chunks with m = 0 take no work
+    std::vector<int64_t> cost(nchunks);
+    int64_t nmax = 0;
+    for (int i = 0; i < nchunks; ++i) {
+        cost[i] = m[i] > 0 ? predict_item_dims(f->ncomp, f->chunks[i].N, m[i]).Nt : 0;
+        if (m[i] > 0) nmax = std::max(nmax, (int64_t)f->chunks[i].N);
+    }
+    for (int it = 0; it < nitems; ++it) {
+        const psoap_chunk& ch = f->chunks[it % nchunks];
+        hd[it].dates = ch.dates; hd[it].vel = q->item_vel[it]; hd[it].flag = q->flags + it;
+        hd[it].n_epochs = ch.n_epochs; hd[it].p_off = (it / nchunks) * P_STRIDE;
+    }
+    cudaError_t e = cudaMemcpy(q->descs, hd.data(), (size_t)nitems * sizeof(OrbitDesc), cudaMemcpyHostToDevice);
+    // the records of items with m = 0 are never written by the graph: they read 0 (lnlike, logdet, quad, info)
+    if (e == cudaSuccess) e = cudaMemset(q->results, 0, (size_t)nitems * 4 * 8);
+    if (e != cudaSuccess) { delete q; return fail(PSOAP_ERR_CUDA, std::string("farm predict descs: ") + cudaGetErrorString(e)); }
+    q->branch_items = lpt_items(cost, nitems, nbranch);
+    attached_graph_modes(f, q->g, nmax);
+    create_farm_streams(q->g);
+    f->pred = q;
+    rc = capture_farm_graph(q->g, [f, q](cudaStream_t s0, int pdl) {
+        return farm_predict_issue(f, s0, pdl, q->cap_delta, q->cap_sigma);
+    });
+    if (rc != PSOAP_OK) { destroy_farm_predict(q); f->pred = nullptr; return rc; }
+    std::copy(q->delta_off.begin(), q->delta_off.end(), offsets_out);
+    std::copy(q->sigma_off.begin(), q->sigma_off.end(), offsets_out + nitems + 1);
+    return PSOAP_OK;
+}
+
+int psoap_farm_predict(psoap_farm* f, const double* p_dev, double* delta_dev, double* sigma_dev,
+                       psoap_result* results_dev, void* stream) {
+    if (!f || !p_dev || !delta_dev || !sigma_dev || !results_dev)
+        return fail(PSOAP_ERR_ARG, "psoap_farm_predict: bad arguments");
+    if (!f->pred) return fail(PSOAP_ERR_ARG, "psoap_farm_predict: no prediction graph (psoap_farm_predict_attach first)");
+    FarmPredict& q = *f->pred;
+    cudaStream_t st = (cudaStream_t)stream;
+    const int np = f->norb + 2 * f->ncomp;
+    CUDA_TRY(cudaMemcpy2DAsync(q.p_buf, P_STRIDE * 8, p_dev, (size_t)np * 8, (size_t)np * 8, f->nprop,
+                               cudaMemcpyDeviceToDevice, st));
+    // direct issue writes into the caller's buffers; the captured graph into its own, copied out after the replay
+    int rc = run_farm_graph(q.g, st, [f, delta_dev, sigma_dev](cudaStream_t s0, int pdl) {
+        return farm_predict_issue(f, s0, pdl, delta_dev, sigma_dev);
+    });
+    if (rc) return rc;
+    if (!q.g.direct) {
+        CUDA_TRY(cudaMemcpyAsync(delta_dev, q.cap_delta, (size_t)q.delta_off[f->nitems] * 8, cudaMemcpyDeviceToDevice, st));
+        CUDA_TRY(cudaMemcpyAsync(sigma_dev, q.cap_sigma, (size_t)q.sigma_off[f->nitems] * 8, cudaMemcpyDeviceToDevice, st));
+    }
+    CUDA_TRY(cudaMemcpyAsync(results_dev, q.results, (size_t)f->nitems * sizeof(psoap_result), cudaMemcpyDeviceToDevice, st));
     return PSOAP_OK;
 }
 

@@ -4,6 +4,8 @@
 // leading block is eliminated with the likelihood's kernels, and what is left in the trailing block is
 // Sigma = A - C K^-1 C^T while the carried residual holds -C K^-1 (fl - mu).
 #pragma once
+#include <math_constants.h>
+
 #include "common.cuh"
 
 namespace psoap {
@@ -21,22 +23,30 @@ struct PredictSrc {
     int n, m, M;             // M = border size: ncomp * m (mode 0) or m
     int pad, Nn, Nt;         // front padding of the data block, its padded size, total padded size
     double nugget;
+    __device__ __forceinline__ double data_z(int c, int j) const { return data[c][j]; }
 };
 
-template <int NCOMP>
-__device__ __forceinline__ double predict_entry(const PredictSrc& ps, const double (&amp2)[NCOMP], const double (&p2)[NCOMP],
+// The chunk farm's source (psoap_farm_predict): the data's ln-wavelengths are the chunk's resident pixels shifted by
+// the item's epoch velocities on the fly, z_at(zs, c, j), the very values the data block's fill reads; data[] is unused.
+struct PredictFarmSrc : PredictSrc {
+    ZSource zs;
+    __device__ __forceinline__ double data_z(int c, int j) const { return z_at(zs, c, j); }
+};
+
+template <int NCOMP, class Src>
+__device__ __forceinline__ double predict_entry(const Src& ps, const double (&amp2)[NCOMP], const double (&p2)[NCOMP],
                                                 int a, int c, int ap, int col, const double* __restrict__ etab) {
     // border row a (< M; mode 0: component c, grid point ap) against physical column `col`: a data pixel
     // (pad <= col < Nn) or a border column (col >= Nn)
     if (col < ps.Nn) {
         const int j = col - ps.pad;
         if (j < 0) return 0.0;
-        if (ps.mode == 0) return se_term(amp2[c], p2[c], ps.data[c][j], ps.pred[c][ap], etab);
+        if (ps.mode == 0) return se_term(amp2[c], p2[c], ps.data_z(c, j), ps.pred[c][ap], etab);
         double cov = 0.0;
 #pragma unroll
         for (int c = 0; c < NCOMP; ++c) {
-            const double t = (ps.mode == 1) ? se_term(amp2[c], p2[c], ps.data[c][j], ps.pred[c][a], etab)
-                                            : se_term(amp2[c], p2[c], ps.data[c][a], ps.pred[c][j], etab);
+            const double t = (ps.mode == 1) ? se_term(amp2[c], p2[c], ps.data_z(c, j), ps.pred[c][a], etab)
+                                            : se_term(amp2[c], p2[c], ps.data_z(c, a), ps.pred[c][j], etab);
             cov = (c == 0) ? t : __dadd_rn(cov, t);
         }
         return cov;
@@ -59,9 +69,11 @@ __device__ __forceinline__ double predict_entry(const PredictSrc& ps, const doub
 
 // Border rows of S: one CTA per 128 x 128 tile (bi in [Nn/128, Nt/128), bj <= bi), thread = 2 consecutive rows.
 // Rows past M (dead padding of the border) get zeros and a unit diagonal; the residual of all border rows is zeroed.
-template <int NCOMP>
-__global__ void __launch_bounds__(256) predict_border_kernel(double* __restrict__ S, int64_t ld, PredictSrc ps, GpParams gp,
-                                                             double* __restrict__ rvec) {
+// Src says where the data's ln-wavelengths come from (PredictSrc: per-component arrays; PredictFarmSrc: shifted on the
+// fly), as gemm_persistent takes its operand source.
+template <int NCOMP, class Src>
+__device__ __forceinline__ void predict_border_tile(double* __restrict__ S, int64_t ld, Src ps, GpParams gp,
+                                                    double* __restrict__ rvec) {
     __shared__ double etab[64];
     load_exp_table(etab);
     const int Tn = ps.Nn / NB;
@@ -99,6 +111,18 @@ __global__ void __launch_bounds__(256) predict_border_kernel(double* __restrict_
     }
 }
 
+template <int NCOMP>
+__global__ void __launch_bounds__(256) predict_border_kernel(double* __restrict__ S, int64_t ld, PredictSrc ps, GpParams gp,
+                                                             double* __restrict__ rvec) {
+    predict_border_tile<NCOMP>(S, ld, ps, gp, rvec);
+}
+
+template <int NCOMP>
+__global__ void __launch_bounds__(256) predict_border_farm_kernel(double* __restrict__ S, int64_t ld, PredictFarmSrc ps,
+                                                                  GpParams gp, double* __restrict__ rvec) {
+    predict_border_tile<NCOMP>(S, ld, ps, gp, rvec);
+}
+
 // Sigma [M, M] row-major (both triangles) from the lower triangle of the trailing block, delta[a] = -r[Nn + a].
 __global__ void predict_readout_kernel(const double* __restrict__ S, int64_t ld, int Nn, int M, const double* __restrict__ rvec,
                                        double* __restrict__ Sigma, double* __restrict__ delta) {
@@ -129,6 +153,46 @@ __global__ void predict_readout_kernel(const double* __restrict__ S, int64_t ld,
     if (bj == 0 && delta != nullptr && threadIdx.x < 32) {
         const int a = bi * 32 + threadIdx.x;
         if (a < M) delta[a] = -rvec[Nn + a];
+    }
+}
+
+// One farm item's outputs from its trailing block: Sigma row-major [M, M] (diag = 0) or its diagonal [M] (diag = 1), and
+// delta [M] as predict_readout_kernel writes them.  Every output is NaN when the item's sentinel fired (|v| >= c, a
+// negative GP hyper-parameter) or its elimination failed (info != 0): the words grad_flagged reads.  Grid (nb, nb) for
+// Sigma, (1, nb) for its diagonal, nb = ceil(M / 32).
+__global__ void __launch_bounds__(256) predict_farm_readout_kernel(const double* __restrict__ S, int64_t ld, int Nn, int M,
+                                                                   const double* __restrict__ rvec, const int* __restrict__ info,
+                                                                   const int* __restrict__ sentinel, int diag,
+                                                                   double* __restrict__ Sigma, double* __restrict__ delta) {
+    __shared__ double tile[32][33];
+    const bool bad = info[0] != 0 || sentinel[0] != 0;
+    const int bi = blockIdx.y, bj = blockIdx.x;
+    const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;   // 32 x 8
+    if (bj > bi) return;
+    if (diag) {
+        const int a = bi * 32 + threadIdx.x;
+        if (threadIdx.x < 32 && a < M) Sigma[a] = bad ? CUDART_NAN : S[(Nn + a) + (int64_t)(Nn + a) * ld];
+    } else {
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            const int c = bj * 32 + ty + 8 * k, r = bi * 32 + tx;
+            tile[ty + 8 * k][tx] = (r < M && c < M && r >= c) ? (bad ? CUDART_NAN : S[(Nn + r) + (int64_t)(Nn + c) * ld]) : 0.0;
+        }
+        __syncthreads();
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            const int r = bi * 32 + ty + 8 * k, c = bj * 32 + tx;
+            if (r < M && c < M && r >= c) Sigma[(int64_t)r * M + c] = tile[tx][ty + 8 * k];
+        }
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            const int c = bj * 32 + ty + 8 * k, r = bi * 32 + tx;
+            if (r < M && c < M && r > c) Sigma[(int64_t)c * M + r] = tile[ty + 8 * k][tx];
+        }
+    }
+    if (bj == 0 && threadIdx.x < 32) {
+        const int a = bi * 32 + threadIdx.x;
+        if (a < M) delta[a] = bad ? CUDART_NAN : -rvec[Nn + a];
     }
 }
 

@@ -50,6 +50,41 @@ def chunk_cost(N):
 # branches beyond 16 buy nothing the SMs could use, so 16, at half the memory of 32.
 GRAD_NBRANCH = 16
 
+# Default (proposal, chunk) items in flight in the prediction graph (capped by the number of items).  The gradient
+# graph's default; the best value for prediction is not measured.
+PREDICT_NBRANCH = 16
+
+
+def prediction_grids(grids, n_pix, ncomp):
+    """The per-chunk grids of ChunkFarm.attach_prediction_grids as [ncomp, m] float64 arrays: a 1-D entry serves every
+    component, a 2-D one is [ncomp, m] (lwl_f_predict, lwl_g_predict[, lwl_h_predict] of predict_f_g / _f_g_h).
+    n_pix: the number of pixels of every chunk, in global chunk order."""
+    if len(grids) != len(n_pix):
+        raise ValueError("one prediction grid per chunk: got %d grids for %d chunks" % (len(grids), len(n_pix)))
+    out = []
+    for i, (g, n) in enumerate(zip(grids, n_pix)):
+        a = np.asarray(g, dtype=np.float64)
+        if a.ndim == 1:
+            a = np.broadcast_to(a, (ncomp, a.size))
+        if a.ndim != 2 or a.shape[0] != ncomp:
+            raise ValueError("chunk %d: a prediction grid is 1-D or [%d, m], not of shape %s" % (i, ncomp, np.shape(g)))
+        if not np.all(np.isfinite(a)):
+            raise ValueError("chunk %d: the prediction grid holds non-finite values" % i)
+        if n == 0 and a.shape[1] != 0:
+            raise ValueError("chunk %d has no pixels: its prediction grid must be empty" % i)
+        out.append(np.ascontiguousarray(a))
+    return out
+
+
+def combine_predictions(mu, var):
+    """Posterior-averaged spectrum and its variance over K samples by the law of total variance: mean of the variances
+    plus the variance of the means.  mu, var: [K, M] (one chunk's outputs of predict_components, var the diagonal of
+    Sigma).  Sums over the samples run in sample order."""
+    mu, var = np.asarray(mu, dtype=np.float64), np.asarray(var, dtype=np.float64)
+    K = mu.shape[0]
+    mean = np.add.reduce(mu, axis=0) / K
+    return mean, np.add.reduce(var, axis=0) / K + np.add.reduce((mu - mean) ** 2, axis=0) / K
+
 
 class ChunkFarm:
     """model: "SB1" | "SB2" | "ST1" | "ST2" | "ST3".
@@ -142,6 +177,8 @@ class ChunkFarm:
         self._n_epochs = nes
         self._grad_ws = None         # allocated by the first lnprob_and_grad call
         self._grad_farm_ws = None    # allocated, and the gradient graph attached, by the first *_many gradient call
+        self._n_pix = [len(ch["fl"]) for ch in chunks]
+        self._pred = None            # attach_prediction_grids
         self._farm = _lib.vp(None)
         K = self.n_proposals
         self._results = torch.zeros((K, max(1, len(self.mine)), 4), dtype=torch.float64, device="cuda")
@@ -355,11 +392,131 @@ class ChunkFarm:
         lnp = np.array([float(np.sum(hk[:, 0])) for hk in h])
         return lnp, np.stack([np.sum(hk[:, 1:], axis=0) for hk in h])
 
+    def attach_prediction_grids(self, grids, sigma="full", predict_nbranch=None):
+        """Attach the prediction graph (psoap_farm_predict_attach) for predict_components: grids holds one entry per
+        chunk in global chunk order, a 1-D rest-frame ln-wavelength grid used for every component or an [ncomp, m]
+        array (lwl_f_predict, lwl_g_predict[, lwl_h_predict] of predict_f_g / _f_g_h); a chunk without pixels takes an
+        empty grid.  sigma: "full" (Sigma) or "diag" (its diagonal).  predict_nbranch: (proposal, chunk) items in
+        flight (default PREDICT_NBRANCH); each branch holds the bordered matrix of the largest item,
+        8 (padded(N) + padded(ncomp m))^2 bytes.  The grids are uploaded once; a farm that never calls this allocates
+        and captures nothing for prediction."""
+        if self._pred is not None:
+            raise RuntimeError("the prediction grids are already attached to this farm")
+        if sigma not in ("full", "diag"):
+            raise ValueError('sigma must be "full" or "diag", not %r' % (sigma,))
+        nb = int(predict_nbranch) if predict_nbranch is not None else PREDICT_NBRANCH
+        if nb < 1:
+            raise ValueError("predict_nbranch must be at least 1")
+        ncomp = _lib.NCOMP[self.model]
+        gr = prediction_grids(grids, self._n_pix, ncomp)
+        lib = _lib.load()
+        torch = _lib.torch_cuda()
+        K, mode = self.n_proposals, (0 if sigma == "full" else 1)
+        m_all = [g.shape[1] for g in gr]
+        M_all = [ncomp * m for m in m_all]
+        size = [M * M if mode == 0 else M for M in M_all]
+        # the outputs of all chunks in one flat buffer per kind, chunk after chunk and each chunk's proposals side by
+        # side: the layout psoap_farm_predict_attach returns for a farm that holds every chunk
+        d0 = np.concatenate([[0], np.cumsum([K * M for M in M_all])]).astype(np.int64)
+        s0 = np.concatenate([[0], np.cumsum([K * x for x in size])]).astype(np.int64)
+        pred = dict(mode=mode, m=m_all, M=M_all, d0=d0, s0=s0, ws=None, grids=None, off=None)
+        if self.mine:
+            total, offs = 0, []
+            for i in self.mine:
+                offs.append(total)
+                total += (gr[i].nbytes + 255) // 256 * 256
+            gdev = torch.empty(max(total, 256), dtype=torch.uint8, device="cuda")
+            host = np.zeros(max(total, 256), dtype=np.uint8)
+            for i, o in zip(self.mine, offs):
+                host[o:o + gr[i].nbytes] = gr[i].view(np.uint8).reshape(-1)
+            gdev.copy_(torch.from_numpy(host))
+            base = gdev.data_ptr()
+            ptrs = (_lib.vp * (len(self.mine) * ncomp))(
+                *[_lib.vp(base + o + c * m_all[i] * 8) for i, o in zip(self.mine, offs) for c in range(ncomp)])
+            m_mine = (ctypes.c_int64 * len(self.mine))(*[m_all[i] for i in self.mine])
+            nbytes = lib.psoap_farm_predict_workspace_bytes(self._farm, nb, m_mine, mode)
+            try:
+                ws = torch.empty(nbytes + 256, dtype=torch.uint8, device="cuda")
+            except torch.cuda.OutOfMemoryError as e:
+                raise MemoryError("the prediction graph needs %d bytes of device memory for predict_nbranch = %d (one "
+                                  "bordered matrix of the largest item per branch); pass a smaller predict_nbranch"
+                                  % (nbytes, nb)) from e
+            nitems = K * len(self.mine)
+            off = (ctypes.c_int64 * (2 * (nitems + 1)))()
+            _lib.check(lib.psoap_farm_predict_attach(self._farm, nb, m_mine, ptrs, mode, _lib.ptr(ws), nbytes, off))
+            off = np.frombuffer(off, dtype=np.int64).reshape(2, nitems + 1).copy()
+            pred.update(ws=ws, grids=gdev, off=off)
+        self._pred = pred
+
+    def predict_components(self, P, mus):
+        """The component spectra of every chunk at the n_proposals registered vectors P ([n_proposals, n_params]), as
+        predict_f_g / predict_f_g_h compute them from the chunk's pixels shifted by each proposal's velocities, with one
+        launch of the prediction graph (attach_prediction_grids first).  mus: the ncomp component means (mu_f, mu_g[,
+        mu_h]).  Returns, per chunk in global chunk order, (mu [n_proposals, ncomp m], Sigma [n_proposals, M, M]) or,
+        with sigma="diag", (mu, var [n_proposals, M]), M = ncomp m, as device tensors.  Each rank fills its own chunks
+        into one flat buffer per kind, which is all-reduced once (exact: every entry has one contributor).  Raises
+        numpy.linalg.LinAlgError for an item whose data block is not positive definite and ValueError for one whose
+        velocities reach c or whose GP parameters are negative, naming the proposal and the chunk."""
+        ncomp = _lib.NCOMP[self.model]
+        K, npar = self.n_proposals, self.n_params
+        P = np.asarray(P, dtype=np.float64)
+        if P.size != K * npar:
+            raise ValueError("P must hold %d x %d registered parameters of %s" % (K, npar, self.model))
+        mus = np.asarray(mus, dtype=np.float64).reshape(-1)
+        if mus.size != ncomp:
+            raise ValueError("mus must hold the %d component means of %s" % (ncomp, self.model))
+        if self._pred is None:
+            raise RuntimeError("attach_prediction_grids must be called before predict_components")
+        q = self._pred
+        lib = _lib.load()
+        torch = _lib.torch_cuda()
+        delta = torch.zeros(int(q["d0"][-1]), dtype=torch.float64, device="cuda")
+        sig = torch.zeros(int(q["s0"][-1]), dtype=torch.float64, device="cuda")
+        res = torch.zeros((K, self.n_chunks, 4), dtype=torch.float64, device="cuda")
+        if self.mine:
+            off = q["off"]
+            n_mine = len(self.mine)
+            p_dev = torch.from_numpy(np.ascontiguousarray(P.reshape(K, npar))).cuda()
+            dl = torch.empty(max(1, int(off[0, -1])), dtype=torch.float64, device="cuda")
+            sl = torch.empty(max(1, int(off[1, -1])), dtype=torch.float64, device="cuda")
+            rl = torch.empty((K, n_mine, 4), dtype=torch.float64, device="cuda")
+            _lib.check(lib.psoap_farm_predict(self._farm, _lib.ptr(p_dev), _lib.ptr(dl), _lib.ptr(sl), _lib.ptr(rl),
+                                              _lib.stream_ptr()))
+            # each own chunk's proposals are contiguous in the attach layout: one copy per chunk and kind
+            for k, i in enumerate(self.mine):
+                nd, ns = K * q["M"][i], int(q["s0"][i + 1] - q["s0"][i])
+                delta[q["d0"][i]:q["d0"][i] + nd].copy_(dl[off[0, k]:off[0, k] + nd])
+                sig[q["s0"][i]:q["s0"][i] + ns].copy_(sl[off[1, k]:off[1, k] + ns])
+            res.index_copy_(1, self._mine_idx, rl)
+        if self.world_size > 1:
+            self._allreduce(delta)
+            self._allreduce(sig)
+            self._allreduce(res)
+        h = res.cpu().numpy()
+        for k in range(K):
+            for i in range(self.n_chunks):
+                if q["m"][i] == 0:
+                    continue
+                if h[k, i, 3] != 0.0:
+                    raise np.linalg.LinAlgError("proposal %d, chunk %d: %d-th leading minor of the data block is not "
+                                                "positive definite" % (k, i, int(h[k, i, 3])))
+                if h[k, i, 0] == -np.inf:
+                    raise ValueError("proposal %d, chunk %d: a velocity reaches the speed of light or a GP parameter is "
+                                     "negative" % (k, i))
+        out = []
+        for i in range(self.n_chunks):
+            M, m = q["M"][i], q["m"][i]
+            mu = delta[q["d0"][i]:q["d0"][i + 1]].view(K, M) + torch.from_numpy(np.repeat(mus, m)).cuda()
+            s = sig[q["s0"][i]:q["s0"][i + 1]]
+            out.append((mu, s.view(K, M, M) if q["mode"] == 0 else s.view(K, M)))
+        return out
+
     def close(self):
         if self._farm:
             _lib.load().psoap_farm_destroy(self._farm)
             self._farm = _lib.vp(None)
         self._grad_farm_ws = None
+        self._pred = None
 
     def __del__(self):
         try:
