@@ -428,18 +428,21 @@ int launch_factor(const Lanes& ln, double* W, int64_t ld, int T_elim, int T_tota
     return PSOAP_OK;
 }
 
-template <int NCOMP>
-void launch_fill_lower_t(cudaStream_t st, double* W, int64_t ld, int T, int pad, const ZSource& zs,
-                         const double* sigma, const double* fl, double mu, const GpParams& gp, const FactorWs& ws) {
-    launch_k(fill_lower_kernel<NCOMP>, (unsigned)(T * (T + 1) / 2), 256, 0, st, 0, W, ld, pad, zs, sigma, fl, mu, gp, ws.rvec,
-             ws.acc, ws.info, ws.nz);
+// Calls fn(nc) with nc a std::integral_constant<int, ncomp> (1, 2 or 3): the one place where a run-time number of
+// components picks the instantiation of a kernel template.
+template <class Fn>
+void with_ncomp(int ncomp, Fn&& fn) {
+    if (ncomp == 1) fn(std::integral_constant<int, 1>{});
+    else if (ncomp == 2) fn(std::integral_constant<int, 2>{});
+    else fn(std::integral_constant<int, 3>{});
 }
 
 int launch_fill_lower(int ncomp, cudaStream_t st, double* W, int64_t ld, int T, int pad, const ZSource& zs,
                       const double* sigma, const double* fl, double mu, const GpParams& gp, const FactorWs& ws) {
-    if (ncomp == 1) launch_fill_lower_t<1>(st, W, ld, T, pad, zs, sigma, fl, mu, gp, ws);
-    else if (ncomp == 2) launch_fill_lower_t<2>(st, W, ld, T, pad, zs, sigma, fl, mu, gp, ws);
-    else launch_fill_lower_t<3>(st, W, ld, T, pad, zs, sigma, fl, mu, gp, ws);
+    with_ncomp(ncomp, [&](auto nc) {
+        launch_k(fill_lower_kernel<nc>, (unsigned)(T * (T + 1) / 2), 256, 0, st, 0, W, ld, pad, zs, sigma, fl, mu, gp,
+                 ws.rvec, ws.acc, ws.info, ws.nz);
+    });
     LAUNCH_CHECK();
     return PSOAP_OK;
 }
@@ -482,10 +485,17 @@ __global__ void write_result_kernel(double* result, double lnlike, double logdet
     result[0] = lnlike; result[1] = logdet; result[2] = quad; result[3] = info;
 }
 
+// GP hyper-parameters read on the device from dev ([amp, l] per component; null: from amp / l), unused components inert
+GpParams gp_params(const double* dev) {
+    GpParams gp;
+    gp.dev = dev;
+    for (int c = 0; c < 3; ++c) { gp.amp[c] = 0; gp.l[c] = 1; }
+    return gp;
+}
+
 bool make_gp(int ncomp, const double* amp, const double* l, GpParams* gp) {
     bool neg = false;
-    gp->dev = nullptr;
-    for (int c = 0; c < 3; ++c) { gp->amp[c] = 0; gp->l[c] = 1; }
+    *gp = gp_params(nullptr);
     for (int c = 0; c < ncomp; ++c) {
         gp->amp[c] = amp[c];
         gp->l[c] = l[c];
@@ -498,6 +508,13 @@ ZSource direct_z(const double* f, const double* g, const double* h) {
     ZSource zs;
     zs.lwl[0] = f; zs.lwl[1] = g; zs.lwl[2] = h;
     zs.epoch = nullptr; zs.vel = nullptr; zs.n_epochs = 0; zs.shift = 0;
+    return zs;
+}
+
+// the chunk's pixels shifted by a velocity table on the device [ncomp][n_epochs], as the farm and the chunk entries read them
+ZSource farm_z(const psoap_chunk& ch, const double* vel) {
+    ZSource zs = direct_z(ch.lwl, nullptr, nullptr);
+    zs.epoch = ch.epoch; zs.vel = vel; zs.n_epochs = ch.n_epochs; zs.shift = 1;
     return zs;
 }
 
@@ -530,9 +547,7 @@ int psoap_fill_v11(int ncomp, double* mat, int64_t ld, int64_t N, const double* 
     cudaStream_t st = (cudaStream_t)stream;
     const int T = (int)((N + 63) / 64);
     const unsigned grid = (unsigned)((int64_t)T * (T + 1) / 2);
-    if (ncomp == 1) fill_full_kernel<1><<<grid, 256, 0, st>>>(mat, ld, (int)N, zs, gp);
-    else if (ncomp == 2) fill_full_kernel<2><<<grid, 256, 0, st>>>(mat, ld, (int)N, zs, gp);
-    else fill_full_kernel<3><<<grid, 256, 0, st>>>(mat, ld, (int)N, zs, gp);
+    with_ncomp(ncomp, [&](auto nc) { fill_full_kernel<nc><<<grid, 256, 0, st>>>(mat, ld, (int)N, zs, gp); });
     LAUNCH_CHECK();
     return PSOAP_OK;
 }
@@ -582,9 +597,7 @@ int psoap_fill_v12n(int ncomp, double* mat, int64_t ld, int64_t M, int64_t N, co
     }
     dim3 grid((unsigned)((N + 63) / 64), (unsigned)((M + 63) / 64));
     cudaStream_t st = (cudaStream_t)stream;
-    if (ncomp == 1) fill_v12_kernel<1><<<grid, 256, 0, st>>>(mat, ld, (int)M, (int)N, src, gp);
-    else if (ncomp == 2) fill_v12_kernel<2><<<grid, 256, 0, st>>>(mat, ld, (int)M, (int)N, src, gp);
-    else fill_v12_kernel<3><<<grid, 256, 0, st>>>(mat, ld, (int)M, (int)N, src, gp);
+    with_ncomp(ncomp, [&](auto nc) { fill_v12_kernel<nc><<<grid, 256, 0, st>>>(mat, ld, (int)M, (int)N, src, gp); });
     LAUNCH_CHECK();
     return PSOAP_OK;
 }
@@ -805,9 +818,9 @@ int launch_grad(const Lanes& ln, int ncomp, int64_t N, const ZSource& zs, const 
     rc = launch_factor(ln, g.S, g.Nt, Tn, Tt, pad, g.f, sentinel, result, true);
     if (rc) return rc;
     const GradOut out{g.tile, g.slot, g.Tb};
-    if (ncomp == 1) lnlike_grad_kernel<1><<<g.ntiles, 256, 0, st>>>(g.S, g.Nt, (int)g.Nn, (int)N, g.f.rvec, zs, gp, out);
-    else if (ncomp == 2) lnlike_grad_kernel<2><<<g.ntiles, 256, 0, st>>>(g.S, g.Nt, (int)g.Nn, (int)N, g.f.rvec, zs, gp, out);
-    else lnlike_grad_kernel<3><<<g.ntiles, 256, 0, st>>>(g.S, g.Nt, (int)g.Nn, (int)N, g.f.rvec, zs, gp, out);
+    with_ncomp(ncomp, [&](auto nc) {
+        lnlike_grad_kernel<nc><<<g.ntiles, 256, 0, st>>>(g.S, g.Nt, (int)g.Nn, (int)N, g.f.rvec, zs, gp, out);
+    });
     LAUNCH_CHECK();
     grad_hyp_kernel<<<1, 256, 0, st>>>(g.tile, g.ntiles, ncomp, g.f.rvec, (int)g.Nn, (int)N, gp, g.f.info, sentinel, grad_hyp);
     LAUNCH_CHECK();
@@ -886,44 +899,33 @@ extern "C" size_t psoap_chunk_lnprob_grad_workspace_bytes(int model, int64_t N, 
 }
 
 namespace {
-// the chunk's pixels shifted by its epoch velocities (the farm's fused Doppler-shifted fill, farm_issue) and its GP
-// values on the device, as psoap_chunk_lnprob_grad and psoap_chunk_fisher see them
-ZSource chunk_zsource(const psoap_chunk* chunk, const GradWs& g) {
-    ZSource zs;
-    zs.lwl[0] = chunk->lwl; zs.lwl[1] = nullptr; zs.lwl[2] = nullptr;
-    zs.epoch = chunk->epoch; zs.vel = g.vel; zs.n_epochs = chunk->n_epochs; zs.shift = 1;
-    return zs;
-}
-GpParams chunk_gp(const double* p_dev, int norb) {
-    GpParams gp;
-    gp.dev = p_dev + norb;
-    for (int c = 0; c < 3; ++c) { gp.amp[c] = 0; gp.l[c] = 1; }
-    return gp;
+// the per-epoch sums and the chain rule of one gradient problem (the last steps of psoap_chunk_lnprob_grad)
+int launch_grad_chain(cudaStream_t st, int ncomp, int norb, const psoap_chunk& ch, const GradWs& w, const double* jac,
+                      const int* sentinel, double* grad_p) {
+    grad_epoch_kernel<<<(unsigned)(ncomp * ch.n_epochs), 256, 0, st>>>(w.gz, ch.epoch, ch.N, ch.n_epochs, w.gv);
+    LAUNCH_CHECK();
+    grad_chain_kernel<<<1, 32, 0, st>>>(w.gv, jac, w.hyp, ncomp, ch.n_epochs, norb, w.f.info, sentinel, grad_p);
+    LAUNCH_CHECK();
+    return PSOAP_OK;
 }
 
 // The launches of psoap_chunk_lnprob_grad on a carved workspace: orbit velocities and sentinel, fill, identity border,
-// restricted elimination, contraction, reductions, per-epoch sum, orbit Jacobian and chain rule.
+// restricted elimination, contraction, reductions, orbit Jacobian, per-epoch sum and chain rule.
 int launch_chunk_grad(int model, const psoap_chunk* chunk, const double* p_dev, double mu_GP, const GradWs& g,
                       cudaStream_t st, double* result, double* grad_p) {
-    const int64_t N = chunk->N;
     const int ne = chunk->n_epochs, ncomp = model_ncomp(model), norb = model_norb(model);
     // orbit velocities and the sentinel (|v| >= c, or a negative GP hyper-parameter), as the farm's orbit kernel
     orbit_kernel<<<1, 128, 0, st>>>(model, p_dev, chunk->dates, ne, g.vel, g.flag, 1);
     LAUNCH_CHECK();
-    const ZSource zs = chunk_zsource(chunk, g);
-    const GpParams gp = chunk_gp(p_dev, norb);
     Lanes ln;
     int rc = get_lanes(st, &ln);
     if (rc) return rc;
-    rc = launch_grad(ln, ncomp, N, zs, chunk->fl, chunk->sigma, mu_GP, gp, g, g.flag, result, g.hyp, g.gz);
+    rc = launch_grad(ln, ncomp, chunk->N, farm_z(*chunk, g.vel), chunk->fl, chunk->sigma, mu_GP, gp_params(p_dev + norb),
+                     g, g.flag, result, g.hyp, g.gz);
     if (rc) return rc;
-    grad_epoch_kernel<<<(unsigned)(ncomp * ne), 256, 0, st>>>(g.gz, chunk->epoch, N, ne, g.gv);
-    LAUNCH_CHECK();
     orbit_jacobian_kernel<<<1, 128, 0, st>>>(model, p_dev, chunk->dates, ne, g.jac);
     LAUNCH_CHECK();
-    grad_chain_kernel<<<1, 32, 0, st>>>(g.gv, g.jac, g.hyp, ncomp, ne, norb, g.f.info, g.flag, grad_p);
-    LAUNCH_CHECK();
-    return PSOAP_OK;
+    return launch_grad_chain(st, ncomp, norb, *chunk, g, g.jac, g.flag, grad_p);
 }
 
 bool chunk_args_ok(int model, const psoap_chunk* chunk) {
@@ -976,12 +978,6 @@ size_t carve_fisher_ws(char* base, int model, int64_t N, int n_epochs, GradWs* g
     return off;
 }
 
-template <int NCOMP>
-void launch_dk(cudaStream_t st, const GradWs& g, int N, const ZSource& zs, const GpParams& gp, int norb, int a,
-               uint8_t* flags) {
-    fisher_dk_kernel<NCOMP><<<(unsigned)(g.Tb * g.Tb), 256, 0, st>>>(g.S, g.Nt, g.Tb, N, zs, gp, g.jac, norb, a, flags);
-}
-
 // the Fisher steps after launch_chunk_grad (fisher.cuh): mirror K^-1, then per parameter D_a and A_a = K^-1 D_a, then
 // the tile-pair contraction and the fixed-order reduction into fisher [P][P]
 int launch_fisher(int model, const psoap_chunk* chunk, const double* p_dev, const GradWs& g, const FisherWs& f,
@@ -996,14 +992,14 @@ int launch_fisher(int model, const psoap_chunk* chunk, const double* p_dev, cons
     int rc = make_tensor_map(&mapS, kinv, (uint64_t)Nn, (uint64_t)Nn, (uint64_t)g.Nt, SA);
     if (!rc) rc = make_tensor_map(&mapD, g.S, (uint64_t)Nn, (uint64_t)Nn, (uint64_t)g.Nt, SB);
     if (rc) return rc;
-    const ZSource zs = chunk_zsource(chunk, g);
-    const GpParams gp = chunk_gp(p_dev, norb);
+    const ZSource zs = farm_z(*chunk, g.vel);
+    const GpParams gp = gp_params(p_dev + norb);
     const int ntiles = g.Tb * 2 * g.Tb;
     for (int a = 0; a < P; ++a) {
         uint8_t* flags = (a == 0) ? f.flags : nullptr;   // the zero pattern is the same for every parameter
-        if (ncomp == 1) launch_dk<1>(st, g, N, zs, gp, norb, a, flags);
-        else if (ncomp == 2) launch_dk<2>(st, g, N, zs, gp, norb, a, flags);
-        else launch_dk<3>(st, g, N, zs, gp, norb, a, flags);
+        with_ncomp(ncomp, [&](auto nc) {
+            fisher_dk_kernel<nc><<<(unsigned)(g.Tb * g.Tb), 256, 0, st>>>(g.S, g.Nt, g.Tb, N, zs, gp, g.jac, norb, a, flags);
+        });
         LAUNCH_CHECK();
         if (a == 0) {
             fisher_krange_kernel<<<1, 256, 0, st>>>(f.flags, g.Tb, f.krange);
@@ -1121,9 +1117,7 @@ extern "C" int psoap_predict(int ncomp, int mode, int64_t n, int64_t m, const do
     ps.pad = pad; ps.Nn = (int)Nn; ps.Nt = (int)Nt; ps.nugget = nugget;
     const int Tn = (int)(Nn / NB), Tt = (int)(Nt / NB);
     const unsigned ntile = (unsigned)((int64_t)Tt * (Tt + 1) / 2 - (int64_t)Tn * (Tn + 1) / 2);
-    if (ncomp == 1) predict_border_kernel<1><<<ntile, 256, 0, st>>>(S, Nt, ps, gp, ws.rvec);
-    else if (ncomp == 2) predict_border_kernel<2><<<ntile, 256, 0, st>>>(S, Nt, ps, gp, ws.rvec);
-    else predict_border_kernel<3><<<ntile, 256, 0, st>>>(S, Nt, ps, gp, ws.rvec);
+    with_ncomp(ncomp, [&](auto nc) { predict_border_kernel<nc><<<ntile, 256, 0, st>>>(S, Nt, ps, gp, ws.rvec); });
     LAUNCH_CHECK();
     Lanes ln;
     rc = get_lanes(st, &ln);
@@ -1193,9 +1187,10 @@ extern "C" int psoap_predict_host(int ncomp, int mode, int64_t n, int64_t m, con
 // ======================================================================================================
 constexpr int P_STRIDE = 32;  // doubles reserved per proposal in the parameter buffer
 namespace {
-// One CUDA graph of a farm and what issues it: the branch streams (+ the root stream at index nbranch), their events,
-// the high-priority side streams of look-ahead, and whether calls replay the captured graph or issue the kernels
-// directly.  The likelihood graph, the gradient graph and the prediction graph each own one.
+// One CUDA graph of a farm: the state of its work items (item = proposal * nchunks + chunk), the branch scratch, and
+// what issues it: the branch streams (+ the root stream at index nbranch), their events, the high-priority side streams
+// of look-ahead, and whether calls replay the captured graph or issue the kernels directly.  The likelihood graph, the
+// gradient graph and the prediction graph each own one; it releases its streams, events and graph with it.
 struct FarmGraph {
     int nbranch = 0;
     bool lookahead = false;
@@ -1207,44 +1202,46 @@ struct FarmGraph {
     std::vector<cudaEvent_t> events;
     std::vector<cudaEvent_t> side_events;
     int launches = 0;                 // kernels one evaluation launches
-};
-
-// The optional gradient graph of a farm (psoap_farm_grad_attach): its own parameter buffer, velocity tables,
-// sentinels, orbit Jacobians and outputs per (proposal, chunk) item, and one GradWs region per branch, carved for
-// each item in turn (items of a branch run in stream order).
-struct FarmGrad {
-    FarmGraph g;
-    double* p_buf = nullptr;          // [nprop][P_STRIDE]
+    double* p_buf = nullptr;          // [nprop][P_STRIDE] parameter vectors the graph reads
     double* results = nullptr;        // [nitems][4]
-    double* grad = nullptr;           // [nitems][n_params]
     int* flags = nullptr;             // per item sentinel
     OrbitDesc* descs = nullptr;       // device, per item
-    JacDesc* jdescs = nullptr;        // device, per item
-    std::vector<double*> item_vel;    // [ncomp][n_epochs] per item
-    std::vector<double*> item_jac;    // [ncomp][n_epochs][norb] per item
-    std::vector<char*> branch_base;   // GradWs region of each branch
-    std::vector<std::vector<int>> branch_items;
+    std::vector<double*> item_vel;    // device velocity table of each item
+    std::vector<char*> branch_base;   // scratch region of each branch, carved for each of its items in turn (items of
+                                      // a branch run in stream order)
+    std::vector<std::vector<int>> branch_items;   // LPT order
+
+    FarmGraph() = default;
+    FarmGraph(const FarmGraph&) = delete;
+    FarmGraph& operator=(const FarmGraph&) = delete;
+    ~FarmGraph() {
+        if (exec) cudaGraphExecDestroy(exec);
+        if (graph) cudaGraphDestroy(graph);
+        for (auto& s : streams) if (s) cudaStreamDestroy(s);
+        for (auto& s : side_streams) if (s) cudaStreamDestroy(s);
+        for (auto& ev : events) if (ev) cudaEventDestroy(ev);
+        for (auto& ev : side_events) if (ev) cudaEventDestroy(ev);
+    }
 };
 
-// The optional prediction graph of a farm (psoap_farm_predict_attach): its own parameter buffer, velocity tables,
-// sentinels and result records per (proposal, chunk) item, the caller's grids, the output offsets of every item, and
-// one bordered-matrix region per branch (S of the largest item, then its FactorWs), carved for each item in turn.
+// The optional gradient graph of a farm (psoap_farm_grad_attach): besides the item state, the gradient rows and orbit
+// Jacobians of every item.  Each branch region holds one GradWs.
+struct FarmGrad {
+    FarmGraph g;
+    double* grad = nullptr;           // [nitems][n_params]
+    JacDesc* jdescs = nullptr;        // device, per item
+    std::vector<double*> item_jac;    // [ncomp][n_epochs][norb] per item
+};
+
+// The optional prediction graph of a farm (psoap_farm_predict_attach): besides the item state, the caller's grids and
+// the output offsets of every item.  Each branch region holds the bordered matrix of an item (S, then its FactorWs).
 struct FarmPredict {
     FarmGraph g;
     int sigma_mode = 0;               // 0: Sigma [M][M], 1: its diagonal [M]
-    double* p_buf = nullptr;          // [nprop][P_STRIDE]
-    double* results = nullptr;        // [nitems][4]
-    int* flags = nullptr;             // per item sentinel
-    OrbitDesc* descs = nullptr;       // device, per item
-    std::vector<double*> item_vel;    // [ncomp][n_epochs] per item
     std::vector<int64_t> m;           // grid points per component, per chunk
     std::vector<const double*> grids; // [nchunks][ncomp] device pointers
     std::vector<int64_t> delta_off;   // [nitems + 1] offsets (doubles) into delta_dev; the last one is its length
     std::vector<int64_t> sigma_off;   // [nitems + 1] the same into sigma_dev
-    std::vector<char*> branch_base;
-    std::vector<std::vector<int>> branch_items;
-    double* delta = nullptr;          // the caller's buffers of the call being issued (direct issue)
-    double* sigma = nullptr;
     double* cap_delta = nullptr;      // scratch outputs the captured graph writes; copied out after a replay
     double* cap_sigma = nullptr;
 };
@@ -1254,130 +1251,92 @@ struct psoap_farm {
     int model = 0, ncomp = 0, norb = 0, nchunks = 0, nprop = 1, nitems = 0;
     double mu = 1.0;
     std::vector<psoap_chunk> chunks;
-    std::vector<FactorWs> branch_ws;
-    std::vector<std::vector<int>> branch_items;
-    double* p_buf = nullptr;          // [nprop][P_STRIDE] parameter vectors the graph reads
-    double* results = nullptr;        // [nprop][nchunks][4]
-    double* vel = nullptr;            // per item [3 * n_epochs]
-    int* flags = nullptr;             // per item sentinel
-    OrbitDesc* descs = nullptr;       // device, per item
-    std::vector<size_t> vel_off;
-    std::vector<double*> item_vel;    // device velocity table of each item
     FarmGraph g;                      // the likelihood graph
     int chain_hint = 0;               // psoap_chunk.reserved of the first chunk, low byte: 3 | 7 forces the chain links
     int group_hint = 0;               // ... bits 8 and up: 2 | 4 | 8 forces the panels per trailing update
     FarmGrad* grad = nullptr;         // psoap_farm_grad_attach; null until then
     FarmPredict* pred = nullptr;      // psoap_farm_predict_attach; null until then
+    ~psoap_farm() { delete grad; delete pred; }
 };
 
 namespace {
-// The launch plan of one work item on branch b, shared by the likelihood, gradient and prediction graphs so that they
-// cannot drift apart.  `nbranch` and `lookahead` are the issuing graph's.
-Lanes farm_lanes(const psoap_farm* f, int nbranch, bool lookahead, cudaStream_t main, cudaStream_t side, cudaEvent_t e1,
-                 cudaEvent_t e2, int pdl) {
+// The launch plan of one work item on branch b of graph g, shared by the likelihood, gradient and prediction graphs so
+// that they cannot drift apart.
+Lanes farm_lanes(const psoap_farm* f, const FarmGraph& g, int b, int pdl) {
     Lanes ln;
-    ln.main = main;
-    ln.side = lookahead ? side : nullptr;
-    ln.e1 = e1; ln.e2 = e2;
+    ln.main = g.streams[b];
+    ln.side = g.lookahead ? g.side_streams[b] : nullptr;
+    ln.e1 = g.side_events[2 * b]; ln.e2 = g.side_events[2 * b + 1];
     // panels per update: the caller's choice (bits 8.. of psoap_chunk.reserved: 2, 4 or 8, again the same on every
     // rank), else by the number of chunks in flight: rank-1024 updates need many to hide their 8-panel heads (C1
     // x 8 proposals on 8 branches: 1121 evals/s against 1149 with rank-512)
-    ln.group = lookahead ? 0
+    ln.group = g.lookahead ? 0
              : (f->group_hint == 2 || f->group_hint == 4 || f->group_hint == 8) ? f->group_hint
-             : (nbranch >= 32 ? 8 : 4);
+             : (g.nbranch >= 32 ? 8 : 4);
     ln.pdl = pdl;
     // chain links: the caller's choice (psoap_chunk.reserved = 3 | 7, the same on every rank of a partitioned
     // farm so that the bits do not depend on the number of GPUs), else by exposure of the chain latency
-    ln.chain = (f->chain_hint == 3 || f->chain_hint == 7) ? f->chain_hint : (lookahead ? 0 : 3);
+    ln.chain = (f->chain_hint == 3 || f->chain_hint == 7) ? f->chain_hint : (g.lookahead ? 0 : 3);
     return ln;
 }
-Lanes farm_lanes(const psoap_farm* f, const FarmGraph& g, int b, int pdl) {
-    return farm_lanes(f, g.nbranch, g.lookahead, g.streams[b], g.side_streams[b], g.side_events[2 * b],
-                      g.side_events[2 * b + 1], pdl);
+
+// the GP values of item it's proposal, as every farm graph reads them
+GpParams farm_gp(const psoap_farm* f, const FarmGraph& g, int it) {
+    return gp_params(g.p_buf + (size_t)(it / f->nchunks) * P_STRIDE + f->norb);
 }
 
-// The GP values of proposal k and the chunk's pixels shifted by the item's velocity table, as every farm graph reads them
-GpParams farm_gp(const psoap_farm* f, const double* p_buf, int k) {
-    GpParams gp;
-    gp.dev = p_buf + (size_t)k * P_STRIDE + f->norb;
-    for (int c = 0; c < 3; ++c) { gp.amp[c] = 0; gp.l[c] = 1; }
-    return gp;
-}
-ZSource farm_z(const psoap_chunk& ch, const double* vel) {
-    ZSource zs;
-    zs.lwl[0] = ch.lwl; zs.lwl[1] = nullptr; zs.lwl[2] = nullptr;
-    zs.epoch = ch.epoch; zs.vel = vel; zs.n_epochs = ch.n_epochs; zs.shift = 1;
-    return zs;
-}
-
-// Issues one evaluation onto the farm's streams, rooted at s0: the orbit kernel for every item, then the per-chunk
-// pipelines on the branch streams, joined back into s0.  Runs under stream capture (graph mode) or for real
-// (direct mode, which adds programmatic dependent launch on the small grids).
-int farm_issue(psoap_farm* f, cudaStream_t s0, int pdl) {
-    const int nbranch = f->g.nbranch, nchunks = f->nchunks;
-    orbit_farm_kernel<<<f->nitems, 64, 0, s0>>>(f->model, f->p_buf, f->descs);
-    ++g_launches;
-    cudaEventRecord(f->g.events[nbranch], s0);
+// Forks g's branches from s0, after the root kernels the caller launched there, issues the items of each branch in LPT
+// order through item(b, branch stream, it), and joins the branches back into s0.
+template <class Item>
+int issue_branches(const FarmGraph& g, cudaStream_t s0, Item&& item) {
+    const cudaEvent_t fork = g.events[g.nbranch];
+    CUDA_TRY(cudaEventRecord(fork, s0));
     int rc = PSOAP_OK;
-    for (int b = 0; b < nbranch && rc == PSOAP_OK; ++b) {
-        cudaStream_t sb = f->g.streams[b];
-        cudaStreamWaitEvent(sb, f->g.events[nbranch], 0);
-        for (int it : f->branch_items[b]) {
-            const psoap_chunk& ch = f->chunks[it % nchunks];
-            const GpParams gp = farm_gp(f, f->p_buf, it / nchunks);
-            const ZSource zs = farm_z(ch, f->item_vel[it]);
-            FactorWs ws = f->branch_ws[b];
-            ws.Nt = padded_dim(ch.N);
-            rc = launch_chunk(farm_lanes(f, f->g, b, pdl), f->ncomp, ch.N, zs, ch.fl, ch.sigma, f->mu, gp, ws, f->flags + it,
-                              f->results + 4 * it);
-            if (rc) break;
-        }
-        cudaEventRecord(f->g.events[b], sb);
-        cudaStreamWaitEvent(s0, f->g.events[b], 0);
+    for (int b = 0; b < g.nbranch && rc == PSOAP_OK; ++b) {
+        const cudaStream_t sb = g.streams[b];
+        CUDA_TRY(cudaStreamWaitEvent(sb, fork, 0));
+        for (int it : g.branch_items[b])
+            if ((rc = item(b, sb, it)) != PSOAP_OK) break;
+        CUDA_TRY(cudaEventRecord(g.events[b], sb));
+        CUDA_TRY(cudaStreamWaitEvent(s0, g.events[b], 0));
     }
     return rc;
 }
 
-// the per-epoch sums and the chain rule of one gradient item (steps 7 and 8 of psoap_chunk_lnprob_grad)
-int launch_grad_chain(cudaStream_t st, int ncomp, int norb, const psoap_chunk& ch, const GradWs& w, const double* jac,
-                      const int* sentinel, double* grad_p) {
-    grad_epoch_kernel<<<(unsigned)(ncomp * ch.n_epochs), 256, 0, st>>>(w.gz, ch.epoch, ch.N, ch.n_epochs, w.gv);
-    LAUNCH_CHECK();
-    grad_chain_kernel<<<1, 32, 0, st>>>(w.gv, jac, w.hyp, ncomp, ch.n_epochs, norb, w.f.info, sentinel, grad_p);
-    LAUNCH_CHECK();
-    return PSOAP_OK;
-}
-
-// The gradient counterpart of farm_issue: velocities, sentinels and orbit Jacobians of every item, then per branch,
-// item after item in LPT order, the steps of psoap_chunk_lnprob_grad into the item's result and gradient rows.
-int farm_grad_issue(psoap_farm* f, cudaStream_t s0, int pdl) {
-    FarmGrad& g = *f->grad;
-    const int nbranch = g.g.nbranch, nchunks = f->nchunks, np = f->norb + 2 * f->ncomp;
+// Issues one evaluation onto the likelihood graph's streams, rooted at s0: the orbit kernel for every item, then the
+// per-chunk pipelines on the branch streams.  Runs under stream capture (graph mode) or for real (direct mode, which
+// adds programmatic dependent launch on the small grids).
+int farm_issue(const psoap_farm* f, cudaStream_t s0, int pdl) {
+    const FarmGraph& g = f->g;
     orbit_farm_kernel<<<f->nitems, 64, 0, s0>>>(f->model, g.p_buf, g.descs);
-    ++g_launches;
-    orbit_jacobian_farm_kernel<<<f->nitems, 64, 0, s0>>>(f->model, g.p_buf, g.jdescs);
-    ++g_launches;
-    cudaEventRecord(g.g.events[nbranch], s0);
-    int rc = PSOAP_OK;
-    for (int b = 0; b < nbranch && rc == PSOAP_OK; ++b) {
-        cudaStream_t sb = g.g.streams[b];
-        cudaStreamWaitEvent(sb, g.g.events[nbranch], 0);
-        for (int it : g.branch_items[b]) {
-            const psoap_chunk& ch = f->chunks[it % nchunks];
-            const GpParams gp = farm_gp(f, g.p_buf, it / nchunks);
-            const ZSource zs = farm_z(ch, g.item_vel[it]);
-            GradWs w;
-            carve_grad_ws(g.branch_base[b], f->ncomp, ch.N, ch.n_epochs, f->norb, &w);
-            rc = launch_grad(farm_lanes(f, g.g, b, pdl), f->ncomp, ch.N, zs, ch.fl, ch.sigma, f->mu, gp, w, g.flags + it,
-                             g.results + 4 * it, w.hyp, w.gz);
-            if (!rc) rc = launch_grad_chain(sb, f->ncomp, f->norb, ch, w, g.item_jac[it], g.flags + it,
-                                            g.grad + (size_t)it * np);
-            if (rc) break;
-        }
-        cudaEventRecord(g.g.events[b], sb);
-        cudaStreamWaitEvent(s0, g.g.events[b], 0);
-    }
-    return rc;
+    LAUNCH_CHECK();
+    return issue_branches(g, s0, [&](int b, cudaStream_t, int it) {
+        const psoap_chunk& ch = f->chunks[it % f->nchunks];
+        FactorWs ws;
+        carve_factor_ws(g.branch_base[b], padded_dim(ch.N), &ws, true);
+        return launch_chunk(farm_lanes(f, g, b, pdl), f->ncomp, ch.N, farm_z(ch, g.item_vel[it]), ch.fl, ch.sigma, f->mu,
+                            farm_gp(f, g, it), ws, g.flags + it, g.results + 4 * it);
+    });
+}
+
+// The gradient counterpart of farm_issue: velocities, sentinels and orbit Jacobians of every item, then per branch the
+// steps of psoap_chunk_lnprob_grad into the item's result and gradient rows.
+int farm_grad_issue(const psoap_farm* f, const FarmGrad& q, cudaStream_t s0, int pdl) {
+    const FarmGraph& g = q.g;
+    const int np = f->norb + 2 * f->ncomp;
+    orbit_farm_kernel<<<f->nitems, 64, 0, s0>>>(f->model, g.p_buf, g.descs);
+    LAUNCH_CHECK();
+    orbit_jacobian_farm_kernel<<<f->nitems, 64, 0, s0>>>(f->model, g.p_buf, q.jdescs);
+    LAUNCH_CHECK();
+    return issue_branches(g, s0, [&](int b, cudaStream_t sb, int it) {
+        const psoap_chunk& ch = f->chunks[it % f->nchunks];
+        GradWs w;
+        carve_grad_ws(g.branch_base[b], f->ncomp, ch.N, ch.n_epochs, f->norb, &w);
+        int rc = launch_grad(farm_lanes(f, g, b, pdl), f->ncomp, ch.N, farm_z(ch, g.item_vel[it]), ch.fl, ch.sigma, f->mu,
+                             farm_gp(f, g, it), w, g.flags + it, g.results + 4 * it, w.hyp, w.gz);
+        if (!rc) rc = launch_grad_chain(sb, f->ncomp, f->norb, ch, w, q.item_jac[it], g.flags + it, q.grad + (size_t)it * np);
+        return rc;
+    });
 }
 
 // Bordered dimensions of one prediction item: data block Nn (front-padded), border M = ncomp m, total Nt.
@@ -1387,57 +1346,43 @@ PredictDims predict_item_dims(int ncomp, int64_t N, int64_t m) {
     return {Nn, M, Nn + padded_dim(M)};
 }
 
-template <int NCOMP>
-void launch_predict_border_farm(cudaStream_t st, double* S, int64_t ld, const PredictFarmSrc& ps, const GpParams& gp,
-                                double* rvec, unsigned ntile) {
-    predict_border_farm_kernel<NCOMP><<<ntile, 256, 0, st>>>(S, ld, ps, gp, rvec);
-}
-
-// The prediction counterpart of farm_issue: velocities and sentinels of every item, then per branch, item after item in
-// LPT order, the steps of psoap_predict (mode 0) on the item's shifted pixels: data fill, border fill, elimination of
-// the data block, read-out into the item's offsets of delta and sigma.
-int farm_predict_issue(psoap_farm* f, cudaStream_t s0, int pdl, double* delta, double* sigma) {
-    FarmPredict& q = *f->pred;
-    const int nbranch = q.g.nbranch, nchunks = f->nchunks, ncomp = f->ncomp;
-    orbit_farm_kernel<<<f->nitems, 64, 0, s0>>>(f->model, q.p_buf, q.descs);
-    ++g_launches;
-    cudaEventRecord(q.g.events[nbranch], s0);
-    int rc = PSOAP_OK;
-    for (int b = 0; b < nbranch && rc == PSOAP_OK; ++b) {
-        cudaStream_t sb = q.g.streams[b];
-        cudaStreamWaitEvent(sb, q.g.events[nbranch], 0);
-        for (int it : q.branch_items[b]) {
-            const int ci = it % nchunks;
-            const psoap_chunk& ch = f->chunks[ci];
-            const PredictDims d = predict_item_dims(ncomp, ch.N, q.m[ci]);
-            const int Tn = (int)(d.Nn / NB), Tt = (int)(d.Nt / NB), pad = (int)(d.Nn - ch.N);
-            FactorWs ws;
-            carve_factor_ws(q.branch_base[b], d.Nt, &ws, true);
-            const GpParams gp = farm_gp(f, q.p_buf, it / nchunks);
-            const ZSource zs = farm_z(ch, q.item_vel[it]);
-            rc = launch_fill_lower(ncomp, sb, ws.W, d.Nt, Tn, pad, zs, ch.sigma, ch.fl, f->mu, gp, ws);
-            if (rc) break;
-            PredictFarmSrc ps;
-            for (int c = 0; c < 3; ++c) { ps.data[c] = nullptr; ps.pred[c] = c < ncomp ? q.grids[(size_t)ci * ncomp + c] : nullptr; }
-            ps.ncomp = ncomp; ps.mode = 0; ps.n = (int)ch.N; ps.m = (int)q.m[ci]; ps.M = (int)d.M;
-            ps.pad = pad; ps.Nn = (int)d.Nn; ps.Nt = (int)d.Nt; ps.nugget = 0.0; ps.zs = zs;
-            const unsigned ntile = (unsigned)((int64_t)Tt * (Tt + 1) / 2 - (int64_t)Tn * (Tn + 1) / 2);
-            if (ncomp == 1) launch_predict_border_farm<1>(sb, ws.W, d.Nt, ps, gp, ws.rvec, ntile);
-            else if (ncomp == 2) launch_predict_border_farm<2>(sb, ws.W, d.Nt, ps, gp, ws.rvec, ntile);
-            else launch_predict_border_farm<3>(sb, ws.W, d.Nt, ps, gp, ws.rvec, ntile);
-            LAUNCH_CHECK();
-            rc = launch_factor(farm_lanes(f, q.g, b, pdl), ws.W, d.Nt, Tn, Tt, pad, ws, q.flags + it, q.results + 4 * it);
-            if (rc) break;
-            const unsigned nb = (unsigned)((d.M + 31) / 32);
-            predict_farm_readout_kernel<<<dim3(q.sigma_mode ? 1u : nb, nb), 256, 0, sb>>>(
-                ws.W, d.Nt, (int)d.Nn, (int)d.M, ws.rvec, ws.info, q.flags + it, q.sigma_mode, sigma + q.sigma_off[it],
-                delta + q.delta_off[it]);
-            LAUNCH_CHECK();
-        }
-        cudaEventRecord(q.g.events[b], sb);
-        cudaStreamWaitEvent(s0, q.g.events[b], 0);
-    }
-    return rc;
+// The prediction counterpart of farm_issue: velocities and sentinels of every item, then per branch the steps of
+// psoap_predict (mode 0) on the item's shifted pixels: data fill, border fill, elimination of the data block, read-out
+// into the item's offsets of delta and sigma.
+int farm_predict_issue(const psoap_farm* f, const FarmPredict& q, cudaStream_t s0, int pdl, double* delta, double* sigma) {
+    const FarmGraph& g = q.g;
+    const int nchunks = f->nchunks, ncomp = f->ncomp;
+    orbit_farm_kernel<<<f->nitems, 64, 0, s0>>>(f->model, g.p_buf, g.descs);
+    LAUNCH_CHECK();
+    return issue_branches(g, s0, [&](int b, cudaStream_t sb, int it) {
+        const int ci = it % nchunks;
+        const psoap_chunk& ch = f->chunks[ci];
+        const PredictDims d = predict_item_dims(ncomp, ch.N, q.m[ci]);
+        const int Tn = (int)(d.Nn / NB), Tt = (int)(d.Nt / NB), pad = (int)(d.Nn - ch.N);
+        FactorWs ws;
+        carve_factor_ws(g.branch_base[b], d.Nt, &ws, true);
+        const GpParams gp = farm_gp(f, g, it);
+        const ZSource zs = farm_z(ch, g.item_vel[it]);
+        int rc = launch_fill_lower(ncomp, sb, ws.W, d.Nt, Tn, pad, zs, ch.sigma, ch.fl, f->mu, gp, ws);
+        if (rc) return rc;
+        PredictFarmSrc ps;
+        for (int c = 0; c < 3; ++c) { ps.data[c] = nullptr; ps.pred[c] = c < ncomp ? q.grids[(size_t)ci * ncomp + c] : nullptr; }
+        ps.ncomp = ncomp; ps.mode = 0; ps.n = (int)ch.N; ps.m = (int)q.m[ci]; ps.M = (int)d.M;
+        ps.pad = pad; ps.Nn = (int)d.Nn; ps.Nt = (int)d.Nt; ps.nugget = 0.0; ps.zs = zs;
+        const unsigned ntile = (unsigned)((int64_t)Tt * (Tt + 1) / 2 - (int64_t)Tn * (Tn + 1) / 2);
+        with_ncomp(ncomp, [&](auto nc) {
+            predict_border_farm_kernel<nc><<<ntile, 256, 0, sb>>>(ws.W, d.Nt, ps, gp, ws.rvec);
+        });
+        LAUNCH_CHECK();
+        rc = launch_factor(farm_lanes(f, g, b, pdl), ws.W, d.Nt, Tn, Tt, pad, ws, g.flags + it, g.results + 4 * it);
+        if (rc) return rc;
+        const unsigned nb = (unsigned)((d.M + 31) / 32);
+        predict_farm_readout_kernel<<<dim3(q.sigma_mode ? 1u : nb, nb), 256, 0, sb>>>(
+            ws.W, d.Nt, (int)d.Nn, (int)d.M, ws.rvec, ws.info, g.flags + it, q.sigma_mode, sigma + q.sigma_off[it],
+            delta + q.delta_off[it]);
+        LAUNCH_CHECK();
+        return PSOAP_OK;
+    });
 }
 
 // LPT (longest processing time first) assignment of work items (item = prop * nchunks + chunk) to branches by N^3;
@@ -1460,44 +1405,29 @@ std::vector<std::vector<int>> lpt_items(const std::vector<int64_t>& Ns, int nite
 }
 
 // Branch streams (+ the root stream at index nbranch), their events, and the high-priority side streams of look-ahead
-void create_farm_streams(FarmGraph& g) {
+int create_farm_streams(FarmGraph& g) {
     const int nbranch = g.nbranch;
     g.streams.resize(nbranch + 1);
     g.events.resize(nbranch + 1);
-    {
-        // Branch b carries the b-th largest items first (LPT order): its stream gets the matching priority level, which a
-        // captured kernel node inherits.  Measured neutral on a B200 against all-equal priorities (one rank's share of
-        // an 8-GPU run: 28.50 ms either way; a launch-attribute variant likewise): the drain at the end of an evaluation
-        // is not a matter of which chunk gets the free SM slots first.
-        int lo = 0, hi = 0;
-        cudaDeviceGetStreamPriorityRange(&lo, &hi);
-        const int nlev = lo - hi + 1;
-        for (int b = 0; b <= nbranch; ++b) {
-            // (a look-ahead farm's branch streams carry the bulk updates: lowest priority, below their side streams, where
-            // the chain links run; with both at the top C2 ran at 95.5 instead of 104 evals/s)
-            const int pr = (b < nbranch && nlev > 1 && !g.lookahead) ? hi + (int)((int64_t)b * nlev / nbranch) : lo;
-            cudaStreamCreateWithPriority(&g.streams[b], cudaStreamNonBlocking, pr);
-        }
-    }
-    for (auto& ev : g.events) cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
     g.side_streams.resize(nbranch);
     g.side_events.resize(2 * nbranch);
-    {
-        int lo = 0, hi = 0;
-        cudaDeviceGetStreamPriorityRange(&lo, &hi);
-        for (auto& s : g.side_streams) cudaStreamCreateWithPriority(&s, cudaStreamNonBlocking, hi);
-        for (auto& ev : g.side_events) cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
+    int lo = 0, hi = 0;
+    CUDA_TRY(cudaDeviceGetStreamPriorityRange(&lo, &hi));
+    // Branch b carries the b-th largest items first (LPT order): its stream gets the matching priority level, which a
+    // captured kernel node inherits.  Measured neutral on a B200 against all-equal priorities (one rank's share of
+    // an 8-GPU run: 28.50 ms either way; a launch-attribute variant likewise): the drain at the end of an evaluation
+    // is not a matter of which chunk gets the free SM slots first.
+    const int nlev = lo - hi + 1;
+    for (int b = 0; b <= nbranch; ++b) {
+        // (a look-ahead farm's branch streams carry the bulk updates: lowest priority, below their side streams, where
+        // the chain links run; with both at the top C2 ran at 95.5 instead of 104 evals/s)
+        const int pr = (b < nbranch && nlev > 1 && !g.lookahead) ? hi + (int)((int64_t)b * nlev / nbranch) : lo;
+        CUDA_TRY(cudaStreamCreateWithPriority(&g.streams[b], cudaStreamNonBlocking, pr));
     }
-}
-
-void destroy_farm_graph(FarmGraph& g) {
-    if (g.exec) cudaGraphExecDestroy(g.exec);
-    if (g.graph) cudaGraphDestroy(g.graph);
-    g.exec = nullptr; g.graph = nullptr;
-    for (auto& s : g.streams) if (s) cudaStreamDestroy(s);
-    for (auto& s : g.side_streams) if (s) cudaStreamDestroy(s);
-    for (auto& ev : g.events) if (ev) cudaEventDestroy(ev);
-    for (auto& ev : g.side_events) if (ev) cudaEventDestroy(ev);
+    for (auto& s : g.side_streams) CUDA_TRY(cudaStreamCreateWithPriority(&s, cudaStreamNonBlocking, hi));
+    for (auto& ev : g.events) CUDA_TRY(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+    for (auto& ev : g.side_events) CUDA_TRY(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+    return PSOAP_OK;
 }
 
 using FarmIssue = std::function<int(cudaStream_t s0, int pdl)>;
@@ -1520,9 +1450,48 @@ int capture_farm_graph(FarmGraph& g, const FarmIssue& issue) {
     return PSOAP_OK;
 }
 
-// One evaluation on the caller's stream st: the captured graph's replay, or (direct mode) the kernels issued on g's
-// own streams, forked from st and joined back into it.
-int run_farm_graph(FarmGraph& g, cudaStream_t st, const FarmIssue& issue) {
+// The setup of every farm graph once its workspace is carved: the orbit descriptors of its items, their LPT assignment
+// to the branches by `cost` (per chunk, cubed by lpt_items; 0: no work), look-ahead and direct issue, the streams, and
+// the capture.  On failure the caller deletes the graph's owner, which releases what was created.
+int attach_farm_graph(const psoap_farm* f, FarmGraph& g, const std::vector<int64_t>& cost, bool attached,
+                      const FarmIssue& issue) {
+    std::vector<OrbitDesc> hd(f->nitems);
+    for (int it = 0; it < f->nitems; ++it) {
+        const psoap_chunk& ch = f->chunks[it % f->nchunks];
+        hd[it] = {ch.dates, g.item_vel[it], g.flags + it, ch.n_epochs, (it / f->nchunks) * P_STRIDE};
+    }
+    CUDA_TRY(cudaMemcpy(g.descs, hd.data(), hd.size() * sizeof(OrbitDesc), cudaMemcpyHostToDevice));
+    g.branch_items = lpt_items(cost, f->nitems, g.nbranch);
+    int64_t nmax = 0;   // the largest chunk that takes work
+    for (int i = 0; i < f->nchunks; ++i)
+        if (cost[i] > 0) nmax = std::max(nmax, f->chunks[i].N);
+    // Look-ahead changes the panel groups of the elimination, hence its bits.  When the caller passes the chain links
+    // (psoap_chunk.reserved, chosen from the global problem: 7 for fewer than 8 (proposal, chunk) pairs in all), an
+    // attached graph (gradient, prediction) takes look-ahead exactly there, so that its outputs depend neither on the
+    // branch count nor on the number of GPUs; without that hint it decides by branch count.  The likelihood graph always
+    // decides by branch count: taking the hint there would change the likelihood's bits on some partitioned farms.
+    const char* la_env = getenv("PSOAP_FARM_LOOKAHEAD");
+    const bool hinted = attached && (f->chain_hint == 3 || f->chain_hint == 7);
+    g.lookahead = la_env ? (atoi(la_env) != 0) : hinted ? (f->chain_hint == 7) : (g.nbranch < 8);
+    // Graph replay removes every launch gap, which wins for short chains (N = 4000: 2.57 vs 2.75 ms); for a farm of
+    // a few LARGE chunks the directly issued pipeline is faster (N = 9000: 10.5 vs 11.3 ms: the side stream's
+    // priority and the pre-staged small grids do their job there).  PSOAP_FARM_DIRECT=0|1 overrides.
+    const char* de = getenv("PSOAP_FARM_DIRECT");
+    g.direct = de ? (atoi(de) != 0) : (g.lookahead && nmax >= 7000);
+    int rc = create_farm_streams(g);
+    if (rc) return rc;
+    return capture_farm_graph(g, issue);
+}
+
+// One evaluation of graph g at the parameters p_dev on the caller's stream st: the parameter upload, the captured
+// graph's replay or (direct mode) the kernels issued on g's own streams, forked from st and joined back into it, and
+// the copy of the result records.
+int run_farm_graph(const psoap_farm* f, FarmGraph& g, const double* p_dev, psoap_result* results_dev, cudaStream_t st,
+                   const FarmIssue& issue) {
+    const int np = f->norb + 2 * f->ncomp;
+    // p_dev: [nprop][np] contiguous -> [nprop][P_STRIDE]
+    CUDA_TRY(cudaMemcpy2DAsync(g.p_buf, P_STRIDE * 8, p_dev, (size_t)np * 8, (size_t)np * 8, f->nprop,
+                               cudaMemcpyDeviceToDevice, st));
     if (g.direct) {
         cudaStream_t s0 = g.streams[g.nbranch];
         cudaEvent_t fork = g.events[g.nbranch];
@@ -1536,130 +1505,92 @@ int run_farm_graph(FarmGraph& g, cudaStream_t st, const FarmIssue& issue) {
         CUDA_TRY(cudaGraphLaunch(g.exec, st));
         g_launches += g.launches;
     }
+    CUDA_TRY(cudaMemcpyAsync(results_dev, g.results, (size_t)f->nitems * sizeof(psoap_result), cudaMemcpyDeviceToDevice, st));
     return PSOAP_OK;
 }
 
-// Look-ahead and direct issue of a graph attached to a farm (gradient, prediction).  Look-ahead changes the panel
-// groups of the elimination, hence its bits.  When the caller passes the chain links (psoap_chunk.reserved, chosen from
-// the global problem: 7 for fewer than 8 (proposal, chunk) pairs in all), the attached graph takes look-ahead exactly
-// there, so that its outputs depend neither on the branch count nor on the number of GPUs; without that hint it decides
-// by branch count, as the likelihood graph does.
-void attached_graph_modes(const psoap_farm* f, FarmGraph& g, int64_t nmax) {
-    const char* la_env = getenv("PSOAP_FARM_LOOKAHEAD");
-    g.lookahead = la_env ? (atoi(la_env) != 0)
-                : (f->chain_hint == 3 || f->chain_hint == 7) ? (f->chain_hint == 7) : (g.nbranch < 8);
-    const char* de = getenv("PSOAP_FARM_DIRECT");
-    g.direct = de ? (atoi(de) != 0) : (g.lookahead && nmax >= 7000);
+// Bump allocation of 256-byte aligned pieces from base (null: offsets only, for the size queries)
+struct Carver {
+    char* base;
+    size_t off = 0;
+    char* take(size_t bytes) { char* r = base ? base + off : nullptr; off += align_up(bytes, 256); return r; }
+};
+
+// Layout of the part of a workspace every farm graph has: the parameter buffer, the result records, sentinels and orbit
+// descriptors of the items, vel_rows x n_epochs velocity doubles per item, then nbranch regions of branch_bytes.  The
+// graph's own buffers follow at c.off.
+void carve_farm_items(Carver& c, FarmGraph& g, int nprop, int nchunks, const int32_t* n_epochs, int vel_rows,
+                      size_t branch_bytes) {
+    const int nitems = nchunks * nprop;
+    g.p_buf = (double*)c.take((size_t)nprop * P_STRIDE * 8);
+    g.results = (double*)c.take((size_t)nitems * 4 * 8);
+    g.flags = (int*)c.take((size_t)nitems * 4);
+    g.descs = (OrbitDesc*)c.take((size_t)nitems * sizeof(OrbitDesc));
+    g.item_vel.resize(nitems);
+    for (int it = 0; it < nitems; ++it) g.item_vel[it] = (double*)c.take((size_t)vel_rows * n_epochs[it % nchunks] * 8);
+    g.branch_base.resize(g.nbranch);
+    for (auto& r : g.branch_base) r = c.take(branch_bytes);
 }
 
-// Layout of a gradient workspace (base null: sizes only): the per-item buffers, then nbranch GradWs regions sized for
-// the largest chunk and the most epochs (every GradWs buffer grows with N and with n_epochs, so an item's carve fits).
-size_t carve_farm_grad(const psoap_farm* f, int nbranch, char* base, FarmGrad* g) {
+// Layout of a likelihood workspace: each branch holds the FactorWs of the largest chunk.  The size query takes no
+// model, so every item reserves the velocity table of three components.
+size_t carve_farm_lnprob(char* base, FarmGraph& g, int nchunks, const int64_t* N, const int32_t* n_epochs, int nprop) {
+    int64_t nmax = 0;
+    for (int i = 0; i < nchunks; ++i) nmax = std::max(nmax, N[i]);
+    Carver c{base};
+    carve_farm_items(c, g, nprop, nchunks, n_epochs, 3, factor_ws_bytes(padded_dim(nmax)));
+    return c.off;
+}
+
+std::vector<int32_t> farm_epochs(const psoap_farm* f) {
+    std::vector<int32_t> nes;
+    for (const psoap_chunk& ch : f->chunks) nes.push_back(ch.n_epochs);
+    return nes;
+}
+
+// Layout of a gradient workspace: each branch holds a GradWs sized for the largest chunk and the most epochs (every
+// GradWs buffer grows with N and with n_epochs, so an item's carve fits), then the gradient rows, Jacobian descriptors
+// and Jacobians of the items.
+size_t carve_farm_grad(const psoap_farm* f, char* base, FarmGrad& q) {
     const int nitems = f->nitems, np = f->norb + 2 * f->ncomp;
-    size_t off = 0;
-    auto take = [&](size_t bytes) { char* r = base ? base + off : nullptr; off += align_up(bytes, 256); return r; };
-    char* p_buf = take((size_t)f->nprop * P_STRIDE * 8);
-    char* results = take((size_t)nitems * 4 * 8);
-    char* grad = take((size_t)nitems * np * 8);
-    char* flags = take((size_t)nitems * 4);
-    char* descs = take((size_t)nitems * sizeof(OrbitDesc));
-    char* jdescs = take((size_t)nitems * sizeof(JacDesc));
-    if (g) {
-        g->p_buf = (double*)p_buf; g->results = (double*)results; g->grad = (double*)grad; g->flags = (int*)flags;
-        g->descs = (OrbitDesc*)descs; g->jdescs = (JacDesc*)jdescs;
-        g->item_vel.resize(nitems); g->item_jac.resize(nitems); g->branch_base.resize(nbranch);
-    }
+    const std::vector<int32_t> nes = farm_epochs(f);
     int64_t nmax = 1;
     int nemax = 1;
-    for (int it = 0; it < nitems; ++it) {
-        const psoap_chunk& ch = f->chunks[it % f->nchunks];
-        nmax = std::max<int64_t>(nmax, ch.N);
-        nemax = std::max(nemax, (int)ch.n_epochs);
-        char* vel = take((size_t)f->ncomp * ch.n_epochs * 8);
-        char* jac = take((size_t)f->ncomp * ch.n_epochs * f->norb * 8);
-        if (g) { g->item_vel[it] = (double*)vel; g->item_jac[it] = (double*)jac; }
-    }
+    for (const psoap_chunk& ch : f->chunks) { nmax = std::max<int64_t>(nmax, ch.N); nemax = std::max(nemax, (int)ch.n_epochs); }
     GradWs probe;
-    const size_t per_branch = carve_grad_ws(nullptr, f->ncomp, nmax, nemax, f->norb, &probe);
-    for (int b = 0; b < nbranch; ++b) {
-        char* r = take(per_branch);
-        if (g) g->branch_base[b] = r;
-    }
-    return off;
+    Carver c{base};
+    carve_farm_items(c, q.g, f->nprop, f->nchunks, nes.data(), f->ncomp,
+                     carve_grad_ws(nullptr, f->ncomp, nmax, nemax, f->norb, &probe));
+    q.grad = (double*)c.take((size_t)nitems * np * 8);
+    q.jdescs = (JacDesc*)c.take((size_t)nitems * sizeof(JacDesc));
+    q.item_jac.resize(nitems);
+    for (int it = 0; it < nitems; ++it) q.item_jac[it] = (double*)c.take((size_t)f->ncomp * nes[it % f->nchunks] * f->norb * 8);
+    return c.off;
 }
 
-void destroy_farm_grad(FarmGrad* g) {
-    if (!g) return;
-    destroy_farm_graph(g->g);
-    delete g;
-}
-
-// Layout of a prediction workspace (base null: sizes only): the per-item buffers, the graph's scratch outputs, then
-// nbranch regions of factor_ws_bytes(Nt) for the largest bordered item (S first, then its FactorWs).
-size_t carve_farm_predict(const psoap_farm* f, int nbranch, const int64_t* m, int sigma_mode, char* base, FarmPredict* q) {
+// Layout of a prediction workspace: each branch holds factor_ws_bytes(Nt) for the largest bordered item, then the
+// graph's scratch outputs.  Also sets the output offsets of the items.
+size_t carve_farm_predict(const psoap_farm* f, const int64_t* m, int sigma_mode, char* base, FarmPredict& q) {
     const int nitems = f->nitems, nchunks = f->nchunks;
-    size_t off = 0;
-    auto take = [&](size_t bytes) { char* r = base ? base + off : nullptr; off += align_up(bytes, 256); return r; };
-    char* p_buf = take((size_t)f->nprop * P_STRIDE * 8);
-    char* results = take((size_t)nitems * 4 * 8);
-    char* flags = take((size_t)nitems * 4);
-    char* descs = take((size_t)nitems * sizeof(OrbitDesc));
     // output layout: chunk after chunk, each chunk's proposals side by side, so that a chunk's outputs are contiguous
-    std::vector<int64_t> doff(nitems + 1), soff(nitems + 1);
+    q.delta_off.resize(nitems + 1);
+    q.sigma_off.resize(nitems + 1);
     int64_t nd = 0, ns = 0, ntmax = 0;
     for (int ci = 0; ci < nchunks; ++ci) {
         const PredictDims d = predict_item_dims(f->ncomp, f->chunks[ci].N, m[ci]);
         if (m[ci] > 0) ntmax = std::max(ntmax, d.Nt);
         for (int k = 0; k < f->nprop; ++k) {
             const int it = k * nchunks + ci;
-            doff[it] = nd; soff[it] = ns;
+            q.delta_off[it] = nd; q.sigma_off[it] = ns;
             nd += d.M; ns += sigma_mode ? d.M : d.M * d.M;
         }
     }
-    doff[nitems] = nd; soff[nitems] = ns;
-    char* cap_delta = take((size_t)nd * 8);
-    char* cap_sigma = take((size_t)ns * 8);
-    if (q) {
-        q->p_buf = (double*)p_buf; q->results = (double*)results; q->flags = (int*)flags; q->descs = (OrbitDesc*)descs;
-        q->cap_delta = (double*)cap_delta; q->cap_sigma = (double*)cap_sigma;
-        q->delta_off = doff; q->sigma_off = soff;
-        q->item_vel.resize(nitems); q->branch_base.resize(nbranch);
-    }
-    for (int it = 0; it < nitems; ++it) {
-        char* vel = take((size_t)f->ncomp * f->chunks[it % nchunks].n_epochs * 8);
-        if (q) q->item_vel[it] = (double*)vel;
-    }
-    const size_t per_branch = ntmax ? factor_ws_bytes(ntmax) : 0;
-    for (int b = 0; b < nbranch; ++b) {
-        char* r = take(per_branch);
-        if (q) q->branch_base[b] = r;
-    }
-    return off;
-}
-
-void destroy_farm_predict(FarmPredict* q) {
-    if (!q) return;
-    destroy_farm_graph(q->g);
-    delete q;
-}
-}  // namespace
-
-namespace {
-// item = prop * nchunks + chunk
-size_t farm_small_bytes(int nchunks, int nprop, const int32_t* n_epochs, std::vector<size_t>* vel_off) {
-    const size_t nitems = (size_t)nchunks * nprop;
-    size_t b = 0;
-    b += align_up((size_t)nprop * P_STRIDE * 8, 256);  // p_buf
-    b += align_up(nitems * 4 * 8, 256);                // results
-    b += align_up(nitems * 4, 256);                    // flags
-    b += align_up(nitems * sizeof(OrbitDesc), 256);
-    size_t v = 0;
-    for (int k = 0; k < nprop; ++k)
-        for (int i = 0; i < nchunks; ++i) {
-            if (vel_off) vel_off->push_back(v);
-            v += align_up((size_t)3 * n_epochs[i] * 8, 256);
-        }
-    return b + v;
+    q.delta_off[nitems] = nd; q.sigma_off[nitems] = ns;
+    Carver c{base};
+    carve_farm_items(c, q.g, f->nprop, nchunks, farm_epochs(f).data(), f->ncomp, ntmax ? factor_ws_bytes(ntmax) : 0);
+    q.cap_delta = (double*)c.take((size_t)nd * 8);
+    q.cap_sigma = (double*)c.take((size_t)ns * 8);
+    return c.off;
 }
 }  // namespace
 
@@ -1668,10 +1599,9 @@ extern "C" {
 size_t psoap_farm_workspace_bytes_batched(int nchunks, const int64_t* N, const int32_t* n_epochs, int nprop,
                                           int nbranch) {
     if (nchunks < 1 || nprop < 1 || !N || !n_epochs) return 0;
-    nbranch = std::max(1, std::min(nbranch, nchunks * nprop));
-    int64_t nmax = 0;
-    for (int i = 0; i < nchunks; ++i) nmax = std::max(nmax, N[i]);
-    return farm_small_bytes(nchunks, nprop, n_epochs, nullptr) + (size_t)nbranch * factor_ws_bytes(padded_dim(nmax));
+    FarmGraph probe;
+    probe.nbranch = std::max(1, std::min(nbranch, nchunks * nprop));
+    return carve_farm_lnprob(nullptr, probe, nchunks, N, n_epochs, nprop);
 }
 size_t psoap_farm_workspace_bytes(int nchunks, const int64_t* N, const int32_t* n_epochs, int nbranch) {
     return psoap_farm_workspace_bytes_batched(nchunks, N, n_epochs, 1, nbranch);
@@ -1703,50 +1633,9 @@ int psoap_farm_create_batched(psoap_farm** out, int model, int nchunks, const ps
     f->chunks.assign(chunks, chunks + nchunks);
     f->chain_hint = chunks[0].reserved & 0xff;
     f->group_hint = (chunks[0].reserved >> 8) & 0xff;
-    char* p = (char*)workspace;
-    auto take = [&](size_t bytes) { char* r = p; p += align_up(bytes, 256); return r; };
-    f->p_buf = (double*)take((size_t)nprop * P_STRIDE * 8);
-    f->results = (double*)take((size_t)nitems * 4 * 8);
-    f->flags = (int*)take((size_t)nitems * 4);
-    f->descs = (OrbitDesc*)take((size_t)nitems * sizeof(OrbitDesc));
-    const size_t small = farm_small_bytes(nchunks, nprop, nes.data(), &f->vel_off);
-    f->vel = (double*)p;
-    p = (char*)workspace + small;
-    int64_t nmax = *std::max_element(Ns.begin(), Ns.end());
-    const size_t per_branch = factor_ws_bytes(padded_dim(nmax));
-    f->branch_ws.resize(nbranch);
-    for (int b = 0; b < nbranch; ++b) carve_factor_ws(p + (size_t)b * per_branch, padded_dim(nmax), &f->branch_ws[b], true);
-
-    // orbit descriptors, one per (proposal, chunk)
-    std::vector<OrbitDesc> hd(nitems);
-    for (int it = 0; it < nitems; ++it) {
-        const int ci = it % nchunks, k = it / nchunks;
-        hd[it].dates = chunks[ci].dates;
-        hd[it].vel = (double*)((char*)f->vel + f->vel_off[it]);
-        hd[it].flag = f->flags + it;
-        hd[it].n_epochs = chunks[ci].n_epochs;
-        hd[it].p_off = k * P_STRIDE;
-    }
-    cudaError_t e = cudaMemcpy(f->descs, hd.data(), (size_t)nitems * sizeof(OrbitDesc), cudaMemcpyHostToDevice);
-    if (e != cudaSuccess) { delete f; return fail(PSOAP_ERR_CUDA, std::string("farm descs: ") + cudaGetErrorString(e)); }
-
-    f->branch_items = lpt_items(Ns, nitems, nbranch);
-
-    const char* la_env = getenv("PSOAP_FARM_LOOKAHEAD");
-    f->g.lookahead = la_env ? (atoi(la_env) != 0) : (nbranch < 8);
-    // capture the whole evaluation into one CUDA graph
-    create_farm_streams(f->g);
-    f->item_vel.resize(nitems);
-    for (int it = 0; it < nitems; ++it) f->item_vel[it] = hd[it].vel;
-    // Graph replay removes every launch gap, which wins for short chains (N = 4000: 2.57 vs 2.75 ms); for a farm of
-    // a few LARGE chunks the directly issued pipeline is faster (N = 9000: 10.5 vs 11.3 ms: the side stream's
-    // priority and the pre-staged small grids do their job there).  PSOAP_FARM_DIRECT=0|1 overrides.
-    {
-        const char* de = getenv("PSOAP_FARM_DIRECT");
-        f->g.direct = de ? (atoi(de) != 0) : (f->g.lookahead && nmax >= 7000);
-    }
-    rc = capture_farm_graph(f->g, [f](cudaStream_t s0, int pdl) { return farm_issue(f, s0, pdl); });
-    if (rc != PSOAP_OK) { psoap_farm_destroy(f); return rc; }
+    carve_farm_lnprob((char*)workspace, f->g, nchunks, Ns.data(), nes.data(), nprop);
+    rc = attach_farm_graph(f, f->g, Ns, false, [f](cudaStream_t s0, int pdl) { return farm_issue(f, s0, pdl); });
+    if (rc != PSOAP_OK) { delete f; return rc; }
     *out = f;
     return PSOAP_OK;
 }
@@ -1758,24 +1647,13 @@ int psoap_farm_create(psoap_farm** out, int model, int nchunks, const psoap_chun
 
 int psoap_farm_lnprob(psoap_farm* f, const double* p_dev, psoap_result* results_dev, void* stream) {
     if (!f || !p_dev || !results_dev) return fail(PSOAP_ERR_ARG, "psoap_farm_lnprob: bad arguments");
-    cudaStream_t st = (cudaStream_t)stream;
-    const int np = f->norb + 2 * f->ncomp;
-    // p_dev: [nprop][np] contiguous -> [nprop][P_STRIDE]
-    CUDA_TRY(cudaMemcpy2DAsync(f->p_buf, P_STRIDE * 8, p_dev, (size_t)np * 8, (size_t)np * 8, f->nprop,
-                               cudaMemcpyDeviceToDevice, st));
-    int rc = run_farm_graph(f->g, st, [f](cudaStream_t s0, int pdl) { return farm_issue(f, s0, pdl); });
-    if (rc) return rc;
-    CUDA_TRY(cudaMemcpyAsync(results_dev, f->results, (size_t)f->nitems * sizeof(psoap_result), cudaMemcpyDeviceToDevice, st));
-    return PSOAP_OK;
+    return run_farm_graph(f, f->g, p_dev, results_dev, (cudaStream_t)stream,
+                          [f](cudaStream_t s0, int pdl) { return farm_issue(f, s0, pdl); });
 }
 
 int psoap_farm_launches_per_eval(const psoap_farm* f) { return f ? f->g.launches : 0; }
 
 int psoap_farm_destroy(psoap_farm* f) {
-    if (!f) return PSOAP_OK;
-    destroy_farm_graph(f->g);
-    destroy_farm_grad(f->grad);
-    destroy_farm_predict(f->pred);
     delete f;
     return PSOAP_OK;
 }
@@ -1783,7 +1661,9 @@ int psoap_farm_destroy(psoap_farm* f) {
 // ---- gradient graph of a farm -----------------------------------------------------------------------------------
 size_t psoap_farm_grad_workspace_bytes(const psoap_farm* f, int nbranch) {
     if (!f || nbranch < 1) return 0;
-    return carve_farm_grad(f, std::min(nbranch, f->nitems), nullptr, nullptr);
+    FarmGrad probe;
+    probe.g.nbranch = std::min(nbranch, f->nitems);
+    return carve_farm_grad(f, nullptr, probe);
 }
 
 int psoap_farm_grad_attach(psoap_farm* f, int nbranch, void* workspace, size_t workspace_bytes) {
@@ -1794,47 +1674,35 @@ int psoap_farm_grad_attach(psoap_farm* f, int nbranch, void* workspace, size_t w
         return fail(PSOAP_ERR_WORKSPACE, "psoap_farm_grad_attach: workspace too small or not 256-byte aligned");
     int rc = set_kernel_attributes();
     if (rc) return rc;
-    FarmGrad* g = new FarmGrad();
-    g->g.nbranch = nbranch;
-    carve_farm_grad(f, nbranch, (char*)workspace, g);
-    const int nitems = f->nitems, nchunks = f->nchunks;
-    std::vector<OrbitDesc> hd(nitems);
-    std::vector<JacDesc> hj(nitems);
-    std::vector<int64_t> Ns(nchunks);
-    int64_t nmax = 0;
-    for (int i = 0; i < nchunks; ++i) { Ns[i] = f->chunks[i].N; nmax = std::max(nmax, Ns[i]); }
-    for (int it = 0; it < nitems; ++it) {
-        const psoap_chunk& ch = f->chunks[it % nchunks];
-        const int k = it / nchunks;
-        hd[it].dates = ch.dates; hd[it].vel = g->item_vel[it]; hd[it].flag = g->flags + it;
-        hd[it].n_epochs = ch.n_epochs; hd[it].p_off = k * P_STRIDE;
-        hj[it].dates = ch.dates; hj[it].jac = g->item_jac[it]; hj[it].n_epochs = ch.n_epochs; hj[it].p_off = k * P_STRIDE;
+    FarmGrad* q = new FarmGrad();
+    q->g.nbranch = nbranch;
+    carve_farm_grad(f, (char*)workspace, *q);
+    std::vector<JacDesc> hj(f->nitems);
+    std::vector<int64_t> Ns;
+    for (const psoap_chunk& ch : f->chunks) Ns.push_back(ch.N);
+    for (int it = 0; it < f->nitems; ++it) {
+        const psoap_chunk& ch = f->chunks[it % f->nchunks];
+        hj[it] = {ch.dates, q->item_jac[it], ch.n_epochs, (it / f->nchunks) * P_STRIDE};
     }
-    cudaError_t e = cudaMemcpy(g->descs, hd.data(), (size_t)nitems * sizeof(OrbitDesc), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaMemcpy(g->jdescs, hj.data(), (size_t)nitems * sizeof(JacDesc), cudaMemcpyHostToDevice);
-    if (e != cudaSuccess) { delete g; return fail(PSOAP_ERR_CUDA, std::string("farm grad descs: ") + cudaGetErrorString(e)); }
-    g->branch_items = lpt_items(Ns, nitems, nbranch);
-    attached_graph_modes(f, g->g, nmax);
-    create_farm_streams(g->g);
-    f->grad = g;
-    rc = capture_farm_graph(g->g, [f](cudaStream_t s0, int pdl) { return farm_grad_issue(f, s0, pdl); });
-    if (rc != PSOAP_OK) { destroy_farm_grad(g); f->grad = nullptr; }
-    return rc;
+    cudaError_t e = cudaMemcpy(q->jdescs, hj.data(), hj.size() * sizeof(JacDesc), cudaMemcpyHostToDevice);
+    rc = e != cudaSuccess ? fail(PSOAP_ERR_CUDA, std::string("farm grad descs: ") + cudaGetErrorString(e))
+                          : attach_farm_graph(f, q->g, Ns, true,
+                                              [f, q](cudaStream_t s0, int pdl) { return farm_grad_issue(f, *q, s0, pdl); });
+    if (rc != PSOAP_OK) { delete q; return rc; }
+    f->grad = q;
+    return PSOAP_OK;
 }
 
 int psoap_farm_lnprob_grad(psoap_farm* f, const double* p_dev, psoap_result* results_dev, double* grad_dev,
                            void* stream) {
     if (!f || !p_dev || !results_dev || !grad_dev) return fail(PSOAP_ERR_ARG, "psoap_farm_lnprob_grad: bad arguments");
     if (!f->grad) return fail(PSOAP_ERR_ARG, "psoap_farm_lnprob_grad: no gradient graph (psoap_farm_grad_attach first)");
-    FarmGrad& g = *f->grad;
+    FarmGrad& q = *f->grad;
     cudaStream_t st = (cudaStream_t)stream;
-    const int np = f->norb + 2 * f->ncomp;
-    CUDA_TRY(cudaMemcpy2DAsync(g.p_buf, P_STRIDE * 8, p_dev, (size_t)np * 8, (size_t)np * 8, f->nprop,
-                               cudaMemcpyDeviceToDevice, st));
-    int rc = run_farm_graph(g.g, st, [f](cudaStream_t s0, int pdl) { return farm_grad_issue(f, s0, pdl); });
+    int rc = run_farm_graph(f, q.g, p_dev, results_dev, st,
+                            [f, &q](cudaStream_t s0, int pdl) { return farm_grad_issue(f, q, s0, pdl); });
     if (rc) return rc;
-    CUDA_TRY(cudaMemcpyAsync(results_dev, g.results, (size_t)f->nitems * sizeof(psoap_result), cudaMemcpyDeviceToDevice, st));
-    CUDA_TRY(cudaMemcpyAsync(grad_dev, g.grad, (size_t)f->nitems * np * 8, cudaMemcpyDeviceToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(grad_dev, q.grad, (size_t)f->nitems * (f->norb + 2 * f->ncomp) * 8, cudaMemcpyDeviceToDevice, st));
     return PSOAP_OK;
 }
 
@@ -1851,7 +1719,9 @@ bool predict_args_ok(const psoap_farm* f, int nbranch, const int64_t* m, int sig
 
 size_t psoap_farm_predict_workspace_bytes(const psoap_farm* f, int nbranch, const int64_t* m, int sigma_mode) {
     if (!predict_args_ok(f, nbranch, m, sigma_mode)) return 0;
-    return carve_farm_predict(f, std::min(nbranch, f->nitems), m, sigma_mode, nullptr, nullptr);
+    FarmPredict probe;
+    probe.g.nbranch = std::min(nbranch, f->nitems);
+    return carve_farm_predict(f, m, sigma_mode, nullptr, probe);
 }
 
 int psoap_farm_predict_attach(psoap_farm* f, int nbranch, const int64_t* m, const double* const* grids, int sigma_mode,
@@ -1868,38 +1738,24 @@ int psoap_farm_predict_attach(psoap_farm* f, int nbranch, const int64_t* m, cons
         return fail(PSOAP_ERR_WORKSPACE, "psoap_farm_predict_attach: workspace too small or not 256-byte aligned");
     int rc = set_kernel_attributes();
     if (rc) return rc;
+    const int nitems = f->nitems, nchunks = f->nchunks;
     FarmPredict* q = new FarmPredict();
     q->g.nbranch = nbranch;
     q->sigma_mode = sigma_mode;
-    const int nitems = f->nitems, nchunks = f->nchunks;
     q->m.assign(m, m + nchunks);
     q->grids.assign(grids, grids + (size_t)nchunks * f->ncomp);
-    carve_farm_predict(f, nbranch, m, sigma_mode, (char*)workspace, q);
-    std::vector<OrbitDesc> hd(nitems);
+    carve_farm_predict(f, m, sigma_mode, (char*)workspace, *q);
     // the LPT weight of an item is its bordered dimension Nt (cubed by lpt_items); items of chunks with m = 0 take no work
     std::vector<int64_t> cost(nchunks);
-    int64_t nmax = 0;
-    for (int i = 0; i < nchunks; ++i) {
-        cost[i] = m[i] > 0 ? predict_item_dims(f->ncomp, f->chunks[i].N, m[i]).Nt : 0;
-        if (m[i] > 0) nmax = std::max(nmax, (int64_t)f->chunks[i].N);
-    }
-    for (int it = 0; it < nitems; ++it) {
-        const psoap_chunk& ch = f->chunks[it % nchunks];
-        hd[it].dates = ch.dates; hd[it].vel = q->item_vel[it]; hd[it].flag = q->flags + it;
-        hd[it].n_epochs = ch.n_epochs; hd[it].p_off = (it / nchunks) * P_STRIDE;
-    }
-    cudaError_t e = cudaMemcpy(q->descs, hd.data(), (size_t)nitems * sizeof(OrbitDesc), cudaMemcpyHostToDevice);
+    for (int i = 0; i < nchunks; ++i) cost[i] = m[i] > 0 ? predict_item_dims(f->ncomp, f->chunks[i].N, m[i]).Nt : 0;
     // the records of items with m = 0 are never written by the graph: they read 0 (lnlike, logdet, quad, info)
-    if (e == cudaSuccess) e = cudaMemset(q->results, 0, (size_t)nitems * 4 * 8);
-    if (e != cudaSuccess) { delete q; return fail(PSOAP_ERR_CUDA, std::string("farm predict descs: ") + cudaGetErrorString(e)); }
-    q->branch_items = lpt_items(cost, nitems, nbranch);
-    attached_graph_modes(f, q->g, nmax);
-    create_farm_streams(q->g);
+    cudaError_t e = cudaMemset(q->g.results, 0, (size_t)nitems * 4 * 8);
+    rc = e != cudaSuccess ? fail(PSOAP_ERR_CUDA, std::string("farm predict results: ") + cudaGetErrorString(e))
+                          : attach_farm_graph(f, q->g, cost, true, [f, q](cudaStream_t s0, int pdl) {
+                                return farm_predict_issue(f, *q, s0, pdl, q->cap_delta, q->cap_sigma);
+                            });
+    if (rc != PSOAP_OK) { delete q; return rc; }
     f->pred = q;
-    rc = capture_farm_graph(q->g, [f, q](cudaStream_t s0, int pdl) {
-        return farm_predict_issue(f, s0, pdl, q->cap_delta, q->cap_sigma);
-    });
-    if (rc != PSOAP_OK) { destroy_farm_predict(q); f->pred = nullptr; return rc; }
     std::copy(q->delta_off.begin(), q->delta_off.end(), offsets_out);
     std::copy(q->sigma_off.begin(), q->sigma_off.end(), offsets_out + nitems + 1);
     return PSOAP_OK;
@@ -1912,19 +1768,15 @@ int psoap_farm_predict(psoap_farm* f, const double* p_dev, double* delta_dev, do
     if (!f->pred) return fail(PSOAP_ERR_ARG, "psoap_farm_predict: no prediction graph (psoap_farm_predict_attach first)");
     FarmPredict& q = *f->pred;
     cudaStream_t st = (cudaStream_t)stream;
-    const int np = f->norb + 2 * f->ncomp;
-    CUDA_TRY(cudaMemcpy2DAsync(q.p_buf, P_STRIDE * 8, p_dev, (size_t)np * 8, (size_t)np * 8, f->nprop,
-                               cudaMemcpyDeviceToDevice, st));
     // direct issue writes into the caller's buffers; the captured graph into its own, copied out after the replay
-    int rc = run_farm_graph(q.g, st, [f, delta_dev, sigma_dev](cudaStream_t s0, int pdl) {
-        return farm_predict_issue(f, s0, pdl, delta_dev, sigma_dev);
+    int rc = run_farm_graph(f, q.g, p_dev, results_dev, st, [f, &q, delta_dev, sigma_dev](cudaStream_t s0, int pdl) {
+        return farm_predict_issue(f, q, s0, pdl, delta_dev, sigma_dev);
     });
     if (rc) return rc;
     if (!q.g.direct) {
         CUDA_TRY(cudaMemcpyAsync(delta_dev, q.cap_delta, (size_t)q.delta_off[f->nitems] * 8, cudaMemcpyDeviceToDevice, st));
         CUDA_TRY(cudaMemcpyAsync(sigma_dev, q.cap_sigma, (size_t)q.sigma_off[f->nitems] * 8, cudaMemcpyDeviceToDevice, st));
     }
-    CUDA_TRY(cudaMemcpyAsync(results_dev, q.results, (size_t)f->nitems * sizeof(psoap_result), cudaMemcpyDeviceToDevice, st));
     return PSOAP_OK;
 }
 
