@@ -39,6 +39,12 @@ extern "C" {
 #define PSOAP_ST1 3
 #define PSOAP_ST2 4
 #define PSOAP_ST3 5
+/* free per-epoch velocities of 1, 2 or 3 components, no orbit: the vector is [v_0[0..n), .., v_{ncomp-1}[0..n), amp_f, l_f,
+ * (amp_g, l_g, (amp_h, l_h))] in km/s, n the chunk's own epochs (chunk entries) or the farm's Ng global epochs
+ * (psoap_farm_create_free).  Adding one constant to all of a component's velocities leaves the likelihood unchanged. */
+#define PSOAP_FREE1 6
+#define PSOAP_FREE2 7
+#define PSOAP_FREE3 8
 
 /* Result record written (on the device) by psoap_lnlike and, per chunk, by the farm. */
 typedef struct {
@@ -98,8 +104,8 @@ int psoap_replicate_wls(double *out_dev, const double *lwl_dev, const int32_t *e
  * vel_dev: [ncomp, n_epochs].  flag_dev (may be NULL): set to 1 if any |v| >= c_kms (sample_parallel.py:186). */
 int psoap_orbit_velocities(int model, const double *p_orb_dev, const double *dates_dev, int n_epochs,
                            double *vel_dev, int *flag_dev, void *stream);
-int psoap_model_ncomp(int model);
-int psoap_model_norb(int model);
+int psoap_model_ncomp(int model);   /* also for PSOAP_FREE1..3 */
+int psoap_model_norb(int model);    /* 0 for the free models (they have no orbit) */
 
 /* ---- likelihood: psoap/covariance.py:299-376 --------------------------------------------------------- */
 size_t psoap_lnlike_workspace_bytes(int64_t N);
@@ -179,6 +185,8 @@ int psoap_lnlike_grad_views(void *workspace_dev, int64_t N, double **neg_kinv_de
  * elimination, the contraction, the per-epoch sum and the orbit Jacobian.  grad_p_dev [norb + 2 ncomp]; NaN when
  * lnlike is -inf (|v| >= c, a negative GP hyper-parameter, info != 0).  chunk->reserved is ignored (the direct API's
  * launch choices apply).  workspace_dev: >= psoap_chunk_lnprob_grad_workspace_bytes(model, N, n_epochs) bytes. */
+/* PSOAP_FREE1..3: p_dev and grad_p_dev are [ncomp n_epochs + 2 ncomp], the chunk's own velocities then GP; the velocity
+ * entries of grad_p_dev are the per-epoch sums d lnlike / d v_c[e] (no Jacobian). */
 size_t psoap_chunk_lnprob_grad_workspace_bytes(int model, int64_t N, int32_t n_epochs);
 int psoap_chunk_lnprob_grad(int model, const psoap_chunk *chunk, const double *p_dev, double mu_GP, void *workspace_dev,
                             size_t workspace_bytes, psoap_result *result_dev, double *grad_p_dev, void *stream);
@@ -194,6 +202,8 @@ int psoap_orbit_jacobian(int model, const double *p_orb_dev, const double *dates
  * Bit-reproducible: no floating-point atomics.  workspace_dev: >= psoap_chunk_fisher_workspace_bytes(model, N,
  * n_epochs) bytes, 256-byte aligned: the gradient's identity-bordered matrix plus one N x N product per parameter,
  * about (4 + n_params) 8 N^2 bytes. */
+/* PSOAP_FREE1..3: n_params = ncomp n_epochs + 2 ncomp (the chunk's own velocities, then GP), workspace still about
+ * (4 + n_params) 8 N^2 bytes; a component's velocity block has zero row sums up to rounding (the gauge). */
 size_t psoap_chunk_fisher_workspace_bytes(int model, int64_t N, int32_t n_epochs);
 int psoap_chunk_fisher(int model, const psoap_chunk *chunk, const double *p_dev, double mu_GP, void *workspace_dev,
                        size_t workspace_bytes, psoap_result *result_dev, double *grad_p_dev, double *fisher_dev,
@@ -222,6 +232,19 @@ size_t psoap_farm_workspace_bytes_batched(int nchunks, const int64_t *N, const i
                                           int nbranch);
 int psoap_farm_create_batched(psoap_farm **farm, int model, int nchunks, const psoap_chunk *chunks, int nprop,
                               int nbranch, double mu_GP, void *workspace_dev, size_t workspace_bytes);
+/* A farm with free per-epoch velocities (PSOAP_FREE1..3 layout) over Ng global epochs.  epoch_map_dev: HOST array of
+ * nchunks DEVICE pointers, chunk i's map int32 [chunks[i].n_epochs] from its local epoch to its global epoch in [0, Ng),
+ * no global epoch twice in a chunk (checked here); the maps stay valid for the farm's life.  The result is an ordinary
+ * farm: psoap_farm_lnprob, psoap_farm_grad_attach / psoap_farm_lnprob_grad and psoap_farm_predict_attach /
+ * psoap_farm_predict work on it unchanged, with p_dev [nprop][ncomp Ng + 2 ncomp] and gradient rows of that length.  An
+ * item's velocity table is gathered as v_c[map[e]] (sentinel as the orbit's: |v| >= c_kms or a negative GP value gives
+ * -inf and NaN for that item only); its gradient row holds d lnlike / d v_c[e] at c Ng + map[e] and exactly 0 at the
+ * global epochs the chunk does not observe. */
+size_t psoap_farm_free_workspace_bytes(int ncomp, int Ng, int nchunks, const int64_t *N, const int32_t *n_epochs,
+                                       int nprop, int nbranch);
+int psoap_farm_create_free(psoap_farm **farm, int ncomp, int Ng, int nchunks, const psoap_chunk *chunks,
+                           const int32_t *const *epoch_map_dev, int nprop, int nbranch, double mu_GP,
+                           void *workspace_dev, size_t workspace_bytes);
 int psoap_farm_launches_per_eval(const psoap_farm *farm);
 /* Frees the farm's streams, events and graph, and its gradient and prediction graphs when attached (not the workspaces). */
 int psoap_farm_destroy(psoap_farm *farm);

@@ -20,6 +20,7 @@ vp = ctypes.c_void_p
 MODELS = {"SB1": 1, "SB2": 2, "ST1": 3, "ST2": 4, "ST3": 5}
 NCOMP = {"SB1": 1, "SB2": 2, "ST1": 1, "ST2": 2, "ST3": 3}
 N_ORB = {"SB1": 6, "SB2": 7, "ST1": 11, "ST2": 12, "ST3": 13}  # psoap/utils.py:14
+FREE_MODELS = {1: 6, 2: 7, 3: 8}  # ncomp -> PSOAP_FREE1..3 (per-epoch velocities, no orbit)
 
 
 class PsoapResult(ctypes.Structure):
@@ -89,6 +90,11 @@ SIGNATURES = {
     "psoap_farm_create_batched": (ctypes.c_int, [ctypes.POINTER(vp), ctypes.c_int, ctypes.c_int,
                                                  ctypes.POINTER(PsoapChunk), ctypes.c_int, ctypes.c_int,
                                                  ctypes.c_double, vp, ctypes.c_size_t]),
+    "psoap_farm_free_workspace_bytes": (ctypes.c_size_t, [ctypes.c_int, ctypes.c_int, ctypes.c_int, c_i64_p, c_i32_p,
+                                                          ctypes.c_int, ctypes.c_int]),
+    "psoap_farm_create_free": (ctypes.c_int, [ctypes.POINTER(vp), ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                              ctypes.POINTER(PsoapChunk), ctypes.POINTER(vp), ctypes.c_int, ctypes.c_int,
+                                              ctypes.c_double, vp, ctypes.c_size_t]),
     "psoap_farm_lnprob": (ctypes.c_int, [vp, vp, vp, vp]),
     "psoap_farm_launches_per_eval": (ctypes.c_int, [vp]),
     "psoap_farm_destroy": (ctypes.c_int, [vp]),

@@ -518,6 +518,13 @@ ZSource farm_z(const psoap_chunk& ch, const double* vel) {
     return zs;
 }
 
+// Model ids of the chunk entries: an orbit (PSOAP_SB1 .. PSOAP_ST3) or free per-epoch velocities (PSOAP_FREE1 .. 3).
+// nvel: the parameters before the GP block of one chunk, the orbit's or the chunk's own ncomp n_epochs velocities.
+bool model_valid(int m) { return m >= PSOAP_SB1 && m <= PSOAP_FREE3; }
+bool model_free(int m) { return m >= PSOAP_FREE1 && m <= PSOAP_FREE3; }
+int dims_ncomp(int m) { return model_free(m) ? m - PSOAP_FREE1 + 1 : model_ncomp(m); }
+int dims_nvel(int m, int n_epochs) { return model_free(m) ? dims_ncomp(m) * n_epochs : model_norb(m); }
+
 }  // namespace
 
 // ======================================================================================================
@@ -531,7 +538,7 @@ int psoap_device_count(void) {
     return n;
 }
 int64_t psoap_launch_count(void) { return g_launches.load(); }
-int psoap_model_ncomp(int model) { return (model >= 1 && model <= 5) ? model_ncomp(model) : 0; }
+int psoap_model_ncomp(int model) { return model_valid(model) ? dims_ncomp(model) : 0; }
 int psoap_model_norb(int model) { return (model >= 1 && model <= 5) ? model_norb(model) : 0; }
 
 // ---- fills ------------------------------------------------------------------------------------------
@@ -893,9 +900,9 @@ extern "C" int psoap_lnlike_grad_views(void* workspace, int64_t N, double** neg_
 }
 
 extern "C" size_t psoap_chunk_lnprob_grad_workspace_bytes(int model, int64_t N, int32_t n_epochs) {
-    if (model < 1 || model > 5 || N < 1 || n_epochs < 1) return 0;
+    if (!model_valid(model) || N < 1 || n_epochs < 1) return 0;
     GradWs g;
-    return carve_grad_ws(nullptr, model_ncomp(model), N, n_epochs, model_norb(model), &g);
+    return carve_grad_ws(nullptr, dims_ncomp(model), N, n_epochs, dims_nvel(model, n_epochs), &g);
 }
 
 namespace {
@@ -909,13 +916,30 @@ int launch_grad_chain(cudaStream_t st, int ncomp, int norb, const psoap_chunk& c
     return PSOAP_OK;
 }
 
+// The free-velocity counterpart of launch_grad_chain: the per-epoch sums scattered into the row of the vector with Ng
+// global epochs through the chunk's epoch map (null: the chunk's own epochs), no Jacobian.
+int launch_grad_free(cudaStream_t st, int ncomp, const psoap_chunk& ch, const GradWs& w, int Ng, const int32_t* map,
+                     const int* sentinel, double* grad_p) {
+    grad_epoch_kernel<<<(unsigned)(ncomp * ch.n_epochs), 256, 0, st>>>(w.gz, ch.epoch, ch.N, ch.n_epochs, w.gv);
+    LAUNCH_CHECK();
+    const int n = ncomp * Ng + 2 * ncomp;
+    grad_free_kernel<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(w.gv, w.hyp, ncomp, ch.n_epochs, Ng, map, w.f.info,
+                                                                  sentinel, grad_p);
+    LAUNCH_CHECK();
+    return PSOAP_OK;
+}
+
 // The launches of psoap_chunk_lnprob_grad on a carved workspace: orbit velocities and sentinel, fill, identity border,
-// restricted elimination, contraction, reductions, orbit Jacobian, per-epoch sum and chain rule.
+// restricted elimination, contraction, reductions, orbit Jacobian, per-epoch sum and chain rule.  A free model reads
+// the chunk's velocities from p_dev instead and ends with the per-epoch sums.
 int launch_chunk_grad(int model, const psoap_chunk* chunk, const double* p_dev, double mu_GP, const GradWs& g,
                       cudaStream_t st, double* result, double* grad_p) {
-    const int ne = chunk->n_epochs, ncomp = model_ncomp(model), norb = model_norb(model);
-    // orbit velocities and the sentinel (|v| >= c, or a negative GP hyper-parameter), as the farm's orbit kernel
-    orbit_kernel<<<1, 128, 0, st>>>(model, p_dev, chunk->dates, ne, g.vel, g.flag, 1);
+    const int ne = chunk->n_epochs, ncomp = dims_ncomp(model), norb = dims_nvel(model, ne);
+    // velocities and the sentinel (|v| >= c, or a negative GP hyper-parameter), as the farm's velocity kernels
+    if (model_free(model))
+        free_velocity_kernel<<<1, 128, 0, st>>>(ncomp, ne, p_dev, nullptr, ne, g.vel, g.flag, 1);
+    else
+        orbit_kernel<<<1, 128, 0, st>>>(model, p_dev, chunk->dates, ne, g.vel, g.flag, 1);
     LAUNCH_CHECK();
     Lanes ln;
     int rc = get_lanes(st, &ln);
@@ -923,13 +947,14 @@ int launch_chunk_grad(int model, const psoap_chunk* chunk, const double* p_dev, 
     rc = launch_grad(ln, ncomp, chunk->N, farm_z(*chunk, g.vel), chunk->fl, chunk->sigma, mu_GP, gp_params(p_dev + norb),
                      g, g.flag, result, g.hyp, g.gz);
     if (rc) return rc;
+    if (model_free(model)) return launch_grad_free(st, ncomp, *chunk, g, ne, nullptr, g.flag, grad_p);
     orbit_jacobian_kernel<<<1, 128, 0, st>>>(model, p_dev, chunk->dates, ne, g.jac);
     LAUNCH_CHECK();
     return launch_grad_chain(st, ncomp, norb, *chunk, g, g.jac, g.flag, grad_p);
 }
 
 bool chunk_args_ok(int model, const psoap_chunk* chunk) {
-    return model >= 1 && model <= 5 && chunk && chunk->N >= 1 && chunk->N <= 200000 && chunk->n_epochs >= 1 &&
+    return model_valid(model) && chunk && chunk->N >= 1 && chunk->N <= 200000 && chunk->n_epochs >= 1 &&
            chunk->lwl && chunk->epoch && chunk->fl && chunk->sigma && chunk->dates;
 }
 }  // namespace
@@ -940,7 +965,7 @@ extern "C" int psoap_chunk_lnprob_grad(int model, const psoap_chunk* chunk, cons
     if (!chunk_args_ok(model, chunk) || !p_dev || !result || !grad_p)
         return fail(PSOAP_ERR_ARG, "psoap_chunk_lnprob_grad: bad arguments");
     const int64_t N = chunk->N;
-    const int ne = chunk->n_epochs, ncomp = model_ncomp(model), norb = model_norb(model);
+    const int ne = chunk->n_epochs, ncomp = dims_ncomp(model), norb = dims_nvel(model, ne);
     if (!workspace || workspace_bytes < psoap_chunk_lnprob_grad_workspace_bytes(model, N, ne) ||
         ((uintptr_t)workspace & 255))
         return fail(PSOAP_ERR_WORKSPACE, "psoap_chunk_lnprob_grad: workspace too small or not 256-byte aligned");
@@ -964,7 +989,7 @@ struct FisherWs {
     int P, npairs;
 };
 size_t carve_fisher_ws(char* base, int model, int64_t N, int n_epochs, GradWs* g, FisherWs* f) {
-    const int ncomp = model_ncomp(model), norb = model_norb(model);
+    const int ncomp = dims_ncomp(model), norb = dims_nvel(model, n_epochs);
     size_t off = carve_grad_ws(base, ncomp, N, n_epochs, norb, g);
     auto take = [&](size_t bytes) { char* r = base ? base + off : nullptr; off += align_up(bytes, 256); return r; };
     const int64_t Tb = g->Tb;
@@ -979,15 +1004,20 @@ size_t carve_fisher_ws(char* base, int model, int64_t N, int n_epochs, GradWs* g
 }
 
 // the Fisher steps after launch_chunk_grad (fisher.cuh): mirror K^-1, then per parameter D_a and A_a = K^-1 D_a, then
-// the tile-pair contraction and the fixed-order reduction into fisher [P][P]
+// the tile-pair contraction and the fixed-order reduction into fisher [P][P].  A free model's velocities enter D_a
+// through the identity Jacobian.
 int launch_fisher(int model, const psoap_chunk* chunk, const double* p_dev, const GradWs& g, const FisherWs& f,
                   cudaStream_t st, double* fisher) {
-    const int N = (int)chunk->N, ncomp = model_ncomp(model), norb = model_norb(model), P = f.P;
+    const int N = (int)chunk->N, ncomp = dims_ncomp(model), norb = dims_nvel(model, chunk->n_epochs), P = f.P;
     const int64_t Nn = g.Nn;
     double* kinv = g.S + Nn + Nn * g.Nt;
     const int T32 = (int)(Nn / 32);
     fisher_mirror_kernel<<<(unsigned)((int64_t)T32 * (T32 + 1) / 2), 256, 0, st>>>(kinv, g.Nt, N);
     LAUNCH_CHECK();
+    if (model_free(model)) {
+        free_jacobian_kernel<<<(unsigned)std::min<int64_t>(((int64_t)norb * norb + 255) / 256, 1024), 256, 0, st>>>(norb, g.jac);
+        LAUNCH_CHECK();
+    }
     CUtensorMap mapS, mapD;
     int rc = make_tensor_map(&mapS, kinv, (uint64_t)Nn, (uint64_t)Nn, (uint64_t)g.Nt, SA);
     if (!rc) rc = make_tensor_map(&mapD, g.S, (uint64_t)Nn, (uint64_t)Nn, (uint64_t)g.Nt, SB);
@@ -1010,7 +1040,13 @@ int launch_fisher(int model, const psoap_chunk* chunk, const double* p_dev, cons
         fisher_gemm_kernel<<<persistent_ctas(ntiles), 256, GEMM_SMEM, st>>>(src, ntiles, mapS, mapD);
         LAUNCH_CHECK();
     }
-    fisher_pair_kernel<<<(unsigned)f.npairs, 256, fisher_pair_smem(P), st>>>(f.prod, Nn * Nn, Nn, P, f.part);
+    if (P <= FISHER_MAXP) {
+        fisher_pair_kernel<<<(unsigned)f.npairs, 256, fisher_pair_smem(P), st>>>(f.prod, Nn * Nn, Nn, P, f.part);
+    } else {   // a free chunk with many epochs: 16-parameter blocks
+        const int nblk = (P + FISHER_PB - 1) / FISHER_PB;
+        fisher_pair_blocked_kernel<<<dim3((unsigned)f.npairs, (unsigned)(nblk * (nblk + 1) / 2)), 256, 0, st>>>(
+            f.prod, Nn * Nn, Nn, P, f.part);
+    }
     LAUNCH_CHECK();
     fisher_reduce_kernel<<<1, 256, 0, st>>>(f.part, f.npairs, P, g.f.info, g.flag, fisher);
     LAUNCH_CHECK();
@@ -1019,7 +1055,7 @@ int launch_fisher(int model, const psoap_chunk* chunk, const double* p_dev, cons
 }  // namespace
 
 extern "C" size_t psoap_chunk_fisher_workspace_bytes(int model, int64_t N, int32_t n_epochs) {
-    if (model < 1 || model > 5 || N < 1 || N > 200000 || n_epochs < 1) return 0;
+    if (!model_valid(model) || N < 1 || N > 200000 || n_epochs < 1) return 0;
     GradWs g;
     FisherWs f;
     return carve_fisher_ws(nullptr, model, N, n_epochs, &g, &f);
@@ -1046,7 +1082,7 @@ extern "C" int psoap_chunk_fisher(int model, const psoap_chunk* chunk, const dou
 
 extern "C" int psoap_chunk_fisher_views(void* workspace, int model, int64_t N, int32_t n_epochs, uint8_t** flags,
                                         int** krange, int* Tb) {
-    if (!workspace || model < 1 || model > 5 || N < 1 || n_epochs < 1)
+    if (!workspace || !model_valid(model) || N < 1 || n_epochs < 1)
         return fail(PSOAP_ERR_ARG, "psoap_chunk_fisher_views: bad arguments");
     GradWs g;
     FisherWs f;
@@ -1202,10 +1238,11 @@ struct FarmGraph {
     std::vector<cudaEvent_t> events;
     std::vector<cudaEvent_t> side_events;
     int launches = 0;                 // kernels one evaluation launches
-    double* p_buf = nullptr;          // [nprop][P_STRIDE] parameter vectors the graph reads
+    double* p_buf = nullptr;          // [nprop][pstride] parameter vectors the graph reads
     double* results = nullptr;        // [nitems][4]
     int* flags = nullptr;             // per item sentinel
     OrbitDesc* descs = nullptr;       // device, per item
+    FreeDesc* fdescs = nullptr;       // device, per item, in place of descs on a free-velocity farm
     std::vector<double*> item_vel;    // device velocity table of each item
     std::vector<char*> branch_base;   // scratch region of each branch, carved for each of its items in turn (items of
                                       // a branch run in stream order)
@@ -1248,9 +1285,13 @@ struct FarmPredict {
 }  // namespace
 
 struct psoap_farm {
-    int model = 0, ncomp = 0, norb = 0, nchunks = 0, nprop = 1, nitems = 0;
+    int model = 0, ncomp = 0, norb = 0, nchunks = 0, nprop = 1, nitems = 0;   // norb: parameters before the GP block
     double mu = 1.0;
     std::vector<psoap_chunk> chunks;
+    bool free = false;                // psoap_farm_create_free: norb = ncomp Ng per-epoch velocities, no orbit
+    int Ng = 0;                       // global epochs of a free farm
+    std::vector<const int32_t*> maps; // [nchunks] device epoch maps of a free farm
+    int pstride = P_STRIDE;           // doubles per proposal in the parameter buffers
     FarmGraph g;                      // the likelihood graph
     int chain_hint = 0;               // psoap_chunk.reserved of the first chunk, low byte: 3 | 7 forces the chain links
     int group_hint = 0;               // ... bits 8 and up: 2 | 4 | 8 forces the panels per trailing update
@@ -1282,8 +1323,22 @@ Lanes farm_lanes(const psoap_farm* f, const FarmGraph& g, int b, int pdl) {
 
 // the GP values of item it's proposal, as every farm graph reads them
 GpParams farm_gp(const psoap_farm* f, const FarmGraph& g, int it) {
-    return gp_params(g.p_buf + (size_t)(it / f->nchunks) * P_STRIDE + f->norb);
+    return gp_params(g.p_buf + (size_t)(it / f->nchunks) * f->pstride + f->norb);
 }
+
+// the first step of every farm graph: the velocity table and sentinel of every item, from its orbit or (free farm)
+// gathered through its chunk's epoch map
+int launch_item_velocities(const psoap_farm* f, const FarmGraph& g, cudaStream_t s0) {
+    if (f->free)
+        free_velocity_farm_kernel<<<f->nitems, 64, 0, s0>>>(f->ncomp, f->Ng, g.p_buf, g.fdescs);
+    else
+        orbit_farm_kernel<<<f->nitems, 64, 0, s0>>>(f->model, g.p_buf, g.descs);
+    LAUNCH_CHECK();
+    return PSOAP_OK;
+}
+
+// orbit Jacobian columns a gradient workspace holds: none on a free farm
+int jac_cols(const psoap_farm* f) { return f->free ? 0 : f->norb; }
 
 // Forks g's branches from s0, after the root kernels the caller launched there, issues the items of each branch in LPT
 // order through item(b, branch stream, it), and joins the branches back into s0.
@@ -1308,8 +1363,8 @@ int issue_branches(const FarmGraph& g, cudaStream_t s0, Item&& item) {
 // adds programmatic dependent launch on the small grids).
 int farm_issue(const psoap_farm* f, cudaStream_t s0, int pdl) {
     const FarmGraph& g = f->g;
-    orbit_farm_kernel<<<f->nitems, 64, 0, s0>>>(f->model, g.p_buf, g.descs);
-    LAUNCH_CHECK();
+    const int rc = launch_item_velocities(f, g, s0);
+    if (rc) return rc;
     return issue_branches(g, s0, [&](int b, cudaStream_t, int it) {
         const psoap_chunk& ch = f->chunks[it % f->nchunks];
         FactorWs ws;
@@ -1324,17 +1379,22 @@ int farm_issue(const psoap_farm* f, cudaStream_t s0, int pdl) {
 int farm_grad_issue(const psoap_farm* f, const FarmGrad& q, cudaStream_t s0, int pdl) {
     const FarmGraph& g = q.g;
     const int np = f->norb + 2 * f->ncomp;
-    orbit_farm_kernel<<<f->nitems, 64, 0, s0>>>(f->model, g.p_buf, g.descs);
-    LAUNCH_CHECK();
-    orbit_jacobian_farm_kernel<<<f->nitems, 64, 0, s0>>>(f->model, g.p_buf, q.jdescs);
-    LAUNCH_CHECK();
+    int rc = launch_item_velocities(f, g, s0);
+    if (rc) return rc;
+    if (!f->free) {
+        orbit_jacobian_farm_kernel<<<f->nitems, 64, 0, s0>>>(f->model, g.p_buf, q.jdescs);
+        LAUNCH_CHECK();
+    }
     return issue_branches(g, s0, [&](int b, cudaStream_t sb, int it) {
         const psoap_chunk& ch = f->chunks[it % f->nchunks];
         GradWs w;
-        carve_grad_ws(g.branch_base[b], f->ncomp, ch.N, ch.n_epochs, f->norb, &w);
+        carve_grad_ws(g.branch_base[b], f->ncomp, ch.N, ch.n_epochs, jac_cols(f), &w);
         int rc = launch_grad(farm_lanes(f, g, b, pdl), f->ncomp, ch.N, farm_z(ch, g.item_vel[it]), ch.fl, ch.sigma, f->mu,
                              farm_gp(f, g, it), w, g.flags + it, g.results + 4 * it, w.hyp, w.gz);
-        if (!rc) rc = launch_grad_chain(sb, f->ncomp, f->norb, ch, w, q.item_jac[it], g.flags + it, q.grad + (size_t)it * np);
+        double* row = q.grad + (size_t)it * np;
+        if (!rc)
+            rc = f->free ? launch_grad_free(sb, f->ncomp, ch, w, f->Ng, f->maps[it % f->nchunks], g.flags + it, row)
+                         : launch_grad_chain(sb, f->ncomp, f->norb, ch, w, q.item_jac[it], g.flags + it, row);
         return rc;
     });
 }
@@ -1352,8 +1412,8 @@ PredictDims predict_item_dims(int ncomp, int64_t N, int64_t m) {
 int farm_predict_issue(const psoap_farm* f, const FarmPredict& q, cudaStream_t s0, int pdl, double* delta, double* sigma) {
     const FarmGraph& g = q.g;
     const int nchunks = f->nchunks, ncomp = f->ncomp;
-    orbit_farm_kernel<<<f->nitems, 64, 0, s0>>>(f->model, g.p_buf, g.descs);
-    LAUNCH_CHECK();
+    const int rc0 = launch_item_velocities(f, g, s0);
+    if (rc0) return rc0;
     return issue_branches(g, s0, [&](int b, cudaStream_t sb, int it) {
         const int ci = it % nchunks;
         const psoap_chunk& ch = f->chunks[ci];
@@ -1455,12 +1515,21 @@ int capture_farm_graph(FarmGraph& g, const FarmIssue& issue) {
 // the capture.  On failure the caller deletes the graph's owner, which releases what was created.
 int attach_farm_graph(const psoap_farm* f, FarmGraph& g, const std::vector<int64_t>& cost, bool attached,
                       const FarmIssue& issue) {
-    std::vector<OrbitDesc> hd(f->nitems);
-    for (int it = 0; it < f->nitems; ++it) {
-        const psoap_chunk& ch = f->chunks[it % f->nchunks];
-        hd[it] = {ch.dates, g.item_vel[it], g.flags + it, ch.n_epochs, (it / f->nchunks) * P_STRIDE};
+    if (f->free) {
+        std::vector<FreeDesc> hd(f->nitems);
+        for (int it = 0; it < f->nitems; ++it) {
+            const psoap_chunk& ch = f->chunks[it % f->nchunks];
+            hd[it] = {f->maps[it % f->nchunks], g.item_vel[it], g.flags + it, ch.n_epochs, (it / f->nchunks) * f->pstride};
+        }
+        CUDA_TRY(cudaMemcpy(g.fdescs, hd.data(), hd.size() * sizeof(FreeDesc), cudaMemcpyHostToDevice));
+    } else {
+        std::vector<OrbitDesc> hd(f->nitems);
+        for (int it = 0; it < f->nitems; ++it) {
+            const psoap_chunk& ch = f->chunks[it % f->nchunks];
+            hd[it] = {ch.dates, g.item_vel[it], g.flags + it, ch.n_epochs, (it / f->nchunks) * f->pstride};
+        }
+        CUDA_TRY(cudaMemcpy(g.descs, hd.data(), hd.size() * sizeof(OrbitDesc), cudaMemcpyHostToDevice));
     }
-    CUDA_TRY(cudaMemcpy(g.descs, hd.data(), hd.size() * sizeof(OrbitDesc), cudaMemcpyHostToDevice));
     g.branch_items = lpt_items(cost, f->nitems, g.nbranch);
     int64_t nmax = 0;   // the largest chunk that takes work
     for (int i = 0; i < f->nchunks; ++i)
@@ -1489,8 +1558,8 @@ int attach_farm_graph(const psoap_farm* f, FarmGraph& g, const std::vector<int64
 int run_farm_graph(const psoap_farm* f, FarmGraph& g, const double* p_dev, psoap_result* results_dev, cudaStream_t st,
                    const FarmIssue& issue) {
     const int np = f->norb + 2 * f->ncomp;
-    // p_dev: [nprop][np] contiguous -> [nprop][P_STRIDE]
-    CUDA_TRY(cudaMemcpy2DAsync(g.p_buf, P_STRIDE * 8, p_dev, (size_t)np * 8, (size_t)np * 8, f->nprop,
+    // p_dev: [nprop][np] contiguous -> [nprop][pstride]
+    CUDA_TRY(cudaMemcpy2DAsync(g.p_buf, (size_t)f->pstride * 8, p_dev, (size_t)np * 8, (size_t)np * 8, f->nprop,
                                cudaMemcpyDeviceToDevice, st));
     if (g.direct) {
         cudaStream_t s0 = g.streams[g.nbranch];
@@ -1516,16 +1585,19 @@ struct Carver {
     char* take(size_t bytes) { char* r = base ? base + off : nullptr; off += align_up(bytes, 256); return r; }
 };
 
-// Layout of the part of a workspace every farm graph has: the parameter buffer, the result records, sentinels and orbit
-// descriptors of the items, vel_rows x n_epochs velocity doubles per item, then nbranch regions of branch_bytes.  The
-// graph's own buffers follow at c.off.
+// Layout of the part of a workspace every farm graph has: the parameter buffer (pstride doubles per proposal), the result
+// records, sentinels and velocity descriptors of the items (orbit, or with free_vel the epoch-map ones), vel_rows x
+// n_epochs velocity doubles per item, then nbranch regions of branch_bytes.  The graph's own buffers follow at c.off.
 void carve_farm_items(Carver& c, FarmGraph& g, int nprop, int nchunks, const int32_t* n_epochs, int vel_rows,
-                      size_t branch_bytes) {
+                      size_t branch_bytes, int pstride = P_STRIDE, bool free_vel = false) {
     const int nitems = nchunks * nprop;
-    g.p_buf = (double*)c.take((size_t)nprop * P_STRIDE * 8);
+    g.p_buf = (double*)c.take((size_t)nprop * pstride * 8);
     g.results = (double*)c.take((size_t)nitems * 4 * 8);
     g.flags = (int*)c.take((size_t)nitems * 4);
-    g.descs = (OrbitDesc*)c.take((size_t)nitems * sizeof(OrbitDesc));
+    if (free_vel)
+        g.fdescs = (FreeDesc*)c.take((size_t)nitems * sizeof(FreeDesc));
+    else
+        g.descs = (OrbitDesc*)c.take((size_t)nitems * sizeof(OrbitDesc));
     g.item_vel.resize(nitems);
     for (int it = 0; it < nitems; ++it) g.item_vel[it] = (double*)c.take((size_t)vel_rows * n_epochs[it % nchunks] * 8);
     g.branch_base.resize(g.nbranch);
@@ -1534,11 +1606,12 @@ void carve_farm_items(Carver& c, FarmGraph& g, int nprop, int nchunks, const int
 
 // Layout of a likelihood workspace: each branch holds the FactorWs of the largest chunk.  The size query takes no
 // model, so every item reserves the velocity table of three components.
-size_t carve_farm_lnprob(char* base, FarmGraph& g, int nchunks, const int64_t* N, const int32_t* n_epochs, int nprop) {
+size_t carve_farm_lnprob(char* base, FarmGraph& g, int nchunks, const int64_t* N, const int32_t* n_epochs, int nprop,
+                         int pstride = P_STRIDE, bool free_vel = false) {
     int64_t nmax = 0;
     for (int i = 0; i < nchunks; ++i) nmax = std::max(nmax, N[i]);
     Carver c{base};
-    carve_farm_items(c, g, nprop, nchunks, n_epochs, 3, factor_ws_bytes(padded_dim(nmax)));
+    carve_farm_items(c, g, nprop, nchunks, n_epochs, 3, factor_ws_bytes(padded_dim(nmax)), pstride, free_vel);
     return c.off;
 }
 
@@ -1560,11 +1633,11 @@ size_t carve_farm_grad(const psoap_farm* f, char* base, FarmGrad& q) {
     GradWs probe;
     Carver c{base};
     carve_farm_items(c, q.g, f->nprop, f->nchunks, nes.data(), f->ncomp,
-                     carve_grad_ws(nullptr, f->ncomp, nmax, nemax, f->norb, &probe));
+                     carve_grad_ws(nullptr, f->ncomp, nmax, nemax, jac_cols(f), &probe), f->pstride, f->free);
     q.grad = (double*)c.take((size_t)nitems * np * 8);
     q.jdescs = (JacDesc*)c.take((size_t)nitems * sizeof(JacDesc));
     q.item_jac.resize(nitems);
-    for (int it = 0; it < nitems; ++it) q.item_jac[it] = (double*)c.take((size_t)f->ncomp * nes[it % f->nchunks] * f->norb * 8);
+    for (int it = 0; it < nitems; ++it) q.item_jac[it] = (double*)c.take((size_t)f->ncomp * nes[it % f->nchunks] * jac_cols(f) * 8);
     return c.off;
 }
 
@@ -1587,7 +1660,8 @@ size_t carve_farm_predict(const psoap_farm* f, const int64_t* m, int sigma_mode,
     }
     q.delta_off[nitems] = nd; q.sigma_off[nitems] = ns;
     Carver c{base};
-    carve_farm_items(c, q.g, f->nprop, nchunks, farm_epochs(f).data(), f->ncomp, ntmax ? factor_ws_bytes(ntmax) : 0);
+    carve_farm_items(c, q.g, f->nprop, nchunks, farm_epochs(f).data(), f->ncomp, ntmax ? factor_ws_bytes(ntmax) : 0,
+                     f->pstride, f->free);
     q.cap_delta = (double*)c.take((size_t)nd * 8);
     q.cap_sigma = (double*)c.take((size_t)ns * 8);
     return c.off;
@@ -1645,6 +1719,65 @@ int psoap_farm_create(psoap_farm** out, int model, int nchunks, const psoap_chun
     return psoap_farm_create_batched(out, model, nchunks, chunks, 1, nbranch, mu_GP, workspace, workspace_bytes);
 }
 
+// ---- free-velocity farm ---------------------------------------------------------------------------------------------
+size_t psoap_farm_free_workspace_bytes(int ncomp, int Ng, int nchunks, const int64_t* N, const int32_t* n_epochs,
+                                       int nprop, int nbranch) {
+    if (ncomp < 1 || ncomp > 3 || Ng < 1 || nchunks < 1 || nprop < 1 || !N || !n_epochs) return 0;
+    FarmGraph probe;
+    probe.nbranch = std::max(1, std::min(nbranch, nchunks * nprop));
+    const int np = ncomp * Ng + 2 * ncomp;
+    return carve_farm_lnprob(nullptr, probe, nchunks, N, n_epochs, nprop, (np + 3) / 4 * 4, true);
+}
+
+int psoap_farm_create_free(psoap_farm** out, int ncomp, int Ng, int nchunks, const psoap_chunk* chunks,
+                           const int32_t* const* epoch_map_dev, int nprop, int nbranch, double mu_GP, void* workspace,
+                           size_t workspace_bytes) {
+    if (!out || ncomp < 1 || ncomp > 3 || Ng < 1 || nchunks < 1 || nprop < 1 || !chunks || !epoch_map_dev || !workspace ||
+        ((uintptr_t)workspace & 255))
+        return fail(PSOAP_ERR_ARG, "psoap_farm_create_free: bad arguments");
+    const int nitems = nchunks * nprop;
+    nbranch = std::max(1, std::min(nbranch, nitems));
+    std::vector<int64_t> Ns(nchunks);
+    std::vector<int32_t> nes(nchunks);
+    for (int i = 0; i < nchunks; ++i) {
+        if (chunks[i].N < 1 || chunks[i].n_epochs < 1 || !chunks[i].lwl || !chunks[i].epoch || !chunks[i].fl ||
+            !chunks[i].sigma || !chunks[i].dates || !epoch_map_dev[i])
+            return fail(PSOAP_ERR_ARG, "psoap_farm_create_free: bad chunk descriptor or null epoch map");
+        Ns[i] = chunks[i].N;
+        nes[i] = chunks[i].n_epochs;
+    }
+    if (workspace_bytes < psoap_farm_free_workspace_bytes(ncomp, Ng, nchunks, Ns.data(), nes.data(), nprop, nbranch))
+        return fail(PSOAP_ERR_WORKSPACE, "psoap_farm_create_free: workspace too small");
+    int rc = set_kernel_attributes();
+    if (rc) return rc;
+    // every map entry in [0, Ng), and no global epoch twice in one chunk (each gradient slot then has one source epoch)
+    for (int i = 0; i < nchunks; ++i) {
+        std::vector<int32_t> m(nes[i]);
+        CUDA_TRY(cudaMemcpy(m.data(), epoch_map_dev[i], m.size() * 4, cudaMemcpyDeviceToHost));
+        std::vector<char> seen(Ng, 0);
+        for (int32_t g : m) {
+            if (g < 0 || g >= Ng || seen[g])
+                return fail(PSOAP_ERR_ARG, "psoap_farm_create_free: the epoch map of chunk " + std::to_string(i) +
+                                               " leaves [0, Ng) or repeats a global epoch");
+            seen[g] = 1;
+        }
+    }
+
+    psoap_farm* f = new psoap_farm();
+    f->model = PSOAP_FREE1 + ncomp - 1; f->ncomp = ncomp; f->norb = ncomp * Ng;
+    f->free = true; f->Ng = Ng; f->maps.assign(epoch_map_dev, epoch_map_dev + nchunks);
+    f->pstride = (f->norb + 2 * ncomp + 3) / 4 * 4;
+    f->nchunks = nchunks; f->nprop = nprop; f->nitems = nitems; f->g.nbranch = nbranch; f->mu = mu_GP;
+    f->chunks.assign(chunks, chunks + nchunks);
+    f->chain_hint = chunks[0].reserved & 0xff;
+    f->group_hint = (chunks[0].reserved >> 8) & 0xff;
+    carve_farm_lnprob((char*)workspace, f->g, nchunks, Ns.data(), nes.data(), nprop, f->pstride, true);
+    rc = attach_farm_graph(f, f->g, Ns, false, [f](cudaStream_t s0, int pdl) { return farm_issue(f, s0, pdl); });
+    if (rc != PSOAP_OK) { delete f; return rc; }
+    *out = f;
+    return PSOAP_OK;
+}
+
 int psoap_farm_lnprob(psoap_farm* f, const double* p_dev, psoap_result* results_dev, void* stream) {
     if (!f || !p_dev || !results_dev) return fail(PSOAP_ERR_ARG, "psoap_farm_lnprob: bad arguments");
     return run_farm_graph(f, f->g, p_dev, results_dev, (cudaStream_t)stream,
@@ -1682,9 +1815,11 @@ int psoap_farm_grad_attach(psoap_farm* f, int nbranch, void* workspace, size_t w
     for (const psoap_chunk& ch : f->chunks) Ns.push_back(ch.N);
     for (int it = 0; it < f->nitems; ++it) {
         const psoap_chunk& ch = f->chunks[it % f->nchunks];
-        hj[it] = {ch.dates, q->item_jac[it], ch.n_epochs, (it / f->nchunks) * P_STRIDE};
+        hj[it] = {ch.dates, q->item_jac[it], ch.n_epochs, (it / f->nchunks) * f->pstride};
     }
-    cudaError_t e = cudaMemcpy(q->jdescs, hj.data(), hj.size() * sizeof(JacDesc), cudaMemcpyHostToDevice);
+    // a free farm has no orbit Jacobian
+    cudaError_t e = f->free ? cudaSuccess
+                            : cudaMemcpy(q->jdescs, hj.data(), hj.size() * sizeof(JacDesc), cudaMemcpyHostToDevice);
     rc = e != cudaSuccess ? fail(PSOAP_ERR_CUDA, std::string("farm grad descs: ") + cudaGetErrorString(e))
                           : attach_farm_graph(f, q->g, Ns, true,
                                               [f, q](cudaStream_t s0, int pdl) { return farm_grad_issue(f, *q, s0, pdl); });

@@ -240,6 +240,54 @@ __global__ void __launch_bounds__(256) fisher_pair_kernel(const double* __restri
     }
 }
 
+// fisher_pair_kernel for any P (a free-velocity chunk has ncomp n_epochs + 2 ncomp parameters, beyond the 512 G entries
+// one CTA of that kernel holds): block (t, u) takes tile pair t and the u-th pair (A, B), A <= B, of 16-parameter
+// blocks.  Thread (a, b) of the 16 x 16 block sums G_ab = sum_e X_a[e] Y_b[e] and G_ba = sum_e X_b[e] Y_a[e] in element
+// order, FISHER_PC elements staged per step, and writes part[t][tri(a, b)] for a <= b as fisher_pair_kernel does.
+constexpr int FISHER_PB = 16;   // parameters per block
+constexpr int FISHER_PC = 64;   // tile-pair elements staged per step
+__global__ void __launch_bounds__(256) fisher_pair_blocked_kernel(const double* __restrict__ A, int64_t stride,
+                                                                  int64_t ld, int P, double* __restrict__ part) {
+    const int t = blockIdx.x;
+    int I = (int)((sqrtf(8.0f * (float)t + 1.0f) - 1.0f) * 0.5f);
+    while ((I + 1) * (I + 2) / 2 <= t) ++I;
+    while (I * (I + 1) / 2 > t) --I;
+    const int J = t - I * (I + 1) / 2;
+    const int nblk = (P + FISHER_PB - 1) / FISHER_PB;
+    int u = blockIdx.y, ba = 0;
+    while (u >= nblk - ba) { u -= nblk - ba; ++ba; }
+    const int bb = ba + u;
+    __shared__ double XA[FISHER_PC][FISHER_PB + 1], YA[FISHER_PC][FISHER_PB + 1];
+    __shared__ double XB[FISHER_PC][FISHER_PB + 1], YB[FISHER_PC][FISHER_PB + 1];
+    const int tid = threadIdx.x;
+    const int al = tid >> 4, bl = tid & 15;
+    const int a = ba * FISHER_PB + al, b = bb * FISHER_PB + bl;
+    double gab = 0.0, gba = 0.0;
+#pragma unroll 1
+    for (int e0 = 0; e0 < NB * NB; e0 += FISHER_PC) {
+        for (int q = tid; q < FISHER_PC * FISHER_PB; q += 256) {
+            const int k = q / FISHER_PC, e = q % FISHER_PC;
+            const int el = e0 + e, i = el % NB, j = el / NB;
+            const int64_t ox = (int64_t)(I * NB + i) + (int64_t)(J * NB + j) * ld;
+            const int64_t oy = (int64_t)(J * NB + j) + (int64_t)(I * NB + i) * ld;
+            const int pa = ba * FISHER_PB + k, pb = bb * FISHER_PB + k;
+            XA[e][k] = pa < P ? A[pa * stride + ox] : 0.0;
+            YA[e][k] = pa < P ? A[pa * stride + oy] : 0.0;
+            XB[e][k] = pb < P ? A[pb * stride + ox] : 0.0;
+            YB[e][k] = pb < P ? A[pb * stride + oy] : 0.0;
+        }
+        __syncthreads();
+#pragma unroll 8
+        for (int e = 0; e < FISHER_PC; ++e) {
+            gab = fma(XA[e][al], YB[e][bl], gab);
+            gba = fma(XB[e][bl], YA[e][al], gba);
+        }
+        __syncthreads();
+    }
+    if (a < P && b < P && a <= b)
+        part[(int64_t)t * (P * (P + 1) / 2) + fisher_tri(a, b, P)] = (I == J) ? gab : gab + gba;
+}
+
 // F (row-major P x P) = 1/2 sum over the tile pairs, in pair order, of the partials; both triangles from one value.
 // NaN everywhere when the likelihood is -inf (info != 0, or the sentinel of the orbit / hyper-parameter check fired),
 // the words the gradient reads.

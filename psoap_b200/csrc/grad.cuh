@@ -276,6 +276,38 @@ __global__ void grad_chain_kernel(const double* __restrict__ grad_v, const doubl
     grad_p[k] = grad_flagged(info, sentinel) ? CUDART_NAN : g;
 }
 
+// The free-velocity counterpart of grad_chain_kernel (the Jacobian is the identity): the gradient row for the vector
+// [v_0[0..Ng), .., v_{ncomp-1}[0..Ng), GP] of a chunk whose local epoch e is global epoch map[e] (map null: the
+// identity, Ng = n_epochs):  grad_p[c Ng + g] = sum_{e : map[e] = g} dlnlike/dv_c[e] (in e order; exactly 0 for an epoch
+// the chunk does not observe),  grad_p[ncomp Ng + j] = grad_hyp[j].  NaN everywhere when the item's sentinel or pivot
+// fired.  One writer per entry: no atomics.
+__global__ void __launch_bounds__(128) grad_free_kernel(const double* __restrict__ grad_v,
+                                                        const double* __restrict__ grad_hyp, int ncomp, int n_epochs,
+                                                        int Ng, const int32_t* __restrict__ map,
+                                                        const int* __restrict__ info, const int* __restrict__ sentinel,
+                                                        double* __restrict__ grad_p) {
+    const int nv = ncomp * Ng;
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= nv + 2 * ncomp) return;
+    double g = 0.0;
+    if (k < nv) {
+        const int c = k / Ng, gl = k - c * Ng;
+        for (int e = 0; e < n_epochs; ++e)
+            if ((map ? map[e] : e) == gl) g += grad_v[c * n_epochs + e];
+    } else {
+        g = grad_hyp[k - nv];
+    }
+    grad_p[k] = grad_flagged(info, sentinel) ? CUDART_NAN : g;
+}
+
+// dv_c[e] / dv_{c'}[e'] of a free chunk in the layout of orbit_jacobian_block, jac [ncomp][n_epochs][ncomp n_epochs]:
+// the identity, so that the Fisher steps read free velocities as they read orbital parameters.
+__global__ void free_jacobian_kernel(int nv, double* __restrict__ jac) {
+    const int64_t n = (int64_t)nv * nv;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
+        jac[i] = (i / nv == i % nv) ? 1.0 : 0.0;
+}
+
 // -inf likelihood found on the host (negative hyper-parameters): NaN in every gradient entry.
 __global__ void grad_fill_kernel(double* __restrict__ out, int64_t n, double v) {
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) out[i] = v;

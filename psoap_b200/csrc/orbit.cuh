@@ -194,4 +194,56 @@ __global__ void orbit_farm_kernel(int model, const double* __restrict__ p, const
     orbit_block(model, p + d.p_off, d.dates, d.n_epochs, d.vel, d.flag, 1);
 }
 
+// Free velocities (no orbit): the parameter vector starts with ncomp blocks of Ng per-epoch velocities, v_c[g] at
+// p[c Ng + g], followed by the GP values.  An item's table is gathered through its chunk's epoch map,
+// vel[c][e] = p[c Ng + map[e]] (map null: the identity, Ng = n_epochs), with the sentinel of orbit_block: flag[0] = 1
+// when any gathered |v| >= c_kms or, with check_gp, a GP value is negative; else 0.  One block; threads stride over
+// epochs.
+__device__ inline void free_velocity_block(int ncomp, int Ng, const double* __restrict__ p,
+                                           const int32_t* __restrict__ map, int n_epochs, double* __restrict__ vel,
+                                           int* __restrict__ flag, int check_gp) {
+    __shared__ int s_flag;
+    if (threadIdx.x == 0) {
+        int f = 0;
+        if (check_gp) {
+            const double* gp = p + (int64_t)ncomp * Ng;
+            for (int c = 0; c < 2 * ncomp; ++c)
+                if (gp[c] < 0.0) f = 1;
+        }
+        s_flag = f;
+    }
+    __syncthreads();
+    for (int ep = threadIdx.x; ep < n_epochs; ep += blockDim.x) {
+        const int g = map ? map[ep] : ep;
+        bool fast = false;
+        for (int c = 0; c < ncomp; ++c) {
+            const double v = p[(int64_t)c * Ng + g];
+            vel[(int64_t)c * n_epochs + ep] = v;
+            if (!(fabs(v) < C_KMS)) fast = true;
+        }
+        if (fast) atomicExch(&s_flag, 1);
+    }
+    __syncthreads();
+    if (threadIdx.x == 0 && flag) flag[0] = s_flag;
+}
+
+__global__ void free_velocity_kernel(int ncomp, int Ng, const double* __restrict__ p, const int32_t* __restrict__ map,
+                                     int n_epochs, double* __restrict__ vel, int* __restrict__ flag, int check_gp) {
+    free_velocity_block(ncomp, Ng, p, map, n_epochs, vel, flag, check_gp);
+}
+
+// Chunk farm with free velocities: the OrbitDesc of an item with the chunk's epoch map in place of its dates.
+struct FreeDesc {
+    const int32_t* map;
+    double* vel;
+    int* flag;
+    int n_epochs;
+    int p_off;
+};
+__global__ void free_velocity_farm_kernel(int ncomp, int Ng, const double* __restrict__ p,
+                                          const FreeDesc* __restrict__ descs) {
+    const FreeDesc d = descs[blockIdx.x];
+    free_velocity_block(ncomp, Ng, p + d.p_off, d.map, d.n_epochs, d.vel, d.flag, 1);
+}
+
 }  // namespace psoap

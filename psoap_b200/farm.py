@@ -76,6 +76,38 @@ def prediction_grids(grids, n_pix, ncomp):
     return out
 
 
+def global_epochs(dates):
+    """The global epoch list of a free-velocity farm: the sorted unique values of every chunk's date1D."""
+    if not len(dates):
+        return np.zeros(0)
+    return np.unique(np.concatenate([np.asarray(d, dtype=np.float64).reshape(-1) for d in dates]))
+
+
+def epoch_maps(dates, epochs):
+    """Per chunk, the int32 index of each of its dates in the global list `epochs` (exact match).  Raises ValueError for
+    a date that is not in the list or a date a chunk lists twice (each global velocity then has one source epoch)."""
+    epochs = np.asarray(epochs, dtype=np.float64)
+    maps = []
+    for i, d in enumerate(dates):
+        d = np.asarray(d, dtype=np.float64).reshape(-1)
+        idx = np.searchsorted(epochs, d)
+        ok = idx < len(epochs)
+        ok[ok] = epochs[idx[ok]] == d[ok]
+        if not np.all(ok):
+            raise ValueError("chunk %d: date %r is not in the global epoch list" % (i, float(d[~ok][0])))
+        if len(np.unique(idx)) != len(idx):
+            raise ValueError("chunk %d: date1D lists an epoch twice" % i)
+        maps.append(idx.astype(np.int32))
+    return maps
+
+
+def free_index(ncomp, Ng, emap):
+    """Positions in the farm's free vector [v_0[0..Ng), .., GP] of a chunk's own vector [v_0[e].., .., GP] (PSOAP_FREEn
+    at chunk level) for its epoch map."""
+    emap = np.asarray(emap, dtype=np.int64)
+    return np.concatenate([c * Ng + emap for c in range(ncomp)] + [ncomp * Ng + np.arange(2 * ncomp)])
+
+
 def combine_predictions(mu, var):
     """Posterior-averaged spectrum and its variance over K samples by the law of total variance: mean of the variances
     plus the variance of the means.  mu, var: [K, M] (one chunk's outputs of predict_components, var the diagonal of
@@ -93,10 +125,15 @@ class ChunkFarm:
     rank/world_size: static partition of the chunks over GPUs; process_group: torch.distributed group (or None).
     grad_nbranch: (proposal, chunk) pairs in flight in the gradient graph of chunk_lnlike_grads_many (default
     GRAD_NBRANCH, at most nbranch); each branch holds the identity-bordered matrix of the largest chunk, 8 (2 N)^2 bytes.
+    free_velocities: fit the radial velocity of each component at each epoch instead of an orbit (the model then only
+    gives the number of components).  The global epochs are the sorted unique dates of all chunks (`epochs`, Ng of them),
+    and every method takes p = [v_0[0..Ng), .., v_{ncomp-1}[0..Ng), amp_f, l_f, ...] in km/s, n_params = ncomp Ng +
+    2 ncomp, in place of the registered vector.  Adding one constant to all of a component's velocities leaves the
+    likelihood unchanged (sample.fit_epoch_velocities fixes that gauge).
     """
 
     def __init__(self, model, chunks, mu_GP=1.0, soften=1.0, nbranch=32, rank=0, world_size=1, process_group=None,
-                 n_proposals=1, grad_nbranch=None):
+                 n_proposals=1, grad_nbranch=None, free_velocities=False):
         self.grad_nbranch = int(grad_nbranch) if grad_nbranch is not None else min(nbranch, GRAD_NBRANCH)
         if self.grad_nbranch < 1:
             raise ValueError("grad_nbranch must be at least 1")
@@ -105,7 +142,14 @@ class ChunkFarm:
         self.model = model
         self.n_proposals = int(n_proposals)
         self.n_chunks = len(chunks)
-        self.n_params = _lib.N_ORB[model] + 2 * _lib.NCOMP[model]
+        self.free = bool(free_velocities)
+        ncomp = _lib.NCOMP[model]
+        if self.free:
+            self.epochs = global_epochs([ch["date1D"] for ch in chunks])
+            maps = epoch_maps([ch["date1D"] for ch in chunks], self.epochs)
+            self.n_params = ncomp * len(self.epochs) + 2 * ncomp
+        else:
+            self.n_params = _lib.N_ORB[model] + 2 * ncomp
         self.rank, self.world_size, self.group = rank, world_size, process_group
         self.parts = lpt_partition([chunk_cost(len(ch["fl"])) for ch in chunks], world_size)
         # a chunk whose mask removed every pixel contributes -0.0 in the reference (sums over nothing): it takes no
@@ -123,6 +167,8 @@ class ChunkFarm:
                         sigma=np.ascontiguousarray(np.asarray(ch["sigma"], dtype=np.float64) * soften),
                         dates=np.ascontiguousarray(ch["date1D"], dtype=np.float64),
                         epoch=np.ascontiguousarray(ep, dtype=np.int32))
+            if self.free:
+                host["map"] = maps[idx]
             N = len(host["fl"])
             if not (len(host["lwl"]) == len(host["sigma"]) == len(host["epoch"]) == N):
                 raise ValueError("chunk %d: lwl, fl, sigma and the mask must select the same number of pixels" % idx)
@@ -179,6 +225,11 @@ class ChunkFarm:
         self._grad_farm_ws = None    # allocated, and the gradient graph attached, by the first *_many gradient call
         self._n_pix = [len(ch["fl"]) for ch in chunks]
         self._pred = None            # attach_prediction_grids
+        # free velocities: each own chunk's epoch map (device, in the resident buffer) and the positions of its own
+        # vector (velocities at its epochs, then GP) in the farm's vector
+        if self.free:
+            self._free_idx = [torch.from_numpy(free_index(ncomp, len(self.epochs), maps[i])).cuda() for i in self.mine]
+            self._map_ptrs = (_lib.vp * max(1, len(self.mine)))(*[_lib.vp(base + off["map"]) for off in offsets])
         self._farm = _lib.vp(None)
         K = self.n_proposals
         self._results = torch.zeros((K, max(1, len(self.mine)), 4), dtype=torch.float64, device="cuda")
@@ -191,12 +242,30 @@ class ChunkFarm:
         self.launches_per_eval = 0
         if self.mine:
             nb = max(1, min(nbranch, len(self.mine) * K))
-            nbytes = lib.psoap_farm_workspace_bytes_batched(len(self.mine), (ctypes.c_int64 * len(Ns))(*Ns),
-                                                            (ctypes.c_int32 * len(nes))(*nes), K, nb)
-            self._ws = torch.empty(nbytes + 256, dtype=torch.uint8, device="cuda")
-            _lib.check(lib.psoap_farm_create_batched(ctypes.byref(self._farm), _lib.MODELS[model], len(self.mine),
-                                                     descs, K, nb, float(mu_GP), _lib.ptr(self._ws), nbytes))
+            Ns_c, nes_c = (ctypes.c_int64 * len(Ns))(*Ns), (ctypes.c_int32 * len(nes))(*nes)
+            if self.free:
+                Ng = len(self.epochs)
+                nbytes = lib.psoap_farm_free_workspace_bytes(ncomp, Ng, len(self.mine), Ns_c, nes_c, K, nb)
+                self._ws = torch.empty(nbytes + 256, dtype=torch.uint8, device="cuda")
+                _lib.check(lib.psoap_farm_create_free(ctypes.byref(self._farm), ncomp, Ng, len(self.mine), descs,
+                                                      self._map_ptrs, K, nb, float(mu_GP), _lib.ptr(self._ws), nbytes))
+            else:
+                nbytes = lib.psoap_farm_workspace_bytes_batched(len(self.mine), Ns_c, nes_c, K, nb)
+                self._ws = torch.empty(nbytes + 256, dtype=torch.uint8, device="cuda")
+                _lib.check(lib.psoap_farm_create_batched(ctypes.byref(self._farm), _lib.MODELS[model], len(self.mine),
+                                                         descs, K, nb, float(mu_GP), _lib.ptr(self._ws), nbytes))
             self.launches_per_eval = lib.psoap_farm_launches_per_eval(self._farm)
+
+    free = False   # free_velocities
+
+    @property
+    def _pname(self):
+        """What the parameter vector is, for the error messages."""
+        return "%s with free velocities at %d epochs" % (self.model, len(self.epochs)) if self.free else self.model
+
+    def _chunk_model(self):
+        """The model id of the chunk entries: the orbit's, or PSOAP_FREEn (each chunk's own epochs)."""
+        return _lib.FREE_MODELS[_lib.NCOMP[self.model]] if self.free else _lib.MODELS[self.model]
 
     # -- per-rank work --------------------------------------------------------------------------------
     def cost_of_mine(self):
@@ -239,8 +308,7 @@ class ChunkFarm:
         p = np.asarray(p, dtype=np.float64).reshape(-1, self.n_params) if np.size(p) == self.n_proposals * self.n_params \
             else None
         if p is None:
-            raise ValueError("p must hold %d x %d registered parameters of %s"
-                             % (self.n_proposals, self.n_params, self.model))
+            raise ValueError("p must hold %d x %d parameters of %s" % (self.n_proposals, self.n_params, self._pname))
         # the previous call's asynchronous upload may still be reading the pinned staging buffer
         if self._p_event is not None:
             self._p_event.synchronize()
@@ -273,11 +341,11 @@ class ChunkFarm:
         torch = _lib.torch_cuda()
         p = np.asarray(p, dtype=np.float64)
         if p.size != self.n_params:
-            raise ValueError("p must hold the %d registered parameters of %s" % (self.n_params, self.model))
+            raise ValueError("p must hold the %d parameters of %s" % (self.n_params, self._pname))
         npar = self.n_params
         rows = torch.zeros((self.n_chunks, npar + 1), dtype=torch.float64, device="cuda")
         if self.mine:
-            model = _lib.MODELS[self.model]
+            model = self._chunk_model()
             if self._grad_ws is None:
                 need = max(lib.psoap_chunk_lnprob_grad_workspace_bytes(model, N, ne)
                            for N, ne in zip(self.Ns, self._n_epochs))
@@ -287,6 +355,16 @@ class ChunkFarm:
             res = torch.empty((len(self.mine), 4), dtype=torch.float64, device="cuda")
             base, stride = rows.data_ptr(), (npar + 1) * 8
             for k, idx in enumerate(self.mine):
+                if self.free:   # the chunk's own vector in, its row scattered to the global epochs (the rest stay 0)
+                    gi = self._free_idx[k]
+                    g_loc = torch.empty(gi.numel(), dtype=torch.float64, device="cuda")
+                    _lib.check(lib.psoap_chunk_lnprob_grad(model, ctypes.byref(self._descs[k]),
+                                                           _lib.ptr(p_dev[gi].contiguous()), self.mu_GP, _lib.ptr(ws),
+                                                           nbytes, _lib.ptr(res[k]), _lib.ptr(g_loc), _lib.stream_ptr()))
+                    rows[idx, 1:].index_copy_(0, gi, g_loc)
+                    # a -inf chunk's row is NaN throughout, as the farm's gradient graph writes it
+                    rows[idx, 1:].masked_fill_(torch.isneginf(res[k, 0]), float("nan"))
+                    continue
                 _lib.check(lib.psoap_chunk_lnprob_grad(model, ctypes.byref(self._descs[k]), _lib.ptr(p_dev),
                                                        self.mu_GP, _lib.ptr(ws), nbytes, _lib.ptr(res[k]),
                                                        _lib.vp(base + idx * stride + 8), _lib.stream_ptr()))
@@ -312,11 +390,11 @@ class ChunkFarm:
         torch = _lib.torch_cuda()
         p = np.asarray(p, dtype=np.float64)
         if p.size != self.n_params:
-            raise ValueError("p must hold the %d registered parameters of %s" % (self.n_params, self.model))
+            raise ValueError("p must hold the %d parameters of %s" % (self.n_params, self._pname))
         npar = self.n_params
         out = torch.zeros((self.n_chunks, npar, npar), dtype=torch.float64, device="cuda")
         if self.mine:
-            model = _lib.MODELS[self.model]
+            model = self._chunk_model()
             nbytes = max(lib.psoap_chunk_fisher_workspace_bytes(model, N, ne) for N, ne in zip(self.Ns, self._n_epochs))
             try:
                 ws = torch.empty(nbytes, dtype=torch.uint8, device="cuda")
@@ -326,6 +404,14 @@ class ChunkFarm:
             p_dev = torch.from_numpy(p.reshape(-1).copy()).cuda()
             res = torch.empty(4, dtype=torch.float64, device="cuda")
             for k, idx in enumerate(self.mine):
+                if self.free:   # the chunk's own matrix, scattered to the global epochs on the device
+                    gi = self._free_idx[k]
+                    F_loc = torch.empty((gi.numel(), gi.numel()), dtype=torch.float64, device="cuda")
+                    _lib.check(lib.psoap_chunk_fisher(model, ctypes.byref(self._descs[k]),
+                                                      _lib.ptr(p_dev[gi].contiguous()), self.mu_GP, _lib.ptr(ws),
+                                                      nbytes, _lib.ptr(res), None, _lib.ptr(F_loc), _lib.stream_ptr()))
+                    out[idx][gi[:, None], gi[None, :]] = F_loc
+                    continue
                 _lib.check(lib.psoap_chunk_fisher(model, ctypes.byref(self._descs[k]), _lib.ptr(p_dev), self.mu_GP,
                                                   _lib.ptr(ws), nbytes, _lib.ptr(res), None, _lib.ptr(out[idx]),
                                                   _lib.stream_ptr()))
@@ -369,7 +455,7 @@ class ChunkFarm:
         P = np.asarray(P, dtype=np.float64)
         K, npar = self.n_proposals, self.n_params
         if P.size != K * npar:
-            raise ValueError("P must hold %d x %d registered parameters of %s" % (K, npar, self.model))
+            raise ValueError("P must hold %d x %d parameters of %s" % (K, npar, self._pname))
         rows = torch.zeros((K, self.n_chunks, npar + 1), dtype=torch.float64, device="cuda")
         if self.mine:
             if self._grad_farm_ws is None:
@@ -461,7 +547,7 @@ class ChunkFarm:
         K, npar = self.n_proposals, self.n_params
         P = np.asarray(P, dtype=np.float64)
         if P.size != K * npar:
-            raise ValueError("P must hold %d x %d registered parameters of %s" % (K, npar, self.model))
+            raise ValueError("P must hold %d x %d parameters of %s" % (K, npar, self._pname))
         mus = np.asarray(mus, dtype=np.float64).reshape(-1)
         if mus.size != ncomp:
             raise ValueError("mus must hold the %d component means of %s" % (ncomp, self.model))

@@ -7,6 +7,7 @@ proposals with a fixed covariance, `sample(p0, iterations)` generator, `flatchai
 `acceptance_fraction`).  Under torchrun every rank runs the same chain from the same seed (the proposals and the
 all-reduced likelihoods are identical on all ranks, so are the accept decisions); rank 0 writes the outputs.
 """
+import collections
 import os
 import shutil
 
@@ -179,6 +180,81 @@ def fisher_jump(F, model, fix_params):
     except np.linalg.LinAlgError as e:
         raise ValueError("the Fisher information of the sampled parameters %s is not positive definite" % names) from e
     return 2.38 ** 2 / len(idx) * np.linalg.inv(F_fit)
+
+
+# --------------------------------------------------------------------------------------------------
+# Per-epoch radial velocities without an orbit (ChunkFarm(..., free_velocities=True))
+# --------------------------------------------------------------------------------------------------
+# fit_epoch_velocities' result: v [ncomp, Ng] (km/s, at farm.epochs), gp [2 ncomp], cov (the Cramer-Rao covariance of
+# the fitted entries, in the order of `free`), free (their positions in the farm's vector), sigma_v [ncomp, Ng] (the
+# square root of cov's diagonal at each velocity; 0 at the reference epoch), lnprob, and scipy's OptimizeResult
+EpochFit = collections.namedtuple("EpochFit", "v gp cov free sigma_v lnprob opt")
+
+
+def epoch_fit_free(ncomp, Ng, ref_epoch=0, fix_gp=False):
+    """Positions in the free vector [v_0[0..Ng), .., GP] that fit_epoch_velocities varies: every velocity except each
+    component's v_c[ref_epoch] (the gauge: the likelihood depends on velocity differences within a component only),
+    and the 2 ncomp GP values unless fix_gp."""
+    if not 0 <= ref_epoch < Ng:
+        raise ValueError("ref_epoch must lie in [0, %d)" % Ng)
+    fixed = {c * Ng + ref_epoch for c in range(ncomp)}
+    n = ncomp * Ng + (0 if fix_gp else 2 * ncomp)
+    return np.array([k for k in range(n) if k not in fixed], dtype=np.int64)
+
+
+def fit_epoch_velocities(farm, v0, gp0, ref_epoch=0, fix_gp=False, options=None):
+    """Maximum-likelihood radial velocity of every component at every epoch, without an orbit: L-BFGS-B (scipy) on
+    farm.lnprob_and_grad for a ChunkFarm built with free_velocities=True.  v0: [ncomp, Ng] starting velocities (km/s,
+    at farm.epochs), gp0: the 2 ncomp GP values.  Each component's v_c[ref_epoch] is held at its v0 value, which fixes
+    the gauge (a constant added to all of a component's velocities leaves the likelihood unchanged); with fix_gp the GP
+    values are held too.  The GP values are bounded below by 0.  Returns an EpochFit; its covariance is the inverse of
+    farm.fisher at the optimum with the fixed rows and columns removed (the Cramer-Rao bound)."""
+    from scipy.optimize import minimize
+    from . import _lib
+    if not getattr(farm, "free", False):
+        raise ValueError("fit_epoch_velocities needs a ChunkFarm built with free_velocities=True")
+    ncomp, Ng = _lib.NCOMP[farm.model], len(farm.epochs)
+    v0 = np.asarray(v0, dtype=np.float64)
+    gp0 = np.asarray(gp0, dtype=np.float64).reshape(-1)
+    if v0.shape != (ncomp, Ng) or gp0.size != 2 * ncomp:
+        raise ValueError("v0 must be [%d, %d] and gp0 hold %d values" % (ncomp, Ng, 2 * ncomp))
+    p0 = np.concatenate([v0.reshape(-1), gp0])
+    free = epoch_fit_free(ncomp, Ng, ref_epoch, fix_gp)
+    nv = ncomp * Ng
+
+    def full(x):
+        p = p0.copy()
+        p[free] = x
+        return p
+
+    def f(x):
+        lnp, g = farm.lnprob_and_grad(full(x))
+        if not np.isfinite(lnp):
+            return np.inf, np.zeros_like(x)
+        return -lnp, -g[free]
+
+    bounds = [(None, None) if k < nv else (0.0, None) for k in free]
+    opt = minimize(f, p0[free], jac=True, method="L-BFGS-B", bounds=bounds, options=options or {})
+    p = full(opt.x)
+    F = np.asarray(farm.fisher(p), dtype=np.float64)[np.ix_(free, free)]
+    cov = np.linalg.inv(F)
+    sig = np.zeros(nv)
+    vfree = free < nv
+    sig[free[vfree]] = np.sqrt(np.diag(cov)[vfree])
+    return EpochFit(p[:nv].reshape(ncomp, Ng), p[nv:], cov, free, sig.reshape(ncomp, Ng), -float(opt.fun), opt)
+
+
+def fit_sb1_epoch_velocities(chunks, v0, amp_f, l_f, ref_epoch=0, mu_GP=1.0, soften=1.0, fix_gp=False, **farm_kw):
+    """Single-lined per-epoch velocities on the dense GP: the counterpart of the reference's celerite per-epoch fit
+    (psoap/covariance.py:426-494), with the velocities at the sorted unique dates of all chunks.  v0: [Ng] starting
+    velocities (km/s).  Builds a one-component free-velocity farm, runs fit_epoch_velocities and releases the farm."""
+    from .farm import ChunkFarm
+    farm = ChunkFarm("SB1", chunks, mu_GP=mu_GP, soften=soften, free_velocities=True, **farm_kw)
+    try:
+        return fit_epoch_velocities(farm, np.asarray(v0, dtype=np.float64).reshape(1, -1), [amp_f, l_f], ref_epoch,
+                                    fix_gp)
+    finally:
+        farm.close()
 
 
 def run(config, chunks, run_index=0, seed=0, rank=0, world_size=1, process_group=None, verbose=True, workdir=None):
