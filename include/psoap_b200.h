@@ -125,6 +125,10 @@ int psoap_lnlike_host(int ncomp, int64_t N, const double *lwl_f, const double *l
  * (T = padded(N) / 128 row blocks); tend[e], e >= 1, is the first row block from which every row of K is exactly zero
  * in block columns [0, e).  The factorisation's launches for panels before e stop there. */
 int psoap_lnlike_envelope_view(void *workspace_dev, int64_t N, int **tend_dev, int *T);
+/* The row profile the same call computed: *profile_dev points at int[T]; profile[I] is the first block column in which
+ * row block I can hold a non-zero (the suffix minimum over rows >= I of each row block's first non-zero block column).
+ * The update tiles of row block I start their k loop at that panel. */
+int psoap_lnlike_profile_view(void *workspace_dev, int64_t N, int **profile_dev, int *T);
 
 /* ---- prediction: psoap/covariance.py:81-297 (Schur complement of a bordered matrix) ------------------- */
 /* In place on a column-major device matrix S [n + m, ld]: the leading n x n block (lower triangle) is
@@ -326,6 +330,14 @@ int psoap_bench_fill(int kind, int ncomp, int64_t N, const double *lwl_f_dev, co
  * (row tile r, 64-column tile jrel) of every tile of a launch over R row tiles for part 0 (all), 1 (first ncol1
  * column tiles of every row) or 2 (the rest).  Returns the tile count, -1 if cap is too small. */
 int psoap_debug_syrk_tiles(int R, int part, int ncol1, int *rows_out, int *cols_out, int cap);
+/* Host-side replay of the k ranges of a trailing-update launch (csrc/gemm.cuh SyrkSrc::kfirst; no device work): R row
+ * blocks from row block row0, tile shape sh (1: 128 x 64, 2: 64 x 32), k range [kbeg, kend) of the group buffer, and
+ * either no profile (prof null: every tile runs [kbeg, kend)) or the row profile prof (host memory, int[T]) with the
+ * group's first panel panel0.  Per tile: row tile and column tile (in units of the shape), first k column and number of
+ * 16-column stages.  Returns the tile count, -1 if cap is too small or an argument is out of range (row0 + R > T with
+ * a profile). */
+int psoap_debug_syrk_tile_k(int R, int part, int ncol1, int sh, int row0, int kbeg, int kend, const int *prof, int T,
+                            int panel0, int *rows_out, int *cols_out, int *kbeg_out, int *kt_out, int cap);
 /* Number of kernels launched by this library since load (for bench.py's gpu_launches). */
 int64_t psoap_launch_count(void);
 

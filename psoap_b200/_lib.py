@@ -59,6 +59,7 @@ SIGNATURES = {
     "psoap_schur_workspace_bytes": (ctypes.c_size_t, [ctypes.c_int64, ctypes.c_int64]),
     "psoap_schur": (ctypes.c_int, [vp, ctypes.c_int64, ctypes.c_int64, ctypes.c_int64, vp, ctypes.c_size_t, vp, vp]),
     "psoap_lnlike_envelope_view": (ctypes.c_int, [vp, ctypes.c_int64, ctypes.POINTER(vp), c_int_p]),
+    "psoap_lnlike_profile_view": (ctypes.c_int, [vp, ctypes.c_int64, ctypes.POINTER(vp), c_int_p]),
     "psoap_schur_views": (ctypes.c_int, [vp, ctypes.c_int64, ctypes.c_int64, ctypes.POINTER(vp), ctypes.POINTER(vp),
                                          ctypes.POINTER(vp)]),
     "psoap_lnlike_grad_workspace_bytes": (ctypes.c_size_t, [ctypes.c_int, ctypes.c_int64]),
@@ -113,6 +114,8 @@ SIGNATURES = {
     "psoap_bench_fill": (ctypes.c_int, [ctypes.c_int, ctypes.c_int, ctypes.c_int64, vp, vp, vp, c_double_p, c_double_p,
                                         ctypes.c_int, c_double_p]),
     "psoap_debug_syrk_tiles": (ctypes.c_int, [ctypes.c_int, ctypes.c_int, ctypes.c_int, c_int_p, c_int_p, ctypes.c_int]),
+    "psoap_debug_syrk_tile_k": (ctypes.c_int, [ctypes.c_int] * 7 + [c_int_p] + [ctypes.c_int] * 2 + [c_int_p] * 4
+                                + [ctypes.c_int]),
     "psoap_launch_count": (ctypes.c_int64, []),
 }
 

@@ -108,8 +108,10 @@ int set_kernel_attributes() {
         if (e == cudaSuccess) e = cudaFuncSetAttribute(potrf_diag7_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, POTRF7_SMEM);
         if (e == cudaSuccess) e = cudaFuncSetAttribute(trsm7_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TRSM7_SMEM);
         if (e == cudaSuccess) e = cudaFuncSetAttribute(trsm3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(syrk3_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, SYRK1_SMEM);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(syrk3_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, Shape<2>::SMEM);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(syrk3_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SYRK1_SMEM);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(syrk3_kernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, Shape<2>::SMEM);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(syrk3_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SYRK1_SMEM);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(syrk3_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Shape<2>::SMEM);
         if (e == cudaSuccess) e = cudaFuncSetAttribute(fisher_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM);
         if (e == cudaSuccess)
             e = cudaFuncSetAttribute(fisher_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, fisher_pair_smem(FISHER_MAXP));
@@ -119,8 +121,10 @@ int set_kernel_attributes() {
         if (e == cudaSuccess) e = cudaFuncSetAttribute(potrf_diag7_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
         if (e == cudaSuccess) e = cudaFuncSetAttribute(trsm7_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
         if (e == cudaSuccess) e = cudaFuncSetAttribute(trsm3_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(syrk3_kernel<1>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(syrk3_kernel<2>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(syrk3_kernel<1, false>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(syrk3_kernel<2, false>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(syrk3_kernel<1, true>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(syrk3_kernel<2, true>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
         int dev = 0;
         if (e == cudaSuccess) e = cudaGetDevice(&dev);
         if (e == cudaSuccess) e = cudaDeviceGetAttribute(&g_num_sms, cudaDevAttrMultiProcessorCount, dev);
@@ -169,6 +173,7 @@ struct FactorWs {
     int* info;
     uint8_t* nz;    // fill_lower_kernel: one byte per lower tile, T (T + 1) / 2 (T = Nt / 128)
     int* tend;      // envelope_kernel: int[T + 1], tend[e] = first row block of the envelope of panels [0, e)
+    int* prof;      // envelope_kernel: int[T], prof[I] = first block column in which row block I can be non-zero
     int64_t Nt;
 };
 
@@ -184,6 +189,7 @@ size_t factor_ws_bytes(int64_t Nt) {
     const int64_t T = Nt / NB;
     b += align_up((size_t)(T * (T + 1) / 2), 256);
     b += align_up((size_t)(T + 1) * 4, 256);
+    b += align_up((size_t)T * 4, 256);
     return b;
 }
 
@@ -203,6 +209,7 @@ void carve_factor_ws(char* base, int64_t Nt, FactorWs* ws, bool with_W) {
     const int64_t T = Nt / NB;
     ws->nz = (uint8_t*)take((size_t)(T * (T + 1) / 2));
     ws->tend = (int*)take((size_t)(T + 1) * 4);
+    ws->prof = (int*)take((size_t)T * 4);
 }
 
 // Streams of one factorisation pipeline: the caller's stream plus a high-priority side stream on which the next
@@ -269,11 +276,17 @@ cudaError_t launch_k(void (*kernel)(KArgs...), unsigned grid, unsigned block, si
 // the update C - 0 leaves C as it is, except that the sign of a zero can differ inside entries that stay zero and are
 // never pivoted.  The kernels read the entry after pdl_wait() and stop their rows there (gemm.cuh row_limit); the grids,
 // the group boundaries and every other host-side choice stay those of the full launch, which bound them from above.
+// profile (with envelope): profile[I] (envelope_kernel's F) is the first block column in which row block I can be
+// non-zero.  The same argument holds along k: the panels of row block I before panel profile[I] are exact +-0, so with
+// groups of 4 panels or more every update tile of row block I (the group update, its look-ahead parts and the in-group
+// column updates) starts its k loop there (gemm.cuh SyrkSrc::kfirst).  A skipped stage would only have added +-0 products to the accumulator: again only
+// the sign of zeros that are never pivoted can differ.  The panel solves and the residual blocks run their full k range.
 // The likelihood is the same bits as the unrestricted factorisation in the same row order.  Rows sorted by wavelength
 // give a narrow envelope (squared-exponential entries underflow to +0 beyond about 38.6 length scales); in any other
 // order it is T_total everywhere and every launch runs in full.
 int launch_factor(const Lanes& ln, double* W, int64_t ld, int T_elim, int T_total, int pad, const FactorWs& ws,
-                  const int* sentinel, double* result, bool identity_border = false, const int* envelope = nullptr) {
+                  const int* sentinel, double* result, bool identity_border = false, const int* envelope = nullptr,
+                  const int* profile = nullptr) {
     const int64_t ldp = ws.Nt;
     CUtensorMap mapW, mapLinv, mapPa[2], mapPb[2], mapPas[2], mapPbs[2];   // ..s: boxes of the small tile shape
     CUtensorMap mapWblk, mapWt, mapL7[3];                                   // chain 7: diagonal block, panel tile, L_kk below its sub-blocks
@@ -301,6 +314,10 @@ int launch_factor(const Lanes& ln, double* W, int64_t ld, int T_elim, int T_tota
     const int G = g_group ? g_group : (ln.group ? ln.group : (T_total >= 96 ? 4 : 2));
     auto pbuf = [&](int q) { return ws.P[q & 1]; };
     auto kbeg_of = [&](int q) { return q == 0 ? (pad / BK) * BK : 0; };
+    // The profile's k start (SyrkSrc<true>) from groups of 4 panels on: C4 (G = 8) 144.7 -> 120.1 ms, C5 (G = 4) 55.4 ->
+    // 53.5 ms.  With G = 2 a tile can skip at most one of its two panels, and the per-tile profile read on a lone
+    // matrix's chain cost more than that saved (C1 1.34 -> 1.36 ms, C3 6.05 -> 6.16 ms); those launches keep SyrkSrc<false>.
+    const bool kstart = profile != nullptr && G >= 4;
     // a very large matrix has hundreds of 32-row panel-solve tiles per panel: the GEMM panel solve wins again
     // (N = 32768: 342 vs 350 ms)
     const int chain = ln.chain ? ln.chain : (T_total >= 192 ? 3 : g_potrf_version);
@@ -339,10 +356,6 @@ int launch_factor(const Lanes& ln, double* W, int64_t ld, int T_elim, int T_tota
         // part 1 (the block columns the next diagonal blocks wait for) of a matrix factored on its own: 64 x 32 tiles,
         // four times the CTAs at a quarter of the latency each
         const int sh = (part == 1 && chain == 7) ? 2 : 1;
-        SyrkSrc src;
-        src.W = W; src.ld = ld; src.row0 = sh * row0; src.res_row0 = row0; src.kbeg = kbeg_of(q); src.kend = kend;
-        src.P = pbuf(q); src.ldp = ldp; src.part = part; src.ncol1 = sh * ncol1;
-        src.tend = envelope; src.tend_at = gstart[q + 1];
         const int ntiles = syrk_ntiles(sh * R, part, sh * ncol1);
         const int nres = (part == 2 || ykb < 0) ? 0 : R;
         if (ntiles + nres == 0) return;
@@ -357,16 +370,28 @@ int launch_factor(const Lanes& ln, double* W, int64_t ld, int T_elim, int T_tota
         const int yield_mode = g_yield_lookahead ? g_yield_lookahead : (T_total >= 96 ? 1 : 2);
         const bool yield_slots = (part == 2 && ln.side != nullptr);
         const double* yk = ws.y + (int64_t)std::max(ykb, 0) * NB;
-        if (sh == 2) {
-            const int nctas = persistent_ctas(ntiles);
-            launch_k(syrk3_kernel<2>, nctas + nres, 256, Shape<2>::SMEM, s, ln.pdl, src, ntiles, nctas, nres, yk, ws.rvec,
-                     res_col0, mapPas[q & 1], mapPbs[q & 1], mapPas[q & 1], mapPbs[q & 1]);
-        } else {
-            SyrkSplit sp = syrk_split(ntiles, yield_slots && yield_mode == 1, part != 1 && g_tail_split != 0);
-            if (yield_slots && yield_mode == 2) sp.nctas = std::min(sp.nmain, g_num_sms - 1);
-            launch_k(syrk3_kernel<1>, nres + sp.nctas + sp.nquarters, 256, sp.nquarters ? SYRK1_SMEM : GEMM_SMEM, s, ln.pdl, src, sp.nmain, sp.nctas, nres,
-                     yk, ws.rvec, res_col0, mapPa[q & 1], mapPb[q & 1], mapPas[q & 1], mapPbs[q & 1]);
-        }
+        // the same launch with (KS) or without the profile's k start
+        auto go = [&](auto ks_tag) {
+            constexpr bool KS = decltype(ks_tag)::value;
+            SyrkSrc<KS> ks;
+            ks.W = W; ks.ld = ld; ks.row0 = sh * row0; ks.res_row0 = row0; ks.kbeg = kbeg_of(q); ks.kend = kend;
+            ks.P = pbuf(q); ks.ldp = ldp; ks.part = part; ks.ncol1 = sh * ncol1;
+            ks.tend = envelope; ks.tend_at = gstart[q + 1];
+            if (KS) { ks.prof = profile; ks.panel0 = gstart[q]; }
+            if (sh == 2) {
+                const int nctas = persistent_ctas(ntiles);
+                launch_k(syrk3_kernel<2, KS>, nctas + nres, 256, Shape<2>::SMEM, s, ln.pdl, ks, ntiles, nctas, nres, yk,
+                         ws.rvec, res_col0, mapPas[q & 1], mapPbs[q & 1], mapPas[q & 1], mapPbs[q & 1]);
+            } else {
+                SyrkSplit sp = syrk_split(ntiles, yield_slots && yield_mode == 1, part != 1 && g_tail_split != 0);
+                if (yield_slots && yield_mode == 2) sp.nctas = std::min(sp.nmain, g_num_sms - 1);
+                launch_k(syrk3_kernel<1, KS>, nres + sp.nctas + sp.nquarters, 256, sp.nquarters ? SYRK1_SMEM : GEMM_SMEM, s,
+                         ln.pdl, ks, sp.nmain, sp.nctas, nres, yk, ws.rvec, res_col0, mapPa[q & 1], mapPb[q & 1],
+                         mapPas[q & 1], mapPbs[q & 1]);
+            }
+        };
+        if (kstart) go(std::true_type{});
+        else go(std::false_type{});
         ++g_launches;
     };
     // Group boundaries.  Uniform groups of G, except at the END of a matrix factored on its own (look-ahead, chain 7):
@@ -456,9 +481,9 @@ int launch_chunk(const Lanes& ln, int ncomp, int64_t N, const ZSource& zs, const
     int rc = launch_fill_lower(ncomp, ln.main, ws.W, Np, T, pad, zs, sigma, fl, mu, gp, ws);
     if (rc) return rc;
     if (T > ENV_MAX_T) return fail(PSOAP_ERR_ARG, "launch_chunk: matrix too large for the envelope");
-    launch_k(envelope_kernel, 1, 256, 0, ln.main, ln.pdl, (const uint8_t*)ws.nz, T, ws.tend);
+    launch_k(envelope_kernel, 1, 256, 0, ln.main, ln.pdl, (const uint8_t*)ws.nz, T, ws.tend, ws.prof);
     LAUNCH_CHECK();
-    return launch_factor(ln, ws.W, Np, T, T, pad, ws, sentinel, result, false, ws.tend);
+    return launch_factor(ln, ws.W, Np, T, T, pad, ws, sentinel, result, false, ws.tend, ws.prof);
 }
 
 // Side stream + events for calls on a caller-provided stream (one set per host thread).
@@ -531,7 +556,7 @@ int dims_nvel(int m, int n_epochs) { return model_free(m) ? dims_ncomp(m) * n_ep
 extern "C" {
 
 const char* psoap_last_error(void) { return g_err.c_str(); }
-int psoap_version(void) { return 104; }
+int psoap_version(void) { return 105; }
 int psoap_device_count(void) {
     int n = 0;
     if (cudaGetDeviceCount(&n) != cudaSuccess) { cudaGetLastError(); return 0; }
@@ -675,6 +700,17 @@ int psoap_lnlike_envelope_view(void* workspace, int64_t N, int** tend, int* T) {
     FactorWs ws;
     carve_factor_ws((char*)workspace, padded_dim(N), &ws, true);
     *tend = ws.tend;
+    *T = (int)(padded_dim(N) / NB);
+    return PSOAP_OK;
+}
+
+// The row profile of the last psoap_lnlike call in `workspace`: int[T] on the device, profile[I] = first block column
+// in which row block I can hold a non-zero (the suffix minimum of the first non-zero block columns, envelope_kernel).
+int psoap_lnlike_profile_view(void* workspace, int64_t N, int** profile, int* T) {
+    if (!workspace || N < 1 || !profile || !T) return fail(PSOAP_ERR_ARG, "psoap_lnlike_profile_view: bad arguments");
+    FactorWs ws;
+    carve_factor_ws((char*)workspace, padded_dim(N), &ws, true);
+    *profile = ws.prof;
     *T = (int)(padded_dim(N) / NB);
     return PSOAP_OK;
 }
@@ -1945,7 +1981,7 @@ int psoap_bench_syrk_split(int64_t m, int K, int reps, int tail_split, double* a
     CUDA_TRY(cudaEventCreate(&e0));
     CUDA_TRY(cudaEventCreate(&e1));
     const int R = (int)(m / NB), ntiles = R * (R + 1);
-    SyrkSrc src;
+    SyrkSrc<> src;
     src.W = W; src.ld = m; src.row0 = 0; src.res_row0 = 0; src.kbeg = 0; src.kend = K; src.P = P; src.ldp = m; src.part = 0; src.ncol1 = 2;
     const SyrkSplit sp = syrk_split(ntiles, false, tail_split != 0);
     CUtensorMap mapPa, mapPb, mapQa, mapQb;
@@ -1955,7 +1991,7 @@ int psoap_bench_syrk_split(int64_t m, int K, int reps, int tail_split, double* a
     if (!rc) rc = make_tensor_map(&mapQb, P, (uint64_t)m, (uint64_t)K, (uint64_t)m, Shape<2>::SB);
     if (rc) return rc;
     auto launch = [&]() {
-        syrk3_kernel<1><<<R + sp.nctas + sp.nquarters, 256, SYRK1_SMEM, st>>>(src, sp.nmain, sp.nctas, R, y, r, 0, mapPa, mapPb,
+        syrk3_kernel<1, false><<<R + sp.nctas + sp.nquarters, 256, SYRK1_SMEM, st>>>(src, sp.nmain, sp.nctas, R, y, r, 0, mapPa, mapPb,
                                                                               mapQa, mapQb);
         ++g_launches;
     };
@@ -2051,11 +2087,38 @@ int psoap_bench_fill(int kind, int ncomp, int64_t N, const double* lwl_f, const 
 // Host-side replay of the trailing-update tile enumeration (no device work): writes (row, column-tile) of every
 // tile of a launch over R row tiles; returns the tile count, or -1 when `cap` is too small.
 int psoap_debug_syrk_tiles(int R, int part, int ncol1, int* rows_out, int* cols_out, int cap) {
-    SyrkSrc src{};
+    SyrkSrc<> src{};
     src.part = part; src.ncol1 = ncol1;
     const int n = syrk_ntiles(R, part, ncol1);
     if (n > cap) return -1;
     for (int t = 0; t < n; ++t) src.decode(t, rows_out[t], cols_out[t]);
+    return n;
+}
+
+// Host-side replay of the k ranges of a trailing-update launch (no device work), as launch_factor sets it up: R row
+// blocks from row block row0, tile shape sh (1: 128 x 64, 2: 64 x 32), k range [kbeg, kend) of the group buffer, and
+// either no profile (prof null: SyrkSrc<false>) or the row profile prof[0 .. T) in host memory with the group's first
+// panel panel0 (SyrkSrc<true>).  Writes, per tile, its row tile (in units of the shape's rows), 64/sh-column tile,
+// first k column and number of 16-column stages; returns the tile count, or -1 when `cap` is too small or an argument
+// is out of range.
+int psoap_debug_syrk_tile_k(int R, int part, int ncol1, int sh, int row0, int kbeg, int kend, const int* prof, int T,
+                            int panel0, int* rows_out, int* cols_out, int* kbeg_out, int* kt_out, int cap) {
+    if (R < 0 || row0 < 0 || (sh != 1 && sh != 2) || part < 0 || part > 2 || kend < BK || kbeg < 0 || kbeg >= kend)
+        return -1;
+    if (prof && (row0 + R > T || panel0 < 0)) return -1;
+    SyrkSrc<true> src{};
+    src.row0 = sh * row0; src.kbeg = kbeg; src.kend = kend; src.part = part; src.ncol1 = sh * ncol1;
+    src.prof = prof; src.panel0 = panel0;
+    const int n = syrk_ntiles(sh * R, part, sh * ncol1);
+    if (n > cap) return -1;
+    for (int t = 0; t < n; ++t) {
+        int r, jrel;
+        src.decode(t, r, jrel);
+        const int I = src.row0 + r;
+        rows_out[t] = I; cols_out[t] = 2 * src.row0 + jrel;
+        kbeg_out[t] = prof ? src.kfirst(I / sh) : kbeg;
+        kt_out[t] = (kend - kbeg_out[t]) / BK;
+    }
     return n;
 }
 

@@ -125,9 +125,12 @@ __global__ void __launch_bounds__(256) fill_lower_kernel(double* __restrict__ W,
 // Row blocks I >= tend[e] are exactly zero in block columns < e, in K and so in L (Cholesky keeps a row's leading
 // zeros), so the launches of a panel group ending at panel e stop at row block tend[e] (api.cu launch_factor).
 // tend does not decrease with e.  Unsorted data has tend = T everywhere: every launch runs in full.
+// F itself is stored too (prof, int[T]): row block I is exactly zero in block columns < F[I], so the update tiles of
+// row block I start their k loop at panel F[I] (gemm.cuh SyrkSrc::kfirst).
 // ------------------------------------------------------------------------------------------------------
 constexpr int ENV_MAX_T = 2048;   // shared-memory suffix minima: matrices up to 262144 rows
-__global__ void __launch_bounds__(256) envelope_kernel(const uint8_t* __restrict__ nz, int T, int* __restrict__ tend) {
+__global__ void __launch_bounds__(256) envelope_kernel(const uint8_t* __restrict__ nz, int T, int* __restrict__ tend,
+                                                       int* __restrict__ prof) {
     __shared__ int F[ENV_MAX_T];
     pdl_wait();
     const int tid = threadIdx.x;
@@ -141,6 +144,7 @@ __global__ void __launch_bounds__(256) envelope_kernel(const uint8_t* __restrict
     if (tid == 0)
         for (int I = T - 2; I >= 0; --I) F[I] = min(F[I], F[I + 1]);
     __syncthreads();
+    for (int I = tid; I < T; I += blockDim.x) prof[I] = F[I];
     for (int e = tid; e <= T; e += blockDim.x) {
         int I = e;
         if (e > 0)

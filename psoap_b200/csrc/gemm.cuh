@@ -115,6 +115,9 @@ struct TrsmSrc {
 //   part 0: all of them
 //   part 1: jrel < ncol1 (ncol1 = 2 per panel of the next group: its block columns, for look-ahead)
 //   part 2: jrel >= ncol1
+// KSTART: every tile starts its k loop at its row block's profile (kfirst).  A compile-time choice, so that the launches
+// without a profile run the same code as before it existed.
+template <bool KSTART = false>
 struct SyrkSrc {
     double* W;
     int64_t ld;
@@ -125,6 +128,11 @@ struct SyrkSrc {
     int part, ncol1;
     const int* tend = nullptr;   // envelope (may be null): row blocks from tend[tend_at] on are skipped (see row_limit)
     int tend_at = 0;
+    // row profile (KSTART only): prof[I] = first block column in which row block I can hold a non-zero (envelope_kernel's
+    // suffix minimum F); panel0 = the block column of the buffer's first panel.  A tile of row block I starts its k
+    // loop at panel prof[I]: before it P_I is exactly zero (Cholesky keeps a row's leading zeros).
+    const int* prof = nullptr;
+    int panel0 = 0;
     static constexpr bool PREFETCH_C = true;   // the next tile's C lines are pulled towards L2 (gemm_persistent)
     // tile index -> (row r, 64-column tile jrel); host-callable so the CPU tests can check the coverage
     __host__ __device__ __forceinline__ void decode(int t, int& r, int& jrel) const {
@@ -153,6 +161,17 @@ struct SyrkSrc {
             r = v + (ncol1 >> 1) - 1;
         }
     }
+    // first k column of the tiles of row block I (128 rows): kbeg, or later where the profile says the row block's
+    // panels are exactly zero.  At least one stage stays (KT >= 1): a row block that is zero in every panel of an in-group
+    // column update runs one stage of +-0 products, which leaves C as it is, instead of none, which would store -C.
+    __host__ __device__ __forceinline__ int kfirst(int I) const {
+#ifdef __CUDA_ARCH__
+        const int F = __ldg(prof + I);
+#else
+        const int F = prof[I];
+#endif
+        return min(max(kbeg, NB * (F - panel0)), kend - BK);
+    }
     // SH = 2: the same enumeration in units of 64-row / 32-column tiles (row0, R, ncol1 are then given in those units;
     // a row tile still owns 2 r + 2 column tiles because TI = 2 TJ in both shapes)
     template <int SH = 1>
@@ -167,8 +186,13 @@ struct SyrkSrc {
         d.lda = ldp;
         d.Bj = P + (int64_t)J * TJ;
         d.ldb = ldp;
-        d.kbeg = kbeg;
-        d.KT = (kend - kbeg) / BK;
+        if constexpr (KSTART) {
+            d.kbeg = kfirst(I / SH);
+            d.KT = (kend - d.kbeg) / BK;
+        } else {
+            d.kbeg = kbeg;
+            d.KT = (kend - kbeg) / BK;
+        }
         d.C = W + (int64_t)I * TI + (int64_t)J * TJ * ld;
         d.ldc = ld;
         d.rowA = I * TI; d.rowB = J * TJ; d.colA0 = d.colB0 = 0;   // both operands: the group buffer's map
@@ -179,8 +203,9 @@ struct SyrkSrc {
 // The last, partial round of a persistent launch as QUARTER tiles (64 x 32, the SH = 2 shape): quarter t of the tail
 // belongs to the 128 x 64 tile first + t / 4.  Each quarter is one CTA behind the persistent ones in the same grid, so
 // the hardware hands them to SM slots as these free up (see syrk3_kernel).  Same k order per entry: same bits.
+template <bool KSTART>
 struct SyrkTailSrc {
-    SyrkSrc base;
+    SyrkSrc<KSTART> base;
     int first;
     static constexpr bool PREFETCH_C = false;   // each quarter CTA reads its one C tile without an L2 prefetch
     template <int SH = 2>
@@ -382,7 +407,8 @@ trsm3_kernel(TrsmSrc src, int ntiles, const __grid_constant__ CUtensorMap mapW, 
 }
 
 // residual block: r_I -= P_I[:, res_col0 .. res_col0+128) y for row tile I = row0 + block (deterministic two-half sum)
-__device__ __forceinline__ void syrk_residual_block(const SyrkSrc& src, const double* __restrict__ yk,
+template <class Src>
+__device__ __forceinline__ void syrk_residual_block(const Src& src, const double* __restrict__ yk,
                                                     double* __restrict__ rvec, int res_col0, double* sm) {
     const int I = src.res_row0 + (int)blockIdx.x;
     const int tid = threadIdx.x;
@@ -402,9 +428,9 @@ __device__ __forceinline__ void syrk_residual_block(const SyrkSrc& src, const do
 // only) each take ONE quarter of the tiles from `ntiles` on: the partial last round of a persistent launch, cut into
 // 64 x 32 pieces that the block scheduler deals out as the persistent CTAs retire (m = 4096, K = 512: 1056 tiles on
 // 296 slots are 3 rounds + 168 tiles; as a 4th round those keep 57 % of the slots busy for a whole tile time).
-template <int SH>
+template <int SH, bool KSTART>
 __global__ void __launch_bounds__(256, CTAS_PER_SM)
-syrk3_kernel(SyrkSrc src, int ntiles, int nctas, int nres, const double* __restrict__ yk, double* __restrict__ rvec,
+syrk3_kernel(SyrkSrc<KSTART> src, int ntiles, int nctas, int nres, const double* __restrict__ yk, double* __restrict__ rvec,
              int res_col0, const __grid_constant__ CUtensorMap mapPa, const __grid_constant__ CUtensorMap mapPb,
              const __grid_constant__ CUtensorMap mapQa, const __grid_constant__ CUtensorMap mapQb) {
     extern __shared__ __align__(128) double sm[];
@@ -425,7 +451,7 @@ syrk3_kernel(SyrkSrc src, int ntiles, int nctas, int nres, const double* __restr
         // same buffer, two boxes: TI + 4 rows for the i operand, TJ + 4 rows for the j operand
         gemm_persistent<1, SH>(src, min(ntiles, ntot), b, nctas, sm, &mapPa, &mapPb);
     } else if constexpr (SH == 1) {
-        SyrkTailSrc tail;
+        SyrkTailSrc<KSTART> tail;
         tail.base = src; tail.first = ntiles;
         const int q = b - nctas;
         if (ntiles + (q >> 2) < ntot) gemm_persistent<1, 2>(tail, q + 1, q, 1 << 30, sm, &mapQa, &mapQb);

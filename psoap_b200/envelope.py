@@ -1,4 +1,5 @@
-"""The factorisation's envelope on the host: exact-zero tile flags, the envelope `tend`, and executed flops.
+"""The factorisation's envelope on the host: exact-zero tile flags, the envelope `tend`, the row profile, and executed
+flops.
 
 The device computes the same envelope from the values its fill stored (fill.cuh envelope_kernel); these functions
 restate it for the tests and for tools/envelope_flops.py.  Tiles are NB x NB with front padding (the first
@@ -46,12 +47,18 @@ def tile_flags_from_z(zs, amps, ls, sigma):
     return flags
 
 
-def tend_by_end(flags):
-    """int[T + 1]: tend[e] = min{I >= e : F[I] >= e} (T when there is none), F the suffix minimum of the first non-zero
-    block column f[I] of every row tile (I itself when the row has no non-zero tile before its diagonal); tend[0] = T."""
+def row_profile(flags):
+    """int[T]: F[I], the suffix minimum of the first non-zero block column f[I] of every row tile (I itself when the
+    row has no non-zero tile before its diagonal).  Row tile I is exactly zero in block columns < F[I], in K and in L."""
     T = flags.shape[0]
     f = np.array([next((J for J in range(I) if flags[I, J]), I) for I in range(T)], dtype=np.int64)
-    F = np.minimum.accumulate(f[::-1])[::-1]
+    return np.minimum.accumulate(f[::-1])[::-1]
+
+
+def tend_by_end(flags):
+    """int[T + 1]: tend[e] = min{I >= e : F[I] >= e} (T when there is none), F = row_profile(flags); tend[0] = T."""
+    T = flags.shape[0]
+    F = row_profile(flags)
     tend = np.full(T + 1, T, dtype=np.int64)
     for e in range(1, T + 1):
         I = e
@@ -65,23 +72,31 @@ def group_starts(T, G):
     return list(range(0, T, G)) + [T]
 
 
-def executed_flops(T, G, tend=None):
+def executed_flops(T, G, tend=None, prof=None):
     """DMMA flops the grouped factorisation executes for T row blocks and groups of G panels (uniform groups; chain 3
     panel solves, 2 * 128 * 64 * (64 + 128) per row block; trailing and in-group updates as 128 x 64 tiles, diagonal
-    tiles in full).  tend None: the dense factorisation."""
+    tiles in full).  tend None: the dense factorisation.  prof (row_profile; with tend): the update tiles of row block
+    I start their k loop at panel max(a, prof[I]) of the group [a, e), and run at least one 16-column stage."""
     gs = group_starts(T, G)
     tile = 2.0 * NB * 64
     total = 0.0
+
+    def k_len(I, a, kb):
+        """k columns a 128 x 64 update tile of row block I runs over the panels [a, kb)."""
+        if prof is None:
+            return NB * (kb - a)
+        return max(16, NB * (kb - max(a, int(prof[I]))))
+
     for q in range(len(gs) - 1):
         a, e = gs[q], gs[q + 1]
         end = T if tend is None else int(tend[e])
         for g in range(e - a):
             kb = a + g
-            if g > 0:
-                total += 2 * (end - kb) * tile * NB * g          # column update of block column kb, K = 128 g
+            if g > 0:                                            # column update of block column kb, K <= 128 g
+                total += sum(2 * tile * k_len(I, a, kb) for I in range(kb, end))
             total += 2 * max(end - kb - 1, 0) * tile * 96        # panel solve: two 128 x 64 tiles, K = 64 and 128
-        R = end - e
-        total += R * (R + 1) * tile * NB * (e - a)                # the group's trailing update
+        # the group's trailing update: row block e + r owns 2 r + 2 tiles
+        total += sum((2 * r + 2) * tile * k_len(e + r, a, e) for r in range(end - e))
     return total
 
 
