@@ -301,6 +301,41 @@ int psoap_farm_predict_attach(psoap_farm *farm, int nbranch, const int64_t *m, c
 int psoap_farm_predict(psoap_farm *farm, const double *p_dev, double *delta_dev, double *sigma_dev,
                        psoap_result *results_dev, void *stream);
 
+/* Posterior draws of the component spectra, in the same prediction graph (one per farm: attach either this or
+ * psoap_farm_predict_attach).  Per item (proposal k, chunk i), after delta and Sigma as psoap_farm_predict writes them:
+ *   L = chol(Sigma + jitter I), factored in place in the item's bordered matrix with the likelihood's kernels;
+ *   X[s] = delta + L z[s], s = 0 .. n_draws - 1, z[s] ~ N(0, I_M), the product on the FP64 tensor pipe (DMMA).
+ * The normals are Philox4x32-10 with key (seed & 0xffffffff, seed >> 32) and counter (a >> 1, s, k, chunk_keys[i]), the
+ * two uniforms u = (((x0 << 32 | x1) >> 11) + 0.5) 2^-53 of outputs (x0, x1) and (x2, x3), and Box-Muller
+ * r = sqrt(-2 log u1), z = r cospi(2 u2) for even a, r sinpi(2 u2) for odd a: a draw's bits depend on (seed, chunk key,
+ * proposal, draw, row) alone, not on nbranch, direct or graph issue, or how the chunks are partitioned over ranks when
+ * chunk_keys holds each chunk's global index.
+ * psoap_farm_predict_draws_workspace_bytes: bytes the attach needs (0 for bad arguments or n_draws outside [1, 2^20]):
+ * psoap_farm_predict_workspace_bytes plus, per branch, Sigma's factorisation scratch and n_draws padded(M) normals of the
+ * largest item, plus the draws n_draws M of every item.
+ * psoap_farm_predict_attach_draws: as psoap_farm_predict_attach, with n_draws >= 1, jitter any finite value (added to
+ * Sigma's diagonal; the Python layer asks for >= 0) and chunk_keys int64 [nchunks] in [0, 2^32) (HOST).  offsets_out:
+ * int64 [3][nitems + 1], rows 0 and 1 as psoap_farm_predict_attach's, row 2 where each item's draws start in draws_dev
+ * (doubles), its last entry that buffer's length. */
+size_t psoap_farm_predict_draws_workspace_bytes(const psoap_farm *farm, int nbranch, const int64_t *m, int sigma_mode,
+                                                int n_draws);
+int psoap_farm_predict_attach_draws(psoap_farm *farm, int nbranch, const int64_t *m, const double *const *grids_dev,
+                                    int sigma_mode, int n_draws, double jitter, const int64_t *chunk_keys,
+                                    void *workspace_dev, size_t workspace_bytes, int64_t *offsets_out);
+/* One call of the draws graph: p_dev, delta_dev, sigma_dev, results_dev as psoap_farm_predict; seed_dev one uint64 on the
+ * device, copied into the graph before the replay (every call may take a new seed).  draws_dev: per item [n_draws][M]
+ * row-major at its offset.  sigma_results_dev [nprop][nchunks]: the record of the factorisation of Sigma + jitter I
+ * (lnlike = -logdet / 2, logdet, quad 0, info: 0 or the 1-based row of Sigma's first non-positive pivot).  Every draw of an
+ * item is NaN when its sentinel fired, its data block's info != 0 or Sigma's info != 0; other items are unaffected.  No
+ * floating-point atomics: bit-identical from call to call.  PSOAP_ERR_ARG on a farm without draws attached;
+ * psoap_farm_predict returns PSOAP_ERR_ARG on a farm with them. */
+int psoap_farm_predict_draws(psoap_farm *farm, const double *p_dev, const uint64_t *seed_dev, double *delta_dev,
+                             double *sigma_dev, double *draws_dev, psoap_result *results_dev,
+                             psoap_result *sigma_results_dev, void *stream);
+/* The draws' generator alone: out_dev [S][M] row-major, z for (seed, chunk_key, proposal) as the draws graph makes them.
+ * Asynchronous on `stream`. */
+int psoap_debug_normals(uint64_t seed, int64_t chunk_key, int proposal, int S, int64_t M, double *out_dev, void *stream);
+
 /* ---- measurement helpers ----------------------------------------------------------------------------- */
 /* Register-resident DMMA.8x8x4 loop on all SMs: measured FP64 tensor-pipe peak in TFLOP/s (synchronous). */
 int psoap_fp64_peak_tflops(double *tflops_out);

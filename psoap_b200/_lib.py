@@ -106,6 +106,13 @@ SIGNATURES = {
     "psoap_farm_predict_attach": (ctypes.c_int, [vp, ctypes.c_int, c_i64_p, ctypes.POINTER(vp), ctypes.c_int, vp,
                                                  ctypes.c_size_t, c_i64_p]),
     "psoap_farm_predict": (ctypes.c_int, [vp, vp, vp, vp, vp, vp]),
+    "psoap_farm_predict_draws_workspace_bytes": (ctypes.c_size_t, [vp, ctypes.c_int, c_i64_p, ctypes.c_int, ctypes.c_int]),
+    "psoap_farm_predict_attach_draws": (ctypes.c_int, [vp, ctypes.c_int, c_i64_p, ctypes.POINTER(vp), ctypes.c_int,
+                                                       ctypes.c_int, ctypes.c_double, c_i64_p, vp, ctypes.c_size_t,
+                                                       c_i64_p]),
+    "psoap_farm_predict_draws": (ctypes.c_int, [vp, vp, vp, vp, vp, vp, vp, vp, vp]),
+    "psoap_debug_normals": (ctypes.c_int, [ctypes.c_uint64, ctypes.c_int64, ctypes.c_int, ctypes.c_int, ctypes.c_int64,
+                                           vp, vp]),
     "psoap_fp64_peak_tflops": (ctypes.c_int, [c_double_p]),
     "psoap_bench_syrk": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int, ctypes.c_int, c_double_p, c_double_p]),
     "psoap_bench_syrk_split": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int, ctypes.c_int, ctypes.c_int, c_double_p, c_double_p]),

@@ -212,6 +212,9 @@ void carve_factor_ws(char* base, int64_t Nt, FactorWs* ws, bool with_W) {
     ws->prof = (int*)take((size_t)T * 4);
 }
 
+// The FactorWs of a matrix factored in place elsewhere (no W): the scratch of Sigma's factorisation in the prediction graph
+size_t sigma_ws_bytes(int64_t Nt) { return factor_ws_bytes(Nt) - align_up((size_t)Nt * Nt * 8, 256); }
+
 // Streams of one factorisation pipeline: the caller's stream plus a high-priority side stream on which the next
 // panel is factored while the bulk of the current trailing update runs (look-ahead).
 struct Lanes {
@@ -284,9 +287,14 @@ cudaError_t launch_k(void (*kernel)(KArgs...), unsigned grid, unsigned block, si
 // The likelihood is the same bits as the unrestricted factorisation in the same row order.  Rows sorted by wavelength
 // give a narrow envelope (squared-exponential entries underflow to +0 beyond about 38.6 length scales); in any other
 // order it is T_total everywhere and every launch runs in full.
+//
+// store_l (T_elim == T_total, no identity border or envelope): W's lower triangle is left holding L itself, the upper
+// triangle of its diagonal tiles exact zeros.  The links keep L only in their scratch (the group buffers, L_kk in Linv),
+// so each finished block column is copied into W behind its panel solve (predict.cuh store_l_kernel); W's block column kb
+// is read by nothing after that solve.  It takes chain 7, whose diagonal kernel leaves L_kk itself (chain 3 its inverse).
 int launch_factor(const Lanes& ln, double* W, int64_t ld, int T_elim, int T_total, int pad, const FactorWs& ws,
                   const int* sentinel, double* result, bool identity_border = false, const int* envelope = nullptr,
-                  const int* profile = nullptr) {
+                  const int* profile = nullptr, bool store_l = false) {
     const int64_t ldp = ws.Nt;
     CUtensorMap mapW, mapLinv, mapPa[2], mapPb[2], mapPas[2], mapPbs[2];   // ..s: boxes of the small tile shape
     CUtensorMap mapWblk, mapWt, mapL7[3];                                   // chain 7: diagonal block, panel tile, L_kk below its sub-blocks
@@ -320,7 +328,7 @@ int launch_factor(const Lanes& ln, double* W, int64_t ld, int T_elim, int T_tota
     const bool kstart = profile != nullptr && G >= 4;
     // a very large matrix has hundreds of 32-row panel-solve tiles per panel: the GEMM panel solve wins again
     // (N = 32768: 342 vs 350 ms)
-    const int chain = ln.chain ? ln.chain : (T_total >= 192 ? 3 : g_potrf_version);
+    const int chain = store_l ? 7 : ln.chain ? ln.chain : (T_total >= 192 ? 3 : g_potrf_version);
     auto potrf = [&](cudaStream_t s, int kb) {
         if (chain == 7)   // blocked: one chain warp, DMMA followers and rank-32 updates (chain.cuh, experimental)
             launch_k(potrf_diag7_kernel, 1, P7_THREADS, POTRF7_SMEM, s, ln.pdl, (const double*)W, ld, kb, pad, ws.Linv,
@@ -421,6 +429,10 @@ int launch_factor(const Lanes& ln, double* W, int64_t ld, int T_elim, int T_tota
             if (g > 0) syrk(s, q, kb, g * NB, 1, 2, kb - 1, (g - 1) * NB);   // block column kb, K = 128 g
             potrf(s, kb); LAUNCH_CHECK();
             if (tend[q] - kb - 1 > 0) { trsm(s, kb, q, g * NB); LAUNCH_CHECK(); }
+            if (store_l) {
+                store_l_kernel<<<tend[q] - kb, 256, 0, s>>>(ws.Linv, pbuf(q) + (int64_t)g * NB * ldp, ldp, W, ld, kb);
+                LAUNCH_CHECK();
+            }
         }
         return PSOAP_OK;
     };
@@ -556,7 +568,7 @@ int dims_nvel(int m, int n_epochs) { return model_free(m) ? dims_ncomp(m) * n_ep
 extern "C" {
 
 const char* psoap_last_error(void) { return g_err.c_str(); }
-int psoap_version(void) { return 105; }
+int psoap_version(void) { return 106; }
 int psoap_device_count(void) {
     int n = 0;
     if (cudaGetDeviceCount(&n) != cudaSuccess) { cudaGetLastError(); return 0; }
@@ -1317,6 +1329,14 @@ struct FarmPredict {
     std::vector<int64_t> sigma_off;   // [nitems + 1] the same into sigma_dev
     double* cap_delta = nullptr;      // scratch outputs the captured graph writes; copied out after a replay
     double* cap_sigma = nullptr;
+    // posterior draws (psoap_farm_predict_attach_draws; n_draws = 0: none, the graph of psoap_farm_predict_attach)
+    int n_draws = 0;
+    double jitter = 0.0;
+    std::vector<uint32_t> chunk_keys; // [nchunks] global chunk index of each of the farm's chunks
+    std::vector<int64_t> draws_off;   // [nitems + 1] offsets (doubles) into draws_dev
+    uint64_t* seed = nullptr;         // the graph's seed word, set from the caller's before every call
+    double* sig_results = nullptr;    // [nitems][4] records of the factorisation of Sigma + jitter I
+    double* cap_draws = nullptr;
 };
 }  // namespace
 
@@ -1445,7 +1465,12 @@ PredictDims predict_item_dims(int ncomp, int64_t N, int64_t m) {
 // The prediction counterpart of farm_issue: velocities and sentinels of every item, then per branch the steps of
 // psoap_predict (mode 0) on the item's shifted pixels: data fill, border fill, elimination of the data block, read-out
 // into the item's offsets of delta and sigma.
-int farm_predict_issue(const psoap_farm* f, const FarmPredict& q, cudaStream_t s0, int pdl, double* delta, double* sigma) {
+//
+// With draws, each item goes on: jitter on Sigma's diagonal in the trailing block (after the read-out, which saw Sigma
+// itself), the factorisation of that block in place into L (launch_factor with store_l, on Sigma's own FactorWs carved
+// behind the data block's), the item's normals Z [S][padded(M)], and X = delta + L Z into the item's offset of draws.
+int farm_predict_issue(const psoap_farm* f, const FarmPredict& q, cudaStream_t s0, int pdl, double* delta, double* sigma,
+                       double* draws = nullptr) {
     const FarmGraph& g = q.g;
     const int nchunks = f->nchunks, ncomp = f->ncomp;
     const int rc0 = launch_item_velocities(f, g, s0);
@@ -1476,6 +1501,24 @@ int farm_predict_issue(const psoap_farm* f, const FarmPredict& q, cudaStream_t s
         predict_farm_readout_kernel<<<dim3(q.sigma_mode ? 1u : nb, nb), 256, 0, sb>>>(
             ws.W, d.Nt, (int)d.Nn, (int)d.M, ws.rvec, ws.info, g.flags + it, q.sigma_mode, sigma + q.sigma_off[it],
             delta + q.delta_off[it]);
+        LAUNCH_CHECK();
+        if (q.n_draws == 0) return PSOAP_OK;
+        const int64_t Mp = d.Nt - d.Nn;
+        double* T = ws.W + d.Nn * (d.Nt + 1);
+        FactorWs sw;
+        carve_factor_ws(g.branch_base[b] + factor_ws_bytes(d.Nt), Mp, &sw, false);
+        double* Z = (double*)(g.branch_base[b] + factor_ws_bytes(d.Nt) + sigma_ws_bytes(Mp));
+        sigma_jitter_kernel<<<1, 256, 0, sb>>>(T, d.Nt, (int)d.M, (int)Mp, q.jitter, sw.rvec, sw.acc, sw.info);
+        LAUNCH_CHECK();
+        rc = launch_factor(farm_lanes(f, g, b, pdl), T, d.Nt, (int)(Mp / NB), (int)(Mp / NB), 0, sw, g.flags + it,
+                           q.sig_results + 4 * it, false, nullptr, nullptr, true);
+        if (rc) return rc;
+        const int S = q.n_draws;
+        normals_kernel<<<dim3((unsigned)((Mp + 255) / 256), (unsigned)std::min(S, 65535)), 128, 0, sb>>>(
+            q.seed, 0, q.chunk_keys[ci], (uint32_t)(it / nchunks), S, (int)d.M, (int)Mp, Z, Mp);
+        LAUNCH_CHECK();
+        predict_draws_kernel<<<dim3((unsigned)(Mp / DR_T), (unsigned)((S + DR_T - 1) / DR_T)), 256, 0, sb>>>(
+            T, d.Nt, (int)d.M, (int)Mp, Z, S, ws.rvec + d.Nn, ws.info, sw.info, g.flags + it, draws + q.draws_off[it]);
         LAUNCH_CHECK();
         return PSOAP_OK;
     });
@@ -1678,28 +1721,41 @@ size_t carve_farm_grad(const psoap_farm* f, char* base, FarmGrad& q) {
 }
 
 // Layout of a prediction workspace: each branch holds factor_ws_bytes(Nt) for the largest bordered item, then the
-// graph's scratch outputs.  Also sets the output offsets of the items.
-size_t carve_farm_predict(const psoap_farm* f, const int64_t* m, int sigma_mode, char* base, FarmPredict& q) {
+// graph's scratch outputs.  Also sets the output offsets of the items.  With n_draws > 0 a branch holds, behind an item's
+// data FactorWs, Sigma's own FactorWs (sigma_ws_bytes) and its normals [n_draws][padded(M)], sized for the largest such
+// sum; the graph adds its seed word, the records of Sigma's factorisation and the draws [n_draws][M] of every item.
+size_t carve_farm_predict(const psoap_farm* f, const int64_t* m, int sigma_mode, int n_draws, char* base, FarmPredict& q) {
     const int nitems = f->nitems, nchunks = f->nchunks;
     // output layout: chunk after chunk, each chunk's proposals side by side, so that a chunk's outputs are contiguous
     q.delta_off.resize(nitems + 1);
     q.sigma_off.resize(nitems + 1);
-    int64_t nd = 0, ns = 0, ntmax = 0;
+    q.draws_off.resize(nitems + 1);
+    int64_t nd = 0, ns = 0, nx = 0, ntmax = 0;
+    size_t branch = 0;
     for (int ci = 0; ci < nchunks; ++ci) {
         const PredictDims d = predict_item_dims(f->ncomp, f->chunks[ci].N, m[ci]);
-        if (m[ci] > 0) ntmax = std::max(ntmax, d.Nt);
+        if (m[ci] > 0) {
+            ntmax = std::max(ntmax, d.Nt);
+            const int64_t Mp = d.Nt - d.Nn;
+            branch = std::max(branch, factor_ws_bytes(d.Nt) + sigma_ws_bytes(Mp) + (size_t)n_draws * Mp * 8);
+        }
         for (int k = 0; k < f->nprop; ++k) {
             const int it = k * nchunks + ci;
-            q.delta_off[it] = nd; q.sigma_off[it] = ns;
-            nd += d.M; ns += sigma_mode ? d.M : d.M * d.M;
+            q.delta_off[it] = nd; q.sigma_off[it] = ns; q.draws_off[it] = nx;
+            nd += d.M; ns += sigma_mode ? d.M : d.M * d.M; nx += (int64_t)n_draws * d.M;
         }
     }
-    q.delta_off[nitems] = nd; q.sigma_off[nitems] = ns;
+    q.delta_off[nitems] = nd; q.sigma_off[nitems] = ns; q.draws_off[nitems] = nx;
+    if (n_draws == 0) branch = ntmax ? factor_ws_bytes(ntmax) : 0;
     Carver c{base};
-    carve_farm_items(c, q.g, f->nprop, nchunks, farm_epochs(f).data(), f->ncomp, ntmax ? factor_ws_bytes(ntmax) : 0,
-                     f->pstride, f->free);
+    carve_farm_items(c, q.g, f->nprop, nchunks, farm_epochs(f).data(), f->ncomp, branch, f->pstride, f->free);
     q.cap_delta = (double*)c.take((size_t)nd * 8);
     q.cap_sigma = (double*)c.take((size_t)ns * 8);
+    if (n_draws > 0) {
+        q.seed = (uint64_t*)c.take(8);
+        q.sig_results = (double*)c.take((size_t)nitems * 4 * 8);
+        q.cap_draws = (double*)c.take((size_t)nx * 8);
+    }
     return c.off;
 }
 }  // namespace
@@ -1888,25 +1944,30 @@ bool predict_args_ok(const psoap_farm* f, int nbranch, const int64_t* m, int sig
 }
 }  // namespace
 
-size_t psoap_farm_predict_workspace_bytes(const psoap_farm* f, int nbranch, const int64_t* m, int sigma_mode) {
+namespace {
+size_t predict_workspace_bytes(const psoap_farm* f, int nbranch, const int64_t* m, int sigma_mode, int n_draws) {
     if (!predict_args_ok(f, nbranch, m, sigma_mode)) return 0;
     FarmPredict probe;
     probe.g.nbranch = std::min(nbranch, f->nitems);
-    return carve_farm_predict(f, m, sigma_mode, nullptr, probe);
+    return carve_farm_predict(f, m, sigma_mode, n_draws, nullptr, probe);
 }
 
-int psoap_farm_predict_attach(psoap_farm* f, int nbranch, const int64_t* m, const double* const* grids, int sigma_mode,
-                              void* workspace, size_t workspace_bytes, int64_t* offsets_out) {
+// The attach both prediction entries share (`who` names the entry in the messages); n_draws = 0: no draws, and
+// chunk_keys / jitter are unused.  offsets_out gets 2 (no draws) or 3 rows of nitems + 1.
+int attach_predict(psoap_farm* f, int nbranch, const int64_t* m, const double* const* grids, int sigma_mode, int n_draws,
+                   double jitter, const int64_t* chunk_keys, void* workspace, size_t workspace_bytes, int64_t* offsets_out,
+                   const char* who) {
+    const std::string w(who);
     if (!predict_args_ok(f, nbranch, m, sigma_mode) || !grids || !workspace || !offsets_out)
-        return fail(PSOAP_ERR_ARG, "psoap_farm_predict_attach: bad arguments");
+        return fail(PSOAP_ERR_ARG, w + ": bad arguments");
     for (int i = 0; i < f->nchunks; ++i)
         for (int c = 0; c < f->ncomp; ++c)
             if (m[i] > 0 && !grids[(size_t)i * f->ncomp + c])
-                return fail(PSOAP_ERR_ARG, "psoap_farm_predict_attach: null grid of chunk " + std::to_string(i));
-    if (f->pred) return fail(PSOAP_ERR_ARG, "psoap_farm_predict_attach: the farm already has a prediction graph");
+                return fail(PSOAP_ERR_ARG, w + ": null grid of chunk " + std::to_string(i));
+    if (f->pred) return fail(PSOAP_ERR_ARG, w + ": the farm already has a prediction graph");
     nbranch = std::min(nbranch, f->nitems);
-    if (((uintptr_t)workspace & 255) || workspace_bytes < psoap_farm_predict_workspace_bytes(f, nbranch, m, sigma_mode))
-        return fail(PSOAP_ERR_WORKSPACE, "psoap_farm_predict_attach: workspace too small or not 256-byte aligned");
+    if (((uintptr_t)workspace & 255) || workspace_bytes < predict_workspace_bytes(f, nbranch, m, sigma_mode, n_draws))
+        return fail(PSOAP_ERR_WORKSPACE, w + ": workspace too small or not 256-byte aligned");
     int rc = set_kernel_attributes();
     if (rc) return rc;
     const int nitems = f->nitems, nchunks = f->nchunks;
@@ -1915,21 +1976,56 @@ int psoap_farm_predict_attach(psoap_farm* f, int nbranch, const int64_t* m, cons
     q->sigma_mode = sigma_mode;
     q->m.assign(m, m + nchunks);
     q->grids.assign(grids, grids + (size_t)nchunks * f->ncomp);
-    carve_farm_predict(f, m, sigma_mode, (char*)workspace, *q);
+    q->n_draws = n_draws;
+    q->jitter = jitter;
+    if (n_draws > 0) q->chunk_keys.assign(chunk_keys, chunk_keys + nchunks);
+    carve_farm_predict(f, m, sigma_mode, n_draws, (char*)workspace, *q);
     // the LPT weight of an item is its bordered dimension Nt (cubed by lpt_items); items of chunks with m = 0 take no work
     std::vector<int64_t> cost(nchunks);
     for (int i = 0; i < nchunks; ++i) cost[i] = m[i] > 0 ? predict_item_dims(f->ncomp, f->chunks[i].N, m[i]).Nt : 0;
     // the records of items with m = 0 are never written by the graph: they read 0 (lnlike, logdet, quad, info)
     cudaError_t e = cudaMemset(q->g.results, 0, (size_t)nitems * 4 * 8);
-    rc = e != cudaSuccess ? fail(PSOAP_ERR_CUDA, std::string("farm predict results: ") + cudaGetErrorString(e))
+    if (e == cudaSuccess && n_draws > 0) e = cudaMemset(q->sig_results, 0, (size_t)nitems * 4 * 8);
+    rc = e != cudaSuccess ? fail(PSOAP_ERR_CUDA, w + " results: " + cudaGetErrorString(e))
                           : attach_farm_graph(f, q->g, cost, true, [f, q](cudaStream_t s0, int pdl) {
-                                return farm_predict_issue(f, *q, s0, pdl, q->cap_delta, q->cap_sigma);
+                                return farm_predict_issue(f, *q, s0, pdl, q->cap_delta, q->cap_sigma, q->cap_draws);
                             });
     if (rc != PSOAP_OK) { delete q; return rc; }
     f->pred = q;
     std::copy(q->delta_off.begin(), q->delta_off.end(), offsets_out);
     std::copy(q->sigma_off.begin(), q->sigma_off.end(), offsets_out + nitems + 1);
+    if (n_draws > 0) std::copy(q->draws_off.begin(), q->draws_off.end(), offsets_out + 2 * (nitems + 1));
     return PSOAP_OK;
+}
+
+// One call of the prediction graph: outputs of the draws graph when draws_dev is set (the caller has checked which graph
+// the farm holds)
+int run_predict(psoap_farm* f, const double* p_dev, double* delta_dev, double* sigma_dev, double* draws_dev,
+                psoap_result* results_dev, cudaStream_t st) {
+    FarmPredict& q = *f->pred;
+    // direct issue writes into the caller's buffers; the captured graph into its own, copied out after the replay
+    int rc = run_farm_graph(f, q.g, p_dev, results_dev, st, [f, &q, delta_dev, sigma_dev, draws_dev](cudaStream_t s0, int pdl) {
+        return farm_predict_issue(f, q, s0, pdl, delta_dev, sigma_dev, draws_dev);
+    });
+    if (rc) return rc;
+    if (!q.g.direct) {
+        CUDA_TRY(cudaMemcpyAsync(delta_dev, q.cap_delta, (size_t)q.delta_off[f->nitems] * 8, cudaMemcpyDeviceToDevice, st));
+        CUDA_TRY(cudaMemcpyAsync(sigma_dev, q.cap_sigma, (size_t)q.sigma_off[f->nitems] * 8, cudaMemcpyDeviceToDevice, st));
+        if (draws_dev)
+            CUDA_TRY(cudaMemcpyAsync(draws_dev, q.cap_draws, (size_t)q.draws_off[f->nitems] * 8, cudaMemcpyDeviceToDevice, st));
+    }
+    return PSOAP_OK;
+}
+}  // namespace
+
+size_t psoap_farm_predict_workspace_bytes(const psoap_farm* f, int nbranch, const int64_t* m, int sigma_mode) {
+    return predict_workspace_bytes(f, nbranch, m, sigma_mode, 0);
+}
+
+int psoap_farm_predict_attach(psoap_farm* f, int nbranch, const int64_t* m, const double* const* grids, int sigma_mode,
+                              void* workspace, size_t workspace_bytes, int64_t* offsets_out) {
+    return attach_predict(f, nbranch, m, grids, sigma_mode, 0, 0.0, nullptr, workspace, workspace_bytes, offsets_out,
+                          "psoap_farm_predict_attach");
 }
 
 int psoap_farm_predict(psoap_farm* f, const double* p_dev, double* delta_dev, double* sigma_dev,
@@ -1937,17 +2033,59 @@ int psoap_farm_predict(psoap_farm* f, const double* p_dev, double* delta_dev, do
     if (!f || !p_dev || !delta_dev || !sigma_dev || !results_dev)
         return fail(PSOAP_ERR_ARG, "psoap_farm_predict: bad arguments");
     if (!f->pred) return fail(PSOAP_ERR_ARG, "psoap_farm_predict: no prediction graph (psoap_farm_predict_attach first)");
+    if (f->pred->n_draws > 0)
+        return fail(PSOAP_ERR_ARG, "psoap_farm_predict: the farm's prediction graph draws samples: call psoap_farm_predict_draws");
+    return run_predict(f, p_dev, delta_dev, sigma_dev, nullptr, results_dev, (cudaStream_t)stream);
+}
+
+// ---- posterior draws of the prediction graph ----------------------------------------------------------------------
+// n_draws <= DRAWS_MAX keeps the product's grid (64 draws per CTA row) inside gridDim.y
+constexpr int DRAWS_MAX = 1 << 20;
+
+size_t psoap_farm_predict_draws_workspace_bytes(const psoap_farm* f, int nbranch, const int64_t* m, int sigma_mode,
+                                                int n_draws) {
+    if (n_draws < 1 || n_draws > DRAWS_MAX) return 0;
+    return predict_workspace_bytes(f, nbranch, m, sigma_mode, n_draws);
+}
+
+int psoap_farm_predict_attach_draws(psoap_farm* f, int nbranch, const int64_t* m, const double* const* grids,
+                                    int sigma_mode, int n_draws, double jitter, const int64_t* chunk_keys, void* workspace,
+                                    size_t workspace_bytes, int64_t* offsets_out) {
+    if (!f || n_draws < 1 || n_draws > DRAWS_MAX || !std::isfinite(jitter) || !chunk_keys)
+        return fail(PSOAP_ERR_ARG, "psoap_farm_predict_attach_draws: bad arguments");
+    for (int i = 0; i < f->nchunks; ++i)
+        if (chunk_keys[i] < 0 || chunk_keys[i] > (int64_t)UINT32_MAX)
+            return fail(PSOAP_ERR_ARG, "psoap_farm_predict_attach_draws: chunk key " + std::to_string(i) +
+                                           " outside [0, 2^32)");
+    return attach_predict(f, nbranch, m, grids, sigma_mode, n_draws, jitter, chunk_keys, workspace, workspace_bytes,
+                          offsets_out, "psoap_farm_predict_attach_draws");
+}
+
+int psoap_farm_predict_draws(psoap_farm* f, const double* p_dev, const uint64_t* seed_dev, double* delta_dev,
+                             double* sigma_dev, double* draws_dev, psoap_result* results_dev,
+                             psoap_result* sigma_results_dev, void* stream) {
+    if (!f || !p_dev || !seed_dev || !delta_dev || !sigma_dev || !draws_dev || !results_dev || !sigma_results_dev)
+        return fail(PSOAP_ERR_ARG, "psoap_farm_predict_draws: bad arguments");
+    if (!f->pred || f->pred->n_draws == 0)
+        return fail(PSOAP_ERR_ARG, "psoap_farm_predict_draws: no draws attached (psoap_farm_predict_attach_draws first)");
     FarmPredict& q = *f->pred;
     cudaStream_t st = (cudaStream_t)stream;
-    // direct issue writes into the caller's buffers; the captured graph into its own, copied out after the replay
-    int rc = run_farm_graph(f, q.g, p_dev, results_dev, st, [f, &q, delta_dev, sigma_dev](cudaStream_t s0, int pdl) {
-        return farm_predict_issue(f, q, s0, pdl, delta_dev, sigma_dev);
-    });
+    CUDA_TRY(cudaMemcpyAsync(q.seed, seed_dev, 8, cudaMemcpyDeviceToDevice, st));
+    int rc = run_predict(f, p_dev, delta_dev, sigma_dev, draws_dev, results_dev, st);
     if (rc) return rc;
-    if (!q.g.direct) {
-        CUDA_TRY(cudaMemcpyAsync(delta_dev, q.cap_delta, (size_t)q.delta_off[f->nitems] * 8, cudaMemcpyDeviceToDevice, st));
-        CUDA_TRY(cudaMemcpyAsync(sigma_dev, q.cap_sigma, (size_t)q.sigma_off[f->nitems] * 8, cudaMemcpyDeviceToDevice, st));
-    }
+    CUDA_TRY(cudaMemcpyAsync(sigma_results_dev, q.sig_results, (size_t)f->nitems * sizeof(psoap_result),
+                             cudaMemcpyDeviceToDevice, st));
+    return PSOAP_OK;
+}
+
+// The generator of the draws alone: Z[s][a] (row-major [S][M]) for (seed, chunk_key, proposal)
+int psoap_debug_normals(uint64_t seed, int64_t chunk_key, int proposal, int S, int64_t M, double* out_dev, void* stream) {
+    if (chunk_key < 0 || chunk_key > (int64_t)UINT32_MAX || proposal < 0 || S < 1 || M < 1 || M > (int64_t)1 << 30 ||
+        !out_dev)
+        return fail(PSOAP_ERR_ARG, "psoap_debug_normals: bad arguments");
+    normals_kernel<<<dim3((unsigned)((M + 255) / 256), (unsigned)std::min(S, 65535)), 128, 0, (cudaStream_t)stream>>>(
+        nullptr, seed, (uint32_t)chunk_key, (uint32_t)proposal, S, (int)M, (int)M, out_dev, M);
+    LAUNCH_CHECK();
     return PSOAP_OK;
 }
 

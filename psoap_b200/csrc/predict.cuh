@@ -196,4 +196,148 @@ __global__ void __launch_bounds__(256) predict_farm_readout_kernel(const double*
     }
 }
 
+// ---- posterior draws X = delta + L_Sigma Z (psoap_farm_predict_attach_draws) ------------------------------------------
+// Philox4x32-10 (Salmon et al., SC'11; the Random123 constants): counter c, key k.
+__host__ __device__ __forceinline__ void philox4x32_10(uint32_t (&c)[4], uint32_t k0, uint32_t k1) {
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        const uint64_t p0 = (uint64_t)0xD2511F53u * c[0], p1 = (uint64_t)0xCD9E8D57u * c[2];
+        const uint32_t n0 = (uint32_t)(p1 >> 32) ^ c[1] ^ k0, n2 = (uint32_t)(p0 >> 32) ^ c[3] ^ k1;
+        c[0] = n0; c[1] = (uint32_t)p1; c[2] = n2; c[3] = (uint32_t)p0;
+        k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
+    }
+}
+
+// A uniform from two 32-bit outputs: the top 53 bits of (hi << 32 | lo), plus one half, times 2^-53.  Never 0, so the
+// logarithm of Box-Muller is finite; the sum rounds to 2^53 for the top 2^11 words, where u = 1 and the pair is 0.
+__device__ __forceinline__ double philox_uniform(uint32_t hi, uint32_t lo) {
+    const uint64_t v = (((uint64_t)hi << 32) | lo) >> 11;
+    return __dmul_rn(__dadd_rn((double)v, 0.5), 0x1p-53);
+}
+
+// Standard normals of rows a = 2j and 2j + 1 of draw s for (seed, chunk key, proposal): one Philox block with key
+// (seed low, seed high) and counter (j, s, proposal, chunk key), Box-Muller on its two uniforms, the cosine for the
+// even row and the sine for the odd one.  Nothing else enters, so a draw's bits do not depend on where or in which
+// order it is generated.
+__device__ __forceinline__ void normal_pair(uint64_t seed, uint32_t chunk_key, uint32_t proposal, uint32_t s, uint32_t j,
+                                            double& z_even, double& z_odd) {
+    uint32_t c[4] = {j, s, proposal, chunk_key};
+    philox4x32_10(c, (uint32_t)seed, (uint32_t)(seed >> 32));
+    const double u1 = philox_uniform(c[0], c[1]), u2 = philox_uniform(c[2], c[3]);
+    const double r = sqrt(__dmul_rn(-2.0, log(u1)));
+    double sn, cs;
+    sincospi(__dmul_rn(2.0, u2), &sn, &cs);
+    z_even = __dmul_rn(r, cs);
+    z_odd = __dmul_rn(r, sn);
+}
+
+// Z[s][a] (row s at out + s ld) for a < M, zero for M <= a < Mrows, s < S.  The seed is *seed_dev when that is not null
+// (the prediction graph's own word, set before every replay), else `seed`.  Grid (ceil(Mrows / 256), min(S, 65535)).
+__global__ void __launch_bounds__(128) normals_kernel(const uint64_t* __restrict__ seed_dev, uint64_t seed, uint32_t chunk_key,
+                                                      uint32_t proposal, int S, int M, int Mrows, double* __restrict__ out,
+                                                      int64_t ld) {
+    if (seed_dev) seed = *seed_dev;
+    const int j = blockIdx.x * blockDim.x + threadIdx.x, a = 2 * j;
+    if (a >= Mrows) return;
+    for (int s = blockIdx.y; s < S; s += gridDim.y) {
+        double z0 = 0.0, z1 = 0.0;
+        if (a < M) normal_pair(seed, chunk_key, proposal, (uint32_t)s, (uint32_t)j, z0, z1);
+        double* o = out + (int64_t)s * ld;
+        o[a] = z0;
+        if (a + 1 < Mrows) o[a + 1] = (a + 1 < M) ? z1 : 0.0;
+    }
+}
+
+// Before the factorisation of Sigma + jitter I in place (the trailing block T of an item, after the read-out): jitter on
+// the M live diagonal entries, and the residual [Mp], accumulators and info word of Sigma's own FactorWs zeroed.
+__global__ void __launch_bounds__(256) sigma_jitter_kernel(double* __restrict__ T, int64_t ld, int M, int Mp, double jitter,
+                                                           double* __restrict__ rvec, double* __restrict__ acc,
+                                                           int* __restrict__ info) {
+    for (int a = threadIdx.x; a < Mp; a += blockDim.x) {
+        if (a < M) T[a + (int64_t)a * ld] = __dadd_rn(T[a + (int64_t)a * ld], jitter);
+        rvec[a] = 0.0;
+    }
+    if (threadIdx.x < 8) acc[threadIdx.x] = 0.0;
+    if (threadIdx.x < 2) info[threadIdx.x] = 0;
+}
+
+// Block column kb of L into the factored matrix T as its panel finishes (launch_factor's lstore): the diagonal tile from
+// Lkk (potrf_diag7's L_kk, column-major [128, 128]) with exact zeros above the diagonal, the R row blocks below it from
+// the panel P (rows absolute, leading dimension ldp).  Grid R + 1: CTA 0 the diagonal tile, CTA b row block kb + b.
+__global__ void __launch_bounds__(256) store_l_kernel(const double* __restrict__ Lkk, const double* __restrict__ P,
+                                                      int64_t ldp, double* __restrict__ T, int64_t ld, int kb) {
+    const int I = kb + (int)blockIdx.x;
+    const int r = threadIdx.x & (NB - 1);
+    double* dst = T + (int64_t)I * NB + r + (int64_t)kb * NB * ld;
+    for (int c = threadIdx.x >> 7; c < NB; c += 2) {
+        const double v = blockIdx.x == 0 ? (r >= c ? Lkk[r + c * NB] : 0.0) : P[(int64_t)I * NB + r + (int64_t)c * ldp];
+        dst[(int64_t)c * ld] = v;
+    }
+}
+
+// X[s][a] = delta[a] + sum_{k <= a} L[a][k] Z[s][k] for a < M, s < S, row-major at X (row length M); delta[a] = -rtail[a]
+// (the carried residual the read-out negates).  L: the lower triangle of T (column-major, ld), read with k <= a, so
+// whatever lies above the diagonal is never used; Z: [S][Mp], zero in rows M.. of each draw.  A CTA owns 64 rows a and 64
+// draws s; its k loop ends at its diagonal tile.  DMMA m8n8k4 with M <-> s, N <-> a: a thread's two accumulators are
+// two consecutive a of one draw.  Warps 2 (s) x 4 (a), each 32 s x 16 a.  Every draw is NaN when the item's sentinel
+// fired or either factorisation failed (the data block's info, Sigma's info).
+constexpr int DR_T = 64, DR_K = 32, DR_LP = DR_T + 8, DR_ZP = DR_K + 4;
+__global__ void __launch_bounds__(256) predict_draws_kernel(const double* __restrict__ T, int64_t ld, int M, int Mp,
+                                                            const double* __restrict__ Z, int S,
+                                                            const double* __restrict__ rtail, const int* __restrict__ info_data,
+                                                            const int* __restrict__ info_sigma, const int* __restrict__ sentinel,
+                                                            double* __restrict__ X) {
+    __shared__ double sL[DR_K][DR_LP];   // sL[k][a] = L[a0 + a][k0 + k], masked to k <= a
+    __shared__ double sZ[DR_T][DR_ZP];   // sZ[s][k] = Z[s0 + s][k0 + k]
+    const int a0 = blockIdx.x * DR_T, s0 = blockIdx.y * DR_T;
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g4 = lane >> 2, tq = lane & 3;
+    const int ws = warp & 1, wa = warp >> 1;
+    double acc[4][2][2];
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+#pragma unroll
+        for (int j = 0; j < 2; ++j) acc[i][j][0] = acc[i][j][1] = 0.0;
+    const int kend = min(a0 + DR_T, Mp);
+#pragma unroll 1
+    for (int k0 = 0; k0 < kend; k0 += DR_K) {
+#pragma unroll
+        for (int e = tid; e < DR_K * DR_T; e += 256) {
+            const int a = e & (DR_T - 1), k = e / DR_T;
+            sL[k][a] = (k0 + k <= a0 + a) ? T[(a0 + a) + (int64_t)(k0 + k) * ld] : 0.0;
+        }
+#pragma unroll
+        for (int e = tid; e < DR_K * DR_T; e += 256) {
+            const int k = e & (DR_K - 1), s = e / DR_K;
+            sZ[s][k] = (s0 + s < S) ? Z[(k0 + k) + (int64_t)(s0 + s) * Mp] : 0.0;
+        }
+        __syncthreads();
+#pragma unroll
+        for (int kk = 0; kk < DR_K / 4; ++kk) {
+            double fa[4], fb[2];
+#pragma unroll
+            for (int i = 0; i < 4; ++i) fa[i] = sZ[ws * 32 + i * 8 + g4][kk * 4 + tq];
+#pragma unroll
+            for (int j = 0; j < 2; ++j) fb[j] = sL[kk * 4 + tq][wa * 16 + j * 8 + g4];
+#pragma unroll
+            for (int i = 0; i < 4; ++i)
+#pragma unroll
+                for (int j = 0; j < 2; ++j) dmma_8x8x4(acc[i][j][0], acc[i][j][1], fa[i], fb[j]);
+        }
+        __syncthreads();
+    }
+    const bool bad = sentinel[0] != 0 || info_data[0] != 0 || info_sigma[0] != 0;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        const int s = s0 + ws * 32 + i * 8 + g4;
+        if (s >= S) continue;
+#pragma unroll
+        for (int j = 0; j < 2; ++j)
+#pragma unroll
+            for (int e = 0; e < 2; ++e) {
+                const int a = a0 + wa * 16 + j * 8 + 2 * tq + e;
+                if (a < M) X[(int64_t)s * M + a] = bad ? CUDART_NAN : __dadd_rn(-rtail[a], acc[i][j][e]);
+            }
+    }
+}
+
 }  // namespace psoap

@@ -478,18 +478,26 @@ class ChunkFarm:
         lnp = np.array([float(np.sum(hk[:, 0])) for hk in h])
         return lnp, np.stack([np.sum(hk[:, 1:], axis=0) for hk in h])
 
-    def attach_prediction_grids(self, grids, sigma="full", predict_nbranch=None):
+    def attach_prediction_grids(self, grids, sigma="full", predict_nbranch=None, n_draws=0, jitter=1e-8):
         """Attach the prediction graph (psoap_farm_predict_attach) for predict_components: grids holds one entry per
         chunk in global chunk order, a 1-D rest-frame ln-wavelength grid used for every component or an [ncomp, m]
         array (lwl_f_predict, lwl_g_predict[, lwl_h_predict] of predict_f_g / _f_g_h); a chunk without pixels takes an
         empty grid.  sigma: "full" (Sigma) or "diag" (its diagonal).  predict_nbranch: (proposal, chunk) items in
         flight (default PREDICT_NBRANCH); each branch holds the bordered matrix of the largest item,
         8 (padded(N) + padded(ncomp m))^2 bytes.  The grids are uploaded once; a farm that never calls this allocates
-        and captures nothing for prediction."""
+        and captures nothing for prediction.  n_draws > 0 attaches the draws graph instead (psoap_farm_predict_attach_draws),
+        for draw_components: n_draws posterior draws of every item from N(mu, Sigma + jitter I), jitter (absolute, >= 0)
+        the reference's nugget 1e-8 by default; predict_components is then not available on this farm."""
         if self._pred is not None:
             raise RuntimeError("the prediction grids are already attached to this farm")
         if sigma not in ("full", "diag"):
             raise ValueError('sigma must be "full" or "diag", not %r' % (sigma,))
+        if isinstance(n_draws, bool) or not isinstance(n_draws, (int, np.integer)) or n_draws < 0:
+            raise ValueError("n_draws must be an int >= 0, not %r" % (n_draws,))
+        n_draws = int(n_draws)
+        jitter = float(jitter)
+        if not np.isfinite(jitter) or jitter < 0.0:
+            raise ValueError("jitter must be finite and >= 0, not %r" % (jitter,))
         nb = int(predict_nbranch) if predict_nbranch is not None else PREDICT_NBRANCH
         if nb < 1:
             raise ValueError("predict_nbranch must be at least 1")
@@ -505,7 +513,9 @@ class ChunkFarm:
         # side: the layout psoap_farm_predict_attach returns for a farm that holds every chunk
         d0 = np.concatenate([[0], np.cumsum([K * M for M in M_all])]).astype(np.int64)
         s0 = np.concatenate([[0], np.cumsum([K * x for x in size])]).astype(np.int64)
-        pred = dict(mode=mode, m=m_all, M=M_all, d0=d0, s0=s0, ws=None, grids=None, off=None)
+        x0 = np.concatenate([[0], np.cumsum([K * n_draws * M for M in M_all])]).astype(np.int64)
+        pred = dict(mode=mode, m=m_all, M=M_all, d0=d0, s0=s0, x0=x0, n_draws=n_draws, jitter=jitter, ws=None, grids=None,
+                    off=None)
         if self.mine:
             total, offs = 0, []
             for i in self.mine:
@@ -520,7 +530,12 @@ class ChunkFarm:
             ptrs = (_lib.vp * (len(self.mine) * ncomp))(
                 *[_lib.vp(base + o + c * m_all[i] * 8) for i, o in zip(self.mine, offs) for c in range(ncomp)])
             m_mine = (ctypes.c_int64 * len(self.mine))(*[m_all[i] for i in self.mine])
-            nbytes = lib.psoap_farm_predict_workspace_bytes(self._farm, nb, m_mine, mode)
+            if n_draws:
+                nbytes = lib.psoap_farm_predict_draws_workspace_bytes(self._farm, nb, m_mine, mode, n_draws)
+                if nbytes == 0:
+                    raise ValueError("n_draws = %d is out of range" % n_draws)
+            else:
+                nbytes = lib.psoap_farm_predict_workspace_bytes(self._farm, nb, m_mine, mode)
             try:
                 ws = torch.empty(nbytes + 256, dtype=torch.uint8, device="cuda")
             except torch.cuda.OutOfMemoryError as e:
@@ -528,9 +543,16 @@ class ChunkFarm:
                                   "bordered matrix of the largest item per branch); pass a smaller predict_nbranch"
                                   % (nbytes, nb)) from e
             nitems = K * len(self.mine)
-            off = (ctypes.c_int64 * (2 * (nitems + 1)))()
-            _lib.check(lib.psoap_farm_predict_attach(self._farm, nb, m_mine, ptrs, mode, _lib.ptr(ws), nbytes, off))
-            off = np.frombuffer(off, dtype=np.int64).reshape(2, nitems + 1).copy()
+            rows = 3 if n_draws else 2
+            off = (ctypes.c_int64 * (rows * (nitems + 1)))()
+            if n_draws:
+                # the chunks' global indices key the normals: the draws do not depend on the partition over ranks
+                keys = (ctypes.c_int64 * len(self.mine))(*self.mine)
+                _lib.check(lib.psoap_farm_predict_attach_draws(self._farm, nb, m_mine, ptrs, mode, n_draws, jitter, keys,
+                                                               _lib.ptr(ws), nbytes, off))
+            else:
+                _lib.check(lib.psoap_farm_predict_attach(self._farm, nb, m_mine, ptrs, mode, _lib.ptr(ws), nbytes, off))
+            off = np.frombuffer(off, dtype=np.int64).reshape(rows, nitems + 1).copy()
             pred.update(ws=ws, grids=gdev, off=off)
         self._pred = pred
 
@@ -554,6 +576,9 @@ class ChunkFarm:
         if self._pred is None:
             raise RuntimeError("attach_prediction_grids must be called before predict_components")
         q = self._pred
+        if q.get("n_draws"):
+            raise RuntimeError("this farm's prediction graph draws samples (n_draws = %d): call draw_components"
+                               % q["n_draws"])
         lib = _lib.load()
         torch = _lib.torch_cuda()
         delta = torch.zeros(int(q["d0"][-1]), dtype=torch.float64, device="cuda")
@@ -595,6 +620,83 @@ class ChunkFarm:
             mu = delta[q["d0"][i]:q["d0"][i + 1]].view(K, M) + torch.from_numpy(np.repeat(mus, m)).cuda()
             s = sig[q["s0"][i]:q["s0"][i + 1]]
             out.append((mu, s.view(K, M, M) if q["mode"] == 0 else s.view(K, M)))
+        return out
+
+    def draw_components(self, P, mus, seed):
+        """predict_components with posterior draws (attach_prediction_grids with n_draws > 0 first): per chunk in global
+        chunk order (mu [n_proposals, M], Sigma [n_proposals, M, M] or var [n_proposals, M], draws [n_proposals,
+        n_draws, M]) as device tensors, M = ncomp m, draws[k, s] = mu[k] + L_k z (L_k the Cholesky factor of
+        Sigma_k + jitter I, z standard normal).  Draws over all proposals are samples of the posterior predictive.  seed:
+        an int in [0, 2^64); the normals depend only on (seed, chunk, proposal, draw, row), so the draws are the same
+        bits for any predict_nbranch and any number of ranks.  Raises numpy.linalg.LinAlgError for an item whose data
+        block is not positive definite, a separate LinAlgError naming the jitter when Sigma + jitter I is not, and
+        ValueError for a velocity at c or a negative GP value, naming the proposal and the chunk."""
+        ncomp = _lib.NCOMP[self.model]
+        K, npar = self.n_proposals, self.n_params
+        P = np.asarray(P, dtype=np.float64)
+        if P.size != K * npar:
+            raise ValueError("P must hold %d x %d parameters of %s" % (K, npar, self._pname))
+        mus = np.asarray(mus, dtype=np.float64).reshape(-1)
+        if mus.size != ncomp:
+            raise ValueError("mus must hold the %d component means of %s" % (ncomp, self.model))
+        if isinstance(seed, bool) or not isinstance(seed, (int, np.integer)) or not 0 <= int(seed) < 2 ** 64:
+            raise ValueError("seed must be an int in [0, 2^64), not %r" % (seed,))
+        if self._pred is None or not self._pred.get("n_draws"):
+            raise RuntimeError("draw_components needs attach_prediction_grids(..., n_draws > 0) first")
+        q = self._pred
+        S = q["n_draws"]
+        lib = _lib.load()
+        torch = _lib.torch_cuda()
+        delta = torch.zeros(int(q["d0"][-1]), dtype=torch.float64, device="cuda")
+        sig = torch.zeros(int(q["s0"][-1]), dtype=torch.float64, device="cuda")
+        draws = torch.zeros(int(q["x0"][-1]), dtype=torch.float64, device="cuda")
+        res = torch.zeros((2, K, self.n_chunks, 4), dtype=torch.float64, device="cuda")
+        if self.mine:
+            off = q["off"]
+            n_mine = len(self.mine)
+            p_dev = torch.from_numpy(np.ascontiguousarray(P.reshape(K, npar))).cuda()
+            seed_dev = torch.tensor([int(seed) - 2 ** 64 if int(seed) >= 2 ** 63 else int(seed)], dtype=torch.int64,
+                                    device="cuda")
+            dl = torch.empty(max(1, int(off[0, -1])), dtype=torch.float64, device="cuda")
+            sl = torch.empty(max(1, int(off[1, -1])), dtype=torch.float64, device="cuda")
+            xl = torch.empty(max(1, int(off[2, -1])), dtype=torch.float64, device="cuda")
+            rl = torch.empty((2, K, n_mine, 4), dtype=torch.float64, device="cuda")
+            _lib.check(lib.psoap_farm_predict_draws(self._farm, _lib.ptr(p_dev), _lib.ptr(seed_dev), _lib.ptr(dl),
+                                                    _lib.ptr(sl), _lib.ptr(xl), _lib.ptr(rl[0]), _lib.ptr(rl[1]),
+                                                    _lib.stream_ptr()))
+            # each own chunk's proposals are contiguous in the attach layout: one copy per chunk and kind
+            for k, i in enumerate(self.mine):
+                nd, ns, nx = K * q["M"][i], int(q["s0"][i + 1] - q["s0"][i]), K * S * q["M"][i]
+                delta[q["d0"][i]:q["d0"][i] + nd].copy_(dl[off[0, k]:off[0, k] + nd])
+                sig[q["s0"][i]:q["s0"][i] + ns].copy_(sl[off[1, k]:off[1, k] + ns])
+                draws[q["x0"][i]:q["x0"][i] + nx].copy_(xl[off[2, k]:off[2, k] + nx])
+            res.index_copy_(2, self._mine_idx, rl)
+        if self.world_size > 1:
+            for t in (delta, sig, draws, res):
+                self._allreduce(t)
+        h = res.cpu().numpy()
+        for k in range(K):
+            for i in range(self.n_chunks):
+                if q["m"][i] == 0:
+                    continue
+                if h[0, k, i, 3] != 0.0:
+                    raise np.linalg.LinAlgError("proposal %d, chunk %d: %d-th leading minor of the data block is not "
+                                                "positive definite" % (k, i, int(h[0, k, i, 3])))
+                if h[0, k, i, 0] == -np.inf:
+                    raise ValueError("proposal %d, chunk %d: a velocity reaches the speed of light or a GP parameter is "
+                                     "negative" % (k, i))
+                if h[1, k, i, 3] != 0.0:
+                    raise np.linalg.LinAlgError("proposal %d, chunk %d: Sigma + jitter I (jitter = %g) is not positive "
+                                                "definite: its %d-th leading minor; pass a larger jitter"
+                                                % (k, i, q["jitter"], int(h[1, k, i, 3])))
+        out = []
+        for i in range(self.n_chunks):
+            M, m = q["M"][i], q["m"][i]
+            mean = torch.from_numpy(np.repeat(mus, m)).cuda()
+            mu = delta[q["d0"][i]:q["d0"][i + 1]].view(K, M) + mean
+            s = sig[q["s0"][i]:q["s0"][i + 1]]
+            x = draws[q["x0"][i]:q["x0"][i + 1]].view(K, S, M) + mean
+            out.append((mu, s.view(K, M, M) if q["mode"] == 0 else s.view(K, M), x))
         return out
 
     def close(self):
