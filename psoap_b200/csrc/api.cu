@@ -52,6 +52,19 @@ int fail(int code, const std::string& msg) {
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 inline int64_t padded_dim(int64_t n) { return (n + NB - 1) / NB * NB; }
 
+// Bump allocation of 256-byte aligned arrays from base.  A null base measures only: every pointer is null and off ends
+// at the size of the layout, so a size query and the carve it sizes run the same code.
+struct Carver {
+    char* base;
+    size_t off = 0;
+    template <class T>
+    T* take(size_t count) {
+        T* r = base ? (T*)(base + off) : nullptr;
+        off += align_up(count * sizeof(T), 256);
+        return r;
+    }
+};
+
 // ---- 2-D tensor maps for the TMA operand loads (driver entry point fetched at run time: no -lcuda) ----------
 PFN_cuTensorMapEncodeTiled g_encode_tiled = nullptr;
 
@@ -159,11 +172,10 @@ int set_kernel_attributes() {
     return PSOAP_OK;
 }
 
-// Device scratch of one factorisation: W [Nt x Nt] (Nt = padded total dimension), two panel buffers,
-// L_kk^-1, residual, y, accumulators, info, the fill's exact-zero tile flags and the envelope computed from them.
+// Device scratch of the factorisation of an Nt x Nt matrix (Nt = padded total dimension) held elsewhere: two panel
+// buffers, L_kk^-1, residual, y, accumulators, info, the fill's exact-zero tile flags and the envelope computed from them.
 constexpr int MAX_GROUP = 8;  // panels per trailing update (rank 128 * G)
 struct FactorWs {
-    double* W;
     double* P[2];   // two group buffers, each column-major [Nt, 128 * MAX_GROUP] (the adjacent panels of a group)
     double* Linv;   // potrf_diag3: L_kk^-1;  potrf_diag7: L_kk
     double* Xd;     // potrf_diag7: inverses of the four 32 x 32 diagonal sub-blocks of L_kk
@@ -177,43 +189,36 @@ struct FactorWs {
     int64_t Nt;
 };
 
-size_t factor_ws_bytes(int64_t Nt) {
-    size_t b = 0;
-    b += align_up((size_t)Nt * Nt * 8, 256);
-    b += 2 * align_up((size_t)Nt * MAX_GROUP * NB * 8, 256);
-    b += align_up((size_t)NB * NB * 8, 256);
-    b += align_up((size_t)4 * XD_BLOCK * 8, 256);
-    b += 2 * align_up((size_t)Nt * 8, 256);
-    b += align_up(8 * 8, 256);
-    b += align_up(2 * 4, 256);
+FactorWs carve_factor_ws(Carver& c, int64_t Nt) {
+    FactorWs ws;
+    ws.Nt = Nt;
+    ws.P[0] = c.take<double>((size_t)Nt * MAX_GROUP * NB);
+    ws.P[1] = c.take<double>((size_t)Nt * MAX_GROUP * NB);
+    ws.Linv = c.take<double>((size_t)NB * NB);
+    ws.Xd = c.take<double>((size_t)4 * XD_BLOCK);
+    ws.rvec = c.take<double>((size_t)Nt);
+    ws.y = c.take<double>((size_t)Nt);
+    ws.acc = c.take<double>(8);
+    ws.info = c.take<int>(2);
     const int64_t T = Nt / NB;
-    b += align_up((size_t)(T * (T + 1) / 2), 256);
-    b += align_up((size_t)(T + 1) * 4, 256);
-    b += align_up((size_t)T * 4, 256);
-    return b;
+    ws.nz = c.take<uint8_t>((size_t)(T * (T + 1) / 2));
+    ws.tend = c.take<int>((size_t)(T + 1));
+    ws.prof = c.take<int>((size_t)T);
+    return ws;
 }
 
-void carve_factor_ws(char* base, int64_t Nt, FactorWs* ws, bool with_W) {
-    char* p = base;
-    auto take = [&](size_t bytes) { char* r = p; p += align_up(bytes, 256); return r; };
-    ws->Nt = Nt;
-    ws->W = with_W ? (double*)take((size_t)Nt * Nt * 8) : nullptr;
-    ws->P[0] = (double*)take((size_t)Nt * MAX_GROUP * NB * 8);
-    ws->P[1] = (double*)take((size_t)Nt * MAX_GROUP * NB * 8);
-    ws->Linv = (double*)take((size_t)NB * NB * 8);
-    ws->Xd = (double*)take((size_t)4 * XD_BLOCK * 8);
-    ws->rvec = (double*)take((size_t)Nt * 8);
-    ws->y = (double*)take((size_t)Nt * 8);
-    ws->acc = (double*)take(8 * 8);
-    ws->info = (int*)take(2 * 4);
-    const int64_t T = Nt / NB;
-    ws->nz = (uint8_t*)take((size_t)(T * (T + 1) / 2));
-    ws->tend = (int*)take((size_t)(T + 1) * 4);
-    ws->prof = (int*)take((size_t)T * 4);
+// A matrix W [Nt x Nt] and the scratch of its factorisation behind it: the workspace of a likelihood (Nt = padded N),
+// of a prediction (the bordered matrix) and the first part of a farm prediction item.
+struct MatrixWs {
+    double* W;
+    FactorWs f;
+};
+MatrixWs carve_matrix_ws(Carver& c, int64_t Nt) {
+    MatrixWs m;
+    m.W = c.take<double>((size_t)Nt * Nt);
+    m.f = carve_factor_ws(c, Nt);
+    return m;
 }
-
-// The FactorWs of a matrix factored in place elsewhere (no W): the scratch of Sigma's factorisation in the prediction graph
-size_t sigma_ws_bytes(int64_t Nt) { return factor_ws_bytes(Nt) - align_up((size_t)Nt * Nt * 8, 256); }
 
 // Streams of one factorisation pipeline: the caller's stream plus a high-priority side stream on which the next
 // panel is factored while the bulk of the current trailing update runs (look-ahead).
@@ -484,18 +489,18 @@ int launch_fill_lower(int ncomp, cudaStream_t st, double* W, int64_t ld, int T, 
     return PSOAP_OK;
 }
 
-// fill + factor + fused solve of one chunk on stream st
+// fill of W [Np x Np] (Np = padded N) + factor + fused solve of one chunk on stream st
 int launch_chunk(const Lanes& ln, int ncomp, int64_t N, const ZSource& zs, const double* fl, const double* sigma,
-                 double mu, const GpParams& gp, const FactorWs& ws, const int* sentinel, double* result) {
+                 double mu, const GpParams& gp, double* W, const FactorWs& ws, const int* sentinel, double* result) {
     const int64_t Np = padded_dim(N);
     const int T = (int)(Np / NB);
     const int pad = (int)(Np - N);
-    int rc = launch_fill_lower(ncomp, ln.main, ws.W, Np, T, pad, zs, sigma, fl, mu, gp, ws);
+    int rc = launch_fill_lower(ncomp, ln.main, W, Np, T, pad, zs, sigma, fl, mu, gp, ws);
     if (rc) return rc;
     if (T > ENV_MAX_T) return fail(PSOAP_ERR_ARG, "launch_chunk: matrix too large for the envelope");
     launch_k(envelope_kernel, 1, 256, 0, ln.main, ln.pdl, (const uint8_t*)ws.nz, T, ws.tend, ws.prof);
     LAUNCH_CHECK();
-    return launch_factor(ln, ws.W, Np, T, T, pad, ws, sentinel, result, false, ws.tend, ws.prof);
+    return launch_factor(ln, W, Np, T, T, pad, ws, sentinel, result, false, ws.tend, ws.prof);
 }
 
 // Side stream + events for calls on a caller-provided stream (one set per host thread).
@@ -604,20 +609,21 @@ int psoap_fill_v11_host(int ncomp, double* mat, int64_t ld, int64_t N, const dou
         N > (1 << 30) || !amp || !l)
         return fail(PSOAP_ERR_ARG, "psoap_fill_v11_host: bad arguments");
     if (N == 0) return PSOAP_OK;
-    const size_t vec = align_up((size_t)N * 8, 256);
+    double* dmat = nullptr;
+    double* dv[3] = {nullptr, nullptr, nullptr};
+    auto carve = [&](Carver c) {   // the matrix, then the ncomp vectors
+        dmat = c.take<double>((size_t)N * N);
+        for (int k = 0; k < ncomp; ++k) dv[k] = c.take<double>((size_t)N);
+        return c.off;
+    };
     char* base = nullptr;
-    CUDA_TRY(cudaMalloc(&base, (size_t)N * N * 8 + 3 * vec));
-    double* dmat = (double*)base;
-    double* dv[3];
+    CUDA_TRY(cudaMalloc(&base, carve(Carver{nullptr})));
+    carve(Carver{base});
     const double* hv[3] = {lwl_f, lwl_g, lwl_h};
     cudaError_t e = cudaSuccess;
-    for (int c = 0; c < 3; ++c) {
-        dv[c] = (double*)(base + (size_t)N * N * 8 + c * vec);
-        if (c < ncomp && e == cudaSuccess) e = cudaMemcpy(dv[c], hv[c], (size_t)N * 8, cudaMemcpyHostToDevice);
-    }
+    for (int k = 0; k < ncomp && e == cudaSuccess; ++k) e = cudaMemcpy(dv[k], hv[k], (size_t)N * 8, cudaMemcpyHostToDevice);
     int rc = PSOAP_OK;
-    if (e == cudaSuccess)
-        rc = psoap_fill_v11(ncomp, dmat, N, N, dv[0], ncomp > 1 ? dv[1] : nullptr, ncomp > 2 ? dv[2] : nullptr, amp, l, nullptr);
+    if (e == cudaSuccess) rc = psoap_fill_v11(ncomp, dmat, N, N, dv[0], dv[1], dv[2], amp, l, nullptr);
     if (e == cudaSuccess && rc == PSOAP_OK)
         e = cudaMemcpy2D(mat, (size_t)ld * 8, dmat, (size_t)N * 8, (size_t)N * 8, (size_t)N, cudaMemcpyDeviceToHost);
     cudaFree(base);
@@ -674,7 +680,11 @@ int psoap_orbit_velocities(int model, const double* p_orb, const double* dates, 
 }
 
 // ---- likelihood -------------------------------------------------------------------------------------
-size_t psoap_lnlike_workspace_bytes(int64_t N) { return factor_ws_bytes(padded_dim(std::max<int64_t>(N, 1))); }
+size_t psoap_lnlike_workspace_bytes(int64_t N) {
+    Carver c{nullptr};
+    carve_matrix_ws(c, padded_dim(std::max<int64_t>(N, 1)));
+    return c.off;
+}
 
 int psoap_lnlike(int ncomp, int64_t N, const double* lwl_f, const double* lwl_g, const double* lwl_h, const double* fl,
                  const double* sigma, const double* amp, const double* l, double mu_GP, void* workspace,
@@ -699,19 +709,19 @@ int psoap_lnlike(int ncomp, int64_t N, const double* lwl_f, const double* lwl_g,
         return fail(PSOAP_ERR_WORKSPACE, "psoap_lnlike: workspace too small or not 256-byte aligned");
     int rc = set_kernel_attributes();
     if (rc) return rc;
-    FactorWs ws;
-    carve_factor_ws((char*)workspace, padded_dim(N), &ws, true);
+    Carver c{(char*)workspace};
+    const MatrixWs w = carve_matrix_ws(c, padded_dim(N));
     Lanes ln;
     rc = get_lanes(st, &ln);
     if (rc) return rc;
-    return launch_chunk(ln, ncomp, N, direct_z(lwl_f, lwl_g, lwl_h), fl, sigma, mu_GP, gp, ws, nullptr, (double*)result);
+    return launch_chunk(ln, ncomp, N, direct_z(lwl_f, lwl_g, lwl_h), fl, sigma, mu_GP, gp, w.W, w.f, nullptr,
+                        (double*)result);
 }
 
 int psoap_lnlike_envelope_view(void* workspace, int64_t N, int** tend, int* T) {
     if (!workspace || N < 1 || !tend || !T) return fail(PSOAP_ERR_ARG, "psoap_lnlike_envelope_view: bad arguments");
-    FactorWs ws;
-    carve_factor_ws((char*)workspace, padded_dim(N), &ws, true);
-    *tend = ws.tend;
+    Carver c{(char*)workspace};
+    *tend = carve_matrix_ws(c, padded_dim(N)).f.tend;
     *T = (int)(padded_dim(N) / NB);
     return PSOAP_OK;
 }
@@ -720,9 +730,8 @@ int psoap_lnlike_envelope_view(void* workspace, int64_t N, int** tend, int* T) {
 // in which row block I can hold a non-zero (the suffix minimum of the first non-zero block columns, envelope_kernel).
 int psoap_lnlike_profile_view(void* workspace, int64_t N, int** profile, int* T) {
     if (!workspace || N < 1 || !profile || !T) return fail(PSOAP_ERR_ARG, "psoap_lnlike_profile_view: bad arguments");
-    FactorWs ws;
-    carve_factor_ws((char*)workspace, padded_dim(N), &ws, true);
-    *profile = ws.prof;
+    Carver c{(char*)workspace};
+    *profile = carve_matrix_ws(c, padded_dim(N)).f.prof;
     *T = (int)(padded_dim(N) / NB);
     return PSOAP_OK;
 }
@@ -750,8 +759,17 @@ int psoap_lnlike_host(int ncomp, int64_t N, const double* lwl_f, const double* l
     if (!lwl_f || !fl || !sigma || (ncomp > 1 && !lwl_g) || (ncomp > 2 && !lwl_h))
         return fail(PSOAP_ERR_ARG, "psoap_lnlike_host: null vector");
     std::lock_guard<std::mutex> lock(g_hc.mu);
-    const size_t vec = align_up((size_t)N * 8, 256);
-    const size_t need = psoap_lnlike_workspace_bytes(N) + 5 * vec + 256;
+    double* d[5];
+    psoap_result* dres = nullptr;
+    char* wsp = nullptr;
+    const size_t wsb = psoap_lnlike_workspace_bytes(N);
+    auto carve = [&](Carver c) {   // the five vectors, the result record, then the likelihood's workspace
+        for (double*& p : d) p = c.take<double>((size_t)N);
+        dres = c.take<psoap_result>(1);
+        wsp = c.take<char>(wsb);
+        return c.off;
+    };
+    const size_t need = carve(Carver{nullptr});
     if (g_hc.bytes < need) {
         if (g_hc.buf) cudaFree(g_hc.buf);
         g_hc.buf = nullptr; g_hc.bytes = 0;
@@ -759,17 +777,12 @@ int psoap_lnlike_host(int ncomp, int64_t N, const double* lwl_f, const double* l
         g_hc.bytes = need;
     }
     if (!g_hc.st) CUDA_TRY(cudaStreamCreateWithFlags(&g_hc.st, cudaStreamNonBlocking));
-    char* base = (char*)g_hc.buf;
-    double* d[5];
+    carve(Carver{(char*)g_hc.buf});
     const double* h[5] = {lwl_f, lwl_g, lwl_h, fl, sigma};
-    for (int i = 0; i < 5; ++i) {
-        d[i] = (double*)(base + i * vec);
+    for (int i = 0; i < 5; ++i)
         if (h[i] && (i >= 3 || i < ncomp)) CUDA_TRY(cudaMemcpyAsync(d[i], h[i], (size_t)N * 8, cudaMemcpyHostToDevice, g_hc.st));
-    }
-    psoap_result* dres = (psoap_result*)(base + 5 * vec);
-    void* wsp = base + 5 * vec + 256;
     int rc = psoap_lnlike(ncomp, N, d[0], ncomp > 1 ? d[1] : nullptr, ncomp > 2 ? d[2] : nullptr, d[3], d[4], amp, l, mu_GP,
-                          wsp, g_hc.bytes - 5 * vec - 256, dres, g_hc.st);
+                          wsp, wsb, dres, g_hc.st);
     if (rc) return rc;
     CUDA_TRY(cudaMemcpyAsync(result, dres, sizeof(psoap_result), cudaMemcpyDeviceToHost, g_hc.st));
     CUDA_TRY(cudaStreamSynchronize(g_hc.st));
@@ -778,8 +791,9 @@ int psoap_lnlike_host(int ncomp, int64_t N, const double* lwl_f, const double* l
 
 // ---- Schur complement of a bordered matrix (prediction) -----------------------------------------------
 size_t psoap_schur_workspace_bytes(int64_t n, int64_t m) {
-    const int64_t Nt = padded_dim(n) + padded_dim(std::max<int64_t>(m, 0));
-    return factor_ws_bytes(Nt) - align_up((size_t)Nt * Nt * 8, 256);
+    Carver c{nullptr};
+    carve_factor_ws(c, padded_dim(n) + padded_dim(std::max<int64_t>(m, 0)));
+    return c.off;
 }
 
 // S: column-major [Nt, ld] with Nt = padded(n) + padded(m).  The caller lays the leading block out with
@@ -795,8 +809,8 @@ int psoap_schur(double* S, int64_t ld, int64_t n, int64_t m, void* workspace, si
         return fail(PSOAP_ERR_WORKSPACE, "psoap_schur: workspace too small or misaligned");
     int rc = set_kernel_attributes();
     if (rc) return rc;
-    FactorWs ws;
-    carve_factor_ws((char*)workspace, Nt, &ws, false);
+    Carver c{(char*)workspace};
+    const FactorWs ws = carve_factor_ws(c, Nt);
     Lanes ln;
     rc = get_lanes((cudaStream_t)stream, &ln);
     if (rc) return rc;
@@ -807,9 +821,8 @@ int psoap_schur(double* S, int64_t ld, int64_t n, int64_t m, void* workspace, si
 
 // The residual / accumulator part of a Schur workspace, for the host-side prediction code.
 extern "C" int psoap_schur_views(void* workspace, int64_t n, int64_t m, double** rvec, double** acc, int** info) {
-    const int64_t Nt = padded_dim(n) + padded_dim(std::max<int64_t>(m, 0));
-    FactorWs ws;
-    carve_factor_ws((char*)workspace, Nt, &ws, false);
+    Carver c{(char*)workspace};
+    const FactorWs ws = carve_factor_ws(c, padded_dim(n) + padded_dim(std::max<int64_t>(m, 0)));
     if (rvec) *rvec = ws.rvec;
     if (acc) *acc = ws.acc;
     if (info) *info = ws.info;
@@ -836,26 +849,21 @@ struct GradWs {
     int64_t Nn, Nt;
     int Tb, ntiles;
 };
-size_t carve_grad_ws(char* base, int ncomp, int64_t N, int n_epochs, int norb, GradWs* g) {
+void carve_grad_ws(Carver& c, int ncomp, int64_t N, int n_epochs, int norb, GradWs* g) {
     g->Nn = padded_dim(std::max<int64_t>(N, 1));
     g->Nt = 2 * g->Nn;
     g->Tb = (int)(g->Nn / NB);
     g->ntiles = g->Tb * (g->Tb + 1) / 2;
-    size_t off = 0;
-    auto take = [&](size_t bytes) { char* r = base ? base + off : nullptr; off += align_up(bytes, 256); return r; };
-    g->S = (double*)take((size_t)g->Nt * g->Nt * 8);
-    const size_t fbytes = factor_ws_bytes(g->Nt) - align_up((size_t)g->Nt * g->Nt * 8, 256);
-    char* fb = take(fbytes);
-    if (base) carve_factor_ws(fb, g->Nt, &g->f, false);
-    g->tile = (double*)take((size_t)g->ntiles * 2 * ncomp * 8);
-    g->slot = (double*)take((size_t)g->Tb * g->Tb * ncomp * NB * 8);
-    g->hyp = (double*)take(8 * 8);
-    g->vel = (double*)take((size_t)3 * n_epochs * 8);
-    g->flag = (int*)take(4);
-    g->jac = (double*)take((size_t)3 * n_epochs * norb * 8);
-    g->gz = (double*)take((size_t)ncomp * N * 8);
-    g->gv = (double*)take((size_t)3 * n_epochs * 8);
-    return off;
+    g->S = c.take<double>((size_t)g->Nt * g->Nt);
+    g->f = carve_factor_ws(c, g->Nt);
+    g->tile = c.take<double>((size_t)g->ntiles * 2 * ncomp);
+    g->slot = c.take<double>((size_t)g->Tb * g->Tb * ncomp * NB);
+    g->hyp = c.take<double>(8);
+    g->vel = c.take<double>((size_t)3 * n_epochs);
+    g->flag = c.take<int>(1);
+    g->jac = c.take<double>((size_t)3 * n_epochs * norb);
+    g->gz = c.take<double>((size_t)ncomp * N);
+    g->gv = c.take<double>((size_t)3 * n_epochs);
 }
 
 // fill, identity border, restricted elimination, contraction and the hyper-parameter reduction (+ the per-pixel
@@ -897,7 +905,9 @@ int fill_value(double* p, int64_t n, double v, cudaStream_t st) {
 extern "C" size_t psoap_lnlike_grad_workspace_bytes(int ncomp, int64_t N) {
     if (ncomp < 1 || ncomp > 3 || N < 0) return 0;
     GradWs g;
-    return carve_grad_ws(nullptr, ncomp, N, 0, 0, &g);
+    Carver c{nullptr};
+    carve_grad_ws(c, ncomp, N, 0, 0, &g);
+    return c.off;
 }
 
 extern "C" int psoap_lnlike_grad(int ncomp, int64_t N, const double* lwl_f, const double* lwl_g, const double* lwl_h,
@@ -928,7 +938,8 @@ extern "C" int psoap_lnlike_grad(int ncomp, int64_t N, const double* lwl_f, cons
     int rc = set_kernel_attributes();
     if (rc) return rc;
     GradWs g;
-    carve_grad_ws((char*)workspace, ncomp, N, 0, 0, &g);
+    Carver c{(char*)workspace};
+    carve_grad_ws(c, ncomp, N, 0, 0, &g);
     Lanes ln;
     rc = get_lanes(st, &ln);
     if (rc) return rc;
@@ -940,7 +951,8 @@ extern "C" int psoap_lnlike_grad_views(void* workspace, int64_t N, double** neg_
                                        double** neg_alpha_dev) {
     if (!workspace || N < 0) return fail(PSOAP_ERR_ARG, "psoap_lnlike_grad_views: bad arguments");
     GradWs g;
-    carve_grad_ws((char*)workspace, 1, N, 0, 0, &g);
+    Carver c{(char*)workspace};
+    carve_grad_ws(c, 1, N, 0, 0, &g);
     if (neg_kinv_dev) *neg_kinv_dev = g.S + g.Nn + g.Nn * g.Nt;
     if (ld) *ld = g.Nt;
     if (neg_alpha_dev) *neg_alpha_dev = g.f.rvec + g.Nn;
@@ -950,7 +962,9 @@ extern "C" int psoap_lnlike_grad_views(void* workspace, int64_t N, double** neg_
 extern "C" size_t psoap_chunk_lnprob_grad_workspace_bytes(int model, int64_t N, int32_t n_epochs) {
     if (!model_valid(model) || N < 1 || n_epochs < 1) return 0;
     GradWs g;
-    return carve_grad_ws(nullptr, dims_ncomp(model), N, n_epochs, dims_nvel(model, n_epochs), &g);
+    Carver c{nullptr};
+    carve_grad_ws(c, dims_ncomp(model), N, n_epochs, dims_nvel(model, n_epochs), &g);
+    return c.off;
 }
 
 namespace {
@@ -1020,7 +1034,8 @@ extern "C" int psoap_chunk_lnprob_grad(int model, const psoap_chunk* chunk, cons
     int rc = set_kernel_attributes();
     if (rc) return rc;
     GradWs g;
-    carve_grad_ws((char*)workspace, ncomp, N, ne, norb, &g);
+    Carver c{(char*)workspace};
+    carve_grad_ws(c, ncomp, N, ne, norb, &g);
     return launch_chunk_grad(model, chunk, p_dev, mu_GP, g, (cudaStream_t)stream, (double*)result, grad_p);
 }
 
@@ -1036,19 +1051,17 @@ struct FisherWs {
     double* prod;     // [P][Nn][Nn]
     int P, npairs;
 };
-size_t carve_fisher_ws(char* base, int model, int64_t N, int n_epochs, GradWs* g, FisherWs* f) {
+void carve_fisher_ws(Carver& c, int model, int64_t N, int n_epochs, GradWs* g, FisherWs* f) {
     const int ncomp = dims_ncomp(model), norb = dims_nvel(model, n_epochs);
-    size_t off = carve_grad_ws(base, ncomp, N, n_epochs, norb, g);
-    auto take = [&](size_t bytes) { char* r = base ? base + off : nullptr; off += align_up(bytes, 256); return r; };
+    carve_grad_ws(c, ncomp, N, n_epochs, norb, g);
     const int64_t Tb = g->Tb;
     f->P = norb + 2 * ncomp;
     f->npairs = (int)(Tb * (Tb + 1) / 2);
-    f->flags = (uint8_t*)take((size_t)(Tb * Tb));
-    f->krange = (int*)take((size_t)Tb * 2 * 4);
-    f->part = (double*)take((size_t)f->npairs * (f->P * (f->P + 1) / 2) * 8);
-    f->grad_p = (double*)take((size_t)f->P * 8);
-    f->prod = (double*)take((size_t)f->P * g->Nn * g->Nn * 8);
-    return off;
+    f->flags = c.take<uint8_t>((size_t)(Tb * Tb));
+    f->krange = c.take<int>((size_t)Tb * 2);
+    f->part = c.take<double>((size_t)f->npairs * (f->P * (f->P + 1) / 2));
+    f->grad_p = c.take<double>((size_t)f->P);
+    f->prod = c.take<double>((size_t)f->P * g->Nn * g->Nn);
 }
 
 // the Fisher steps after launch_chunk_grad (fisher.cuh): mirror K^-1, then per parameter D_a and A_a = K^-1 D_a, then
@@ -1106,7 +1119,9 @@ extern "C" size_t psoap_chunk_fisher_workspace_bytes(int model, int64_t N, int32
     if (!model_valid(model) || N < 1 || N > 200000 || n_epochs < 1) return 0;
     GradWs g;
     FisherWs f;
-    return carve_fisher_ws(nullptr, model, N, n_epochs, &g, &f);
+    Carver c{nullptr};
+    carve_fisher_ws(c, model, N, n_epochs, &g, &f);
+    return c.off;
 }
 
 extern "C" int psoap_chunk_fisher(int model, const psoap_chunk* chunk, const double* p_dev, double mu_GP,
@@ -1121,7 +1136,8 @@ extern "C" int psoap_chunk_fisher(int model, const psoap_chunk* chunk, const dou
     if (rc) return rc;
     GradWs g;
     FisherWs f;
-    carve_fisher_ws((char*)workspace, model, chunk->N, chunk->n_epochs, &g, &f);
+    Carver c{(char*)workspace};
+    carve_fisher_ws(c, model, chunk->N, chunk->n_epochs, &g, &f);
     const cudaStream_t st = (cudaStream_t)stream;
     rc = launch_chunk_grad(model, chunk, p_dev, mu_GP, g, st, (double*)result, grad_p ? grad_p : f.grad_p);
     if (rc) return rc;
@@ -1134,7 +1150,8 @@ extern "C" int psoap_chunk_fisher_views(void* workspace, int model, int64_t N, i
         return fail(PSOAP_ERR_ARG, "psoap_chunk_fisher_views: bad arguments");
     GradWs g;
     FisherWs f;
-    carve_fisher_ws((char*)workspace, model, N, n_epochs, &g, &f);
+    Carver c{(char*)workspace};
+    carve_fisher_ws(c, model, N, n_epochs, &g, &f);
     if (flags) *flags = f.flags;
     if (krange) *krange = f.krange;
     if (Tb) *Tb = g.Tb;
@@ -1166,7 +1183,9 @@ int predict_dims(int ncomp, int mode, int64_t n, int64_t m, int64_t* M, int64_t*
 extern "C" size_t psoap_predict_workspace_bytes(int ncomp, int mode, int64_t n, int64_t m) {
     int64_t M, Nn, Nt;
     if (predict_dims(ncomp, mode, n, m, &M, &Nn, &Nt)) return 0;
-    return align_up((size_t)Nt * Nt * 8, 256) + psoap_schur_workspace_bytes(n, M);
+    Carver c{nullptr};
+    carve_matrix_ws(c, Nt);
+    return c.off;
 }
 
 extern "C" int psoap_predict(int ncomp, int mode, int64_t n, int64_t m, const double* const* lwl_data,
@@ -1184,9 +1203,10 @@ extern "C" int psoap_predict(int ncomp, int mode, int64_t n, int64_t m, const do
     int rc = set_kernel_attributes();
     if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
-    double* S = (double*)workspace;
-    FactorWs ws;
-    carve_factor_ws((char*)workspace + align_up((size_t)Nt * Nt * 8, 256), Nt, &ws, false);
+    Carver c{(char*)workspace};
+    const MatrixWs w = carve_matrix_ws(c, Nt);
+    double* S = w.W;
+    const FactorWs& ws = w.f;
     GpParams gp;
     make_gp(ncomp, amp, l, &gp);
     const int pad = (int)(Nn - n);
@@ -1226,31 +1246,35 @@ extern "C" int psoap_predict_host(int ncomp, int mode, int64_t n, int64_t m, con
     for (int c = 0; c < ncomp; ++c)
         if (!lwl_data[c] || !lwl_predict[c]) return fail(PSOAP_ERR_ARG, "psoap_predict_host: null vector");
     const size_t wsb = psoap_predict_workspace_bytes(ncomp, mode, n, m);
-    const size_t vn = align_up((size_t)n * 8, 256), vm = align_up((size_t)m * 8, 256), vM = align_up((size_t)M * 8, 256);
-    const size_t sig = Sigma_out ? align_up((size_t)M * M * 8, 256) : 0;
-    const size_t total = wsb + (size_t)(ncomp + 2) * vn + (size_t)ncomp * vm + vM + sig + 512;
+    char* wsp = nullptr;
+    double *dd[3] = {nullptr, nullptr, nullptr}, *dp[3] = {nullptr, nullptr, nullptr};
+    double *dfl = nullptr, *dsg = nullptr, *ddelta = nullptr, *dSig = nullptr;
+    psoap_result* dres = nullptr;
+    auto carve = [&](Carver c) {   // the prediction's workspace, then the staging of its inputs and outputs
+        wsp = c.take<char>(wsb);
+        for (int k = 0; k < ncomp; ++k) { dd[k] = c.take<double>((size_t)n); dp[k] = c.take<double>((size_t)m); }
+        dfl = c.take<double>((size_t)n);
+        dsg = c.take<double>((size_t)n);
+        ddelta = c.take<double>((size_t)M);
+        if (Sigma_out) dSig = c.take<double>((size_t)M * M);
+        dres = c.take<psoap_result>(1);
+        return c.off;
+    };
     char* base = nullptr;
-    CUDA_TRY(cudaMalloc(&base, total));
+    CUDA_TRY(cudaMalloc(&base, carve(Carver{nullptr})));
+    carve(Carver{base});
     cudaStream_t st = nullptr;
     cudaError_t e = cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking);
     int rc = PSOAP_OK;
     if (e == cudaSuccess) {
-        char* p = base + wsb;
-        auto take = [&](size_t b) { char* r = p; p += b; return (double*)r; };
-        const double *dd[3] = {nullptr, nullptr, nullptr}, *dp[3] = {nullptr, nullptr, nullptr};
-        for (int c = 0; c < ncomp && e == cudaSuccess; ++c) {
-            double* x = take(vn); dd[c] = x;
-            e = cudaMemcpyAsync(x, lwl_data[c], (size_t)n * 8, cudaMemcpyHostToDevice, st);
-            double* y = take(vm); dp[c] = y;
-            if (e == cudaSuccess) e = cudaMemcpyAsync(y, lwl_predict[c], (size_t)m * 8, cudaMemcpyHostToDevice, st);
+        for (int k = 0; k < ncomp && e == cudaSuccess; ++k) {
+            e = cudaMemcpyAsync(dd[k], lwl_data[k], (size_t)n * 8, cudaMemcpyHostToDevice, st);
+            if (e == cudaSuccess) e = cudaMemcpyAsync(dp[k], lwl_predict[k], (size_t)m * 8, cudaMemcpyHostToDevice, st);
         }
-        double* dfl = take(vn); double* dsg = take(vn); double* ddelta = take(vM);
-        double* dSig = Sigma_out ? take(sig) : nullptr;
-        psoap_result* dres = (psoap_result*)take(256);
         if (e == cudaSuccess) e = cudaMemcpyAsync(dfl, fl, (size_t)n * 8, cudaMemcpyHostToDevice, st);
         if (e == cudaSuccess) e = cudaMemcpyAsync(dsg, sigma, (size_t)n * 8, cudaMemcpyHostToDevice, st);
         if (e == cudaSuccess)
-            rc = psoap_predict(ncomp, mode, n, m, dd, dfl, dsg, dp, amp, l, resid_mu, nugget, ddelta, dSig, base, wsb, dres, st);
+            rc = psoap_predict(ncomp, mode, n, m, dd, dfl, dsg, dp, amp, l, resid_mu, nugget, ddelta, dSig, wsp, wsb, dres, st);
         if (e == cudaSuccess && rc == PSOAP_OK) {
             e = cudaMemcpyAsync(delta_out, ddelta, (size_t)M * 8, cudaMemcpyDeviceToHost, st);
             if (e == cudaSuccess && Sigma_out) e = cudaMemcpyAsync(Sigma_out, dSig, (size_t)M * M * 8, cudaMemcpyDeviceToHost, st);
@@ -1319,7 +1343,7 @@ struct FarmGrad {
 };
 
 // The optional prediction graph of a farm (psoap_farm_predict_attach): besides the item state, the caller's grids and
-// the output offsets of every item.  Each branch region holds the bordered matrix of an item (S, then its FactorWs).
+// the output offsets of every item.  Each branch region holds one item at a time (carve_predict_item).
 struct FarmPredict {
     FarmGraph g;
     int sigma_mode = 0;               // 0: Sigma [M][M], 1: its diagonal [M]
@@ -1423,10 +1447,10 @@ int farm_issue(const psoap_farm* f, cudaStream_t s0, int pdl) {
     if (rc) return rc;
     return issue_branches(g, s0, [&](int b, cudaStream_t, int it) {
         const psoap_chunk& ch = f->chunks[it % f->nchunks];
-        FactorWs ws;
-        carve_factor_ws(g.branch_base[b], padded_dim(ch.N), &ws, true);
+        Carver region{g.branch_base[b]};
+        const MatrixWs w = carve_matrix_ws(region, padded_dim(ch.N));
         return launch_chunk(farm_lanes(f, g, b, pdl), f->ncomp, ch.N, farm_z(ch, g.item_vel[it]), ch.fl, ch.sigma, f->mu,
-                            farm_gp(f, g, it), ws, g.flags + it, g.results + 4 * it);
+                            farm_gp(f, g, it), w.W, w.f, g.flags + it, g.results + 4 * it);
     });
 }
 
@@ -1444,7 +1468,8 @@ int farm_grad_issue(const psoap_farm* f, const FarmGrad& q, cudaStream_t s0, int
     return issue_branches(g, s0, [&](int b, cudaStream_t sb, int it) {
         const psoap_chunk& ch = f->chunks[it % f->nchunks];
         GradWs w;
-        carve_grad_ws(g.branch_base[b], f->ncomp, ch.N, ch.n_epochs, jac_cols(f), &w);
+        Carver region{g.branch_base[b]};
+        carve_grad_ws(region, f->ncomp, ch.N, ch.n_epochs, jac_cols(f), &w);
         int rc = launch_grad(farm_lanes(f, g, b, pdl), f->ncomp, ch.N, farm_z(ch, g.item_vel[it]), ch.fl, ch.sigma, f->mu,
                              farm_gp(f, g, it), w, g.flags + it, g.results + 4 * it, w.hyp, w.gz);
         double* row = q.grad + (size_t)it * np;
@@ -1462,13 +1487,32 @@ PredictDims predict_item_dims(int ncomp, int64_t N, int64_t m) {
     return {Nn, M, Nn + padded_dim(M)};
 }
 
+// Layout of one prediction item in its branch region: the bordered matrix and its FactorWs; with draws, behind them,
+// the FactorWs of Sigma's factorisation (in place in the matrix's trailing Mp x Mp block, Mp = Nt - Nn) and the
+// normals Z [n_draws][Mp].
+struct PredictItemWs {
+    MatrixWs m;
+    FactorWs sigma{};
+    double* Z = nullptr;
+};
+PredictItemWs carve_predict_item(Carver& c, const PredictDims& d, int n_draws) {
+    PredictItemWs w;
+    w.m = carve_matrix_ws(c, d.Nt);
+    if (n_draws > 0) {
+        const int64_t Mp = d.Nt - d.Nn;
+        w.sigma = carve_factor_ws(c, Mp);
+        w.Z = c.take<double>((size_t)n_draws * Mp);
+    }
+    return w;
+}
+
 // The prediction counterpart of farm_issue: velocities and sentinels of every item, then per branch the steps of
 // psoap_predict (mode 0) on the item's shifted pixels: data fill, border fill, elimination of the data block, read-out
 // into the item's offsets of delta and sigma.
 //
 // With draws, each item goes on: jitter on Sigma's diagonal in the trailing block (after the read-out, which saw Sigma
-// itself), the factorisation of that block in place into L (launch_factor with store_l, on Sigma's own FactorWs carved
-// behind the data block's), the item's normals Z [S][padded(M)], and X = delta + L Z into the item's offset of draws.
+// itself), the factorisation of that block in place into L (launch_factor with store_l, on Sigma's own FactorWs), the
+// item's normals Z [S][padded(M)], and X = delta + L Z into the item's offset of draws.
 int farm_predict_issue(const psoap_farm* f, const FarmPredict& q, cudaStream_t s0, int pdl, double* delta, double* sigma,
                        double* draws = nullptr) {
     const FarmGraph& g = q.g;
@@ -1480,11 +1524,13 @@ int farm_predict_issue(const psoap_farm* f, const FarmPredict& q, cudaStream_t s
         const psoap_chunk& ch = f->chunks[ci];
         const PredictDims d = predict_item_dims(ncomp, ch.N, q.m[ci]);
         const int Tn = (int)(d.Nn / NB), Tt = (int)(d.Nt / NB), pad = (int)(d.Nn - ch.N);
-        FactorWs ws;
-        carve_factor_ws(g.branch_base[b], d.Nt, &ws, true);
+        Carver region{g.branch_base[b]};
+        const PredictItemWs w = carve_predict_item(region, d, q.n_draws);
+        double* W = w.m.W;
+        const FactorWs& ws = w.m.f;
         const GpParams gp = farm_gp(f, g, it);
         const ZSource zs = farm_z(ch, g.item_vel[it]);
-        int rc = launch_fill_lower(ncomp, sb, ws.W, d.Nt, Tn, pad, zs, ch.sigma, ch.fl, f->mu, gp, ws);
+        int rc = launch_fill_lower(ncomp, sb, W, d.Nt, Tn, pad, zs, ch.sigma, ch.fl, f->mu, gp, ws);
         if (rc) return rc;
         PredictFarmSrc ps;
         for (int c = 0; c < 3; ++c) { ps.data[c] = nullptr; ps.pred[c] = c < ncomp ? q.grids[(size_t)ci * ncomp + c] : nullptr; }
@@ -1492,22 +1538,20 @@ int farm_predict_issue(const psoap_farm* f, const FarmPredict& q, cudaStream_t s
         ps.pad = pad; ps.Nn = (int)d.Nn; ps.Nt = (int)d.Nt; ps.nugget = 0.0; ps.zs = zs;
         const unsigned ntile = (unsigned)((int64_t)Tt * (Tt + 1) / 2 - (int64_t)Tn * (Tn + 1) / 2);
         with_ncomp(ncomp, [&](auto nc) {
-            predict_border_farm_kernel<nc><<<ntile, 256, 0, sb>>>(ws.W, d.Nt, ps, gp, ws.rvec);
+            predict_border_farm_kernel<nc><<<ntile, 256, 0, sb>>>(W, d.Nt, ps, gp, ws.rvec);
         });
         LAUNCH_CHECK();
-        rc = launch_factor(farm_lanes(f, g, b, pdl), ws.W, d.Nt, Tn, Tt, pad, ws, g.flags + it, g.results + 4 * it);
+        rc = launch_factor(farm_lanes(f, g, b, pdl), W, d.Nt, Tn, Tt, pad, ws, g.flags + it, g.results + 4 * it);
         if (rc) return rc;
         const unsigned nb = (unsigned)((d.M + 31) / 32);
         predict_farm_readout_kernel<<<dim3(q.sigma_mode ? 1u : nb, nb), 256, 0, sb>>>(
-            ws.W, d.Nt, (int)d.Nn, (int)d.M, ws.rvec, ws.info, g.flags + it, q.sigma_mode, sigma + q.sigma_off[it],
+            W, d.Nt, (int)d.Nn, (int)d.M, ws.rvec, ws.info, g.flags + it, q.sigma_mode, sigma + q.sigma_off[it],
             delta + q.delta_off[it]);
         LAUNCH_CHECK();
         if (q.n_draws == 0) return PSOAP_OK;
         const int64_t Mp = d.Nt - d.Nn;
-        double* T = ws.W + d.Nn * (d.Nt + 1);
-        FactorWs sw;
-        carve_factor_ws(g.branch_base[b] + factor_ws_bytes(d.Nt), Mp, &sw, false);
-        double* Z = (double*)(g.branch_base[b] + factor_ws_bytes(d.Nt) + sigma_ws_bytes(Mp));
+        double* T = W + d.Nn * (d.Nt + 1);
+        const FactorWs& sw = w.sigma;
         sigma_jitter_kernel<<<1, 256, 0, sb>>>(T, d.Nt, (int)d.M, (int)Mp, q.jitter, sw.rvec, sw.acc, sw.info);
         LAUNCH_CHECK();
         rc = launch_factor(farm_lanes(f, g, b, pdl), T, d.Nt, (int)(Mp / NB), (int)(Mp / NB), 0, sw, g.flags + it,
@@ -1515,10 +1559,10 @@ int farm_predict_issue(const psoap_farm* f, const FarmPredict& q, cudaStream_t s
         if (rc) return rc;
         const int S = q.n_draws;
         normals_kernel<<<dim3((unsigned)((Mp + 255) / 256), (unsigned)std::min(S, 65535)), 128, 0, sb>>>(
-            q.seed, 0, q.chunk_keys[ci], (uint32_t)(it / nchunks), S, (int)d.M, (int)Mp, Z, Mp);
+            q.seed, 0, q.chunk_keys[ci], (uint32_t)(it / nchunks), S, (int)d.M, (int)Mp, w.Z, Mp);
         LAUNCH_CHECK();
         predict_draws_kernel<<<dim3((unsigned)(Mp / DR_T), (unsigned)((S + DR_T - 1) / DR_T)), 256, 0, sb>>>(
-            T, d.Nt, (int)d.M, (int)Mp, Z, S, ws.rvec + d.Nn, ws.info, sw.info, g.flags + it, draws + q.draws_off[it]);
+            T, d.Nt, (int)d.M, (int)Mp, w.Z, S, ws.rvec + d.Nn, ws.info, sw.info, g.flags + it, draws + q.draws_off[it]);
         LAUNCH_CHECK();
         return PSOAP_OK;
     });
@@ -1657,40 +1701,35 @@ int run_farm_graph(const psoap_farm* f, FarmGraph& g, const double* p_dev, psoap
     return PSOAP_OK;
 }
 
-// Bump allocation of 256-byte aligned pieces from base (null: offsets only, for the size queries)
-struct Carver {
-    char* base;
-    size_t off = 0;
-    char* take(size_t bytes) { char* r = base ? base + off : nullptr; off += align_up(bytes, 256); return r; }
-};
-
 // Layout of the part of a workspace every farm graph has: the parameter buffer (pstride doubles per proposal), the result
 // records, sentinels and velocity descriptors of the items (orbit, or with free_vel the epoch-map ones), vel_rows x
 // n_epochs velocity doubles per item, then nbranch regions of branch_bytes.  The graph's own buffers follow at c.off.
 void carve_farm_items(Carver& c, FarmGraph& g, int nprop, int nchunks, const int32_t* n_epochs, int vel_rows,
                       size_t branch_bytes, int pstride = P_STRIDE, bool free_vel = false) {
     const int nitems = nchunks * nprop;
-    g.p_buf = (double*)c.take((size_t)nprop * pstride * 8);
-    g.results = (double*)c.take((size_t)nitems * 4 * 8);
-    g.flags = (int*)c.take((size_t)nitems * 4);
+    g.p_buf = c.take<double>((size_t)nprop * pstride);
+    g.results = c.take<double>((size_t)nitems * 4);
+    g.flags = c.take<int>((size_t)nitems);
     if (free_vel)
-        g.fdescs = (FreeDesc*)c.take((size_t)nitems * sizeof(FreeDesc));
+        g.fdescs = c.take<FreeDesc>((size_t)nitems);
     else
-        g.descs = (OrbitDesc*)c.take((size_t)nitems * sizeof(OrbitDesc));
+        g.descs = c.take<OrbitDesc>((size_t)nitems);
     g.item_vel.resize(nitems);
-    for (int it = 0; it < nitems; ++it) g.item_vel[it] = (double*)c.take((size_t)vel_rows * n_epochs[it % nchunks] * 8);
+    for (int it = 0; it < nitems; ++it) g.item_vel[it] = c.take<double>((size_t)vel_rows * n_epochs[it % nchunks]);
     g.branch_base.resize(g.nbranch);
-    for (auto& r : g.branch_base) r = c.take(branch_bytes);
+    for (auto& r : g.branch_base) r = c.take<char>(branch_bytes);
 }
 
-// Layout of a likelihood workspace: each branch holds the FactorWs of the largest chunk.  The size query takes no
-// model, so every item reserves the velocity table of three components.
+// Layout of a likelihood workspace: each branch holds the likelihood workspace (W and its FactorWs) of the largest
+// chunk.  The size query takes no model, so every item reserves the velocity table of three components.
 size_t carve_farm_lnprob(char* base, FarmGraph& g, int nchunks, const int64_t* N, const int32_t* n_epochs, int nprop,
                          int pstride = P_STRIDE, bool free_vel = false) {
     int64_t nmax = 0;
     for (int i = 0; i < nchunks; ++i) nmax = std::max(nmax, N[i]);
+    Carver branch{nullptr};
+    carve_matrix_ws(branch, padded_dim(nmax));
     Carver c{base};
-    carve_farm_items(c, g, nprop, nchunks, n_epochs, 3, factor_ws_bytes(padded_dim(nmax)), pstride, free_vel);
+    carve_farm_items(c, g, nprop, nchunks, n_epochs, 3, branch.off, pstride, free_vel);
     return c.off;
 }
 
@@ -1710,34 +1749,34 @@ size_t carve_farm_grad(const psoap_farm* f, char* base, FarmGrad& q) {
     int nemax = 1;
     for (const psoap_chunk& ch : f->chunks) { nmax = std::max<int64_t>(nmax, ch.N); nemax = std::max(nemax, (int)ch.n_epochs); }
     GradWs probe;
+    Carver branch{nullptr};
+    carve_grad_ws(branch, f->ncomp, nmax, nemax, jac_cols(f), &probe);
     Carver c{base};
-    carve_farm_items(c, q.g, f->nprop, f->nchunks, nes.data(), f->ncomp,
-                     carve_grad_ws(nullptr, f->ncomp, nmax, nemax, jac_cols(f), &probe), f->pstride, f->free);
-    q.grad = (double*)c.take((size_t)nitems * np * 8);
-    q.jdescs = (JacDesc*)c.take((size_t)nitems * sizeof(JacDesc));
+    carve_farm_items(c, q.g, f->nprop, f->nchunks, nes.data(), f->ncomp, branch.off, f->pstride, f->free);
+    q.grad = c.take<double>((size_t)nitems * np);
+    q.jdescs = c.take<JacDesc>((size_t)nitems);
     q.item_jac.resize(nitems);
-    for (int it = 0; it < nitems; ++it) q.item_jac[it] = (double*)c.take((size_t)f->ncomp * nes[it % f->nchunks] * jac_cols(f) * 8);
+    for (int it = 0; it < nitems; ++it) q.item_jac[it] = c.take<double>((size_t)f->ncomp * nes[it % f->nchunks] * jac_cols(f));
     return c.off;
 }
 
-// Layout of a prediction workspace: each branch holds factor_ws_bytes(Nt) for the largest bordered item, then the
-// graph's scratch outputs.  Also sets the output offsets of the items.  With n_draws > 0 a branch holds, behind an item's
-// data FactorWs, Sigma's own FactorWs (sigma_ws_bytes) and its normals [n_draws][padded(M)], sized for the largest such
-// sum; the graph adds its seed word, the records of Sigma's factorisation and the draws [n_draws][M] of every item.
+// Layout of a prediction workspace: each branch holds the largest item (carve_predict_item over the chunks with m > 0),
+// then the graph's scratch outputs.  Also sets the output offsets of the items.  With n_draws > 0 the graph adds its
+// seed word, the records of Sigma's factorisation and the draws [n_draws][M] of every item.
 size_t carve_farm_predict(const psoap_farm* f, const int64_t* m, int sigma_mode, int n_draws, char* base, FarmPredict& q) {
     const int nitems = f->nitems, nchunks = f->nchunks;
     // output layout: chunk after chunk, each chunk's proposals side by side, so that a chunk's outputs are contiguous
     q.delta_off.resize(nitems + 1);
     q.sigma_off.resize(nitems + 1);
     q.draws_off.resize(nitems + 1);
-    int64_t nd = 0, ns = 0, nx = 0, ntmax = 0;
+    int64_t nd = 0, ns = 0, nx = 0;
     size_t branch = 0;
     for (int ci = 0; ci < nchunks; ++ci) {
         const PredictDims d = predict_item_dims(f->ncomp, f->chunks[ci].N, m[ci]);
         if (m[ci] > 0) {
-            ntmax = std::max(ntmax, d.Nt);
-            const int64_t Mp = d.Nt - d.Nn;
-            branch = std::max(branch, factor_ws_bytes(d.Nt) + sigma_ws_bytes(Mp) + (size_t)n_draws * Mp * 8);
+            Carver item{nullptr};
+            carve_predict_item(item, d, n_draws);
+            branch = std::max(branch, item.off);
         }
         for (int k = 0; k < f->nprop; ++k) {
             const int it = k * nchunks + ci;
@@ -1746,15 +1785,14 @@ size_t carve_farm_predict(const psoap_farm* f, const int64_t* m, int sigma_mode,
         }
     }
     q.delta_off[nitems] = nd; q.sigma_off[nitems] = ns; q.draws_off[nitems] = nx;
-    if (n_draws == 0) branch = ntmax ? factor_ws_bytes(ntmax) : 0;
     Carver c{base};
     carve_farm_items(c, q.g, f->nprop, nchunks, farm_epochs(f).data(), f->ncomp, branch, f->pstride, f->free);
-    q.cap_delta = (double*)c.take((size_t)nd * 8);
-    q.cap_sigma = (double*)c.take((size_t)ns * 8);
+    q.cap_delta = c.take<double>((size_t)nd);
+    q.cap_sigma = c.take<double>((size_t)ns);
     if (n_draws > 0) {
-        q.seed = (uint64_t*)c.take(8);
-        q.sig_results = (double*)c.take((size_t)nitems * 4 * 8);
-        q.cap_draws = (double*)c.take((size_t)nx * 8);
+        q.seed = c.take<uint64_t>(1);
+        q.sig_results = c.take<double>((size_t)nitems * 4);
+        q.cap_draws = c.take<double>((size_t)nx);
     }
     return c.off;
 }
@@ -2165,10 +2203,16 @@ int psoap_debug_fill_lower(int ncomp, int64_t N, const double* lwl_f, const doub
     make_gp(ncomp, amp, l, &gp);
     ZSource zs = direct_z(lwl_f, lwl_g, lwl_h);
     if (epoch && vel) { zs.epoch = epoch; zs.vel = vel; zs.n_epochs = n_epochs; zs.shift = 1; }
-    double* scratch = nullptr;   // accumulators + info word the kernel resets
-    CUDA_TRY(cudaMalloc(&scratch, 256));
-    FactorWs ws{};
-    ws.rvec = rvec; ws.acc = scratch; ws.info = (int*)(scratch + 16); ws.Nt = Np;
+    FactorWs ws{};   // the fill's part only: the caller's residual, the accumulators and info word the kernel resets
+    ws.rvec = rvec; ws.Nt = Np;
+    auto carve = [&](Carver c) {
+        ws.acc = c.take<double>(8);
+        ws.info = c.take<int>(2);
+        return c.off;
+    };
+    char* scratch = nullptr;
+    CUDA_TRY(cudaMalloc(&scratch, carve(Carver{nullptr})));
+    carve(Carver{scratch});
     int rc = launch_fill_lower(ncomp, (cudaStream_t)stream, W, ld, (int)(Np / NB), (int)(Np - N), zs, sigma, fl, mu_GP, gp, ws);
     cudaError_t e = cudaStreamSynchronize((cudaStream_t)stream);
     cudaFree(scratch);
@@ -2186,10 +2230,25 @@ int psoap_bench_fill(int kind, int ncomp, int64_t N, const double* lwl_f, const 
     if (kind < 0 || kind > 1 || ncomp < 1 || ncomp > 3 || N < 1 || !lwl_f || !amp || !l || reps < 1 || !avg_ms_out)
         return fail(PSOAP_ERR_ARG, "psoap_bench_fill: bad arguments");
     const int64_t Np = padded_dim(N);
-    double *W = nullptr, *vec = nullptr;
+    // the fill's part of a FactorWs (residual, accumulators, info word) and zero sigma and fl vectors
+    FactorWs ws{};
+    ws.Nt = Np;
+    double *sigma = nullptr, *fl = nullptr;
+    auto carve = [&](Carver c) {
+        ws.rvec = c.take<double>((size_t)Np);
+        sigma = c.take<double>((size_t)Np);
+        fl = c.take<double>((size_t)Np);
+        ws.acc = c.take<double>(8);
+        ws.info = c.take<int>(2);
+        return c.off;
+    };
+    const size_t vec_bytes = carve(Carver{nullptr});
+    double* W = nullptr;
+    char* vec = nullptr;
     CUDA_TRY(cudaMalloc(&W, (size_t)Np * Np * 8));
-    CUDA_TRY(cudaMalloc(&vec, (size_t)(3 * Np + 64) * 8));
-    CUDA_TRY(cudaMemset(vec, 0, (size_t)(3 * Np + 64) * 8));
+    CUDA_TRY(cudaMalloc(&vec, vec_bytes));
+    CUDA_TRY(cudaMemset(vec, 0, vec_bytes));
+    carve(Carver{vec});
     cudaStream_t st;
     CUDA_TRY(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
     cudaEvent_t e0, e1;
@@ -2198,10 +2257,6 @@ int psoap_bench_fill(int kind, int ncomp, int64_t N, const double* lwl_f, const 
     GpParams gp;
     make_gp(ncomp, amp, l, &gp);
     ZSource zs = direct_z(lwl_f, lwl_g, lwl_h);
-    FactorWs ws{};
-    ws.rvec = vec; ws.acc = vec + 3 * Np; ws.info = (int*)(vec + 3 * Np + 16); ws.Nt = Np;
-    const double* sigma = vec + Np;   // zeros
-    const double* fl = vec + 2 * Np;  // zeros
     int rc = PSOAP_OK;
     auto launch = [&]() {
         if (kind == 0) rc = launch_fill_lower(ncomp, st, W, Np, (int)(Np / NB), (int)(Np - N), zs, sigma, fl, 1.0, gp, ws);
